@@ -213,6 +213,12 @@ int mco_parse_ok(const char* eq) {
     free(t);
     return ok;
 }
+int mco_tokenize_ok(const char* eq) {
+    Tokens* t = (Tokens*)malloc(sizeof(Tokens));
+    int ok = tokenize(eq, t);
+    free(t);
+    return ok;
+}
 int mco_set_equation(mco* m, int slot, const char* eq) {
     if (slot < 0 || slot > 3) return 0;
     Tokens* t = (Tokens*)malloc(sizeof(Tokens));

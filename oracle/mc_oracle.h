@@ -15,6 +15,7 @@ void mco_destroy(mco*);
 /* pow_mode: 0 = libm powf (what the reference calls), 1 = the product's mcb_powf restatement */
 void mco_set_pow_mode(mco*, int mode);
 int mco_parse_ok(const char* eq);                                  /* evaluator.cpp:139-237 */
+int mco_tokenize_ok(const char* eq);                               /* Evaluator::tokenize alone: no operand-underflow check */
 int mco_set_equation(mco*, int slot, const char* eq);              /* slot 0 surface, 1..3 constraint lhs */
 float mco_evaluate(mco*, int slot, float x, float y, float z);     /* evaluator.cpp:53-107 */
 void mco_eval_points(mco*, int slot, const float* xyz, float* out, long n, int apply_scale);

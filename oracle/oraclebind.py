@@ -23,6 +23,7 @@ def lib():
         L.mco_destroy.argtypes = [vp]
         L.mco_set_pow_mode.argtypes = [vp, i]
         L.mco_parse_ok.argtypes = [cp]
+        L.mco_tokenize_ok.argtypes = [cp]
         L.mco_set_equation.argtypes = [vp, i, cp]
         L.mco_evaluate.argtypes = [vp, i, f, f, f]
         L.mco_evaluate.restype = f

@@ -87,6 +87,11 @@ def _p(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
 
+def parse_ok(eq):
+    """Evaluator::tokenize's verdict on `eq`."""
+    return bool(lib().mcref_parse_ok(eq.encode()))
+
+
 def fnv1a64(b: bytes) -> str:
     h = 0xCBF29CE484222325
     for x in b:

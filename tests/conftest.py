@@ -17,6 +17,12 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
 
 
+def pytest_report_header(config):
+    from oracle import refbind
+    return "reference for the `refbind` tests: " + ("the unmodified reference (oracle/_ref)" if refbind.available() else
+                                                    "its plain-C restatement (oracle/restated_ref.py); oracle/_ref is not built")
+
+
 @pytest.fixture(scope="session")
 def mcb():
     if os.environ.get("MCB_TEST_EMU") == "1":
@@ -36,9 +42,23 @@ def mcb_emu():
 
 @pytest.fixture(scope="session")
 def refbind():
+    """The unmodified reference (oracle/_ref) where its sources were there to build it; elsewhere its plain-C
+    restatement, which tests/test_oracle.py pins to the reference's golden vectors (oracle/restated_ref.py)."""
+    from oracle import refbind as R
+    if R.available():
+        return R
+    from oracle import restated_ref
+    if not restated_ref.available():
+        pytest.skip("oracle/libmcoracle.so not built (run __graft_entry__.build())")
+    return restated_ref
+
+
+@pytest.fixture(scope="session")
+def unmodified_reference():
+    """The reference's own build, for what no restatement can stand in for (the restatement checked against it)."""
     from oracle import refbind as R
     if not R.available():
-        pytest.skip("oracle/_ref/libmcref.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libmcref.so not built: the unmodified reference's sources are not part of the repository")
     return R
 
 

@@ -12,6 +12,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import refbind as R  # noqa: E402
+from tests.helpers import save_repeat_golden  # noqa: E402
 
 CASES = {
     # marching_test_drawer.h:238 uses distance 1.5; smaller distances give several nested shells
@@ -49,4 +50,4 @@ for name, c in CASES.items():
     print(name, meta[name]["M"], "M", meta[name]["V"], "vertices", meta[name]["T"], "triangles", meta[name]["active"], "active",
           meta[name]["ambiguous"], "ambiguous")
 out["meta_json"] = np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8)
-np.savez_compressed(os.path.join(ROOT, "tests", "golden", "repeat_cases.npz"), **out)
+save_repeat_golden(os.path.join(ROOT, "tests", "golden", "repeat_cases.npz"), out)

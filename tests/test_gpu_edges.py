@@ -1,7 +1,7 @@
 """-m gpu: edge cases of the path — the finest step the reference accepts (0.001: the fp32-accumulated grid drifts by
 1.9e-5, SURVEY.md A.3), a step below it (2048^3, SURVEY.md D4), the coarsest grids, empty and all-NaN fields,
-capacity growth on the first call, and slabs that do not start at layer 0.  Where oracle/_ref travelled to this box
-the reference is executed live on the same layers."""
+capacity growth on the first call, and slabs that do not start at layer 0.  The reference (or, where oracle/_ref is not
+built, its restatement: see the `refbind` fixture) is executed live on the same layers."""
 import numpy as np
 import pytest
 

@@ -1,5 +1,5 @@
 """-m gpu: larger grids.  256^3 (M=257): counts against SURVEY.md Appendix B (made with the unmodified reference) for
-all eight example equations, plus live per-cube comparison against oracle/_ref on a few z-layers.  1024^3: size-
+all eight example equations, plus live per-cube comparison against the `refbind` fixture on a few z-layers.  1024^3: size-
 independent properties (slab additivity, determinism, symmetric-field symmetry)."""
 import numpy as np
 import pytest

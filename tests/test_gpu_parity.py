@@ -1,6 +1,6 @@
 """-m gpu: the CUDA path, called through the C ABI, against the golden vectors produced by the unmodified reference
-(tests/golden/cases.npz, made by tests/golden/make_golden.py) and, when oracle/_ref travelled to this box, against
-the reference executed live.
+(tests/golden/cases.npz, made by tests/golden/make_golden.py) and against the reference executed live (its
+restatement where oracle/_ref is not built: see the `refbind` fixture).
 
 Bars (north_star): cube_code, table_idx and per-cube triangle counts BIT-EXACT; positions within 1e-5 relative
 (they are in fact required bit-exact here, the tolerance test is the weaker fallback assertion); normals within

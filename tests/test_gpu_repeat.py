@@ -12,7 +12,7 @@ import os
 import numpy as np
 import pytest
 
-from .helpers import same_bits
+from .helpers import load_repeat_golden, same_bits
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -20,7 +20,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 @pytest.fixture(scope="module")
 def rep():
-    return np.load(os.path.join(ROOT, "tests", "golden", "repeat_cases.npz"), allow_pickle=False)
+    return load_repeat_golden(os.path.join(ROOT, "tests", "golden", "repeat_cases.npz"))
 
 
 @pytest.fixture(scope="module")

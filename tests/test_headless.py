@@ -8,7 +8,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from .helpers import load_meta, same_bits
+from .helpers import load_meta, load_repeat_golden, same_bits
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 EXE = os.path.join(ROOT, "marching-cube-for-implicit-surfaces_b200", "mcb_headless")
@@ -66,7 +66,7 @@ def test_headless_finer_than_the_reference_allows(mcb, tmp_path):
 def test_headless_repeating_surface_mode(mcb, tmp_path):
     """The drop-in class in repeating-surface mode (set_surface_repeat_step_distance + repeating_surface_mode, the setting of
     the reference's own test drawer, marching_test_drawer.h:238) against the unmodified reference's Poly_Data."""
-    rep = np.load(os.path.join(ROOT, "tests", "golden", "repeat_cases.npz"), allow_pickle=False)
+    rep = load_repeat_golden(os.path.join(ROOT, "tests", "golden", "repeat_cases.npz"))
     case = json.loads(bytes(rep["meta_json"]).decode())["rep_testdrawer"]
     dump = tmp_path / "m.bin"
     out = subprocess.check_output([EXE, "--eq", case["eq"], "--step", str(case["step"]), "--scale", "1", "1", "1", "--levels", str(case["dist"]),

@@ -63,7 +63,7 @@ def test_tokenizer_matches_reference(mcb, refbind):
                                                      "x(y)", "(x)(y)2", "x^-y", "x*-(y)", "-", "(", "1.2.3", "x+(", "((x))", "x^2^3",
                                                      "3(x)", "x3", "x 3", ".5.5", "x*/y", "+x", "x++y", "-x-y", "(-)", "-.5x"]
     for eq in cases:
-        ref_ok = bool(refbind.lib().mcref_parse_ok(eq.encode()))
+        ref_ok = refbind.parse_ok(eq)
         mine = mcb.parse_ok(eq)
         if ref_ok and not mine:
             # accepted by the reference tokenizer, refused here: only allowed when the reference would underflow its
@@ -123,10 +123,48 @@ def _packed_rows():
     return np.array(rows, np.int32)
 
 
-def test_packed_triangle_table_equals_reference(refbind):
-    tri, _, edge = refbind.tables()
-    assert np.array_equal(_packed_rows(), tri)
-    assert edge.tolist() == [[0, 1], [1, 2], [2, 3], [3, 0], [4, 5], [5, 6], [6, 7], [7, 4], [0, 4], [1, 5], [2, 6], [3, 7]]
+EDGES = [[0, 1], [1, 2], [2, 3], [3, 0], [4, 5], [5, 6], [6, 7], [7, 4], [0, 4], [1, 5], [2, 6], [3, 7]]
+
+
+def _golden_active_cubes(golden):
+    """(case name, case, x, y, z, linear index) of every cube with triangles in the reference's golden runs, in its loop
+    order (x fastest), with the offset of the cube's first triangle in the golden soup."""
+    from .helpers import load_meta
+    for name, case in load_meta(golden).items():
+        M, t = case["M"], 0
+        ntri = golden[name + "/ntri"].astype(np.int64)
+        for lin in np.flatnonzero(ntri):
+            yield name, case, int(lin % M), int(lin // M % M), int(lin // (M * M)), int(lin), t
+            t += int(ntri[lin])
+
+
+def test_packed_triangle_table_equals_reference(golden):
+    """The committed packed table against the reference.  Where oracle/_ref is built: all 256 rows of its tri_table and
+    its edge table.  Always: every row the reference's golden runs used (tests/golden/cases.npz) against the triangles
+    the reference emitted — the row holds its triangle count, and the k-th corner of the soup lies on the row's k-th
+    edge (the two fixed coordinates equal, the third between the edge's corners), which pins edges, order and winding."""
+    from oracle import refbind
+    rows = _packed_rows()
+    if refbind.available():
+        tri, _, edge = refbind.tables()
+        assert np.array_equal(rows, tri)
+        assert edge.tolist() == EDGES
+    rows_seen = set()
+    for name, case, i, j, k, lin, t in _golden_active_cubes(golden):
+        c = golden[name + "/coords"]
+        ti = int(golden[name + "/table_idx"][lin])
+        r = rows[ti][rows[ti] >= 0]
+        assert len(r) == 3 * int(golden[name + "/ntri"][lin]), (name, lin, ti)
+        soup = golden[name + "/soup"][t:t + len(r) // 3].reshape(-1, 3)
+        # corner v at (i,j,k) + bits 0,1,2 of v ^ ((v >> 1) & 1) (mcb_tables.h)
+        P = np.array([[c[i + (o & 1)], c[j + (o >> 1 & 1)], c[k + (o >> 2 & 1)]] for o in (v ^ (v >> 1 & 1) for v in range(8))], np.float32)
+        for p, e in zip(soup, r):
+            a, b = P[EDGES[e][0]], P[EDGES[e][1]]
+            ax = int(np.flatnonzero(a != b)[0])
+            assert all(p[d] == a[d] for d in range(3) if d != ax), (name, lin, ti, e)
+            assert min(a[ax], b[ax]) <= p[ax] <= max(a[ax], b[ax]) or np.isnan(p[ax]), (name, lin, ti, e)
+        rows_seen.add(ti)
+    assert len(rows_seen) >= 228
 
 
 def test_triangle_table_invariants():
@@ -140,21 +178,36 @@ def test_triangle_table_invariants():
             assert ((code >> EA[e]) ^ (code >> EB[e])) & 1, "row references a non-crossing edge"
 
 
-def test_ambiguity_faces_equal_reference(mcb, refbind, golden):
-    """The derived face-per-code table (mcb_tables.h) against the table the reference ships, all 256 rows."""
-    _, amb, _ = refbind.tables()
+def test_ambiguity_faces_equal_reference(mcb, golden):
+    """The derived face-per-code table (mcb_tables.h) against the reference.  Where oracle/_ref is built: all 256 rows of
+    the table it ships.  Always: the reference's golden runs (tests/golden/cases.npz) — the cubes it counted as ambiguous
+    are exactly the active cubes whose code has a face here, and every cube it redirected took row 255 - code."""
+    from oracle import refbind
+    from .helpers import load_meta
     FACE = [(0, 1, 2, 3), (1, 2, 6, 5), (4, 5, 6, 7), (0, 3, 7, 4), (3, 2, 6, 7), (0, 1, 5, 4)]
+    derived = []
     for code in range(256):
         f = -1
         for fi in (0, 1, 2, 3, 5, 4):
             b = [(code >> v) & 1 for v in FACE[fi]]
             if b[0] == b[2] and b[1] == b[3] and b[0] != b[1]:
                 f = fi
-        if f < 0:
-            assert amb[code][0] == -1
-        else:
-            assert amb[code].tolist() == [255 - code] + list(FACE[f])
-    assert int((amb[:, 0] >= 0).sum()) == 120
+        derived.append([-1] if f < 0 else [255 - code] + list(FACE[f]))
+    assert sum(len(d) > 1 for d in derived) == 120
+    if refbind.available():
+        _, amb, _ = refbind.tables()
+        for code in range(256):
+            assert amb[code][0] == -1 if len(derived[code]) == 1 else amb[code].tolist() == derived[code]
+    redirected_seen = 0
+    for name, case in load_meta(golden).items():
+        code, tidx = golden[name + "/code"].astype(np.int64), golden[name + "/table_idx"].astype(np.int64)
+        active = (code != 0) & (code != 255)
+        has_face = np.array([len(d) > 1 for d in derived])[code]
+        assert int((active & has_face).sum()) == case["ambiguous"], name
+        red = tidx != code
+        assert int(red.sum()) == case["redirected"] and np.all(has_face[red]) and np.array_equal(tidx[red], 255 - code[red]), name
+        redirected_seen += int(red.sum())
+    assert redirected_seen > 0
 
 
 def test_lowering_bit_exact_on_host(mcb, refbind):
@@ -342,7 +395,7 @@ def test_random_equations_lower_bit_exactly(mcb, refbind):
                 eq = eq[:i] + eq[i + 1:] if k == 0 else eq[:i] + ch + eq[i:] if k == 1 else eq[:i] + ch + eq[i + 1:]
         if not eq or len(eq) > 120:
             continue
-        ref_ok, ours_ok = bool(refbind.lib().mcref_parse_ok(eq.encode())), mcb.parse_ok(eq)
+        ref_ok, ours_ok = refbind.parse_ok(eq), mcb.parse_ok(eq)
         assert ref_ok or not ours_ok, eq
         if not ref_ok:
             rejected += 1

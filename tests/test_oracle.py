@@ -48,7 +48,8 @@ def test_restatement_repeating_surface_mode_matches_reference_goldens(OB):
     """marching.cpp:481-494 in the restatement: per-cube level for code and ambiguity, Marching::interp's own constant for
     the points — against the unmodified reference's runs (tests/golden/repeat_cases.npz)."""
     import json
-    rep = np.load(os.path.join(ROOT, "tests", "golden", "repeat_cases.npz"), allow_pickle=False)
+    from .helpers import load_repeat_golden
+    rep = load_repeat_golden(os.path.join(ROOT, "tests", "golden", "repeat_cases.npz"))
     for name, case in json.loads(bytes(rep["meta_json"]).decode()).items():
         o = OB.Oracle(case["eq"], case["step"], tuple(case["scale"]), case["iso"], cons=[tuple(c) for c in case["cons"]], repeat=case["dist"])
         sw = o.sweep(nthreads=4)
@@ -80,7 +81,8 @@ def test_restatement_gradient_normals_match_numpy(OB, golden):
         assert same_bits(sw["grad_normals"], nref), name
 
 
-def test_restatement_against_live_reference(OB, refbind):
+def test_restatement_against_live_reference(OB, unmodified_reference):
+    refbind = unmodified_reference
     rng = np.random.default_rng(3)
     pts = (rng.random((3000, 3), dtype=np.float32) * 4 - 2).astype(np.float32)
     eqs = list(refbind.EXAMPLE_EQUATIONS.values()) + [refbind.GYR78, "x-y+z", "x/y*z", "-x^2", "x*-y+z", "x^y^z",
@@ -96,6 +98,22 @@ def test_restatement_against_live_reference(OB, refbind):
     v2, t2 = o.recalculate()
     assert same_bits(v, v2) and np.array_equal(t, t2)
     assert same_bits(r.normals(), o.normals())
+
+
+def test_restatement_tokenizer_against_reference_verdicts(OB):
+    """mco_tokenize_ok, which stands in for Evaluator::tokenize where oracle/_ref is not built, against verdicts of the
+    reference itself: Evaluator::test()'s nine known answers and every equation (and constraint) its golden runs took."""
+    import json
+    from .helpers import load_repeat_golden
+    from .test_host_logic import EVALUATOR_TEST_CASES
+    for eq, ok in EVALUATOR_TEST_CASES:
+        assert bool(OB.lib().mco_tokenize_ok(eq.encode())) == ok, eq
+    metas = [load_meta(np.load(os.path.join(ROOT, "tests", "golden", f + ".npz"), allow_pickle=False)) for f in ("cases", "seed_cases")]
+    metas.append(json.loads(bytes(load_repeat_golden(os.path.join(ROOT, "tests", "golden", "repeat_cases.npz"))["meta_json"]).decode()))
+    eqs = {e for m in metas for case in m.values() for e in [case["eq"]] + [c[0] for c in case.get("cons", [])]}
+    assert len(eqs) >= 15
+    for eq in eqs:
+        assert OB.lib().mco_tokenize_ok(eq.encode()), eq
 
 
 def test_parse_accept_reject_matches_product(OB, mcb):
