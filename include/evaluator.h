@@ -31,15 +31,19 @@ public:
     explicit Evaluator(std::string s) : ctx_(nullptr), equation_("x+y") {
         if (!set_equation(s)) throw std::exception();
     }
-    Evaluator(const Evaluator& o) : ctx_(nullptr), equation_(o.equation_) {}
+    Evaluator(const Evaluator& o) : ctx_(nullptr), equation_(o.equation_), function_grammar_(o.function_grammar_) {}
     Evaluator& operator=(const Evaluator& o) {
-        if (this != &o) { equation_ = o.equation_; if (ctx_) mcb_set_equation(ctx_, 0, equation_.c_str()); }
+        if (this != &o) {
+            equation_ = o.equation_;
+            function_grammar_ = o.function_grammar_;
+            if (ctx_) { mcb_set_grammar(ctx_, grammar()); mcb_set_equation(ctx_, 0, equation_.c_str()); }
+        }
         return *this;
     }
     ~Evaluator() { if (ctx_) mcb_destroy(ctx_); }
 
     bool set_equation(std::string s) {
-        if (mcb_parse(s.c_str()) != MCB_OK) return false;
+        if (mcb_grammar_text(s.c_str(), grammar(), -1, nullptr, 0) != MCB_OK) return false; /* mcb_parse by default */
         std::string cleaned;
         for (char c : s) if (c != ' ') cleaned.push_back(c);
         equation_ = cleaned;
@@ -52,6 +56,7 @@ public:
     float evaluate(float x, float y, float z) {
         if (!ctx_) {
             if (mcb_create(device_from_env(), &ctx_) != MCB_OK) throw std::exception(); /* no CPU fallback */
+            mcb_set_grammar(ctx_, grammar());
             if (mcb_set_equation(ctx_, 0, equation_.c_str()) != MCB_OK) throw std::exception();
         }
         const float p[3] = {x, y, z};
@@ -97,9 +102,19 @@ public:
     /* extension used by Marching: the current (cleaned) equation text */
     const std::string& equation() const { return equation_; }
 
+    /* Extension: on = later set_equation calls accept sin( cos( sqrt( abs( (MCB_GRAMMAR_FUNCTIONS, mcb.h); off (the
+     * default) = exactly the reference's language.  The current equation is kept either way.  test() always checks the
+     * reference grammar. */
+    void set_function_grammar(bool on) {
+        function_grammar_ = on;
+        if (ctx_) mcb_set_grammar(ctx_, grammar());
+    }
+    int grammar() const { return function_grammar_ ? MCB_GRAMMAR_FUNCTIONS : MCB_GRAMMAR_REFERENCE; }
+
 private:
     static int device_from_env() { const char* d = std::getenv("MCB_DEVICE"); return d ? std::atoi(d) : 0; }
     static const char* file_name() { const char* f = std::getenv("MCB_EQUATION_FILE"); return f ? f : "equation.txt"; }
     mcb_ctx* ctx_;
     std::string equation_;
+    bool function_grammar_ = false;
 };

@@ -194,6 +194,8 @@ public:
         Comp_Op o;
         if (op == "<=") o = LE; else if (op == ">=") o = GE; else if (op == "<") o = LT; else if (op == ">") o = GT; else return false;
         if (!ensure_ctx()) return false;
+        /* the left-hand side parses in the grammar of the evaluator set at this time (the reference's without one) */
+        mcb_set_grammar(ctx_, evaluator_ ? evaluator_->grammar() : MCB_GRAMMAR_REFERENCE);
         if (mcb_set_equation(ctx_, i + 1, lhs.c_str()) != MCB_OK) return false;
         cons_valid_[i] = true; cons_op_[i] = o; cons_rhs_[i] = rhs;
         reset_step();
@@ -318,6 +320,7 @@ private:
     }
     bool push_parameters() { return push_parameters(ctx_); }
     bool push_parameters(mcb_ctx* c) {
+        mcb_set_grammar(c, evaluator_->grammar()); /* Evaluator::set_function_grammar */
         if (mcb_set_equation(c, 0, evaluator_->equation().c_str()) != MCB_OK) return false;
         mcb_set_surface_constant(c, iso_);
         mcb_set_scaling(c, sx_, sy_, sz_);

@@ -92,6 +92,21 @@ const char* mcb_build_stamp(void);
 int mcb_struct_size(int which);
 const char* mcb_status_string(int status);
 
+/* Equation grammars (mcb_set_grammar, mcb_grammar_text).
+ *   MCB_GRAMMAR_REFERENCE (default)  the reference's language: numbers, x y z (either case), + - * / ^, brackets.
+ *   MCB_GRAMMAR_FUNCTIONS            the same plus four functions, lowercase, each written with its bracket: sin( cos(
+ *                                    sqrt( abs( (blanks are stripped first, so `sin (x)` is `sin(x)`; `sinx`, `SIN(x)`,
+ *                                    `sin()` are parse errors).  A function bracket is a '(' for every rule of the
+ *                                    reference's tokenizer and evaluator: implicit multiplication before it (`2sin(x)`
+ *                                    is 2*sin(x)), unary minus after it (`sin(-x)`), and `f(E)` is the bracketed operand
+ *                                    (E) with f applied at its ')' — so `-sin(x)^2` is (-sin(x))^2, as `-(x)^2` is (-x)^2.
+ *                                    Every equation of the reference grammar parses to the same tokens, operation order
+ *                                    and bytecode.  sin / cos are glibc's sinf / cosf restated bit for bit on the device
+ *                                    (csrc/mcb_trig.h), sqrt is correctly rounded, abs clears the sign bit; all else is
+ *                                    unchanged fp32 without FMA contraction. */
+#define MCB_GRAMMAR_REFERENCE 0
+#define MCB_GRAMMAR_FUNCTIONS 1
+
 /* Evaluator::tokenize accept/reject (evaluator.cpp:139-237) + the operand-stack check: MCB_OK or MCB_E_PARSE. */
 int mcb_parse(const char* equation);
 /* Token list as text, blank separated, unary minus printed as NEG (evaluator.cpp:165).  Returns MCB_OK,
@@ -103,6 +118,10 @@ int mcb_postfix(const char* equation, char* out, size_t cap);
 /* Bytecode listing; which: 0 = point program, 1 = grid program (postfix), 2 = hoisted slot programs,
  * 3 = grid program in the fused accumulator form the grid kernel executes. */
 int mcb_disassemble(const char* equation, int which, char* out, size_t cap);
+/* The four helpers above under a chosen grammar (MCB_GRAMMAR_*; MCB_E_ARG for another value).  what: -1 = accept/reject
+ * only (out unused; as mcb_parse), 0 = tokens (as mcb_tokens; a function prints as `sin(`), 1 = postfix (as mcb_postfix;
+ * a function follows its operand: `x sin`), 2 + w = bytecode listing w of mcb_disassemble. */
+int mcb_grammar_text(const char* equation, int grammar, int what, char* out, size_t cap);
 /* The reference's grid loop on one axis (marching.cpp:372-377): returns M = number of cubes per axis for `step`
  * and, when coords != NULL and cap >= M+1, the cube origins c[0..M-1] and the far corner c[M] = c[M-1]+step. */
 int mcb_grid_axis(float step, float* coords, int cap);
@@ -127,6 +146,9 @@ int mcb_set_stream(mcb_ctx* ctx, void* cuda_stream);
  * marching.cpp:140-147); slots 1..3 = left-hand sides of constraints 0..2 (marching.cpp:173-200).
  * On MCB_E_PARSE the previous equation of that slot stays in force. */
 int mcb_set_equation(mcb_ctx* ctx, int slot, const char* equation);
+/* MCB_GRAMMAR_REFERENCE (default) or MCB_GRAMMAR_FUNCTIONS for the mcb_set_equation calls that follow, in every slot
+ * (surface and constraint left-hand sides).  Equations already set keep their programs. */
+int mcb_set_grammar(mcb_ctx* ctx, int grammar);
 /* Evaluator::evaluate (evaluator.cpp:53-107) for n points on the GPU.  xyz = 3n floats, out = n floats, host
  * memory.  apply_scale != 0 multiplies by the per-axis scale first, i.e. Marching::evaluate (marching.cpp:209-224). */
 int mcb_eval_points(mcb_ctx* ctx, int slot, const float* xyz, float* out, size_t n, int apply_scale);
@@ -193,7 +215,8 @@ int mcb_set_repeat(mcb_ctx* ctx, int enabled, float distance);
  * dispatch (torus 2.3 -> 1.5 ms, polynomial gyroid 1.3 -> 0.7 ms at 1024^3).  Constants, grid size and scaling are
  * kernel arguments: only a new equation compiles again.
  *   MCB_JIT_AUTO (default)  use it when NVRTC is there, the compile succeeds and the program has at most 8 `^` left after
- *                           hoisting (more: powf dominates either way and compile time grows), else the bytecode
+ *                           hoisting (more: powf dominates either way and compile time grows; sin and cos of the function
+ *                           grammar do not count: the kernel calls one out-of-line copy of each), else the bytecode
  *                           interpreter — both are the same CUDA path with the same results; mcb_counts::jit says which ran.
  *                           The compile runs on a background thread: the first mesh of a new equation does not wait for
  *                           NVRTC, the calls made meanwhile interpret, the first call after the compile has finished
@@ -212,6 +235,8 @@ int mcb_jit_wait(mcb_ctx* ctx);
 /* Host-only: generate and compile the specialised kernel for `equation` (no GPU needed).  Returns the cubin size in
  * bytes (> 0) and the generated CUDA source in `log`, or a negative status with the error / compile log in `log`. */
 int mcb_jit_check(const char* equation, char* log, size_t cap);
+/* The same under a chosen grammar (MCB_GRAMMAR_*). */
+int mcb_jit_check_grammar(const char* equation, int grammar, char* log, size_t cap);
 
 /* MCB_FIELD_DENSE (default), MCB_FIELD_SPARSE or MCB_FIELD_AUTO: whether mcb_polygonise evaluates and writes the whole
  * scalar field or only the blocks of it around the surface (SURVEY §8f N4).  Results are bit-identical.  The C++ drop-in

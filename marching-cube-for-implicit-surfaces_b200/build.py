@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmcb200.so")
 SOURCES = ["mcb_api.cu", "mcb_lower.cpp", "mcb_jit.cpp"]
 HEADERS = [os.path.join("..", "..", "tools", "headless_main.cpp"), os.path.join("..", "..", "include", "marching.h"),
-           os.path.join("..", "..", "include", "evaluator.h"), "mcb_kernels.cuh", "mcb_jit.h", "mcb_bytecode.h", "mcb_pow.h", "mcb_tables.h", "mcb_tri_words.inc", "mcb_lower.h",
+           os.path.join("..", "..", "include", "evaluator.h"), "mcb_kernels.cuh", "mcb_jit.h", "mcb_bytecode.h", "mcb_pow.h", "mcb_trig.h", "mcb_interval.h", "mcb_tables.h", "mcb_tri_words.inc", "mcb_lower.h",
            os.path.join("..", "..", "include", "mcb.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-fmad=false",
@@ -51,9 +51,11 @@ def build(force=False, verbose=False):
         force = True  # a source changed since the library was built, whatever the mtimes say
     if not force and not stale():
         return LIB
-    # mcb_pow.h also travels inside the library as text: the run-time compiled evaluator (mcb_jit.cpp) includes it through NVRTC
-    with open(os.path.join(CSRC, "mcb_pow.h")) as f, open(os.path.join(CSRC, "mcb_pow_src.inc"), "w") as o:
-        o.write('R"MCBPOWSRC(' + f.read() + ')MCBPOWSRC"\n')
+    # mcb_pow.h and mcb_trig.h also travel inside the library as text: the run-time compiled evaluator (mcb_jit.cpp)
+    # includes them through NVRTC
+    for name, inc, tag in (("mcb_pow.h", "mcb_pow_src.inc", "MCBPOWSRC"), ("mcb_trig.h", "mcb_trig_src.inc", "MCBTRIGSRC")):
+        with open(os.path.join(CSRC, name)) as f, open(os.path.join(CSRC, inc), "w") as o:
+            o.write('R"%s(' % tag + f.read() + ')%s"\n' % tag)
     cmd = [NVCC] + FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB] + [os.path.join(CSRC, s) for s in SOURCES] + ["-ldl"]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or r.returncode != 0:

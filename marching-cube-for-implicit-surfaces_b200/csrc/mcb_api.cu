@@ -54,6 +54,7 @@ struct mcb_ctx {
     std::string err;
 
     EqSlot eq[4];
+    int grammar = MCB_GRAMMAR_REFERENCE; /* mcb_set_grammar: how later mcb_set_equation calls parse */
     Constraint cons[3];
     float step = 0.25f;
     int M = 0;
@@ -249,7 +250,7 @@ void free_slot(EqSlot& s) {
 int install_equation(mcb_ctx* ctx, int slot, const char* equation) {
     mcb::Compiled c;
     std::string err;
-    int rc = mcb::compile(equation ? equation : "", c, &err);
+    int rc = mcb::compile(equation ? equation : "", c, &err, ctx->grammar);
     if (rc != MCB_OK) return fail(ctx, rc, err);
 
     EqSlot ns;
@@ -505,34 +506,33 @@ const char* mcb_status_string(int s) {
     }
 }
 
-int mcb_parse(const char* equation) {
-    mcb::Compiled c;
-    return mcb::compile(equation ? equation : "", c, nullptr);
-}
+int mcb_parse(const char* equation) { return mcb_grammar_text(equation, MCB_GRAMMAR_REFERENCE, -1, nullptr, 0); }
 
-int mcb_tokens(const char* equation, char* out, size_t cap) {
-    std::vector<mcb::Token> t;
-    if (!mcb::tokenize(equation ? equation : "", t, nullptr)) return MCB_E_PARSE;
-    std::string s;
-    for (size_t i = 0; i < t.size(); i++) { if (i) s += ' '; s += t[i].text; }
-    return copy_text(s, out, cap);
-}
+int mcb_tokens(const char* equation, char* out, size_t cap) { return mcb_grammar_text(equation, MCB_GRAMMAR_REFERENCE, 0, out, cap); }
 
-int mcb_postfix(const char* equation, char* out, size_t cap) {
-    mcb::Compiled c;
-    int rc = mcb::compile(equation ? equation : "", c, nullptr);
-    if (rc != MCB_OK) return rc;
-    return copy_text(mcb::postfix_text(c.expr), out, cap);
-}
+int mcb_postfix(const char* equation, char* out, size_t cap) { return mcb_grammar_text(equation, MCB_GRAMMAR_REFERENCE, 1, out, cap); }
 
 int mcb_disassemble(const char* equation, int which, char* out, size_t cap) {
+    return mcb_grammar_text(equation, MCB_GRAMMAR_REFERENCE, 2 + (which == 0 || which == 1 || which == 3 ? which : 2), out, cap);
+}
+
+int mcb_grammar_text(const char* equation, int grammar, int what, char* out, size_t cap) {
+    if (grammar != MCB_GRAMMAR_REFERENCE && grammar != MCB_GRAMMAR_FUNCTIONS) return MCB_E_ARG;
+    if (what == 0) {
+        std::vector<mcb::Token> t;
+        if (!mcb::tokenize(equation ? equation : "", t, nullptr, grammar)) return MCB_E_PARSE;
+        std::string s;
+        for (size_t i = 0; i < t.size(); i++) { if (i) s += ' '; s += t[i].text; }
+        return copy_text(s, out, cap);
+    }
     mcb::Compiled c;
-    int rc = mcb::compile(equation ? equation : "", c, nullptr);
-    if (rc != MCB_OK) return rc;
+    int rc = mcb::compile(equation ? equation : "", c, nullptr, grammar);
+    if (rc != MCB_OK || what < 0) return rc;
     std::string s;
-    if (which == 0) s = mcb::disassemble(c.point_code);
-    else if (which == 1) s = mcb::disassemble(c.grid_code);
-    else if (which == 3) s = mcb::disassemble_fused(c.grid_fused);
+    if (what == 1) s = mcb::postfix_text(c.expr);
+    else if (what == 2) s = mcb::disassemble(c.point_code);
+    else if (what == 3) s = mcb::disassemble(c.grid_code);
+    else if (what == 5) s = mcb::disassemble_fused(c.grid_fused);
     else {
         for (const mcb::Slot& sl : c.slots) {
             std::vector<uint32_t> code(c.slot_code.begin() + sl.code_begin, c.slot_code.begin() + sl.code_begin + sl.code_len);
@@ -604,7 +604,8 @@ int mcb_create(int device, mcb_ctx** out) {
     {
         const int stack_bytes = MCB_MAX_STACK * kEvalRows * kEvalThreads * (int)sizeof(float);
         const void* evals[] = {(const void*)eval_field_kernel<true, true>, (const void*)eval_field_kernel<false, true>,
-                               (const void*)eval_blocks_kernel<true>,      (const void*)eval_blocks_kernel<false>};
+                               (const void*)eval_blocks_kernel<true>,      (const void*)eval_blocks_kernel<false>,
+                               (const void*)eval_field_kernel<true, true, true>, (const void*)eval_blocks_kernel<true, true>};
         for (const void* k : evals)
             if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, stack_bytes) != cudaSuccess) return bail(MCB_E_CUDA);
         const char* poison = std::getenv("MCB_POISON_FIELD");
@@ -672,6 +673,13 @@ int mcb_set_equation(mcb_ctx* ctx, int slot, const char* equation) {
     if (rc != MCB_OK) return rc;
     if (slot < 0 || slot > 3) return fail(ctx, MCB_E_ARG, "slot must be 0..3");
     return install_equation(ctx, slot, equation);
+}
+
+int mcb_set_grammar(mcb_ctx* ctx, int grammar) {
+    if (!ctx) return MCB_E_ARG;
+    if (grammar != MCB_GRAMMAR_REFERENCE && grammar != MCB_GRAMMAR_FUNCTIONS) return fail(ctx, MCB_E_ARG, "grammar must be MCB_GRAMMAR_REFERENCE or MCB_GRAMMAR_FUNCTIONS");
+    ctx->grammar = grammar;
+    return MCB_OK;
 }
 
 int mcb_eval_points(mcb_ctx* ctx, int slot, const float* xyz, float* out, size_t n, int apply_scale) {
@@ -815,7 +823,7 @@ struct Run {
     uint32_t launches;
 
     int prepare_buffers();
-    int encode_program(mcb_program& launch, bool& has_pow, bool blocks);
+    int encode_program(mcb_program& launch, bool& has_pow, bool& has_fn, bool blocks);
     int ensure_block_buffers(FieldBlocks* fb, BlockDims* bd);
     int launch_block_eval(const FieldBlocks& fb, const uint32_t* list, const unsigned* count);
     int stage_eval_blocks();
@@ -860,9 +868,10 @@ int Run::prepare_buffers() {
 
 /* Device form of the fused grid program: dense handler numbers, table operands as absolute float offsets into
  * d_tables, and  LOAD/PUSH a ; op b  pairs folded into one two-word instruction (eval_pair). */
-int Run::encode_program(mcb_program& launch, bool& has_pow, bool blocks) {
+int Run::encode_program(mcb_program& launch, bool& has_pow, bool& has_fn, bool blocks) {
     launch = eq.grid;
     has_pow = false;
+    has_fn = false;
     {
         /* operand class of a source as the kernel's lane patch sees it; eval_blocks_kernel's patch is (y, z) per x
          * column, so there the x and z tables trade places */
@@ -882,6 +891,7 @@ int Run::encode_program(mcb_program& launch, bool& has_pow, bool blocks) {
             const uint32_t wd = eq.grid.code[pc], fop = MCB_FINSN_OP(wd), src = MCB_FINSN_SRC(wd);
             has_pow |= fop == MCB_F_POW || fop == MCB_F_RPOW;
             if (fop == MCB_F_NEG) { launch.code[n++] = MCB_HANDLER_NEG; continue; }
+            if (MCB_F_IS_FN(fop)) { launch.code[n++] = MCB_HANDLER_FN(fop); has_fn = true; continue; }
             if (src < MCB_SRC_K || src > MCB_SRC_POP) return fail(ctx, MCB_E_STATE, "internal: raw coordinate operand in a grid program");
             uint32_t arg;
             if (!resolve(src, MCB_FINSN_ARG(wd), &arg)) return fail(ctx, MCB_E_CAPACITY, "axis tables too large for the operand field");
@@ -1064,9 +1074,10 @@ int Run::stage_eval() {
     if (!ctx->jit_used) {
         const size_t smem = (size_t)std::max(1, eq.c.grid_fused_depth) * kEvalRows * kEvalThreads * sizeof(float);
         mcb_program launch;
-        bool has_pow;
-        if ((rc = encode_program(launch, has_pow, false)) != MCB_OK) return rc;
-        if (has_pow) MCB_LAUNCH((eval_field_kernel<true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        bool has_pow, has_fn;
+        if ((rc = encode_program(launch, has_pow, has_fn, false)) != MCB_OK) return rc;
+        if (has_fn) MCB_LAUNCH((eval_field_kernel<true, true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        else if (has_pow) MCB_LAUNCH((eval_field_kernel<true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
         else MCB_LAUNCH((eval_field_kernel<false, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
         launches++;
     }
@@ -1132,10 +1143,11 @@ int Run::launch_block_eval(const FieldBlocks& fb, const uint32_t* list, const un
 #endif
     } else {
         mcb_program launch;
-        bool has_pow;
-        if ((rc = encode_program(launch, has_pow, true)) != MCB_OK) return rc;
+        bool has_pow, has_fn;
+        if ((rc = encode_program(launch, has_pow, has_fn, true)) != MCB_OK) return rc;
         const size_t smem = (size_t)std::max(1, eq.c.grid_fused_depth) * kEvalRows * kEvalThreads * sizeof(float);
-        if (has_pow) MCB_LAUNCH((eval_blocks_kernel<true>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
+        if (has_fn) MCB_LAUNCH((eval_blocks_kernel<true, true>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
+        else if (has_pow) MCB_LAUNCH((eval_blocks_kernel<true>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
         else MCB_LAUNCH((eval_blocks_kernel<false>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
     }
     launches++;
@@ -1610,9 +1622,12 @@ int mcb_jit_wait(mcb_ctx* ctx) {
     return 0;
 }
 
-int mcb_jit_check(const char* equation, char* log, size_t cap) {
+int mcb_jit_check(const char* equation, char* log, size_t cap) { return mcb_jit_check_grammar(equation, MCB_GRAMMAR_REFERENCE, log, cap); }
+
+int mcb_jit_check_grammar(const char* equation, int grammar, char* log, size_t cap) {
+    if (grammar != MCB_GRAMMAR_REFERENCE && grammar != MCB_GRAMMAR_FUNCTIONS) return MCB_E_ARG;
     mcb::Compiled c;
-    int rc = mcb::compile(equation ? equation : "", c, nullptr);
+    int rc = mcb::compile(equation ? equation : "", c, nullptr, grammar);
     if (rc != MCB_OK) return rc;
     std::string err;
     bool has_pow = false;

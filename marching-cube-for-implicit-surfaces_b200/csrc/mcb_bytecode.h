@@ -6,6 +6,8 @@
  *      top (op) second         for the reversed forms OP_RSUB/RDIV/RPOW
  * so the lowering can evaluate the operands of the reference's `val2 (op) val1` (evaluator.cpp:38-40) in either
  * order while each value keeps its role.  All arithmetic is fp32 without FMA contraction; `^` is mcb_powf.
+ * The function grammar's unary operators: sin / cos are mcb_sinf / mcb_cosf (mcb_trig.h, glibc's sinf / cosf), sqrt is
+ * the correctly rounded square root (sqrtf on the host, __fsqrt_rn on the device), abs clears the sign bit.
  *
  * Programs travel to the kernels inside the kernel-parameter block, i.e. in the constant bank: every lane of a
  * warp executes the same instruction word, fetched with a uniform constant load.
@@ -16,6 +18,7 @@
 #include <stdint.h>
 
 #include "mcb_pow.h"
+#include "mcb_trig.h"
 
 enum {
     MCB_OP_END = 0,
@@ -35,8 +38,13 @@ enum {
     MCB_OP_POW,
     MCB_OP_RPOW,
     MCB_OP_NEG,
+    MCB_OP_SIN,  /* function grammar: unary, act on the top of the stack like NEG */
+    MCB_OP_COS,
+    MCB_OP_SQRT,
+    MCB_OP_ABS,
     MCB_OP_COUNT
 };
+#define MCB_OP_IS_UNARY(op) ((op) == MCB_OP_NEG || ((op) >= MCB_OP_SIN && (op) <= MCB_OP_ABS))
 
 #define MCB_MAX_CODE 384   /* instructions per program (a 256-char equation yields < 300) */
 #define MCB_MAX_K 128      /* constant pool entries */
@@ -73,6 +81,27 @@ MCB_BC_FN float mcb_binop(uint32_t op, float second, float top) {
     }
 }
 
+/* The function grammar's functions, fn = 0 sin, 1 cos, 2 sqrt, 3 abs.  Out of line: the scalar interpreters call it
+ * rarely and should not carry the inlined fp64 trigonometry in every kernel that interprets a program. */
+#if defined(__CUDACC__)
+static __host__ __device__ __noinline__
+#else
+static
+#endif
+float mcb_fn(uint32_t fn, float v) {
+    switch (fn) {
+        case 0: return mcb_sinf(v);
+        case 1: return mcb_cosf(v);
+        case 2:
+#if defined(__CUDA_ARCH__)
+            return __fsqrt_rn(v);
+#else
+            return sqrtf(v);
+#endif
+        default: return mcb_u2f(mcb_f2u(v) & 0x7fffffffu);
+    }
+}
+
 /* Plain scalar interpreter: one point, memory stack.  Used for the rare, divergent evaluations (ambiguity face
  * centres, mcb_eval_points, constant folding, axis tables); the per-vertex grid kernel has its own register-cached
  * version.  tx/ty/tz = this point's table values per slot (may be NULL when the program has no table loads). */
@@ -91,6 +120,9 @@ MCB_BC_FN float mcb_interp_scalar(const uint32_t* code, int n, const float* k, f
             case MCB_OP_PUSH_TY: st[sp++] = ty[arg]; break;
             case MCB_OP_PUSH_TZ: st[sp++] = tz[arg]; break;
             case MCB_OP_NEG: st[sp - 1] = -st[sp - 1]; break;
+            case MCB_OP_SIN: case MCB_OP_COS: case MCB_OP_SQRT: case MCB_OP_ABS:
+                st[sp - 1] = mcb_fn(op - MCB_OP_SIN, st[sp - 1]);
+                break;
             case MCB_OP_END: pc = n; break;
             default: {
                 float top = st[--sp];
@@ -112,6 +144,7 @@ MCB_BC_FN float mcb_interp_scalar(const uint32_t* code, int n, const float* k, f
  *      fop LOAD      acc = v                                    fop PUSH    spill acc to the memory stack; acc = v
  *      fop ADD, MUL  acc = acc (op) v                           fop NEG     acc = -acc  (src unused)
  *      fop SUB/DIV/POW  acc = acc (op) v                        fop RSUB/RDIV/RPOW  acc = v (op) acc
+ *      fop SIN, COS, SQRT, ABS  acc = f(acc)  (src unused; the function grammar, like NEG)
  * Every fp32 operation and the role of each operand are those of the postfix program; only pushes and pops of
  * the operand stack disappear.  `x^2+y^2+z^2-0.49` (grid form TX0 TY0 TZ0 K0 - + +) becomes
  *      LOAD TZ0; SUB K0; ADD TY0; ADD TX0 — 4 words and no memory-stack traffic at all.
@@ -119,8 +152,9 @@ MCB_BC_FN float mcb_interp_scalar(const uint32_t* code, int n, const float* k, f
 enum { MCB_SRC_X = 0, MCB_SRC_Y, MCB_SRC_Z, MCB_SRC_K, MCB_SRC_TX, MCB_SRC_TY, MCB_SRC_TZ, MCB_SRC_POP };
 enum {
     MCB_F_LOAD = 0, MCB_F_PUSH, MCB_F_ADD, MCB_F_SUB, MCB_F_RSUB, MCB_F_MUL, MCB_F_DIV, MCB_F_RDIV, MCB_F_POW,
-    MCB_F_RPOW, MCB_F_NEG, MCB_F_COUNT
+    MCB_F_RPOW, MCB_F_NEG, MCB_F_SIN, MCB_F_COS, MCB_F_SQRT, MCB_F_ABS, MCB_F_COUNT
 };
+#define MCB_F_IS_FN(fop) ((fop) >= MCB_F_SIN && (fop) <= MCB_F_ABS)
 #define MCB_FINSN(fop, src, arg) ((uint32_t)(fop) | ((uint32_t)(src) << 4) | ((uint32_t)(arg) << 8))
 #define MCB_FINSN_OP(w) ((w) & 0xFu)
 #define MCB_FINSN_SRC(w) (((w) >> 4) & 0xFu)
@@ -149,6 +183,7 @@ MCB_BC_FN float mcb_interp_fused_scalar(const uint32_t* code, int n, const float
     for (int pc = 0; pc < n; pc++) {
         uint32_t w = code[pc], fop = MCB_FINSN_OP(w), src = MCB_FINSN_SRC(w), arg = MCB_FINSN_ARG(w);
         if (fop == MCB_F_NEG) { acc = -acc; continue; }
+        if (MCB_F_IS_FN(fop)) { acc = mcb_fn(fop - MCB_F_SIN, acc); continue; }
         if (fop == MCB_F_PUSH) st[sp++] = acc;
         float v;
         switch (src) {

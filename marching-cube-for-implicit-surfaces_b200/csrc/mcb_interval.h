@@ -19,6 +19,14 @@
  *   - e a positive integer and any base: odd powers are monotone, even powers are monotone in |x|; widened likewise.
  * Everything else is "unknown".  tests/test_interval.py checks the enclosure and the proof against brute force on the
  * example equations and on random programs.
+ *
+ * The function grammar's functions (tests/test_functions_host.py checks them against brute force likewise):
+ *   - abs: exact, [|lo|, |hi|] ordered, or [0, max(-lo, hi)] when the interval contains 0;
+ *   - sqrt: correctly rounded, hence monotone: [sqrt(lo), sqrt(hi)] when lo >= 0; lo < 0 is "unknown";
+ *   - sin, cos: [-1, 1] for any argument interval.  mcb_sinf / mcb_cosf are not the real functions, so no bound may be
+ *     taken from analysis; this one rests on the exhaustive run of oracle/trig_exhaustive.c (every finite result of
+ *     either function, over all 2^32 inputs, lies in [-1, 1]).  Hoisted sin / cos need no rule at all: their values
+ *     are axis-table entries, whose exact minimum and maximum over the box are the leaves.
  */
 #ifndef MCB_INTERVAL_H
 #define MCB_INTERVAL_H
@@ -108,6 +116,28 @@ MCB_BC_FN mcb_ival mcb_iv_op(uint32_t fop, mcb_ival acc, mcb_ival v, int* bad) {
     return r;
 }
 
+/* f(a) for the function grammar's fop SIN / COS / SQRT / ABS; *bad is set when the rules do not cover the case */
+MCB_BC_FN mcb_ival mcb_iv_fn(uint32_t fop, mcb_ival a, int* bad) {
+    mcb_ival r;
+    switch (fop) {
+        case MCB_F_ABS:
+            if (a.lo >= 0.f) r = a;
+            else if (a.hi <= 0.f) { r.lo = -a.hi; r.hi = -a.lo; }
+            else { r.lo = 0.f; r.hi = mcb_iv_max(-a.lo, a.hi); }
+            break;
+        case MCB_F_SQRT:
+            if (!(a.lo >= 0.f)) { *bad = 1; r.lo = r.hi = 0.f; break; }
+            r.lo = mcb_fn(2, a.lo);
+            r.hi = mcb_fn(2, a.hi);
+            break;
+        default: /* sin, cos */
+            r.lo = -1.f;
+            r.hi = 1.f;
+            break;
+    }
+    return r;
+}
+
 /* Bounds of the axis-table operands over the box: B[(axis * slots_per_axis + slot) * nb + b] = {min, max} of that
  * table over block b of that axis (a non-finite entry makes the pair {-inf, +inf}).  bx, by, bz = the box's block
  * index per axis.  Returns 0 = unknown, 1 = every vertex has sign bit 0 (value > iso is false), 2 = every vertex has
@@ -121,6 +151,7 @@ MCB_BC_FN int mcb_interval_class(const uint32_t* code, int n, const float* k, co
     for (int pc = 0; pc < n && !bad; pc++) {
         const uint32_t w = code[pc], fop = MCB_FINSN_OP(w), src = MCB_FINSN_SRC(w), arg = MCB_FINSN_ARG(w);
         if (fop == MCB_F_NEG) { const float t = acc.lo; acc.lo = -acc.hi; acc.hi = -t; continue; }
+        if (MCB_F_IS_FN(fop)) { acc = mcb_iv_fn(fop, acc, &bad); continue; }
         if (fop == MCB_F_PUSH) { if (sp >= MCB_MAX_STACK) { bad = 1; break; } st[sp++] = acc; }
         mcb_ival v;
         switch (src) {

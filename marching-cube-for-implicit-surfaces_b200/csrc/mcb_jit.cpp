@@ -12,6 +12,9 @@ namespace {
 const char* const kPowHeader =
 #include "mcb_pow_src.inc" /* mcb_pow.h as a raw string literal, written by build.py: one source for nvcc and NVRTC */
     ;
+const char* const kTrigHeader =
+#include "mcb_trig_src.inc" /* mcb_trig.h, likewise */
+    ;
 
 /* Everything around the generated body.  It restates the tile of eval_field_kernel (mcb_kernels.cuh): a warp owns 128
  * columns x 4 rows of one plane, a lane the columns x0 + 32 q; evict-first field stores, sign words by ballot.  The Grid
@@ -33,6 +36,15 @@ __device__ __forceinline__ float op_pow(float a, float b) { /* as fused_op<MCB_F
 }
 #define R(e) ((e) >> 2)
 #define Q(e) ((e) & 3)
+)SRC";
+/* The function grammar's operations, added to the source only when the program uses them: sin / cos out of line (one
+ * copy of the fp64 restatement of glibc's sinf / cosf each), sqrt correctly rounded, abs the sign bit cleared. */
+const char* const kHeadTrig = R"SRC(#include "mcb_trig.h"
+__device__ __noinline__ float op_sin(float a) { return mcb_sinf(a); }
+__device__ __noinline__ float op_cos(float a) { return mcb_cosf(a); }
+)SRC";
+const char* const kHeadSqrtAbs = R"SRC(__device__ __forceinline__ float op_sqrt(float a) { return __fsqrt_rn(a); }
+__device__ __forceinline__ float op_abs(float a) { return __uint_as_float(__float_as_uint(a) & 0x7fffffffu); }
 )SRC";
 const char* const kHeadPlane = R"SRC(
 extern "C" __global__ void __launch_bounds__(128, MCB_MIN_BLOCKS)
@@ -146,7 +158,8 @@ Nvrtc& nvrtc() {
 
 } /* namespace */
 
-static std::string generate_one(const uint32_t* code, int n, int kind /* 0 plane tiles (dense field), 1 listed 32 x 4 x 4 blocks */, bool* has_pow, std::string* err) {
+static std::string generate_one(const uint32_t* code, int n, int kind /* 0 plane tiles (dense field), 1 listed 32 x 4 x 4 blocks */, bool* has_pow,
+                                int* fns /* |= 1: sin or cos, 2: sqrt or abs */, std::string* err) {
     const bool blocks = kind == 1;
     const char* const N = "16";   /* values per lane */
     const char* const I = "e";    /* their index variable */
@@ -199,6 +212,15 @@ static std::string generate_one(const uint32_t* code, int n, int kind /* 0 plane
             acc = t;
             continue;
         }
+        if (MCB_F_IS_FN(fop)) {
+            if (acc.empty()) { *err = "function without a value"; return std::string(); }
+            static const char* const names[] = {"op_sin", "op_cos", "op_sqrt", "op_abs"};
+            *fns |= fop <= MCB_F_COS ? 1 : 2;
+            const std::string t = fresh();
+            body << "    float " << t << "[" << N << "];\n#pragma unroll\n    for (int " << I << " = 0; " << I << " < " << N << "; " << I << "++) " << t << "[" << I << "] = " << names[fop - MCB_F_SIN] << "(" << acc << "[" << I << "]);\n";
+            acc = t;
+            continue;
+        }
         std::string v;
         if (src == MCB_SRC_POP) {
             if (stack.empty()) { *err = "POP from an empty stack"; return std::string(); }
@@ -248,22 +270,27 @@ std::string generate(const uint32_t* code, int n, bool* has_pow, std::string* er
     /* one translation unit, two kernels: mcb_eval_jit (plane tiles: the whole field + signs, MCB_FIELD_DENSE) and
      * mcb_fill_jit (listed 32 x 4 x 4 vertex blocks: field + signs, the block-field mode) — one compile per equation
      * whatever mode runs later */
-    std::string out = kHead;
+    std::string parts;
+    int fns = 0;
     for (int kind = 0; kind < 2; kind++) {
-        const std::string part = generate_one(code, n, kind, has_pow, err);
+        const std::string part = generate_one(code, n, kind, has_pow, &fns, err);
         if (part.empty()) return part;
-        out += part;
+        parts += part;
     }
-    return out;
+    std::string out = kHead;
+    if (fns & 1) out += kHeadTrig;
+    if (fns & 2) out += kHeadSqrtAbs;
+    if ((fns & 1) && has_pow) *has_pow = true; /* out-of-line fp64 calls: the register budget of the powf kernels */
+    return out + parts;
 }
 
 std::string compile(const std::string& source, bool pow, int grid_size, std::vector<char>* cubin) {
     Nvrtc& N = nvrtc();
     if (!N.error.empty()) return N.error;
     void* prog = nullptr;
-    const char* hdr_src[] = {kPowHeader};
-    const char* hdr_name[] = {"mcb_pow.h"};
-    int rc = N.CreateProgram(&prog, source.c_str(), "mcb_eval_jit.cu", 1, hdr_src, hdr_name);
+    const char* hdr_src[] = {kPowHeader, kTrigHeader};
+    const char* hdr_name[] = {"mcb_pow.h", "mcb_trig.h"};
+    int rc = N.CreateProgram(&prog, source.c_str(), "mcb_eval_jit.cu", 2, hdr_src, hdr_name);
     if (rc != 0) return std::string("nvrtcCreateProgram: ") + N.GetErrorString(rc);
     char grid_bytes[64], max_k[64];
     std::snprintf(grid_bytes, sizeof grid_bytes, "-DMCB_GRID_BYTES=%d", grid_size);

@@ -249,6 +249,7 @@ __device__ __forceinline__ void eval_pair(float (&acc)[kEvalRows], uint32_t arg_
         for (int q = 0; q < 4; q++) acc[4 * r + q] = fused_op<FOP>(a.at(r, q), b.at(r, q));
 }
 #define MCB_HANDLER_SPILL 55 /* push the accumulator on the memory stack; the new value comes from the next (pair) word */
+#define MCB_HANDLER_FN(FOP) (56 + (FOP) - MCB_F_SIN) /* sin, cos, sqrt, abs of the accumulator: 56..59 (function grammar) */
 #define MCB_HANDLER_PAIR(FOP, CA, CB) (64 + ((FOP) - MCB_F_ADD) * 16 + (CA) * 4 + (CB))
 
 /* `prog` is the fused grid program with its table operands already resolved by the host for this launch:
@@ -267,9 +268,35 @@ constexpr int kEvalTileX = 128; /* columns per warp tile */
 constexpr int kEvalTileY = 4;   /* rows per warp tile */
 static_assert(kEvalRows == 16, "a lane carries a 4 x 4 patch");
 
+/* The function grammar's functions on the 16 accumulators (handlers 56..59).  sin / cos: the fp64 restatement of glibc's
+ * sinf / cosf (mcb_trig.h) out of line, one copy; sqrt: correctly rounded. */
+__device__ __noinline__ float sinf_call(float a) { return mcb_sinf(a); }
+__device__ __noinline__ float cosf_call(float a) { return mcb_cosf(a); }
+__device__ __forceinline__ void eval_fn(float (&acc)[kEvalRows], uint32_t handler) {
+    switch (handler) {
+        case MCB_HANDLER_FN(MCB_F_SIN):
+#pragma unroll
+            for (int e = 0; e < kEvalRows; e++) acc[e] = sinf_call(acc[e]);
+            break;
+        case MCB_HANDLER_FN(MCB_F_COS):
+#pragma unroll
+            for (int e = 0; e < kEvalRows; e++) acc[e] = cosf_call(acc[e]);
+            break;
+        case MCB_HANDLER_FN(MCB_F_SQRT):
+#pragma unroll
+            for (int e = 0; e < kEvalRows; e++) acc[e] = __fsqrt_rn(acc[e]);
+            break;
+        default: /* abs */
+#pragma unroll
+            for (int e = 0; e < kEvalRows; e++) acc[e] = __uint_as_float(__float_as_uint(acc[e]) & 0x7fffffffu);
+            break;
+    }
+}
+
 /* The interpreter proper: runs the launch program on the lane's 16 accumulators.  QS = distance, in table entries,
- * between the lane's four class-1 operands (32 in the plane-tile kernel, 1 in the block kernel below). */
-template <bool HAS_POW, int QS>
+ * between the lane's four class-1 operands (32 in the plane-tile kernel, 1 in the block kernel below).  HAS_FN: the
+ * program uses a function (handlers 56..59); without it the kernel is exactly the reference grammar's. */
+template <bool HAS_POW, int QS, bool HAS_FN = false>
 __device__ __forceinline__ void eval_run(const mcb_program& prog, const EvalLane& L, float (&acc)[kEvalRows], float* sp) {
 #pragma unroll
     for (int e = 0; e < kEvalRows; e++) acc[e] = 0.f;
@@ -307,7 +334,8 @@ __device__ __forceinline__ void eval_run(const mcb_program& prog, const EvalLane
                 for (int e = 0; e < kEvalRows; e++) sp[e * kEvalThreads] = acc[e];
                 sp += kEvalLevel;
                 break;
-            default: /* MCB_F_NEG */
+            default: /* MCB_F_NEG, and with HAS_FN the functions; HAS_FN = false compiles to NEG alone */
+                if (HAS_FN && (insn & 0xffu) != MCB_HANDLER_NEG) { eval_fn(acc, insn & 0xffu); break; }
 #pragma unroll
                 for (int e = 0; e < kEvalRows; e++) acc[e] = -acc[e];
                 break;
@@ -321,8 +349,9 @@ __device__ __forceinline__ void eval_run(const mcb_program& prog, const EvalLane
 
 /* K1.  STORE_F = false is the sparse-field mode (mcb_set_field_mode): only the sign bit-plane leaves the kernel and
  * eval_blocks_kernel later writes the field where the surface needs it. */
-template <bool HAS_POW, bool STORE_F> /* programs without `^` (after hoisting) get a kernel without the powf paths: fewer registers */
-__global__ void __launch_bounds__(kEvalThreads, HAS_POW ? 8 : 10)
+template <bool HAS_POW, bool STORE_F, bool HAS_FN = false> /* programs without `^` (after hoisting) get a kernel without the powf paths:
+                                                            fewer registers; HAS_FN: with the function grammar's handlers */
+__global__ void __launch_bounds__(kEvalThreads, HAS_POW || HAS_FN ? 8 : 10)
 eval_field_kernel(const __grid_constant__ mcb_program prog, const Grid g, const float* __restrict__ tables,
                   float* __restrict__ F, uint32_t* __restrict__ S, int row_groups) {
     MCB_DYNAMIC_SMEM(float, stack_smem); /* [level][16][kEvalThreads] */
@@ -337,7 +366,7 @@ eval_field_kernel(const __grid_constant__ mcb_program prog, const Grid g, const 
     L.y0 = yq * kEvalTileY;
     L.zi = pz + g.kb;
     float acc[kEvalRows];
-    eval_run<HAS_POW, 32>(prog, L, acc, stack_smem + threadIdx.x);
+    eval_run<HAS_POW, 32, HAS_FN>(prog, L, acc, stack_smem + threadIdx.x);
 
     /* ---- outputs ----
      * A lane's columns are x0 + 32 q: every field store is one fully coalesced 128-byte line per warp, and the warp
@@ -375,8 +404,8 @@ struct FieldBlocks {
     uint8_t* flags;               /* [nbz][nby][nbx] */
     uint32_t* list;               /* flagged blocks, any order */
 };
-template <bool HAS_POW>
-__global__ void __launch_bounds__(kEvalThreads, HAS_POW ? 8 : 10)
+template <bool HAS_POW, bool HAS_FN = false>
+__global__ void __launch_bounds__(kEvalThreads, HAS_POW || HAS_FN ? 8 : 10)
 eval_blocks_kernel(const __grid_constant__ mcb_program prog, const Grid g, const float* __restrict__ tables,
                    float* __restrict__ F, uint32_t* __restrict__ S, const uint32_t* __restrict__ list /* pack_block */,
                    const unsigned* __restrict__ count) {
@@ -393,7 +422,7 @@ eval_blocks_kernel(const __grid_constant__ mcb_program prog, const Grid g, const
         L.y0 = by * kFieldBlockY;        /* class 2: the y tables */
         L.zi = bx * kFieldBlockX + lane; /* class 3: the x tables, this lane's column */
         float acc[kEvalRows];
-        eval_run<HAS_POW, 1>(prog, L, acc, stack_smem + threadIdx.x);
+        eval_run<HAS_POW, 1, HAS_FN>(prog, L, acc, stack_smem + threadIdx.x);
         uint32_t mine = 0; /* lane 4 r + q keeps the sign word of row r, plane q: bit = this column's value > iso */
 #pragma unroll
         for (int e = 0; e < kEvalRows; e++) {

@@ -29,17 +29,23 @@
 
 namespace mcb {
 
-enum TokType { TOK_OP, TOK_NUM, TOK_VAR, TOK_BRAC_O, TOK_BRAC_C, TOK_NEG };
+enum TokType { TOK_OP, TOK_NUM, TOK_VAR, TOK_BRAC_O, TOK_BRAC_C, TOK_NEG, TOK_FUNC };
 struct Token {
     TokType type;
-    std::string text; /* "NEG" for unary minus, like the reference */
+    std::string text; /* "NEG" for unary minus, like the reference; "sin(" etc. for a function and its bracket */
 };
 
+/* Grammars (mcb.h): MCB_GRAMMAR_REFERENCE = the reference's language; MCB_GRAMMAR_FUNCTIONS adds sin( cos( sqrt( abs(.
+ * A function name and its '(' are one TOK_FUNC token that takes part in implicit multiplication, the unary-minus rule
+ * and bracket balance exactly as '(' does; the walk applies the function at the matching ')'. */
+enum { GRAMMAR_REFERENCE = 0, GRAMMAR_FUNCTIONS = 1 };
+
 /* Evaluator::tokenize (evaluator.cpp:139-237). false = parse error. `cleaned` = equation with spaces removed. */
-bool tokenize(const std::string& eq, std::vector<Token>& out, std::string* cleaned);
+bool tokenize(const std::string& eq, std::vector<Token>& out, std::string* cleaned, int grammar = GRAMMAR_REFERENCE);
 
 struct Node {
-    char kind;  /* 'x','y','z' variable; 'c' literal; '+','-','*','/','^' binary (a op b); 'N' negate a */
+    char kind;  /* 'x','y','z' variable; 'c' literal; '+','-','*','/','^' binary (a op b); 'N' negate a;
+                 * 'S' sin a, 'C' cos a, 'Q' sqrt a, 'A' abs a (function grammar) */
     int a, b;   /* children (node ids), -1 when unused */
     float value; /* literal value (strtof, like stof at evaluator.cpp:82) */
     uint8_t mask; /* variables the subtree depends on: 1=x 2=y 4=z */
@@ -82,7 +88,7 @@ struct Compiled {
 };
 
 /* tokenize + build + lower. Returns MCB_OK / MCB_E_PARSE / MCB_E_CAPACITY (program or pool too large). */
-int compile(const std::string& eq, Compiled& out, std::string* err);
+int compile(const std::string& eq, Compiled& out, std::string* err, int grammar = GRAMMAR_REFERENCE);
 
 std::string disassemble(const std::vector<uint32_t>& code);
 

@@ -6,6 +6,7 @@
 //                [--scale sx sy sz] [--iso c] [--constraint i "lhs" "op" rhs]... [--no-normals] [--soup]
 //                [--ply out.ply] [--dump out.bin] [--repeat n] [--levels d]   (--levels: repeating-surface mode, distance d)
 //                [--devices n]   (z-slabs over GPUs 0..n-1 of this box: Marching::set_devices)
+//                [--functions]   (equations and constraints may use sin( cos( sqrt( abs(: Evaluator::set_function_grammar)
 //
 // Defaults are the reference GUI's (drawer.cpp:39-44): equation "x+y", grid 0.2, scale 1.1, iso 0.
 #include <chrono>
@@ -18,7 +19,8 @@
 
 static int usage() {
     std::fprintf(stderr, "usage: mcb_headless [--eq S | --eq-file F] [--step h | --res n] [--scale sx sy sz] [--iso c]\n"
-                         "                    [--constraint i lhs op rhs] [--no-normals] [--soup] [--ply F] [--dump F] [--repeat n] [--levels d] [--devices n]\n");
+                         "                    [--constraint i lhs op rhs] [--no-normals] [--soup] [--ply F] [--dump F] [--repeat n] [--levels d] [--devices n]\n"
+                         "                    [--functions]\n");
     return 2;
 }
 
@@ -29,6 +31,8 @@ int main(int argc, char** argv) {
     float step = 0.2f, sx = 1.1f, sy = 1.1f, sz = 1.1f, iso = 0.f;
     int res = 0, repeat = 1;
     std::string ply, dump;
+    for (int a = 1; a < argc; a++) /* before any equation is parsed, wherever it stands */
+        if (std::strcmp(argv[a], "--functions") == 0) evaluator.set_function_grammar(true);
     for (int a = 1; a < argc; a++) {
         const std::string o = argv[a];
         auto need = [&](int n) { return a + n < argc; };
@@ -49,7 +53,8 @@ int main(int argc, char** argv) {
                 return 1;
             }
             a += 4;
-        } else if (o == "--no-normals") march_maker.set_normals(false);
+        } else if (o == "--functions") continue;
+        else if (o == "--no-normals") march_maker.set_normals(false);
         else if (o == "--soup") march_maker.set_weld(false);
         else if (o == "--ply" && need(1)) ply = argv[++a];
         else if (o == "--dump" && need(1)) dump = argv[++a];
