@@ -168,16 +168,8 @@ struct mcb_ctx {
     bool poison_field = false;     /* $MCB_POISON_FIELD: NaN-fill d_F first, so a read outside the blocks shows (tests) */
     bool decide_blocks = true;     /* $MCB_NO_INTERVAL=1: treat every block as undecided, i.e. evaluate them all (tests) */
     bool stage_timing = true;      /* mcb_set_stage_timing: CUDA events around the stages (mcb_counts::ms_*) */
-    bool weld_exact_only = false;  /* $MCB_WELD_EXACT=1: weld_count_kernel (a thread per crossing edge) on the plain grid too (tests) */
-    int emit_blocks_per_sm = 10;    /* grid of the default emitter: one resident wave, 10 blocks per SM ($MCB_EMIT_BLOCKS_PER_SM: A/B runs) */
     uint32_t index_base = 0;        /* mcb_set_index_base: added to every index mcb_get_indexed_mesh delivers */
     uint32_t index_base_applied = 0; /* what d_tlist currently carries (0 after every polygonisation) */
-    float4* d_edge = nullptr;      /* [cap_edge] edge slots of edge_slots_kernel: 2 float4 per (record, axis) */
-    size_t cap_edge = 0;
-    int emit_variant = 3;          /* $MCB_EMIT: 1 = first-generation emit kernel, 2 / 3 = second generation (128 / 64 cubes per chunk; 3 measured
-                                      fastest on every workload and is the default), 4 = 3 with every crossing grid edge computed once by its
-                                      owner cube (edge_slots_kernel + emit2<OWNED>): same bytes, measured slower (profiles/r02_ab_variants_owned_edges.jsonl),
-                                      9 = second generation with 24 edge slots (tests: forces chunks to be emitted in several runs) */
     uint8_t* d_fflags = nullptr;   /* [cap_fblocks] 2 = evaluated (undecided block), 1 = apron block to refill, 0 = untouched */
     uint8_t* d_bcls = nullptr;     /* [cap_fblocks] interval class of every 32 x 4 x 4 vertex block */
     uint32_t* d_flist = nullptr;   /* [cap_fblocks] apron blocks */
@@ -614,12 +606,6 @@ int mcb_create(int device, mcb_ctx** out) {
         ctx->jit_sync = js && js[0] == '1';
         const char* noiv = std::getenv("MCB_NO_INTERVAL");
         ctx->decide_blocks = !(noiv && noiv[0] == '1');
-        const char* we = std::getenv("MCB_WELD_EXACT");
-        ctx->weld_exact_only = we && we[0] == '1';
-        const char* eb = std::getenv("MCB_EMIT_BLOCKS_PER_SM");
-        if (eb && std::atoi(eb) >= 1 && std::atoi(eb) <= 64) ctx->emit_blocks_per_sm = std::atoi(eb);
-        const char* ev = std::getenv("MCB_EMIT");
-        if (ev && ((ev[0] >= '1' && ev[0] <= '4') || ev[0] == '9') && ev[1] == 0) ctx->emit_variant = ev[0] - '0';
     }
     int rc = install_equation(ctx, 0, "x+y"); /* Evaluator::Evaluator(), evaluator.cpp:6-8 */
     if (rc != MCB_OK) return bail(rc);
@@ -641,7 +627,6 @@ void mcb_destroy(mcb_ctx* ctx) {
     cudaFree(ctx->d_cls); cudaFree(ctx->d_ctr);
     if (ctx->h_ctr) cudaFreeHost(ctx->h_ctr);
     cudaFree(ctx->d_rec); cudaFree(ctx->d_trioff); cudaFree(ctx->d_pos); cudaFree(ctx->d_nrm);
-    cudaFree(ctx->d_edge);
     cudaFree(ctx->d_vlist); cudaFree(ctx->d_vnrm); cudaFree(ctx->d_tlist); cudaFree(ctx->d_item); cudaFree(ctx->d_vinfo);
     cudaFree(ctx->d_chunk_new); cudaFree(ctx->d_fn); cudaFree(ctx->d_nh_count); cudaFree(ctx->d_nh_start); cudaFree(ctx->d_nh_cursor);
     cudaFree(ctx->d_nh_sums); cudaFree(ctx->d_nh_adj);
@@ -836,11 +821,6 @@ struct Run {
     int stage_soup();
     int stage_weld();
     int stage_normal_h();
-    /* K3a + emit2<OWNED>: every crossing grid edge computed once, by the cube it starts at.  The plain grid only: per-cube
-     * levels, constraints and seed mode change which cubes exist around an edge */
-    bool owned_edges() const {
-        return want_soup && ctx->normals == 1 && ctx->emit_variant == 4 && !ctx->seed_on && !any_constraint && !g.repeat;
-    }
 };
 
 int Run::prepare_buffers() {
@@ -1224,7 +1204,7 @@ int Run::stage_classify() {
         launches++;
         cw = ctx->d_cw;
     }
-    const bool need_items = want_indexed || ctx->seed_on || owned_edges(); /* per-word record index for the weld / the seed walk / the edge owners */
+    const bool need_items = want_indexed || ctx->seed_on; /* per-word record index for the weld / the seed walk */
     if (need_items && (rc = ensure_weld_scratch(ctx, g)) != MCB_OK) return rc;
     unsigned long long* items = need_items ? ctx->d_item : nullptr;
     const unsigned amb_ctas = (unsigned)ctx->sm_count * 2;
@@ -1316,49 +1296,13 @@ int Run::stage_seed() {
 int Run::stage_soup() {
     const float* rinv = ctx->d_cs + ctx->rinv_ofs;
     const bool idx32 = (unsigned long long)g.NZ * g.NV * g.P < (1ull << 32) - 2ull * g.NV * g.P; /* offsets +- one plane stay below 2^32 */
-#define MCB_EMIT2_(NRM, CUBES, THREADS, CAP, MINB, MULT, I32)                                                                         \
-    MCB_LAUNCH((emit2_kernel<NRM, CUBES, THREADS, CAP, MINB, I32>), eblocks * MULT, THREADS, 0, s, g, ctx->d_cs, rinv, ctx->d_F, ctx->d_cls, ctx->d_rec, \
-               ctx->d_trioff, ctx->d_ctr, ctx->cap_active, ctx->cap_tris, ctx->d_pos, NRM ? ctx->d_nrm : nullptr)
-#define MCB_EMIT2(NRM, CUBES, THREADS, CAP, MINB, MULT)                                                                               \
-    do { if (idx32) MCB_EMIT2_(NRM, CUBES, THREADS, CAP, MINB, MULT, true); else MCB_EMIT2_(NRM, CUBES, THREADS, CAP, MINB, MULT, false); } while (0)
-    const bool nrm = ctx->normals == 1;
-    if (owned_edges()) {
-        int rc;
-        if ((rc = ensure(ctx, &ctx->d_edge, &ctx->cap_edge, (size_t)ctx->cap_active * 6)) != MCB_OK) return rc;
-        if (idx32) {
-            MCB_LAUNCH((edge_slots_kernel<true>), eblocks * 8, kEdgeCubes, 0, s, g, rinv, ctx->d_F, ctx->d_rec, ctx->d_ctr, ctx->cap_active, ctx->d_edge);
-            MCB_LAUNCH((emit2_kernel<true, 64, 128, 512, 10, true, true>), eblocks * 4, 128, 0, s, g, ctx->d_cs, rinv, ctx->d_F, ctx->d_cls, ctx->d_rec, ctx->d_trioff,
-                       ctx->d_ctr, ctx->cap_active, ctx->cap_tris, ctx->d_pos, ctx->d_nrm, ctx->d_edge, ctx->d_item, cg.WC);
-        } else {
-            MCB_LAUNCH((edge_slots_kernel<false>), eblocks * 8, kEdgeCubes, 0, s, g, rinv, ctx->d_F, ctx->d_rec, ctx->d_ctr, ctx->cap_active, ctx->d_edge);
-            MCB_LAUNCH((emit2_kernel<true, 64, 128, 512, 10, false, true>), eblocks * 4, 128, 0, s, g, ctx->d_cs, rinv, ctx->d_F, ctx->d_cls, ctx->d_rec, ctx->d_trioff,
-                       ctx->d_ctr, ctx->cap_active, ctx->cap_tris, ctx->d_pos, ctx->d_nrm, ctx->d_edge, ctx->d_item, cg.WC);
-        }
-        launches += 2;
-        return MCB_OK;
-    }
-    switch (ctx->emit_variant) {
-        case 1:
-            if (nrm) MCB_LAUNCH((emit_kernel<true>), eblocks, kEmitThreads, 0, s, g, ctx->d_cs, ctx->d_F, ctx->d_rec, ctx->d_trioff, ctx->d_ctr, ctx->cap_active,
-                                ctx->cap_tris, ctx->d_pos, ctx->d_nrm);
-            else MCB_LAUNCH((emit_kernel<false>), eblocks, kEmitThreads, 0, s, g, ctx->d_cs, ctx->d_F, ctx->d_rec, ctx->d_trioff, ctx->d_ctr, ctx->cap_active,
-                            ctx->cap_tris, ctx->d_pos, nullptr);
-            break;
-        case 2: if (nrm) MCB_EMIT2(true, 128, 256, 1024, 6, 2); else MCB_EMIT2(false, 128, 256, 1024, 6, 2); break;
-        case 9: if (nrm) MCB_EMIT2(true, 128, 256, 24, 2, 1); else MCB_EMIT2(false, 128, 256, 24, 2, 1); break;
-        default: {
-            const unsigned grid = (unsigned)ctx->sm_count * (unsigned)ctx->emit_blocks_per_sm;
-#define MCB_EMIT3(NRM, I32)                                                                                                           \
-    MCB_LAUNCH((emit2_kernel<NRM, 64, 128, 512, 10, I32>), grid, 128, 0, s, g, ctx->d_cs, rinv, ctx->d_F, ctx->d_cls, ctx->d_rec, ctx->d_trioff, \
+    const unsigned grid = (unsigned)ctx->sm_count * (unsigned)kEmitBlocksPerSM; /* one resident wave: emit2 hands out chunks itself */
+#define MCB_SOUP(NRM, I32)                                                                                                            \
+    MCB_LAUNCH((emit2_kernel<NRM, I32>), grid, kEmitThreads, 0, s, g, ctx->d_cs, rinv, ctx->d_F, ctx->d_cls, ctx->d_rec, ctx->d_trioff, \
                ctx->d_ctr, ctx->cap_active, ctx->cap_tris, ctx->d_pos, NRM ? ctx->d_nrm : nullptr)
-            if (nrm) { if (idx32) MCB_EMIT3(true, true); else MCB_EMIT3(true, false); }
-            else { if (idx32) MCB_EMIT3(false, true); else MCB_EMIT3(false, false); }
-#undef MCB_EMIT3
-            break;
-        }
-    }
-#undef MCB_EMIT2
-#undef MCB_EMIT2_
+    if (ctx->normals == 1) { if (idx32) MCB_SOUP(true, true); else MCB_SOUP(true, false); }
+    else { if (idx32) MCB_SOUP(false, true); else MCB_SOUP(false, false); }
+#undef MCB_SOUP
     launches++;
     return MCB_OK;
 }
@@ -1371,7 +1315,7 @@ int Run::stage_weld() {
     const WeldViewT<true> WR{W.g, W.cs, W.F, W.V, W.present, W.WC}; /* repeating-surface mode: same view, level checks compiled in */
     const WeldBuffers B{ctx->d_rec, ctx->d_trioff, ctx->d_item, ctx->d_vinfo, ctx->d_chunk_new, cg.WC};
     if (g.repeat) MCB_LAUNCH((weld_count_kernel), eblocks * 2, kWeldThreads, 0, s, WR, B, ctx->d_ctr, ctx->cap_active);
-    else if (W.V != nullptr || W.present != nullptr || ctx->weld_exact_only) MCB_LAUNCH((weld_count_kernel), eblocks * 2, kWeldThreads, 0, s, W, B, ctx->d_ctr, ctx->cap_active);
+    else if (W.V != nullptr || W.present != nullptr) MCB_LAUNCH((weld_count_kernel), eblocks * 2, kWeldThreads, 0, s, W, B, ctx->d_ctr, ctx->cap_active);
     else MCB_LAUNCH((weld_count_fast_kernel), eblocks * 4, kWeldCubes, 0, s, W, B, ctx->d_cls, ctx->d_ctr, ctx->cap_active);
     MCB_LAUNCH((weld_scan_kernel), 1, 1024, 0, s, ctx->d_chunk_new, ctx->d_ctr, ctx->cap_active);
     MCB_LAUNCH((weld_base_kernel), eblocks * 2, kWeldCubes, 0, s, B, ctx->d_ctr, ctx->cap_active);

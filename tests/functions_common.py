@@ -13,6 +13,13 @@ MIXED = "sqrt(abs(x*y)+z^2)-0.4+0.1sin(7x+5y)cos(3z-x)"
 
 FUNCTION_EQUATIONS = [GYROID, TORUS_SDF, NONHOIST, OCTAHEDRON, SCHWARZ_P, MIXED]
 
+# 8 pi = 25.132741: at step 1/8 the product of cosines is +-1 and changes sign at every grid vertex, so every cube is
+# active with 12 crossing edges and a 64-cube chunk of the soup emitter needs 768 edge slots, more than its 512: the
+# chunk is emitted in several runs.  The small polynomial keeps the gradient away from zero, so the normals mean something
+# (the cosines' central differences are 0 at every vertex).  Not +0.1(x+y^2+z^3): there the reference's vertex set keeps
+# 10 duplicate vertices, the documented deviation of the weld (DESIGN.md §5, K4).
+CHECKER = "cos(25.132741x)cos(25.132741y)cos(25.132741z)+0.1(x^3+0.6y+0.3z^2)"
+
 
 def random_function_equation(rng, depth):
     """A random string over the function grammar: the reference's forms (variables, numbers, + - * / ^, brackets,

@@ -128,34 +128,25 @@ def test_layer_histogram_and_balanced_cut(mcb_emu, ctx, golden):
 
 
 @pytest.mark.parametrize("name", ["sphere_17", "gyr78_17", "quirk_div", "nonuniform_scale"])
-def test_owned_edge_emitter_and_index_base_through_the_emulated_kernels(mcb_emu, golden, monkeypatch, name):
-    """The opt-in emitter ($MCB_EMIT=4: edge_slots_kernel + emit2<OWNED>, every crossing grid edge computed once by the cube
-    it starts at) against the default one: positions and normals byte for byte, whole grid and a slab whose boundary edges
-    have no owner; and mcb_set_index_base (the slab's tri_list shifted on the device)."""
+def test_index_base_shifts_the_tri_list_through_the_emulated_kernels(mcb_emu, golden, name):
+    """mcb_set_index_base: the tri_list of the whole grid and of a slab shifted on the device (add_index_base_kernel) and
+    shifted back, the vertices untouched."""
     case = load_meta(golden)[name]
-    res = []
-    for variant in ("4", None):
-        if variant:
-            monkeypatch.setenv("MCB_EMIT", variant)
-        else:
-            monkeypatch.delenv("MCB_EMIT", raising=False)
-        c = mcb_emu.Context(0)
-        c.set_mesh_mode(mcb_emu.MESH_SOUP | mcb_emu.MESH_INDEXED)
-        configure(c, case)
-        for i in range(3):
-            c.set_constraint(i, ">", 0.0, False)
-        c.set_normals(1)
-        out = []
-        for slab in (None, (case["M"] // 3, 2 * case["M"] // 3 + 1)):
-            if slab:
-                c.set_slab(*slab)
-            cnt = c.polygonise()
-            out.append((cnt.triangles,) + c.get_mesh(normals=True))
+    c = mcb_emu.Context(0)
+    c.set_mesh_mode(mcb_emu.MESH_SOUP | mcb_emu.MESH_INDEXED)
+    configure(c, case)
+    for i in range(3):
+        c.set_constraint(i, ">", 0.0, False)
+    c.set_normals(1)
+    for slab in (None, (case["M"] // 3, 2 * case["M"] // 3 + 1)):
+        if slab:
+            c.set_slab(*slab)
+        assert c.polygonise().triangles > 0
         v0, t0 = c.get_indexed_mesh()
         c.set_index_base(123456)
         v1, t1 = c.get_indexed_mesh()
         assert np.array_equal(t1.astype(np.int64), t0.astype(np.int64) + 123456) and same_bits(v0, v1)
-        res.append(out)
-        c.close()
-    for (ta, pa, na), (tb, pb, nb) in zip(*res):
-        assert ta == tb and ta > 0 and same_bits(pa, pb) and same_bits(na, nb)
+        c.set_index_base(0)
+        v2, t2 = c.get_indexed_mesh()
+        assert np.array_equal(t2, t0) and same_bits(v0, v2)
+    c.close()

@@ -9,8 +9,8 @@ import subprocess
 import numpy as np
 import pytest
 
-from .functions_common import (FUNCTION_EQUATIONS, GRAMMAR_FUNCTIONS, GYROID, TORUS_SDF, FnOracle, fn_parse_ok, host_fn_lib,
-                               random_function_equations, trig_exhaustive_exe)
+from .functions_common import (CHECKER, FUNCTION_EQUATIONS, GRAMMAR_FUNCTIONS, GYROID, TORUS_SDF, FnOracle, fn_parse_ok,
+                               host_fn_lib, random_function_equations, trig_exhaustive_exe)
 from .helpers import same_bits
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -268,32 +268,42 @@ def test_generated_kernel_source_executed_on_the_host_equals_the_oracle(mcb, hos
         assert same_bits(Fp[:, :, :NV], ref), (eq, "plane")
 
 
-@pytest.mark.parametrize("eq", [GYROID, TORUS_SDF])
+EMULATED_MESHES = {GYROID: (2.0 / 32, 1.1), TORUS_SDF: (2.0 / 32, 1.1), CHECKER: (0.125, 1.0)}  # equation: (step, scale)
+
+
+@pytest.mark.parametrize("eq", list(EMULATED_MESHES))
 @pytest.mark.parametrize("mode", ["dense", "blocks"])
 def test_emulated_kernels_reproduce_the_oracle_mesh(mcb_emu, eq, mode):
-    """The device code executed on the host (tests/emu) at 33^3, both field modes: per-cube codes, soup and welded
-    Poly_Data equal the oracle's reference pipeline run on the function equation."""
-    step = 2.0 / 32
+    """The device code executed on the host (tests/emu), both field modes: per-cube codes, soup and welded Poly_Data equal
+    the oracle's reference pipeline run on the function equation.  CHECKER makes the soup emitter split every full chunk
+    into several runs, with and without normals."""
+    step, scale = EMULATED_MESHES[eq]
     ctx = mcb_emu.Context(0)
     try:
         ctx.set_mesh_mode(mcb_emu.MESH_SOUP | mcb_emu.MESH_INDEXED)
         ctx.set_grammar(mcb_emu.GRAMMAR_FUNCTIONS)
         assert ctx.set_equation(eq) == 0
         M = ctx.set_grid_step(step)
-        ctx.set_scaling(1.1, 1.1, 1.1)
+        ctx.set_scaling(scale, scale, scale)
         ctx.set_field_mode(mcb_emu.FIELD_DENSE if mode == "dense" else mcb_emu.FIELD_AUTO)
         ctx.set_normals(0)
         cnt = ctx.polygonise()
         code, tidx = ctx.get_cases()
         pos, _ = ctx.get_mesh(normals=False)
         vl, tl = ctx.get_indexed_mesh(normals=False)[:2]
+        if eq == CHECKER:
+            ctx.set_normals(1)
+            ctx.polygonise()
+            assert same_bits(ctx.get_mesh(normals=True)[0], pos)
     finally:
         ctx.close()
-    o = FnOracle(eq, step=step, scale=(1.1, 1.1, 1.1))
+    o = FnOracle(eq, step=step, scale=(scale, scale, scale))
     assert o.M == M
     sw = o.sweep()
     v, t = o.recalculate()
     assert sw["T"] > 1000 and cnt.triangles == sw["T"]
+    if eq == CHECKER:  # every cube active, each with 4 triangles (codes 90 / 165)
+        assert cnt.active == M ** 3 and cnt.triangles == 4 * M ** 3
     assert np.array_equal(code.ravel(), sw["code"]) and np.array_equal(tidx.ravel(), sw["table_idx"])
     assert cnt.ambiguous == sw["ambiguous"] and cnt.redirected == sw["redirected"]
     assert same_bits(pos[:, :, :3], sw["soup"])

@@ -105,39 +105,6 @@ def test_slab_in_the_middle_equals_the_same_layers_of_the_full_grid(mcb):
     c.close()
 
 
-@pytest.mark.parametrize("eq,n,scale", [("x^2+y^2+z^2-0.49", 96, (1.0, 1.0, 1.0)), ("x^2+y^2+z^2-0.49", 40, (1.1, 0.9, 1.3)),
-                                        (None, 48, (1.0, 1.0, 1.0)), ("(x^2+y^2+z^2+0.25-0.0625)^2-(x^2+y^2)", 64, (1.0, 1.0, 1.0)),
-                                        ("x+y", 32, (1.0, 1.0, 1.0)), ("1/(x*y)-z", 24, (1.0, 1.0, 1.0))])
-def test_edges_computed_once_by_their_owner_equal_the_per_cube_computation(mcb, monkeypatch, eq, n, scale):
-    """K3a ($MCB_EMIT=4): a crossing grid edge computed once, in the cube it starts at (edge_slots_kernel), the up to four cubes
-    that share it fetching the result (emit2<OWNED>), against the default emitter, which computes it in every cube.
-    Positions and normals must be the same bytes — on the whole grid, and in a slab whose boundary edges have no owner."""
-    from oracle.refbind import GYR78
-    eq = eq or GYR78
-    res = []
-    for variant in ("4", None):
-        if variant:
-            monkeypatch.setenv("MCB_EMIT", variant)
-        else:
-            monkeypatch.delenv("MCB_EMIT", raising=False)
-        c = mcb.Context(0)
-        assert c.set_equation(eq) == 0
-        M = c.set_grid_step(2.0 / n)
-        c.set_scaling(*scale)
-        c.set_normals(1)
-        out = []
-        for (k0, k1) in ((0, M), (M // 3, 2 * M // 3), (M // 2, M // 2 + 1)):
-            c.set_slab(k0, k1)
-            cnt = c.polygonise()
-            out.append((cnt.triangles,) + c.get_mesh(normals=True))
-        res.append(out)
-        c.close()
-    for (ta, pa, na), (tb, pb, nb) in zip(*res):
-        assert ta == tb and ta > 0
-        assert same_bits(pa, pb)
-        assert same_bits(na, nb)
-
-
 def test_truncated_passes_are_harmless(mcb):
     """A grid that outgrows every buffer: the first pass of the call runs with too small record, soup and mesh buffers and is
     repeated by the host.  Its kernels must stay inside their buffers whatever the truncated state looks like (weld_emit once

@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 from . import mc_numpy
-from .functions_common import FUNCTION_EQUATIONS, GRAMMAR_FUNCTIONS, GYROID, TORUS_SDF, FnOracle, random_function_equations
+from .functions_common import CHECKER, FUNCTION_EQUATIONS, GRAMMAR_FUNCTIONS, GYROID, TORUS_SDF, FnOracle, random_function_equations
 from .helpers import rel_close, same_bits
 from .test_gpu_parity import tri_rows
 
@@ -19,8 +19,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 F = GRAMMAR_FUNCTIONS
 
 # (equation, step, scale, iso, constraints); the steps of gyroid and nonhoist are coarse enough for the face-centre test to
-# redirect cubes (REDIRECTS), the smooth distance fields have no ambiguous faces that flip at any step tried
+# redirect cubes (REDIRECTS), the smooth distance fields have no ambiguous faces that flip at any step tried; checker has
+# only ambiguous cubes and makes the soup emitter split its chunks into several runs
 CASES = {
+    "checker": (CHECKER, 0.125, (1.0, 1.0, 1.0), 0.0, []),
     "gyroid": (GYROID, 0.1, (1.1, 1.1, 1.1), 0.0, []),
     "torus_sdf": (TORUS_SDF, 0.05, (1.0, 1.0, 1.0), 0.0, []),
     "nonhoist": ("sin(6(x^2+y^2+z^2))", 0.15, (1.0, 1.0, 1.0), 0.1, []),
@@ -28,7 +30,7 @@ CASES = {
     "schwarz_cons": (FUNCTION_EQUATIONS[4], 0.09, (1.2, 1.0, 0.9), 0.3, [("abs(x-y)", "<=", 0.9)]),
     "mixed": (FUNCTION_EQUATIONS[5], 0.06, (1.0, 1.0, 1.0), 0.0, []),
 }
-REDIRECTS = {"gyroid", "nonhoist"}
+REDIRECTS = {"checker", "gyroid", "nonhoist"}
 
 
 def _configure(ctx, eq, step, scale, iso, cons):
