@@ -102,7 +102,7 @@ public:
     /* extension used by Marching: the current (cleaned) equation text */
     const std::string& equation() const { return equation_; }
 
-    /* Extension: on = later set_equation calls accept sin( cos( sqrt( abs( (MCB_GRAMMAR_FUNCTIONS, mcb.h); off (the
+    /* Extension: on = later set_equation calls accept sin( cos( sqrt( abs( and min(a,b) max(a,b) (MCB_GRAMMAR_FUNCTIONS, mcb.h); off (the
      * default) = exactly the reference's language.  The current equation is kept either way.  test() always checks the
      * reference grammar. */
     void set_function_grammar(bool on) {

@@ -103,7 +103,15 @@ const char* mcb_status_string(int status);
  *                                    Every equation of the reference grammar parses to the same tokens, operation order
  *                                    and bytecode.  sin / cos are glibc's sinf / cosf restated bit for bit on the device
  *                                    (csrc/mcb_trig.h), sqrt is correctly rounded, abs clears the sign bit; all else is
- *                                    unchanged fp32 without FMA contraction. */
+ *                                    unchanged fp32 without FMA contraction.
+ *                                    Also two functions of two arguments, min( max(, for unions (min), intersections
+ *                                    (max) and differences (max(a,-b)) of signed-distance shapes.  Exactly one ',' goes
+ *                                    directly inside their bracket and nowhere else (`(x,y)`, `sin(x,y)`, `min(x)`,
+ *                                    `min(x,y,z)` are parse errors).  Each argument is a bracketed operand closed at its
+ *                                    ',' or ')', so `max(x-y+z,0)` is max(x-(y+z),0); after the ',' a unary minus is
+ *                                    allowed as after '('.  `max(` is matched as a name, so its x is no variable
+ *                                    (`xmax(y,z)` is x*max(y,z), `maxx(y,z)` an error).  min / max are IEEE 754-2019
+ *                                    minimumNumber / maximumNumber: a NaN operand is ignored, -0 < +0. */
 #define MCB_GRAMMAR_REFERENCE 0
 #define MCB_GRAMMAR_FUNCTIONS 1
 

@@ -25,7 +25,7 @@ LIB_PATH = os.path.join(HERE, "libmcb200.so")
 MESH_SOUP, MESH_INDEXED = 1, 2
 FIELD_DENSE, FIELD_SPARSE, FIELD_AUTO = 0, 1, 2
 JIT_OFF, JIT_ON, JIT_AUTO = 0, 1, 2
-GRAMMAR_REFERENCE, GRAMMAR_FUNCTIONS = 0, 1  # the reference's equation language / the same plus sin( cos( sqrt( abs(
+GRAMMAR_REFERENCE, GRAMMAR_FUNCTIONS = 0, 1  # the reference's equation language / the same plus sin( cos( sqrt( abs( min( max(
 MCB_OK, MCB_E_PARSE, MCB_E_ARG, MCB_E_CUDA, MCB_E_NOMEM, MCB_E_STATE, MCB_E_CAPACITY, MCB_E_NODEVICE = 0, -1, -2, -3, -4, -5, -6, -7
 
 
@@ -263,7 +263,8 @@ class Context:
         return lib.mcb_set_equation(self.h, slot, eq.encode())
 
     def set_grammar(self, grammar):
-        """GRAMMAR_REFERENCE (default) or GRAMMAR_FUNCTIONS for the set_equation calls that follow, in every slot."""
+        """GRAMMAR_REFERENCE (default) or GRAMMAR_FUNCTIONS for the set_equation calls that follow, in every slot.
+        GRAMMAR_FUNCTIONS adds sin( cos( sqrt( abs( and the two-argument min(a,b) max(a,b) (include/mcb.h)."""
         self._ck(lib.mcb_set_grammar(self.h, grammar))
 
     def eval_points(self, xyz, slot=0, apply_scale=False):
@@ -450,7 +451,7 @@ class Evaluator:
             raise ValueError("parse error")  # Evaluator(string) throws on a parse error (evaluator.cpp:10-13)
 
     def set_function_grammar(self, on):
-        """Extension: accept sin( cos( sqrt( abs( in later set_equation calls (GRAMMAR_FUNCTIONS); off by default."""
+        """Extension: accept sin( cos( sqrt( abs( min( max( in later set_equation calls (GRAMMAR_FUNCTIONS); off by default."""
         self.function_grammar = bool(on)
         self._ctx.set_grammar(GRAMMAR_FUNCTIONS if on else GRAMMAR_REFERENCE)
 

@@ -51,9 +51,10 @@ def build(force=False, verbose=False):
         force = True  # a source changed since the library was built, whatever the mtimes say
     if not force and not stale():
         return LIB
-    # mcb_pow.h and mcb_trig.h also travel inside the library as text: the run-time compiled evaluator (mcb_jit.cpp)
-    # includes them through NVRTC
-    for name, inc, tag in (("mcb_pow.h", "mcb_pow_src.inc", "MCBPOWSRC"), ("mcb_trig.h", "mcb_trig_src.inc", "MCBTRIGSRC")):
+    # mcb_pow.h, mcb_trig.h and mcb_bytecode.h also travel inside the library as text: the run-time compiled evaluator
+    # (mcb_jit.cpp) includes them through NVRTC
+    for name, inc, tag in (("mcb_pow.h", "mcb_pow_src.inc", "MCBPOWSRC"), ("mcb_trig.h", "mcb_trig_src.inc", "MCBTRIGSRC"),
+                           ("mcb_bytecode.h", "mcb_bytecode_src.inc", "MCBBCSRC")):
         with open(os.path.join(CSRC, name)) as f, open(os.path.join(CSRC, inc), "w") as o:
             o.write('R"%s(' % tag + f.read() + ')%s"\n' % tag)
     cmd = [NVCC] + FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB] + [os.path.join(CSRC, s) for s in SOURCES] + ["-ldl"]

@@ -597,7 +597,9 @@ int mcb_create(int device, mcb_ctx** out) {
         const int stack_bytes = MCB_MAX_STACK * kEvalRows * kEvalThreads * (int)sizeof(float);
         const void* evals[] = {(const void*)eval_field_kernel<true, true>, (const void*)eval_field_kernel<false, true>,
                                (const void*)eval_blocks_kernel<true>,      (const void*)eval_blocks_kernel<false>,
-                               (const void*)eval_field_kernel<true, true, true>, (const void*)eval_blocks_kernel<true, true>};
+                               (const void*)eval_field_kernel<true, true, true>, (const void*)eval_blocks_kernel<true, true>,
+                               (const void*)eval_field_kernel<true, true, true, true>, (const void*)eval_field_kernel<false, true, false, true>,
+                               (const void*)eval_blocks_kernel<true, true, true>, (const void*)eval_blocks_kernel<false, false, true>};
         for (const void* k : evals)
             if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, stack_bytes) != cudaSuccess) return bail(MCB_E_CUDA);
         const char* poison = std::getenv("MCB_POISON_FIELD");
@@ -808,7 +810,7 @@ struct Run {
     uint32_t launches;
 
     int prepare_buffers();
-    int encode_program(mcb_program& launch, bool& has_pow, bool& has_fn, bool blocks);
+    int encode_program(mcb_program& launch, bool& has_pow, bool& has_fn, bool& has_minmax, bool blocks);
     int ensure_block_buffers(FieldBlocks* fb, BlockDims* bd);
     int launch_block_eval(const FieldBlocks& fb, const uint32_t* list, const unsigned* count);
     int stage_eval_blocks();
@@ -848,10 +850,11 @@ int Run::prepare_buffers() {
 
 /* Device form of the fused grid program: dense handler numbers, table operands as absolute float offsets into
  * d_tables, and  LOAD/PUSH a ; op b  pairs folded into one two-word instruction (eval_pair). */
-int Run::encode_program(mcb_program& launch, bool& has_pow, bool& has_fn, bool blocks) {
+int Run::encode_program(mcb_program& launch, bool& has_pow, bool& has_fn, bool& has_minmax, bool blocks) {
     launch = eq.grid;
     has_pow = false;
     has_fn = false;
+    has_minmax = false;
     {
         /* operand class of a source as the kernel's lane patch sees it; eval_blocks_kernel's patch is (y, z) per x
          * column, so there the x and z tables trade places */
@@ -868,29 +871,39 @@ int Run::encode_program(mcb_program& launch, bool& has_pow, bool& has_fn, bool b
         };
         int n = 0;
         for (int pc = 0; pc < eq.grid.n; pc++) {
-            const uint32_t wd = eq.grid.code[pc], fop = MCB_FINSN_OP(wd), src = MCB_FINSN_SRC(wd);
+            const uint32_t wd = eq.grid.code[pc];
+            uint32_t fop = MCB_FINSN_OP(wd), src = MCB_FINSN_SRC(wd);
+            MCB_FINSN_DECODE(fop, src);
+            const bool minmax = fop == MCB_F_MIN || fop == MCB_F_MAX;
             has_pow |= fop == MCB_F_POW || fop == MCB_F_RPOW;
+            has_minmax |= minmax;
             if (fop == MCB_F_NEG) { launch.code[n++] = MCB_HANDLER_NEG; continue; }
             if (MCB_F_IS_FN(fop)) { launch.code[n++] = MCB_HANDLER_FN(fop); has_fn = true; continue; }
             if (src < MCB_SRC_K || src > MCB_SRC_POP) return fail(ctx, MCB_E_STATE, "internal: raw coordinate operand in a grid program");
             uint32_t arg;
             if (!resolve(src, MCB_FINSN_ARG(wd), &arg)) return fail(ctx, MCB_E_CAPACITY, "axis tables too large for the operand field");
             if ((fop == MCB_F_LOAD || fop == MCB_F_PUSH) && pc + 1 < eq.grid.n) {
-                const uint32_t nx = eq.grid.code[pc + 1], nop = MCB_FINSN_OP(nx), nsrc = MCB_FINSN_SRC(nx);
-                if (nop >= MCB_F_ADD && nop <= MCB_F_RPOW && leaf_class(nsrc) >= 0) {
+                const uint32_t nx = eq.grid.code[pc + 1];
+                uint32_t nop = MCB_FINSN_OP(nx), nsrc = MCB_FINSN_SRC(nx);
+                MCB_FINSN_DECODE(nop, nsrc);
+                const bool nminmax = nop == MCB_F_MIN || nop == MCB_F_MAX;
+                if (((nop >= MCB_F_ADD && nop <= MCB_F_RPOW) || nminmax) && leaf_class(nsrc) >= 0) {
                     uint32_t arg_b;
                     if (!resolve(nsrc, MCB_FINSN_ARG(nx), &arg_b)) return fail(ctx, MCB_E_CAPACITY, "axis tables too large for the operand field");
                     has_pow |= nop == MCB_F_POW || nop == MCB_F_RPOW;
                     if (n + 2 + (fop == MCB_F_PUSH ? 1 : 0) > MCB_MAX_CODE) return fail(ctx, MCB_E_CAPACITY, "program too long");
                     if (fop == MCB_F_PUSH) launch.code[n++] = MCB_HANDLER_SPILL;
-                    launch.code[n++] = (uint32_t)MCB_HANDLER_PAIR(nop, leaf_class(src), leaf_class(nsrc)) | (arg << 8);
+                    has_minmax |= nminmax;
+                    launch.code[n++] = (uint32_t)(nminmax ? MCB_HANDLER_MINMAX_PAIR(nop, leaf_class(src), leaf_class(nsrc))
+                                                          : MCB_HANDLER_PAIR(nop, leaf_class(src), leaf_class(nsrc))) | (arg << 8);
                     launch.code[n++] = arg_b;
                     pc++;
                     continue;
                 }
             }
             if (n + 1 > MCB_MAX_CODE) return fail(ctx, MCB_E_CAPACITY, "program too long");
-            launch.code[n++] = (uint32_t)MCB_HANDLER(fop, role(src)) | (arg << 8); /* dense handler number | operand */
+            const uint32_t cls = src == MCB_SRC_POP ? 4u : (uint32_t)leaf_class(src);
+            launch.code[n++] = (uint32_t)(minmax ? MCB_HANDLER_MINMAX(fop, cls) : MCB_HANDLER(fop, role(src))) | (arg << 8); /* dense handler number | operand */
         }
         launch.n = n;
     }
@@ -1054,9 +1067,11 @@ int Run::stage_eval() {
     if (!ctx->jit_used) {
         const size_t smem = (size_t)std::max(1, eq.c.grid_fused_depth) * kEvalRows * kEvalThreads * sizeof(float);
         mcb_program launch;
-        bool has_pow, has_fn;
-        if ((rc = encode_program(launch, has_pow, has_fn, false)) != MCB_OK) return rc;
-        if (has_fn) MCB_LAUNCH((eval_field_kernel<true, true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        bool has_pow, has_fn, has_minmax;
+        if ((rc = encode_program(launch, has_pow, has_fn, has_minmax, false)) != MCB_OK) return rc;
+        if (has_minmax && (has_pow || has_fn)) MCB_LAUNCH((eval_field_kernel<true, true, true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        else if (has_minmax) MCB_LAUNCH((eval_field_kernel<false, true, false, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        else if (has_fn) MCB_LAUNCH((eval_field_kernel<true, true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
         else if (has_pow) MCB_LAUNCH((eval_field_kernel<true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
         else MCB_LAUNCH((eval_field_kernel<false, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
         launches++;
@@ -1123,10 +1138,12 @@ int Run::launch_block_eval(const FieldBlocks& fb, const uint32_t* list, const un
 #endif
     } else {
         mcb_program launch;
-        bool has_pow, has_fn;
-        if ((rc = encode_program(launch, has_pow, has_fn, true)) != MCB_OK) return rc;
+        bool has_pow, has_fn, has_minmax;
+        if ((rc = encode_program(launch, has_pow, has_fn, has_minmax, true)) != MCB_OK) return rc;
         const size_t smem = (size_t)std::max(1, eq.c.grid_fused_depth) * kEvalRows * kEvalThreads * sizeof(float);
-        if (has_fn) MCB_LAUNCH((eval_blocks_kernel<true, true>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
+        if (has_minmax && (has_pow || has_fn)) MCB_LAUNCH((eval_blocks_kernel<true, true, true>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
+        else if (has_minmax) MCB_LAUNCH((eval_blocks_kernel<false, false, true>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
+        else if (has_fn) MCB_LAUNCH((eval_blocks_kernel<true, true>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
         else if (has_pow) MCB_LAUNCH((eval_blocks_kernel<true>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
         else MCB_LAUNCH((eval_blocks_kernel<false>), fill_ctas, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, list, count);
     }

@@ -8,6 +8,7 @@
  * order while each value keeps its role.  All arithmetic is fp32 without FMA contraction; `^` is mcb_powf.
  * The function grammar's unary operators: sin / cos are mcb_sinf / mcb_cosf (mcb_trig.h, glibc's sinf / cosf), sqrt is
  * the correctly rounded square root (sqrtf on the host, __fsqrt_rn on the device), abs clears the sign bit.
+ * Its two-argument functions min / max are mcb_minf / mcb_maxf below (IEEE 754-2019 minimumNumber / maximumNumber).
  *
  * Programs travel to the kernels inside the kernel-parameter block, i.e. in the constant bank: every lane of a
  * warp executes the same instruction word, fetched with a uniform constant load.
@@ -15,7 +16,9 @@
 #ifndef MCB_BYTECODE_H
 #define MCB_BYTECODE_H
 
+#if !defined(__CUDACC_RTC__) /* the run-time compiled kernels include this file for mcb_minf / mcb_maxf */
 #include <stdint.h>
+#endif
 
 #include "mcb_pow.h"
 #include "mcb_trig.h"
@@ -42,6 +45,8 @@ enum {
     MCB_OP_COS,
     MCB_OP_SQRT,
     MCB_OP_ABS,
+    MCB_OP_MIN,  /* function grammar: binary, commutative (no reversed forms) */
+    MCB_OP_MAX,
     MCB_OP_COUNT
 };
 #define MCB_OP_IS_UNARY(op) ((op) == MCB_OP_NEG || ((op) >= MCB_OP_SIN && (op) <= MCB_OP_ABS))
@@ -68,6 +73,23 @@ typedef struct {
 #define MCB_BC_FN static inline
 #endif
 
+/* min and max of the function grammar: IEEE 754-2019 minimumNumber / maximumNumber.  A NaN operand is ignored (two NaNs
+ * give the canonical quiet NaN), -0 < +0, otherwise the smaller / larger operand exactly.  Both are commutative bit for
+ * bit, so the lowering may order their operands freely.  Explicit compares and selects, not fminf / fmaxf: C leaves the
+ * sign of a zero result of fmin to the implementation.  One source for g++, nvcc and NVRTC (mcb_jit.cpp). */
+MCB_BC_FN float mcb_minf(float a, float b) {
+    const int na = a != a, nb = b != b;
+    if (na || nb) return na && nb ? mcb_u2f(0x7fc00000u) : na ? b : a;
+    if (a == b) return mcb_u2f(mcb_f2u(a) | mcb_f2u(b)); /* equal bits, or +0 and -0: -0 */
+    return a < b ? a : b;
+}
+MCB_BC_FN float mcb_maxf(float a, float b) {
+    const int na = a != a, nb = b != b;
+    if (na || nb) return na && nb ? mcb_u2f(0x7fc00000u) : na ? b : a;
+    if (a == b) return mcb_u2f(mcb_f2u(a) & mcb_f2u(b)); /* equal bits, or +0 and -0: +0 */
+    return a > b ? a : b;
+}
+
 MCB_BC_FN float mcb_binop(uint32_t op, float second, float top) {
     switch (op) {
         case MCB_OP_ADD: return second + top;
@@ -77,6 +99,8 @@ MCB_BC_FN float mcb_binop(uint32_t op, float second, float top) {
         case MCB_OP_DIV: return second / top;
         case MCB_OP_RDIV: return top / second;
         case MCB_OP_POW: return mcb_powf(second, top);
+        case MCB_OP_MIN: return mcb_minf(second, top);
+        case MCB_OP_MAX: return mcb_maxf(second, top);
         default: return mcb_powf(top, second); /* MCB_OP_RPOW */
     }
 }
@@ -145,6 +169,8 @@ MCB_BC_FN float mcb_interp_scalar(const uint32_t* code, int n, const float* k, f
  *      fop ADD, MUL  acc = acc (op) v                           fop NEG     acc = -acc  (src unused)
  *      fop SUB/DIV/POW  acc = acc (op) v                        fop RSUB/RDIV/RPOW  acc = v (op) acc
  *      fop SIN, COS, SQRT, ABS  acc = f(acc)  (src unused; the function grammar, like NEG)
+ *      fop MINMAX    acc = min(acc, v), or max(acc, v) when bit 3 of the src field is set (the function grammar; src
+ *                    takes only 0..7, so that bit is free, and the 4-bit op field has no room for two more ops)
  * Every fp32 operation and the role of each operand are those of the postfix program; only pushes and pops of
  * the operand stack disappear.  `x^2+y^2+z^2-0.49` (grid form TX0 TY0 TZ0 K0 - + +) becomes
  *      LOAD TZ0; SUB K0; ADD TY0; ADD TX0 — 4 words and no memory-stack traffic at all.
@@ -152,13 +178,23 @@ MCB_BC_FN float mcb_interp_scalar(const uint32_t* code, int n, const float* k, f
 enum { MCB_SRC_X = 0, MCB_SRC_Y, MCB_SRC_Z, MCB_SRC_K, MCB_SRC_TX, MCB_SRC_TY, MCB_SRC_TZ, MCB_SRC_POP };
 enum {
     MCB_F_LOAD = 0, MCB_F_PUSH, MCB_F_ADD, MCB_F_SUB, MCB_F_RSUB, MCB_F_MUL, MCB_F_DIV, MCB_F_RDIV, MCB_F_POW,
-    MCB_F_RPOW, MCB_F_NEG, MCB_F_SIN, MCB_F_COS, MCB_F_SQRT, MCB_F_ABS, MCB_F_COUNT
+    MCB_F_RPOW, MCB_F_NEG, MCB_F_SIN, MCB_F_COS, MCB_F_SQRT, MCB_F_ABS, MCB_F_MINMAX,
+    MCB_F_MIN, MCB_F_MAX /* never in a word: what the readers decode an MCB_F_MINMAX word into (MCB_FINSN_DECODE) */
 };
 #define MCB_F_IS_FN(fop) ((fop) >= MCB_F_SIN && (fop) <= MCB_F_ABS)
+#define MCB_SRC_MAX_BIT 8u /* src bit of an MCB_F_MINMAX word that selects max */
 #define MCB_FINSN(fop, src, arg) ((uint32_t)(fop) | ((uint32_t)(src) << 4) | ((uint32_t)(arg) << 8))
 #define MCB_FINSN_OP(w) ((w) & 0xFu)
 #define MCB_FINSN_SRC(w) (((w) >> 4) & 0xFu)
 #define MCB_FINSN_ARG(w) ((w) >> 8)
+/* fop, src of a word with MCB_F_MINMAX resolved into MCB_F_MIN / MCB_F_MAX and a plain src */
+#define MCB_FINSN_DECODE(fop, src)                                        \
+    do {                                                                  \
+        if ((fop) == MCB_F_MINMAX) {                                      \
+            (fop) = ((src) & MCB_SRC_MAX_BIT) ? MCB_F_MAX : MCB_F_MIN;    \
+            (src) &= ~MCB_SRC_MAX_BIT;                                    \
+        }                                                                 \
+    } while (0)
 
 MCB_BC_FN float mcb_fop(uint32_t fop, float acc, float v) {
     switch (fop) {
@@ -170,6 +206,8 @@ MCB_BC_FN float mcb_fop(uint32_t fop, float acc, float v) {
         case MCB_F_RDIV: return v / acc;
         case MCB_F_POW: return mcb_powf(acc, v);
         case MCB_F_RPOW: return mcb_powf(v, acc);
+        case MCB_F_MIN: return mcb_minf(acc, v);
+        case MCB_F_MAX: return mcb_maxf(acc, v);
         default: return v; /* LOAD, PUSH */
     }
 }
@@ -182,6 +220,7 @@ MCB_BC_FN float mcb_interp_fused_scalar(const uint32_t* code, int n, const float
     float acc = 0.f;
     for (int pc = 0; pc < n; pc++) {
         uint32_t w = code[pc], fop = MCB_FINSN_OP(w), src = MCB_FINSN_SRC(w), arg = MCB_FINSN_ARG(w);
+        MCB_FINSN_DECODE(fop, src);
         if (fop == MCB_F_NEG) { acc = -acc; continue; }
         if (MCB_F_IS_FN(fop)) { acc = mcb_fn(fop - MCB_F_SIN, acc); continue; }
         if (fop == MCB_F_PUSH) st[sp++] = acc;

@@ -26,7 +26,12 @@
  *   - sin, cos: [-1, 1] for any argument interval.  mcb_sinf / mcb_cosf are not the real functions, so no bound may be
  *     taken from analysis; this one rests on the exhaustive run of oracle/trig_exhaustive.c (every finite result of
  *     either function, over all 2^32 inputs, lies in [-1, 1]).  Hoisted sin / cos need no rule at all: their values
- *     are axis-table entries, whose exact minimum and maximum over the box are the leaves.
+ *     are axis-table entries, whose exact minimum and maximum over the box are the leaves;
+ *   - min, max (mcb_minf / mcb_maxf): exact and monotone in each argument, [min(a.lo, b.lo), min(a.hi, b.hi)] and the
+ *     same for max.  This rests on the invariant that a known interval never encloses a NaN value: sqrt of a possibly
+ *     negative interval, division across 0 and non-finite end points already make the box unknown, so the NaN-ignoring
+ *     rule of minimumNumber never applies to a value the interval stands for.  An unknown argument makes the result
+ *     unknown (the whole program is).  So a box left undecided for min(A, B) is undecided for A or for B.
  */
 #ifndef MCB_INTERVAL_H
 #define MCB_INTERVAL_H
@@ -110,6 +115,8 @@ MCB_BC_FN mcb_ival mcb_iv_op(uint32_t fop, mcb_ival acc, mcb_ival v, int* bad) {
         }
         case MCB_F_POW: r = mcb_iv_pow(acc, v, bad); break;
         case MCB_F_RPOW: r = mcb_iv_pow(v, acc, bad); break;
+        case MCB_F_MIN: r.lo = mcb_minf(acc.lo, v.lo); r.hi = mcb_minf(acc.hi, v.hi); break;
+        case MCB_F_MAX: r.lo = mcb_maxf(acc.lo, v.lo); r.hi = mcb_maxf(acc.hi, v.hi); break;
         default: r = v; break; /* LOAD, PUSH */
     }
     if (!mcb_iv_finite(r.lo) || !mcb_iv_finite(r.hi)) *bad = 1;
@@ -149,7 +156,9 @@ MCB_BC_FN int mcb_interval_class(const uint32_t* code, int n, const float* k, co
     mcb_ival acc;
     acc.lo = 0.f; acc.hi = 0.f;
     for (int pc = 0; pc < n && !bad; pc++) {
-        const uint32_t w = code[pc], fop = MCB_FINSN_OP(w), src = MCB_FINSN_SRC(w), arg = MCB_FINSN_ARG(w);
+        const uint32_t w = code[pc], arg = MCB_FINSN_ARG(w);
+        uint32_t fop = MCB_FINSN_OP(w), src = MCB_FINSN_SRC(w);
+        MCB_FINSN_DECODE(fop, src);
         if (fop == MCB_F_NEG) { const float t = acc.lo; acc.lo = -acc.hi; acc.hi = -t; continue; }
         if (MCB_F_IS_FN(fop)) { acc = mcb_iv_fn(fop, acc, &bad); continue; }
         if (fop == MCB_F_PUSH) { if (sp >= MCB_MAX_STACK) { bad = 1; break; } st[sp++] = acc; }

@@ -15,6 +15,9 @@ const char* const kPowHeader =
 const char* const kTrigHeader =
 #include "mcb_trig_src.inc" /* mcb_trig.h, likewise */
     ;
+const char* const kBytecodeHeader =
+#include "mcb_bytecode_src.inc" /* mcb_bytecode.h, likewise: mcb_minf / mcb_maxf */
+    ;
 
 /* Everything around the generated body.  It restates the tile of eval_field_kernel (mcb_kernels.cuh): a warp owns 128
  * columns x 4 rows of one plane, a lane the columns x0 + 32 q; evict-first field stores, sign words by ballot.  The Grid
@@ -45,6 +48,11 @@ __device__ __noinline__ float op_cos(float a) { return mcb_cosf(a); }
 )SRC";
 const char* const kHeadSqrtAbs = R"SRC(__device__ __forceinline__ float op_sqrt(float a) { return __fsqrt_rn(a); }
 __device__ __forceinline__ float op_abs(float a) { return __uint_as_float(__float_as_uint(a) & 0x7fffffffu); }
+)SRC";
+/* min / max: the interpreters' own mcb_minf / mcb_maxf (minimumNumber / maximumNumber), also only when used */
+const char* const kHeadMinMax = R"SRC(#include "mcb_bytecode.h"
+__device__ __forceinline__ float op_min(float a, float b) { return mcb_minf(a, b); }
+__device__ __forceinline__ float op_max(float a, float b) { return mcb_maxf(a, b); }
 )SRC";
 const char* const kHeadPlane = R"SRC(
 extern "C" __global__ void __launch_bounds__(128, MCB_MIN_BLOCKS)
@@ -159,7 +167,7 @@ Nvrtc& nvrtc() {
 } /* namespace */
 
 static std::string generate_one(const uint32_t* code, int n, int kind /* 0 plane tiles (dense field), 1 listed 32 x 4 x 4 blocks */, bool* has_pow,
-                                int* fns /* |= 1: sin or cos, 2: sqrt or abs */, std::string* err) {
+                                int* fns /* |= 1: sin or cos, 2: sqrt or abs, 4: min or max */, std::string* err) {
     const bool blocks = kind == 1;
     const char* const N = "16";   /* values per lane */
     const char* const I = "e";    /* their index variable */
@@ -204,7 +212,9 @@ static std::string generate_one(const uint32_t* code, int n, int kind /* 0 plane
     int next = 0;
     auto fresh = [&] { return "v" + std::to_string(next++); };
     for (int pc = 0; pc < n; pc++) {
-        const uint32_t w = code[pc], fop = MCB_FINSN_OP(w), src = MCB_FINSN_SRC(w), arg = MCB_FINSN_ARG(w);
+        const uint32_t w = code[pc], arg = MCB_FINSN_ARG(w);
+        uint32_t fop = MCB_FINSN_OP(w), src = MCB_FINSN_SRC(w);
+        MCB_FINSN_DECODE(fop, src);
         if (fop == MCB_F_NEG) {
             if (acc.empty()) { *err = "NEG without a value"; return std::string(); }
             const std::string t = fresh();
@@ -247,6 +257,8 @@ static std::string generate_one(const uint32_t* code, int n, int kind /* 0 plane
                 case MCB_F_RDIV: expr = "op_div(" + v + ", " + a + ")"; break;
                 case MCB_F_POW: expr = "op_pow(" + a + ", " + v + ")"; pow = true; break;
                 case MCB_F_RPOW: expr = "op_pow(" + v + ", " + a + ")"; pow = true; break;
+                case MCB_F_MIN: expr = "op_min(" + a + ", " + v + ")"; *fns |= 4; break;
+                case MCB_F_MAX: expr = "op_max(" + a + ", " + v + ")"; *fns |= 4; break;
                 default: *err = "unknown operation"; return std::string();
             }
         }
@@ -280,6 +292,7 @@ std::string generate(const uint32_t* code, int n, bool* has_pow, std::string* er
     std::string out = kHead;
     if (fns & 1) out += kHeadTrig;
     if (fns & 2) out += kHeadSqrtAbs;
+    if (fns & 4) out += kHeadMinMax;
     if ((fns & 1) && has_pow) *has_pow = true; /* out-of-line fp64 calls: the register budget of the powf kernels */
     return out + parts;
 }
@@ -288,9 +301,9 @@ std::string compile(const std::string& source, bool pow, int grid_size, std::vec
     Nvrtc& N = nvrtc();
     if (!N.error.empty()) return N.error;
     void* prog = nullptr;
-    const char* hdr_src[] = {kPowHeader, kTrigHeader};
-    const char* hdr_name[] = {"mcb_pow.h", "mcb_trig.h"};
-    int rc = N.CreateProgram(&prog, source.c_str(), "mcb_eval_jit.cu", 2, hdr_src, hdr_name);
+    const char* hdr_src[] = {kPowHeader, kTrigHeader, kBytecodeHeader};
+    const char* hdr_name[] = {"mcb_pow.h", "mcb_trig.h", "mcb_bytecode.h"};
+    int rc = N.CreateProgram(&prog, source.c_str(), "mcb_eval_jit.cu", 3, hdr_src, hdr_name);
     if (rc != 0) return std::string("nvrtcCreateProgram: ") + N.GetErrorString(rc);
     char grid_bytes[64], max_k[64];
     std::snprintf(grid_bytes, sizeof grid_bytes, "-DMCB_GRID_BYTES=%d", grid_size);

@@ -175,6 +175,8 @@ __device__ __forceinline__ float fused_op(float acc, float v) {
             if (__float_as_uint(acc) == 0x40000000u && mcb_pow2_try(v, &r)) return r;
             return powf_call(v, acc);
         }
+        case MCB_F_MIN: return mcb_minf(acc, v);
+        case MCB_F_MAX: return mcb_maxf(acc, v);
         default: return v; /* MCB_F_LOAD, MCB_F_PUSH */
     }
 }
@@ -253,6 +255,10 @@ __device__ __forceinline__ void eval_pair(float (&acc)[kEvalRows], uint32_t arg_
 #define MCB_HANDLER_SPILL 55 /* push the accumulator on the memory stack; the new value comes from the next (pair) word */
 #define MCB_HANDLER_FN(FOP) (56 + (FOP) - MCB_F_SIN) /* sin, cos, sqrt, abs of the accumulator: 56..59 (function grammar) */
 #define MCB_HANDLER_PAIR(FOP, CA, CB) (64 + ((FOP) - MCB_F_ADD) * 16 + (CA) * 4 + (CB))
+/* min and max (function grammar): pairs 192..223, steps 224..233 (operand class as MCB_HANDLER's) */
+#define MCB_HANDLER_MINMAX_FIRST 192
+#define MCB_HANDLER_MINMAX_PAIR(FOP, CA, CB) (192 + ((FOP) - MCB_F_MIN) * 16 + (CA) * 4 + (CB))
+#define MCB_HANDLER_MINMAX(FOP, CLS) (224 + ((FOP) - MCB_F_MIN) * 5 + (CLS))
 
 /* `prog` is the fused grid program with its table operands already resolved by the host for this launch:
  * for src TX/TY/TZ the argument is the float offset of the table row inside `tables` ((axis*slots + slot) * PT),
@@ -295,10 +301,37 @@ __device__ __forceinline__ void eval_fn(float (&acc)[kEvalRows], uint32_t handle
     }
 }
 
+/* min / max steps and  LOAD a ; MIN b  pairs (handlers 192..233), dispatched apart from the main switch so that the
+ * kernels of programs without them keep their code */
+template <int QS>
+__device__ __forceinline__ void eval_minmax(float (&acc)[kEvalRows], float*& sp, const uint32_t insn, const mcb_program& prog,
+                                            const EvalLane& L, int& pc) {
+    const uint32_t arg = MCB_FINSN_ARG(insn);
+    switch (insn & 0xffu) {
+#define MCB_MM_STEP(FOP, SRC, CLS) \
+    case MCB_HANDLER_MINMAX(FOP, CLS): eval_step<FOP, SRC, QS>(acc, sp, arg, prog, L); break;
+#define MCB_MM_STEPS(FOP) MCB_MM_STEP(FOP, MCB_SRC_K, 0) MCB_MM_STEP(FOP, MCB_SRC_TX, 1) MCB_MM_STEP(FOP, MCB_SRC_TY, 2) \
+    MCB_MM_STEP(FOP, MCB_SRC_TZ, 3) MCB_MM_STEP(FOP, MCB_SRC_POP, 4)
+        MCB_MM_STEPS(MCB_F_MIN) MCB_MM_STEPS(MCB_F_MAX)
+#define MCB_MM_PAIR(FOP, CA, CB) \
+    case MCB_HANDLER_MINMAX_PAIR(FOP, CA, CB): eval_pair<FOP, CA, CB, QS>(acc, arg, prog.code[++pc], prog, L); break;
+#define MCB_MM_PAIR_B(FOP, CA) MCB_MM_PAIR(FOP, CA, 0) MCB_MM_PAIR(FOP, CA, 1) MCB_MM_PAIR(FOP, CA, 2) MCB_MM_PAIR(FOP, CA, 3)
+#define MCB_MM_PAIR_AB(FOP) MCB_MM_PAIR_B(FOP, 0) MCB_MM_PAIR_B(FOP, 1) MCB_MM_PAIR_B(FOP, 2) MCB_MM_PAIR_B(FOP, 3)
+        MCB_MM_PAIR_AB(MCB_F_MIN) MCB_MM_PAIR_AB(MCB_F_MAX)
+#undef MCB_MM_STEP
+#undef MCB_MM_STEPS
+#undef MCB_MM_PAIR
+#undef MCB_MM_PAIR_B
+#undef MCB_MM_PAIR_AB
+        default: break;
+    }
+}
+
 /* The interpreter proper: runs the launch program on the lane's 16 accumulators.  QS = distance, in table entries,
  * between the lane's four class-1 operands (32 in the plane-tile kernel, 1 in the block kernel below).  HAS_FN: the
- * program uses a function (handlers 56..59); without it the kernel is exactly the reference grammar's. */
-template <bool HAS_POW, int QS, bool HAS_FN = false>
+ * program uses a function (handlers 56..59); HAS_MINMAX: min or max (handlers 192..233).  Without them the kernel is
+ * exactly the reference grammar's. */
+template <bool HAS_POW, int QS, bool HAS_FN = false, bool HAS_MINMAX = false>
 __device__ __forceinline__ void eval_run(const mcb_program& prog, const EvalLane& L, float (&acc)[kEvalRows], float* sp) {
 #pragma unroll
     for (int e = 0; e < kEvalRows; e++) acc[e] = 0.f;
@@ -336,7 +369,8 @@ __device__ __forceinline__ void eval_run(const mcb_program& prog, const EvalLane
                 for (int e = 0; e < kEvalRows; e++) sp[e * kEvalThreads] = acc[e];
                 sp += kEvalLevel;
                 break;
-            default: /* MCB_F_NEG, and with HAS_FN the functions; HAS_FN = false compiles to NEG alone */
+            default: /* MCB_F_NEG, and with HAS_FN / HAS_MINMAX the functions; both false compiles to NEG alone */
+                if (HAS_MINMAX && (insn & 0xffu) >= MCB_HANDLER_MINMAX_FIRST) { eval_minmax<QS>(acc, sp, insn, prog, L, pc); break; }
                 if (HAS_FN && (insn & 0xffu) != MCB_HANDLER_NEG) { eval_fn(acc, insn & 0xffu); break; }
 #pragma unroll
                 for (int e = 0; e < kEvalRows; e++) acc[e] = -acc[e];
@@ -351,8 +385,8 @@ __device__ __forceinline__ void eval_run(const mcb_program& prog, const EvalLane
 
 /* K1.  STORE_F = false is the sparse-field mode (mcb_set_field_mode): only the sign bit-plane leaves the kernel and
  * eval_blocks_kernel later writes the field where the surface needs it. */
-template <bool HAS_POW, bool STORE_F, bool HAS_FN = false> /* programs without `^` (after hoisting) get a kernel without the powf paths:
-                                                            fewer registers; HAS_FN: with the function grammar's handlers */
+template <bool HAS_POW, bool STORE_F, bool HAS_FN = false, bool HAS_MINMAX = false> /* programs without `^` (after hoisting) get a
+                        kernel without the powf paths: fewer registers; HAS_FN, HAS_MINMAX: with the function grammar's handlers */
 __global__ void __launch_bounds__(kEvalThreads, HAS_POW || HAS_FN ? 8 : 10)
 eval_field_kernel(const __grid_constant__ mcb_program prog, const Grid g, const float* __restrict__ tables,
                   float* __restrict__ F, uint32_t* __restrict__ S, int row_groups) {
@@ -368,7 +402,7 @@ eval_field_kernel(const __grid_constant__ mcb_program prog, const Grid g, const 
     L.y0 = yq * kEvalTileY;
     L.zi = pz + g.kb;
     float acc[kEvalRows];
-    eval_run<HAS_POW, 32, HAS_FN>(prog, L, acc, stack_smem + threadIdx.x);
+    eval_run<HAS_POW, 32, HAS_FN, HAS_MINMAX>(prog, L, acc, stack_smem + threadIdx.x);
 
     /* ---- outputs ----
      * A lane's columns are x0 + 32 q: every field store is one fully coalesced 128-byte line per warp, and the warp
@@ -406,7 +440,7 @@ struct FieldBlocks {
     uint8_t* flags;               /* [nbz][nby][nbx] */
     uint32_t* list;               /* flagged blocks, any order */
 };
-template <bool HAS_POW, bool HAS_FN = false>
+template <bool HAS_POW, bool HAS_FN = false, bool HAS_MINMAX = false>
 __global__ void __launch_bounds__(kEvalThreads, HAS_POW || HAS_FN ? 8 : 10)
 eval_blocks_kernel(const __grid_constant__ mcb_program prog, const Grid g, const float* __restrict__ tables,
                    float* __restrict__ F, uint32_t* __restrict__ S, const uint32_t* __restrict__ list /* pack_block */,
@@ -424,7 +458,7 @@ eval_blocks_kernel(const __grid_constant__ mcb_program prog, const Grid g, const
         L.y0 = by * kFieldBlockY;        /* class 2: the y tables */
         L.zi = bx * kFieldBlockX + lane; /* class 3: the x tables, this lane's column */
         float acc[kEvalRows];
-        eval_run<HAS_POW, 1, HAS_FN>(prog, L, acc, stack_smem + threadIdx.x);
+        eval_run<HAS_POW, 1, HAS_FN, HAS_MINMAX>(prog, L, acc, stack_smem + threadIdx.x);
         uint32_t mine = 0; /* lane 4 r + q keeps the sign word of row r, plane q: bit = this column's value > iso */
 #pragma unroll
         for (int e = 0; e < kEvalRows; e++) {

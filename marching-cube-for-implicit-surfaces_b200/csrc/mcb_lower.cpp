@@ -16,12 +16,15 @@ static inline bool is_operator(char c) { return c == '+' || c == '-' || c == '*'
 static inline bool is_number(char c) { return (c >= '0' && c <= '9') || c == '.'; }
 static inline bool is_variable(char c) { return (c >= 'x' && c <= 'z') || (c >= 'X' && c <= 'Z'); }
 
-/* The function grammar's names, each spelt with its '(' (none contains x, y or z, so none clashes with a variable) */
-static const char* const kFuncNames[4] = {"sin(", "cos(", "sqrt(", "abs("};
-static const char kFuncKinds[4] = {'S', 'C', 'Q', 'A'};
+/* The function grammar's names, each spelt with its '(': the unary ones, then the two-argument min( and max(.  A name
+ * is matched at a lowercase letter that is not a variable, so the x of max( is part of the name. */
+static const int kNumFuncs = 6;
+static const char* const kFuncNames[kNumFuncs] = {"sin(", "cos(", "sqrt(", "abs(", "min(", "max("};
+static const char kFuncKinds[kNumFuncs] = {'S', 'C', 'Q', 'A', 'm', 'M'};
+static inline bool two_args(int f) { return f >= 4; }
 
 /* Accept/reject behaviour of evaluator.cpp:139-237, token for token; under GRAMMAR_FUNCTIONS a function name with its
- * '(' is one more kind of opening bracket. */
+ * '(' is one more kind of opening bracket, and a ',' separates the two arguments of min( / max(. */
 bool tokenize(const std::string& eq_in, std::vector<Token>& out, std::string* cleaned, int grammar) {
     out.clear();
     if (eq_in.empty()) return false; /* evaluator.cpp:141 */
@@ -31,10 +34,12 @@ bool tokenize(const std::string& eq_in, std::vector<Token>& out, std::string* cl
 
     enum { L_OP, L_NUM, L_VAR, L_BO, L_BC, L_NONE } last = L_NONE;
     bool neg = false;
-    int depth = 0;
+    /* per open bracket: 0 plain or one argument, 1 two arguments before the ',', 2 two arguments after it */
+    std::vector<char> open;
     for (size_t i = 0; i < eq.size(); i++) {
         char ch = eq[i];
-        if (ch == '-' && (i == 0 || eq[i - 1] == '(' || is_operator(eq[i - 1]))) { /* :162 unary minus */
+        /* :162 unary minus; a ',' can only have been accepted under GRAMMAR_FUNCTIONS, where it acts as '(' does */
+        if (ch == '-' && (i == 0 || eq[i - 1] == '(' || eq[i - 1] == ',' || is_operator(eq[i - 1]))) {
             if (neg) return false;
             neg = true;
             out.push_back({TOK_NEG, "NEG"});
@@ -43,14 +48,20 @@ bool tokenize(const std::string& eq_in, std::vector<Token>& out, std::string* cl
         if (ch == '(') {
             if (last == L_VAR || last == L_NUM || last == L_BC) out.push_back({TOK_OP, "*"}); /* :172 implicit * */
             out.push_back({TOK_BRAC_O, "("});
-            depth++;
+            open.push_back(0);
             last = L_BO;
         } else if (ch == ')') {
             if (neg || last == L_BO || last == L_OP) return false; /* "-)", "()", "+)" */
-            if (depth == 0) return false;
+            if (open.empty() || open.back() == 1) return false;   /* unbalanced, or min( / max( with one argument */
             out.push_back({TOK_BRAC_C, ")"});
-            depth--;
+            open.pop_back();
             last = L_BC;
+        } else if (ch == ',' && grammar == GRAMMAR_FUNCTIONS) {
+            if (neg || last == L_BO || last == L_OP) return false; /* the rules before ')': "min(,x)", "min(x+,y)" */
+            if (open.empty() || open.back() != 1) return false;   /* only directly inside min( / max(, and only once */
+            out.push_back({TOK_COMMA, ","});
+            open.back() = 2;
+            last = L_BO; /* the rules after '(' */
         } else if (is_operator(ch)) {
             if (neg || last == L_BO || last == L_OP || last == L_NONE) return false;
             out.push_back({TOK_OP, std::string(1, ch)});
@@ -75,19 +86,19 @@ bool tokenize(const std::string& eq_in, std::vector<Token>& out, std::string* cl
             last = L_VAR;
         } else if (grammar == GRAMMAR_FUNCTIONS && ch >= 'a' && ch <= 'z') {
             int f = 0;
-            while (f < 4 && eq.compare(i, std::strlen(kFuncNames[f]), kFuncNames[f]) != 0) f++;
-            if (f == 4) return false; /* not a function name, or a name without its '(' */
+            while (f < kNumFuncs && eq.compare(i, std::strlen(kFuncNames[f]), kFuncNames[f]) != 0) f++;
+            if (f == kNumFuncs) return false; /* not a function name, or a name without its '(' */
             if (last == L_VAR || last == L_NUM || last == L_BC) out.push_back({TOK_OP, "*"}); /* as before '(' */
             out.push_back({TOK_FUNC, kFuncNames[f]});
             i += std::strlen(kFuncNames[f]) - 1; /* eq[i] is now the '(': the unary-minus rule sees it */
-            depth++;
+            open.push_back(two_args(f) ? 1 : 0);
             last = L_BO;
         } else {
             return false; /* :224 unknown character */
         }
         neg = false;
     }
-    if (depth != 0) return false;
+    if (!open.empty()) return false;
     if (cleaned) *cleaned = eq;
     return true;
 }
@@ -129,7 +140,8 @@ int precedence(char c) { /* evaluator.cpp:111-124 */
         default: return 0; /* ( ) and the function markers: the look-back never crosses them */
     }
 }
-bool is_func(char c) { return c == 'S' || c == 'C' || c == 'Q' || c == 'A'; }
+bool is_func(char c) { return c == 'S' || c == 'C' || c == 'Q' || c == 'A' || c == 'm' || c == 'M'; }
+bool is_func2(char c) { return c == 'm' || c == 'M'; } /* min, max: two operands */
 
 struct Machine {
     Builder& b;
@@ -164,7 +176,8 @@ struct Machine {
 
 } /* namespace */
 
-bool build_expr(const std::vector<Token>& toks, Expr& e) { /* f(E) is (E) with f applied at the ')' */
+bool build_expr(const std::vector<Token>& toks, Expr& e) { /* f(E) is (E) with f applied at the ')'; min(A,B) closes A at
+                                                                the ',' as (A) and B at the ')' as (B) */
     e.nodes.clear();
     e.root = -1;
     Builder b(e);
@@ -185,8 +198,12 @@ bool build_expr(const std::vector<Token>& toks, Expr& e) { /* f(E) is (E) with f
             }
             case TOK_BRAC_O: m.ops.push_back('('); break;
             case TOK_FUNC:
-                for (int f = 0; f < 4; f++)
+                for (int f = 0; f < kNumFuncs; f++)
                     if (t.text == kFuncNames[f]) m.ops.push_back(kFuncKinds[f]);
+                break;
+            case TOK_COMMA: /* the first argument is complete: reduce down to the marker, which stays */
+                while (m.ok && !m.ops.empty() && m.ops.back() != '(' && !is_func(m.ops.back())) m.reduce();
+                if (m.ops.empty() || !is_func2(m.ops.back())) m.ok = false;
                 break;
             case TOK_BRAC_C:
                 while (m.ok && !m.ops.empty() && m.ops.back() != '(' && !is_func(m.ops.back())) m.reduce();
@@ -194,7 +211,10 @@ bool build_expr(const std::vector<Token>& toks, Expr& e) { /* f(E) is (E) with f
                 else {
                     const char f = m.ops.back();
                     m.ops.pop_back();
-                    if (is_func(f) && m.ok) {
+                    if (is_func2(f) && m.ok) {
+                        const int v1 = m.pop_val(), v0 = m.pop_val(); /* second argument on top */
+                        if (m.ok) m.vals.push_back(b.make(f, v0, v1, 0.f));
+                    } else if (is_func(f) && m.ok) {
                         const int v = m.pop_val();
                         if (m.ok) m.vals.push_back(b.make(f, v, -1, 0.f));
                     }
@@ -221,6 +241,7 @@ static void postfix_rec(const Expr& e, int n, std::string& s) {
         case 'C': postfix_rec(e, nd.a, s); s += " cos"; return;
         case 'Q': postfix_rec(e, nd.a, s); s += " sqrt"; return;
         case 'A': postfix_rec(e, nd.a, s); s += " abs"; return;
+        case 'm': case 'M': postfix_rec(e, nd.a, s); s += ' '; postfix_rec(e, nd.b, s); s += nd.kind == 'm' ? " min" : " max"; return;
         default: postfix_rec(e, nd.a, s); s += ' '; postfix_rec(e, nd.b, s); s += ' '; s += nd.kind; return;
     }
 }
@@ -342,6 +363,8 @@ struct Lowerer {
             case '*': op = MCB_OP_MUL; break;
             case '-': op = right_first ? MCB_OP_RSUB : MCB_OP_SUB; break;
             case '/': op = right_first ? MCB_OP_RDIV : MCB_OP_DIV; break;
+            case 'm': op = MCB_OP_MIN; break; /* commutative bit for bit (mcb_minf): either order, no reversed form */
+            case 'M': op = MCB_OP_MAX; break;
             default: op = right_first ? MCB_OP_RPOW : MCB_OP_POW; break;
         }
         if (right_first) { gen(nd.b, mode, self, code, memo); gen(nd.a, mode, self, code, memo); }
@@ -420,7 +443,7 @@ int compile(const std::string& eq, Compiled& out, std::string* err, int grammar)
     out = Compiled();
     std::vector<Token> toks;
     if (!tokenize(eq, toks, &out.equation, grammar)) {
-        if (err) *err = grammar == GRAMMAR_FUNCTIONS ? "parse error (function grammar: the reference's language plus sin( cos( sqrt( abs()"
+        if (err) *err = grammar == GRAMMAR_FUNCTIONS ? "parse error (function grammar: the reference's language plus sin( cos( sqrt( abs( min( max()"
                                                      : "parse error (Evaluator::tokenize rejects this equation)";
         return MCB_E_PARSE;
     }
@@ -440,9 +463,14 @@ int compile(const std::string& eq, Compiled& out, std::string* err, int grammar)
 int fuse(const std::vector<uint32_t>& postfix, std::vector<uint32_t>& fused) {
     fused.clear();
     auto is_push = [](uint32_t op) { return op >= MCB_OP_PUSH_X && op <= MCB_OP_PUSH_TZ; };
-    auto is_bin = [](uint32_t op) { return op >= MCB_OP_ADD && op <= MCB_OP_RPOW; };
+    auto is_bin = [](uint32_t op) { return (op >= MCB_OP_ADD && op <= MCB_OP_RPOW) || op == MCB_OP_MIN || op == MCB_OP_MAX; };
     static const int direct[] = {MCB_F_ADD, MCB_F_SUB, MCB_F_RSUB, MCB_F_MUL, MCB_F_DIV, MCB_F_RDIV, MCB_F_POW, MCB_F_RPOW};
     static const int popped[] = {MCB_F_ADD, MCB_F_RSUB, MCB_F_SUB, MCB_F_MUL, MCB_F_RDIV, MCB_F_DIV, MCB_F_RPOW, MCB_F_POW};
+    /* the fused word of binary operator op with operand src; min and max are one op, bit 3 of src picks max */
+    auto bin_word = [](uint32_t op, bool pop, uint32_t src, uint32_t arg) -> uint32_t {
+        if (op == MCB_OP_MIN || op == MCB_OP_MAX) return MCB_FINSN(MCB_F_MINMAX, src | (op == MCB_OP_MAX ? MCB_SRC_MAX_BIT : 0u), arg);
+        return MCB_FINSN((pop ? popped : direct)[op - MCB_OP_ADD], src, arg);
+    };
     int depth = 0, mem = 0, mem_max = 0; /* depth: values on the operand stack (accumulator included) */
     for (size_t i = 0; i < postfix.size(); i++) {
         const uint32_t w = postfix[i], op = MCB_INSN_OP(w), arg = MCB_INSN_ARG(w);
@@ -451,7 +479,7 @@ int fuse(const std::vector<uint32_t>& postfix, std::vector<uint32_t>& fused) {
             const uint32_t src = op - MCB_OP_PUSH_X; /* PUSH_X..PUSH_TZ map onto MCB_SRC_X..MCB_SRC_TZ in order */
             const uint32_t nop = i + 1 < postfix.size() ? MCB_INSN_OP(postfix[i + 1]) : (uint32_t)MCB_OP_END;
             if (depth >= 1 && is_bin(nop)) { /* acc = second, leaf = top */
-                fused.push_back(MCB_FINSN(direct[nop - MCB_OP_ADD], src, arg));
+                fused.push_back(bin_word(nop, false, src, arg));
                 i++;
             } else if (depth == 0) {
                 fused.push_back(MCB_FINSN(MCB_F_LOAD, src, arg));
@@ -466,7 +494,7 @@ int fuse(const std::vector<uint32_t>& postfix, std::vector<uint32_t>& fused) {
         } else if (op >= MCB_OP_SIN && op <= MCB_OP_ABS) {
             fused.push_back(MCB_FINSN(MCB_F_SIN + (op - MCB_OP_SIN), 0, 0));
         } else { /* binary operator on two stacked values: acc = top, popped = second */
-            fused.push_back(MCB_FINSN(popped[op - MCB_OP_ADD], MCB_SRC_POP, 0));
+            fused.push_back(bin_word(op, true, MCB_SRC_POP, 0));
             depth--;
             mem--;
         }
@@ -476,14 +504,15 @@ int fuse(const std::vector<uint32_t>& postfix, std::vector<uint32_t>& fused) {
 
 std::string disassemble_fused(const std::vector<uint32_t>& code) {
     static const char* fops[] = {"LOAD", "PUSH", "ADD", "SUB", "RSUB", "MUL", "DIV", "RDIV", "POW", "RPOW", "NEG",
-                                 "SIN", "COS", "SQRT", "ABS"};
+                                 "SIN", "COS", "SQRT", "ABS", "?", "MIN", "MAX"};
     static const char* srcs[] = {"X", "Y", "Z", "K", "TX", "TY", "TZ", "POP"};
     std::string s;
     char buf[48];
     for (uint32_t w : code) {
         uint32_t fop = MCB_FINSN_OP(w), src = MCB_FINSN_SRC(w);
+        MCB_FINSN_DECODE(fop, src);
         if (!s.empty()) s += "; ";
-        s += fop < MCB_F_COUNT ? fops[fop] : "?";
+        s += fops[fop];
         if (fop == MCB_F_NEG || MCB_F_IS_FN(fop)) continue;
         s += ' ';
         s += src <= MCB_SRC_POP ? srcs[src] : "?";
@@ -497,7 +526,7 @@ std::string disassemble_fused(const std::vector<uint32_t>& code) {
 
 std::string disassemble(const std::vector<uint32_t>& code) {
     static const char* names[] = {"END", "X", "Y", "Z", "K", "TX", "TY", "TZ", "ADD", "SUB", "RSUB",
-                                  "MUL", "DIV", "RDIV", "POW", "RPOW", "NEG", "SIN", "COS", "SQRT", "ABS"};
+                                  "MUL", "DIV", "RDIV", "POW", "RPOW", "NEG", "SIN", "COS", "SQRT", "ABS", "MIN", "MAX"};
     std::string s;
     char buf[32];
     for (uint32_t w : code) {

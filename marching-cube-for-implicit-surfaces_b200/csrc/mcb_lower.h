@@ -29,15 +29,18 @@
 
 namespace mcb {
 
-enum TokType { TOK_OP, TOK_NUM, TOK_VAR, TOK_BRAC_O, TOK_BRAC_C, TOK_NEG, TOK_FUNC };
+enum TokType { TOK_OP, TOK_NUM, TOK_VAR, TOK_BRAC_O, TOK_BRAC_C, TOK_NEG, TOK_FUNC, TOK_COMMA };
 struct Token {
     TokType type;
-    std::string text; /* "NEG" for unary minus, like the reference; "sin(" etc. for a function and its bracket */
+    std::string text; /* "NEG" for unary minus, like the reference; "sin(" etc. for a function and its bracket; "," */
 };
 
-/* Grammars (mcb.h): MCB_GRAMMAR_REFERENCE = the reference's language; MCB_GRAMMAR_FUNCTIONS adds sin( cos( sqrt( abs(.
- * A function name and its '(' are one TOK_FUNC token that takes part in implicit multiplication, the unary-minus rule
- * and bracket balance exactly as '(' does; the walk applies the function at the matching ')'. */
+/* Grammars (mcb.h): MCB_GRAMMAR_REFERENCE = the reference's language; MCB_GRAMMAR_FUNCTIONS adds sin( cos( sqrt( abs(
+ * and the two-argument min( max(.  A function name and its '(' are one TOK_FUNC token that takes part in implicit
+ * multiplication, the unary-minus rule and bracket balance exactly as '(' does; the walk applies the function at the
+ * matching ')'.  Inside a min( / max( bracket exactly one ',' (TOK_COMMA) separates the two arguments: before it the rules
+ * that precede ')' apply, after it those that follow '('; the walk reduces each argument down to the function's marker,
+ * as ')' reduces a bracket, so `max(x-y+z,0)` is max(x-(y+z),0).  A ',' anywhere else is a parse error. */
 enum { GRAMMAR_REFERENCE = 0, GRAMMAR_FUNCTIONS = 1 };
 
 /* Evaluator::tokenize (evaluator.cpp:139-237). false = parse error. `cleaned` = equation with spaces removed. */
@@ -45,7 +48,7 @@ bool tokenize(const std::string& eq, std::vector<Token>& out, std::string* clean
 
 struct Node {
     char kind;  /* 'x','y','z' variable; 'c' literal; '+','-','*','/','^' binary (a op b); 'N' negate a;
-                 * 'S' sin a, 'C' cos a, 'Q' sqrt a, 'A' abs a (function grammar) */
+                 * 'S' sin a, 'C' cos a, 'Q' sqrt a, 'A' abs a, 'm' min(a,b), 'M' max(a,b) (function grammar) */
     int a, b;   /* children (node ids), -1 when unused */
     float value; /* literal value (strtof, like stof at evaluator.cpp:82) */
     uint8_t mask; /* variables the subtree depends on: 1=x 2=y 4=z */

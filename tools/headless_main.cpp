@@ -6,7 +6,7 @@
 //                [--scale sx sy sz] [--iso c] [--constraint i "lhs" "op" rhs]... [--no-normals] [--soup]
 //                [--ply out.ply] [--dump out.bin] [--repeat n] [--levels d]   (--levels: repeating-surface mode, distance d)
 //                [--devices n]   (z-slabs over GPUs 0..n-1 of this box: Marching::set_devices)
-//                [--functions]   (equations and constraints may use sin( cos( sqrt( abs(: Evaluator::set_function_grammar)
+//                [--functions]   (equations and constraints may use sin( cos( sqrt( abs( min( max(: Evaluator::set_function_grammar)
 //
 // Defaults are the reference GUI's (drawer.cpp:39-44): equation "x+y", grid 0.2, scale 1.1, iso 0.
 #include <chrono>
