@@ -122,8 +122,8 @@ public:
              * enough before the mesh size is known: they are whenever the mesh did not grow since the last call — a
              * repeated or shrinking configuration; a growing one takes the plain copy below once, then streams again. */
             const size_t cv = poly_data.vertex_list.size() / 3, ct = poly_data.tri_list.size() / 3;
-            const bool with_n = normals_ && !reference_normals_;
-            bool stream = cv > 0 && ct > 0 && !(normals_ && reference_normals_) && (!with_n || vertex_normals_.size() / 3 >= cv);
+            const bool with_n = normals_mode() == 1;
+            bool stream = cv > 0 && ct > 0 && normals_mode() <= 1 && (!with_n || vertex_normals_.size() / 3 >= cv);
             if (stream) stream = pin(pin_v_, poly_data.vertex_list) && pin(pin_t_, poly_data.tri_list) && (!with_n || pin(pin_n_, vertex_normals_));
             mcb_set_host_output(ctx_, stream ? poly_data.vertex_list.data() : nullptr, stream ? poly_data.tri_list.data() : nullptr,
                                 stream && with_n ? vertex_normals_.data() : nullptr, stream ? cv : 0, stream ? ct : 0);
@@ -276,6 +276,9 @@ public:
     /* true: get_vertex_normals() returns what CalculateNormal(get_poly_data()) would (normal.h:3-42), computed on the GPU,
      * bit for bit; false (default): central-difference gradient normals */
     void set_reference_normals(bool b) { reference_normals_ = b; }
+    /* true: the equation's own gradient at every vertex, soup or welded (mcb_set_normals mode 3, DESIGN.md §12); takes
+     * precedence over set_reference_normals.  false (default): as set_reference_normals says */
+    void set_analytic_normals(bool b) { analytic_normals_ = b; }
     bool set_slab(int k_begin, int k_end) { slab_[0] = k_begin; slab_[1] = k_end; have_slab_ = true; return true; }
     const mcb_counts& last_counts() const { return counts_; }
     /* set_devices(n > 1): wall time of the phases of the last recalculate(), ms: the slabs' polygonisation (+ exchange),
@@ -318,13 +321,14 @@ private:
         if (have_slab_ && mcb_set_slab(ctx_, slab_[0], slab_[1]) != MCB_OK) return false;
         return true;
     }
+    int normals_mode() const { return normals_ ? (analytic_normals_ ? 3 : weld_ && reference_normals_ ? 2 : 1) : 0; }
     bool push_parameters() { return push_parameters(ctx_); }
     bool push_parameters(mcb_ctx* c) {
         mcb_set_grammar(c, evaluator_->grammar()); /* Evaluator::set_function_grammar */
         if (mcb_set_equation(c, 0, evaluator_->equation().c_str()) != MCB_OK) return false;
         mcb_set_surface_constant(c, iso_);
         mcb_set_scaling(c, sx_, sy_, sz_);
-        mcb_set_normals(c, normals_ ? (weld_ && reference_normals_ ? 2 : 1) : 0);
+        mcb_set_normals(c, normals_mode());
         /* marching.cpp:156-170, 481-494.  The reference accepts the mode with its initial distance 0: every cube's iso is
          * then NaN and nothing is drawn; recalculate() short-cuts that case, the GPU only sees positive distances */
         mcb_set_repeat(c, repeat_ && repeat_step_ > 0.f ? 1 : 0, repeat_step_);
@@ -530,6 +534,7 @@ private:
     float step_, iso_, sx_, sy_, sz_;
     bool weld_, normals_, seed_mode_, step_mode_, repeat_;
     bool reference_normals_ = false;
+    bool analytic_normals_ = false;
     float repeat_step_;
     float seed_[3];
     bool cons_valid_[3], cons_use_[3];

@@ -160,6 +160,10 @@ int mcb_set_grammar(mcb_ctx* ctx, int grammar);
 /* Evaluator::evaluate (evaluator.cpp:53-107) for n points on the GPU.  xyz = 3n floats, out = n floats, host
  * memory.  apply_scale != 0 multiplies by the per-axis scale first, i.e. Marching::evaluate (marching.cpp:209-224). */
 int mcb_eval_points(mcb_ctx* ctx, int slot, const float* xyz, float* out, size_t n, int apply_scale);
+/* The gradient of the same point program at n points on the GPU: grad = 3n floats (df/dx, df/dy, df/dz), unnormalised,
+ * host memory; the forward-mode rules of mcb_set_normals mode 3.  With apply_scale != 0 the program runs at (sx*x, sy*y,
+ * sz*z) and the gradient is taken with respect to the unscaled (x, y, z).  Same slots and errors as mcb_eval_points. */
+int mcb_eval_gradients(mcb_ctx* ctx, int slot, const float* xyz, float* grad, size_t n, int apply_scale);
 
 /* ---- marching.h ------------------------------------------------------------------------------------------ */
 
@@ -187,7 +191,18 @@ int mcb_set_constraint(mcb_ctx* ctx, int i, int op, float rhs, int in_use);
 int mcb_set_seed(mcb_ctx* ctx, int enabled, float x, float y, float z);
 /* 0 = positions only; 1 = also normals from central-difference field gradients (per soup vertex and per welded
  * vertex; DESIGN.md, normals); 2 = CalculateNormal of the reference (normal.h:3-42: area-weighted face normals summed
- * per welded vertex in triangle order, glm::normalize), bit-exact, per welded vertex — needs MCB_MESH_INDEXED. */
+ * per welded vertex in triangle order, glm::normalize), bit-exact, per welded vertex — needs MCB_MESH_INDEXED;
+ * 3 = analytic normals (DESIGN.md §12): the equation's own gradient at every soup and welded vertex, by forward-mode
+ * differentiation of the point program in fp32, bit-identical on host and GPU.  Positions, indices and counts are those of
+ * mode 0.  With a the left and b the right operand of each operation of the equation:
+ *     x, y, z -> (sx,0,0), (0,sy,0), (0,0,sz)     constant -> 0           a+-b -> ga+-gb       a*b -> ga*b + a*gb
+ *     a/b -> (ga - q*gb)/b, q = a/b               -a -> -ga               sin a -> cos(a)*ga   cos a -> (-sin(a))*ga
+ *     sqrt a -> ga/(s+s), s = sqrt(a)             abs a -> sign bit of a set ? -ga : ga
+ *     a^b -> gb exactly 0: (b * a^(b-1)) * ga, else a^b * (ln(a)*gb + (b/a)*ga)  (ln from the fp64 log2 of `^`; NaN for a <= 0)
+ *     min / max -> the gradient of the operand whose bits equal the result, (ga+gb)*0.5f when both (or neither) do
+ * Normalisation: m = max |g_i|; (0,0,0) when m is 0, infinite or NaN or a component is NaN; otherwise u = g/m,
+ * d = ux*ux + uy*uy + uz*uz, n = u * (1/sqrt(d)) (correctly rounded square root).  The normal points towards increasing f,
+ * as mode 1's does.  Like mode 2, mode 3 is not streamed through mcb_set_host_output. */
 int mcb_set_normals(mcb_ctx* ctx, int mode);
 
 /* The hot path: Marching::recalculate() (marching.cpp:368-384) for this context's slab, entirely on the GPU.
@@ -256,7 +271,7 @@ int mcb_set_field_mode(mcb_ctx* ctx, int mode);
  * (marching.cpp:599-654, tolerance comparator marching.h:38-54), triangles in emission order. */
 int mcb_set_mesh_mode(mcb_ctx* ctx, int mode);
 /* Copy the indexed mesh to host memory: vertex_list = 3*vertices floats (x,y,z), tri_list = 3*triangles indices,
- * normals = 3*vertices floats (gradient normals per welded vertex; needs mcb_set_normals(1)).  Any may be NULL. */
+ * normals = 3*vertices floats (normals per welded vertex; needs mcb_set_normals 1, 2 or 3).  Any may be NULL. */
 int mcb_get_indexed_mesh(mcb_ctx* ctx, float* vertex_list, uint32_t* tri_list, float* normals, uint64_t cap_vertices,
                          uint64_t cap_triangles);
 /* A mesh assembled from several slabs (one context each) numbers the vertices of slab r from the sum of the earlier slabs'
@@ -268,7 +283,7 @@ int mcb_get_indexed_mesh_device(mcb_ctx* ctx, const float** vertex_list, const u
  * registered, mcb_polygonise in MCB_MESH_INDEXED mode streams vertex_list / normals / tri_list out range by range
  * while the later ranges are still being produced, and returns when the mesh is on the host — one call, like
  * Marching::recalculate() filling Poly_Data.  normals may be NULL when normals are off.  When a device buffer has to
- * grow first, the mesh does not fit the registered capacities, or normal.h normals (mode 2) are on, nothing is
+ * grow first, the mesh does not fit the registered capacities, or normals mode 2 or 3 is on, nothing is
  * streamed: mcb_host_output_filled() returns 0 and mcb_get_indexed_mesh delivers the mesh.  NULL pointers unregister. */
 int mcb_set_host_output(mcb_ctx* ctx, float* vertex_list, uint32_t* tri_list, float* normals, uint64_t cap_vertices,
                         uint64_t cap_triangles);

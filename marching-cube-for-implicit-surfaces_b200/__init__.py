@@ -26,6 +26,7 @@ MESH_SOUP, MESH_INDEXED = 1, 2
 FIELD_DENSE, FIELD_SPARSE, FIELD_AUTO = 0, 1, 2
 JIT_OFF, JIT_ON, JIT_AUTO = 0, 1, 2
 GRAMMAR_REFERENCE, GRAMMAR_FUNCTIONS = 0, 1  # the reference's equation language / the same plus sin( cos( sqrt( abs( min( max(
+NORMALS_ANALYTIC = 3  # set_normals mode: the equation's own gradient at every output vertex (include/mcb.h, DESIGN.md §12)
 MCB_OK, MCB_E_PARSE, MCB_E_ARG, MCB_E_CUDA, MCB_E_NOMEM, MCB_E_STATE, MCB_E_CAPACITY, MCB_E_NODEVICE = 0, -1, -2, -3, -4, -5, -6, -7
 
 
@@ -80,6 +81,7 @@ def _load():
         "mcb_set_equation": ([vp, i, cp], i),
         "mcb_set_grammar": ([vp, i], i),
         "mcb_eval_points": ([vp, i, vp, vp, sz, i], i),
+        "mcb_eval_gradients": ([vp, i, vp, vp, sz, i], i),
         "mcb_set_grid_step": ([vp, f], i),
         "mcb_set_slab": ([vp, i, i], i),
         "mcb_set_surface_constant": ([vp, f], i),
@@ -272,6 +274,15 @@ class Context:
         out = np.empty(len(xyz), np.float32)
         self._ck(lib.mcb_eval_points(self.h, slot, xyz.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p),
                                      len(xyz), int(apply_scale)))
+        return out
+
+    def eval_gradients(self, xyz, slot=0, apply_scale=False):
+        """The gradient (df/dx, df/dy, df/dz) of the slot's equation at n points, unnormalised: [n,3] f32.  Forward-mode
+        differentiation of the same program eval_points runs (include/mcb.h, mcb_eval_gradients)."""
+        xyz = np.ascontiguousarray(xyz, np.float32).reshape(-1, 3)
+        out = np.empty((len(xyz), 3), np.float32)
+        self._ck(lib.mcb_eval_gradients(self.h, slot, xyz.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p),
+                                        len(xyz), int(apply_scale)))
         return out
 
     def set_grid_step(self, step):

@@ -690,6 +690,27 @@ int mcb_eval_points(mcb_ctx* ctx, int slot, const float* xyz, float* out, size_t
     return MCB_OK;
 }
 
+int mcb_eval_gradients(mcb_ctx* ctx, int slot, const float* xyz, float* grad, size_t n, int apply_scale) {
+    int rc = enter(ctx);
+    if (rc != MCB_OK) return rc;
+    if (slot < 0 || slot > 3 || !ctx->eq[slot].valid) return fail(ctx, MCB_E_STATE, "no equation in that slot");
+    if (n == 0) return MCB_OK;
+    if (!xyz || !grad) return fail(ctx, MCB_E_ARG, "null buffer");
+    float *d_in = nullptr, *d_out = nullptr;
+    MCB_CK(cudaMalloc((void**)&d_in, n * 3 * sizeof(float)));
+    cudaError_t e = cudaMalloc((void**)&d_out, n * 3 * sizeof(float));
+    if (e != cudaSuccess) { cudaFree(d_in); return fail(ctx, MCB_E_NOMEM, "cudaMalloc"); }
+    float sx = apply_scale ? ctx->scale[0] : 1.f, sy = apply_scale ? ctx->scale[1] : 1.f, sz = apply_scale ? ctx->scale[2] : 1.f;
+    cudaMemcpyAsync(d_in, xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    MCB_LAUNCH((eval_gradients_kernel), (unsigned)((n + 127) / 128), 128, 0, ctx->stream, ctx->eq[slot].point, d_in, d_out, (long long)n, sx, sy, sz);
+    cudaMemcpyAsync(grad, d_out, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
+    e = cudaStreamSynchronize(ctx->stream);
+    cudaError_t e2 = cudaGetLastError();
+    cudaFree(d_in); cudaFree(d_out);
+    if (e != cudaSuccess || e2 != cudaSuccess) return fail(ctx, MCB_E_CUDA, std::string("eval_gradients: ") + cudaGetErrorString(e != cudaSuccess ? e : e2));
+    return MCB_OK;
+}
+
 int mcb_set_grid_step(mcb_ctx* ctx, float step) {
     if (!ctx) return MCB_E_ARG;
     int M = mcb_grid_axis(step, nullptr, 0);
@@ -786,7 +807,7 @@ int mcb_set_seed(mcb_ctx* ctx, int enabled, float x, float y, float z) {
 }
 
 int mcb_set_normals(mcb_ctx* ctx, int mode) {
-    if (!ctx || mode < 0 || mode > 2) return MCB_E_ARG;
+    if (!ctx || mode < 0 || mode > 3) return MCB_E_ARG;
     ctx->normals = mode;
     ctx->have_result = false;
     return MCB_OK;
@@ -823,6 +844,7 @@ struct Run {
     int stage_soup();
     int stage_weld();
     int stage_normal_h();
+    int stage_grad_normals(bool soup);
 };
 
 int Run::prepare_buffers() {
@@ -1339,7 +1361,7 @@ int Run::stage_weld() {
     /* streaming: with a registered host destination and everything fitting, weld_emit runs range by range and
      * each finished range of vertices / normals / triangles leaves over PCIe on the copy stream meanwhile */
     constexpr int K = 8;
-    bool stream_out = ctx->h_out_v && ctx->h_out_t && ctx->normals != 2 && (ctx->normals == 0 || ctx->h_out_n);
+    bool stream_out = ctx->h_out_v && ctx->h_out_t && ctx->normals <= 1 && (ctx->normals == 0 || ctx->h_out_n);
     ctx->streamed = false;
     if (stream_out) {
         MCB_LAUNCH((weld_bounds_kernel), 1, 32, 0, s, B, ctx->d_ctr, ctx->cap_active, K, ctx->d_bounds);
@@ -1401,6 +1423,19 @@ int Run::stage_normal_h() {
     return MCB_OK;
 }
 
+/* Analytic normals (mcb_set_normals 3): the surface's gradient at every soup or welded vertex, after the emitter / weld */
+int Run::stage_grad_normals(bool soup) {
+    const unsigned grid = (unsigned)ctx->sm_count * 8;
+    if (soup)
+        MCB_LAUNCH((grad_normals_kernel<true>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, ctx->d_ctr, ctx->cap_tris,
+                   (const float*)ctx->d_pos, (float*)ctx->d_nrm);
+    else
+        MCB_LAUNCH((grad_normals_kernel<false>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, ctx->d_ctr, ctx->cap_verts,
+                   ctx->d_vlist, ctx->d_vnrm);
+    launches++;
+    return MCB_OK;
+}
+
 } /* namespace */
 
 extern "C" {
@@ -1458,10 +1493,12 @@ int mcb_polygonise(mcb_ctx* ctx, mcb_counts* out) {
             if (timing) MCB_CK(cudaEventRecord(ctx->ev[3], s));
         }
         if (run.want_soup && (rc = run.stage_soup()) != MCB_OK) return rc;
+        if (run.want_soup && ctx->normals == 3 && (rc = run.stage_grad_normals(true)) != MCB_OK) return rc;
         if (timing) MCB_CK(cudaEventRecord(ctx->ev[4], s));
         if (run.want_indexed) {
             if ((rc = run.stage_weld()) != MCB_OK) return rc;
             if (ctx->normals == 2 && (rc = run.stage_normal_h()) != MCB_OK) return rc;
+            if (ctx->normals == 3 && (rc = run.stage_grad_normals(false)) != MCB_OK) return rc;
         }
         if (timing) MCB_CK(cudaEventRecord(ctx->ev[5], s));
         if (run.want_indexed && ctx->streamed) MCB_CK(cudaStreamWaitEvent(s, ctx->seg_ev[8], 0)); /* return when the mesh is on the host */
@@ -1542,7 +1579,7 @@ int mcb_get_mesh(mcb_ctx* ctx, float* pos4, float* nrm4, uint64_t cap_triangles)
     if (!(ctx->last.mesh_mode & MCB_MESH_SOUP)) return fail(ctx, MCB_E_STATE, "the triangle soup was not requested (mcb_set_mesh_mode)");
     const uint64_t T = ctx->last.triangles;
     if (T > cap_triangles) return fail(ctx, MCB_E_CAPACITY, "mesh buffer too small");
-    if (nrm4 && ctx->normals != 1) return fail(ctx, MCB_E_STATE, "soup normals need mcb_set_normals(ctx, 1)");
+    if (nrm4 && ctx->normals != 1 && ctx->normals != 3) return fail(ctx, MCB_E_STATE, "soup normals need mcb_set_normals(ctx, 1) or 3");
     if (T == 0) return MCB_OK;
     if (pos4) MCB_CK(cudaMemcpyAsync(pos4, ctx->d_pos, T * 3 * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
     if (nrm4) MCB_CK(cudaMemcpyAsync(nrm4, ctx->d_nrm, T * 3 * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1668,7 +1705,7 @@ int mcb_get_mesh_device(mcb_ctx* ctx, const float** pos4, const float** nrm4) {
     if (!ctx) return MCB_E_ARG;
     if (!ctx->have_result) return fail(ctx, MCB_E_STATE, "mcb_polygonise has not run since the last change");
     if (pos4) *pos4 = (const float*)ctx->d_pos;
-    if (nrm4) *nrm4 = ctx->normals == 1 ? (const float*)ctx->d_nrm : nullptr;
+    if (nrm4) *nrm4 = ctx->normals == 1 || ctx->normals == 3 ? (const float*)ctx->d_nrm : nullptr;
     return MCB_OK;
 }
 

@@ -157,6 +157,137 @@ MCB_BC_FN float mcb_interp_scalar(const uint32_t* code, int n, const float* k, f
     return st[0];
 }
 
+/* ---- analytic normals (mcb_set_normals 3, mcb_eval_gradients) ---------------------------------------------------
+ * Forward-mode differentiation of a point program: every stack entry is a dual number, a value and its three partials
+ * with respect to the unscaled coordinates.  The value part runs exactly the operations of mcb_interp_scalar, so its bits
+ * are those of mcb_eval_points.  The partials follow one fixed fp32 rule per operation of the equation, in the order
+ * written, with a the left and b the right operand whatever stack order the lowering chose (the reversed forms swap them
+ * back), so the gradient is a function of the operation graph alone:
+ *      x, y, z  (sx,0,0) (0,sy,0) (0,0,sz)          constant  0
+ *      a+b, a-b ga+-gb                              a*b       ga*b + a*gb
+ *      a/b      (ga - q*gb) / b, q = a/b            -a        -ga
+ *      a^b      gb == 0 exactly: (b * a^(b-1)) * ga, else v * (ln(a)*gb + (b/a)*ga), v = a^b, ln a = mcb_lnf(a)
+ *      sin a    cos(a)*ga      cos a  (-sin(a))*ga  sqrt a    ga / (s+s), s = sqrt(a)
+ *      abs a    sign bit of a set ? -ga : ga
+ *      min, max the gradient of the operand whose bits equal the result; (ga+gb)*0.5f when both or neither do
+ *               (symmetric, so the free operand order of min / max cannot change a bit)
+ * Point programs use no axis tables. */
+
+/* ln x for the x^y rule: mcb_powf_full's fp64 log2 times ln 2, rounded once.  NaN for x <= 0 or NaN, +inf for +inf. */
+MCB_BC_FN float mcb_lnf(float x) {
+    uint32_t ix = mcb_f2u(x);
+    if (!(x > 0.f)) return mcb_u2f(0x7fc00000u);
+    if (ix >= 0x7f800000u) return x;
+    if (ix < 0x00800000u) { /* subnormal: normalised as mcb_powf_full does */
+        ix = mcb_f2u(x * 8388608.0f);
+        ix -= 23u << 23;
+    }
+    return (float)(mcb_pow_log2(ix) * mcb_u2d(0x3fe62e42fefa39efull) /* ln 2 */);
+}
+
+MCB_BC_FN float mcb_interp_grad_scalar(const uint32_t* code, int n, const float* k, float x, float y, float z,
+                                       float sx, float sy, float sz, float g[3]) {
+    float st[MCB_MAX_STACK], gs[MCB_MAX_STACK][3];
+    int sp = 0;
+    for (int pc = 0; pc < n; pc++) {
+        const uint32_t w = code[pc], op = MCB_INSN_OP(w), arg = MCB_INSN_ARG(w);
+        if (op == MCB_OP_END) break;
+        if (op <= MCB_OP_PUSH_K) {
+            st[sp] = op == MCB_OP_PUSH_X ? x : op == MCB_OP_PUSH_Y ? y : op == MCB_OP_PUSH_Z ? z : k[arg];
+            gs[sp][0] = op == MCB_OP_PUSH_X ? sx : 0.f;
+            gs[sp][1] = op == MCB_OP_PUSH_Y ? sy : 0.f;
+            gs[sp][2] = op == MCB_OP_PUSH_Z ? sz : 0.f;
+            sp++;
+            continue;
+        }
+        if (MCB_OP_IS_UNARY(op)) {
+            const float a = st[sp - 1];
+            float* ga = gs[sp - 1];
+            if (op == MCB_OP_NEG) {
+                st[sp - 1] = -a;
+                for (int c = 0; c < 3; c++) ga[c] = -ga[c];
+            } else {
+                const float v = mcb_fn(op - MCB_OP_SIN, a);
+                st[sp - 1] = v;
+                if (op == MCB_OP_SIN || op == MCB_OP_COS) {
+                    const float d = op == MCB_OP_SIN ? mcb_fn(1, a) : -mcb_fn(0, a);
+                    for (int c = 0; c < 3; c++) ga[c] = d * ga[c];
+                } else if (op == MCB_OP_SQRT) {
+                    const float d = v + v;
+                    for (int c = 0; c < 3; c++) ga[c] = ga[c] / d;
+                } else if (mcb_f2u(a) >> 31) {
+                    for (int c = 0; c < 3; c++) ga[c] = -ga[c];
+                }
+            }
+            continue;
+        }
+        const float top = st[--sp], second = st[sp - 1];
+        const bool rev = op == MCB_OP_RSUB || op == MCB_OP_RDIV || op == MCB_OP_RPOW;
+        const float a = rev ? top : second, b = rev ? second : top;
+        float ga[3], gb[3], r[3];
+        for (int c = 0; c < 3; c++) {
+            ga[c] = rev ? gs[sp][c] : gs[sp - 1][c];
+            gb[c] = rev ? gs[sp - 1][c] : gs[sp][c];
+        }
+        const float v = mcb_binop(op, second, top);
+        switch (op) {
+            case MCB_OP_ADD:
+                for (int c = 0; c < 3; c++) r[c] = ga[c] + gb[c];
+                break;
+            case MCB_OP_SUB: case MCB_OP_RSUB:
+                for (int c = 0; c < 3; c++) r[c] = ga[c] - gb[c];
+                break;
+            case MCB_OP_MUL:
+                for (int c = 0; c < 3; c++) r[c] = ga[c] * b + a * gb[c];
+                break;
+            case MCB_OP_DIV: case MCB_OP_RDIV:
+                for (int c = 0; c < 3; c++) r[c] = (ga[c] - v * gb[c]) / b;
+                break;
+            case MCB_OP_MIN: case MCB_OP_MAX: {
+                const uint32_t iv = mcb_f2u(v);
+                const bool ma = mcb_f2u(a) == iv, mb = mcb_f2u(b) == iv;
+                for (int c = 0; c < 3; c++) r[c] = ma && !mb ? ga[c] : mb && !ma ? gb[c] : (ga[c] + gb[c]) * 0.5f;
+                break;
+            }
+            default: /* POW, RPOW */
+                if (gb[0] == 0.f && gb[1] == 0.f && gb[2] == 0.f) {
+                    const float d = b * mcb_powf(a, b - 1.f);
+                    for (int c = 0; c < 3; c++) r[c] = d * ga[c];
+                } else {
+                    const float la = mcb_lnf(a), ba = b / a;
+                    for (int c = 0; c < 3; c++) r[c] = v * (la * gb[c] + ba * ga[c]);
+                }
+        }
+        st[sp - 1] = v;
+        for (int c = 0; c < 3; c++) gs[sp - 1][c] = r[c];
+    }
+    for (int c = 0; c < 3; c++) g[c] = gs[0][c];
+    return st[0];
+}
+
+/* The analytic normal of a gradient: m = max |g_i|; (0,0,0) when m is 0, infinite or NaN or a component is NaN; otherwise
+ * u = g/m, d = ux*ux + uy*uy + uz*uz (left to right), r = 1/sqrt(d) (correctly rounded, no rsqrt), n = u*r.  Scaling by m
+ * first keeps a huge gradient (1/x near 0) a direction instead of an overflow. */
+MCB_BC_FN void mcb_grad_normalise(const float g[3], float out[3]) {
+    const float ax = mcb_u2f(mcb_f2u(g[0]) & 0x7fffffffu), ay = mcb_u2f(mcb_f2u(g[1]) & 0x7fffffffu),
+                az = mcb_u2f(mcb_f2u(g[2]) & 0x7fffffffu);
+    float m = ax > ay ? ax : ay;
+    m = m > az ? m : az;
+    if (g[0] != g[0] || g[1] != g[1] || g[2] != g[2] || !(m > 0.f) || mcb_f2u(m) == 0x7f800000u) {
+        out[0] = out[1] = out[2] = 0.f;
+        return;
+    }
+    const float ux = g[0] / m, uy = g[1] / m, uz = g[2] / m;
+    float d = ux * ux + uy * uy;
+    d = d + uz * uz;
+#if defined(__CUDA_ARCH__)
+    const float r = 1.f / __fsqrt_rn(d);
+#else
+    const float r = 1.f / sqrtf(d);
+#endif
+    out[0] = ux * r; out[1] = uy * r; out[2] = uz * r;
+}
+
 /* ---- fused ("accumulator") form of a grid program -----------------------------------------------------------
  * The grid kernel does not run the postfix words above directly.  mcb::fuse() (mcb_lower.cpp) rewrites them so
  * that a push which is immediately consumed by a binary operator becomes that operator's second operand:

@@ -2518,4 +2518,40 @@ __global__ void eval_points_kernel(const __grid_constant__ mcb_program prog, con
                                nullptr, nullptr, nullptr);
 }
 
+__global__ void eval_gradients_kernel(const __grid_constant__ mcb_program prog, const float* __restrict__ xyz,
+                                      float* __restrict__ grad, long long n, float sx, float sy, float sz) {
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n) return;
+    float gr[3];
+    mcb_interp_grad_scalar(prog.code, prog.n, prog.k, sx * xyz[3 * q], sy * xyz[3 * q + 1], sz * xyz[3 * q + 2], sx, sy, sz, gr);
+    grad[3 * q] = gr[0]; grad[3 * q + 1] = gr[1]; grad[3 * q + 2] = gr[2];
+}
+
+/* Analytic normals (mcb_set_normals 3): the normalised gradient of the surface's point program at every output vertex,
+ * after the emitter (SOUP: float4 (x,y,z,1) -> (nx,ny,nz,0), 3 per triangle) or the weld (float3 -> float3).  A normal is
+ * a function of the position bits, the equation and the scale only.  The element count comes from the device counters,
+ * capped by the buffer, so the pass needs no host synchronisation and runs again in a repeated pass. */
+template <bool SOUP>
+__global__ void __launch_bounds__(256)
+grad_normals_kernel(const __grid_constant__ mcb_program prog, float sx, float sy, float sz, const Counters* __restrict__ ctr,
+                    unsigned long long cap, const float* __restrict__ pos, float* __restrict__ nrm) {
+    unsigned long long n = SOUP ? ctr->triangles : ctr->vertices;
+    if (n > cap) n = cap;
+    if (SOUP) n *= 3;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long q = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += stride) {
+        float p[3], gr[3], o[3];
+        if (SOUP) {
+            const float4 v = reinterpret_cast<const float4*>(pos)[q];
+            p[0] = v.x; p[1] = v.y; p[2] = v.z;
+        } else {
+            p[0] = pos[3 * q]; p[1] = pos[3 * q + 1]; p[2] = pos[3 * q + 2];
+        }
+        mcb_interp_grad_scalar(prog.code, prog.n, prog.k, sx * p[0], sy * p[1], sz * p[2], sx, sy, sz, gr);
+        mcb_grad_normalise(gr, o);
+        if (SOUP) reinterpret_cast<float4*>(nrm)[q] = make_float4(o[0], o[1], o[2], 0.f);
+        else { nrm[3 * q] = o[0]; nrm[3 * q + 1] = o[1]; nrm[3 * q + 2] = o[2]; }
+    }
+}
+
 } /* namespace mcbk */

@@ -120,6 +120,30 @@ MCB_POW_FN int mcb_pow_checkint(uint32_t iy) {
 MCB_POW_FN int mcb_pow_zeroinfnan(uint32_t ix) { return 2 * ix - 1 >= 2u * 0x7f800000u - 1; }
 MCB_POW_FN int mcb_pow_issignaling(uint32_t ix) { return ((ix ^ 0x00400000u) & 0x7fffffffu) > 0x7fc00000u; }
 
+/* log2_inline of the algorithm: log2(x) in fp64 for the bits ix of a positive, normal, finite x (a subnormal x arrives
+ * normalised, its exponent below the range of the field).  mcb_powf_full below and mcb_lnf of the analytic normals. */
+MCB_POW_FN double mcb_pow_log2(uint32_t ix) {
+    uint32_t tmp = ix - 0x3f330000u;
+    int i = (int)((tmp >> 19) & 15u);
+    uint32_t top = tmp & 0xff800000u;
+    uint32_t iz = ix - top;
+    int k = (int32_t)top >> 23;
+    double invc = mcb_log2_tab(2 * i), logc = mcb_log2_tab(2 * i + 1);
+    double z = (double)mcb_u2f(iz);
+    const double A0 = mcb_u2d(0x3fd27616c9496e0bull), A1 = mcb_u2d(0xbfd71969a075c67aull),
+                 A2 = mcb_u2d(0x3fdec70a6ca7baddull), A3 = mcb_u2d(0xbfe7154748bef6c8ull),
+                 A4 = mcb_u2d(0x3ff71547652ab82bull);
+    double r = fma(z, invc, -1.0);
+    double y0 = logc + (double)k;
+    double r2 = r * r;
+    double yy = fma(A0, r, A1);
+    double p = fma(A2, r, A3);
+    double r4 = r2 * r2;
+    double q = fma(A4, r, y0);
+    q = fma(p, r2, q);
+    return fma(yy, r4, q);
+}
+
 MCB_POW_FN float mcb_powf_full(float x, float y) {
     uint32_t sign_bias = 0;
     uint32_t ix = mcb_f2u(x), iy = mcb_f2u(y);
@@ -151,26 +175,7 @@ MCB_POW_FN float mcb_powf_full(float x, float y) {
             ix -= 23u << 23;
         }
     }
-    /* log2_inline */
-    uint32_t tmp = ix - 0x3f330000u;
-    int i = (int)((tmp >> 19) & 15u);
-    uint32_t top = tmp & 0xff800000u;
-    uint32_t iz = ix - top;
-    int k = (int32_t)top >> 23;
-    double invc = mcb_log2_tab(2 * i), logc = mcb_log2_tab(2 * i + 1);
-    double z = (double)mcb_u2f(iz);
-    const double A0 = mcb_u2d(0x3fd27616c9496e0bull), A1 = mcb_u2d(0xbfd71969a075c67aull),
-                 A2 = mcb_u2d(0x3fdec70a6ca7baddull), A3 = mcb_u2d(0xbfe7154748bef6c8ull),
-                 A4 = mcb_u2d(0x3ff71547652ab82bull);
-    double r = fma(z, invc, -1.0);
-    double y0 = logc + (double)k;
-    double r2 = r * r;
-    double yy = fma(A0, r, A1);
-    double p = fma(A2, r, A3);
-    double r4 = r2 * r2;
-    double q = fma(A4, r, y0);
-    q = fma(p, r2, q);
-    double logx = fma(yy, r4, q);
+    double logx = mcb_pow_log2(ix); /* log2_inline */
     double ylogx = (double)y * logx;
     if ((mcb_d2u(ylogx) >> 47 & 0xffff) >= 0x80bfu) { /* |y*log2(x)| >= 126 */
         /* (the round-away check for 0x1.fffffffa3aae2p+6 < ylogx is a no-op in round-to-nearest) */

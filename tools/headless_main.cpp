@@ -7,6 +7,8 @@
 //                [--ply out.ply] [--dump out.bin] [--repeat n] [--levels d]   (--levels: repeating-surface mode, distance d)
 //                [--devices n]   (z-slabs over GPUs 0..n-1 of this box: Marching::set_devices)
 //                [--functions]   (equations and constraints may use sin( cos( sqrt( abs( min( max(: Evaluator::set_function_grammar)
+//                [--analytic-normals]   (normals from the equation's own gradient: Marching::set_analytic_normals)
+//                [--dump-normals out.bin]   (the welded vertex normals, nv*3 f32, or the soup's 3 float4 per triangle)
 //
 // Defaults are the reference GUI's (drawer.cpp:39-44): equation "x+y", grid 0.2, scale 1.1, iso 0.
 #include <chrono>
@@ -20,7 +22,7 @@
 static int usage() {
     std::fprintf(stderr, "usage: mcb_headless [--eq S | --eq-file F] [--step h | --res n] [--scale sx sy sz] [--iso c]\n"
                          "                    [--constraint i lhs op rhs] [--no-normals] [--soup] [--ply F] [--dump F] [--repeat n] [--levels d] [--devices n]\n"
-                         "                    [--functions]\n");
+                         "                    [--functions] [--analytic-normals] [--dump-normals F]\n");
     return 2;
 }
 
@@ -30,7 +32,7 @@ int main(int argc, char** argv) {
     march_maker.set_evaluator(&evaluator);
     float step = 0.2f, sx = 1.1f, sy = 1.1f, sz = 1.1f, iso = 0.f;
     int res = 0, repeat = 1;
-    std::string ply, dump;
+    std::string ply, dump, dump_normals;
     for (int a = 1; a < argc; a++) /* before any equation is parsed, wherever it stands */
         if (std::strcmp(argv[a], "--functions") == 0) evaluator.set_function_grammar(true);
     for (int a = 1; a < argc; a++) {
@@ -55,9 +57,11 @@ int main(int argc, char** argv) {
             a += 4;
         } else if (o == "--functions") continue;
         else if (o == "--no-normals") march_maker.set_normals(false);
+        else if (o == "--analytic-normals") march_maker.set_analytic_normals(true);
         else if (o == "--soup") march_maker.set_weld(false);
         else if (o == "--ply" && need(1)) ply = argv[++a];
         else if (o == "--dump" && need(1)) dump = argv[++a];
+        else if (o == "--dump-normals" && need(1)) dump_normals = argv[++a];
         else if (o == "--repeat" && need(1)) repeat = std::atoi(argv[++a]);
         else if (o == "--devices" && need(1)) { if (!march_maker.set_devices(std::atoi(argv[++a]))) { std::fprintf(stderr, "bad device count\n"); return 1; } }
         else if (o == "--levels" && need(1)) { /* Marching::set_surface_repeat_step_distance + repeating_surface_mode */
@@ -111,6 +115,13 @@ int main(int argc, char** argv) {
         std::fwrite(&nv, 8, 1, fp); std::fwrite(&nt, 8, 1, fp);
         std::fwrite(pData->vertex_list.data(), 4, pData->vertex_list.size(), fp);
         std::fwrite(pData->tri_list.data(), 4, pData->tri_list.size(), fp);
+        std::fclose(fp);
+    }
+    if (!dump_normals.empty()) {
+        const std::vector<float>& n = march_maker.get_vertex_normals().empty() ? march_maker.get_normals() : march_maker.get_vertex_normals();
+        FILE* fp = std::fopen(dump_normals.c_str(), "wb");
+        if (!fp) return 1;
+        std::fwrite(n.data(), 4, n.size(), fp);
         std::fclose(fp);
     }
     return 0;
