@@ -123,7 +123,7 @@ public:
              * repeated or shrinking configuration; a growing one takes the plain copy below once, then streams again. */
             const size_t cv = poly_data.vertex_list.size() / 3, ct = poly_data.tri_list.size() / 3;
             const bool with_n = normals_mode() == 1;
-            bool stream = cv > 0 && ct > 0 && normals_mode() <= 1 && (!with_n || vertex_normals_.size() / 3 >= cv);
+            bool stream = cv > 0 && ct > 0 && normals_mode() <= 1 && !refine_ && (!with_n || vertex_normals_.size() / 3 >= cv);
             if (stream) stream = pin(pin_v_, poly_data.vertex_list) && pin(pin_t_, poly_data.tri_list) && (!with_n || pin(pin_n_, vertex_normals_));
             mcb_set_host_output(ctx_, stream ? poly_data.vertex_list.data() : nullptr, stream ? poly_data.tri_list.data() : nullptr,
                                 stream && with_n ? vertex_normals_.data() : nullptr, stream ? cv : 0, stream ? ct : 0);
@@ -279,6 +279,10 @@ public:
     /* true: the equation's own gradient at every vertex, soup or welded (mcb_set_normals mode 3, DESIGN.md §12); takes
      * precedence over set_reference_normals.  false (default): as set_reference_normals says */
     void set_analytic_normals(bool b) { analytic_normals_ = b; }
+    /* true: every vertex, soup or welded, moved along its grid edge to the equation's root there (mcb_set_refine_vertices,
+     * DESIGN.md §13), on every context of set_devices; indices and counts unchanged.  false (default): the reference's
+     * linear interpolation */
+    void set_refined_vertices(bool b) { refine_ = b; }
     bool set_slab(int k_begin, int k_end) { slab_[0] = k_begin; slab_[1] = k_end; have_slab_ = true; return true; }
     const mcb_counts& last_counts() const { return counts_; }
     /* set_devices(n > 1): wall time of the phases of the last recalculate(), ms: the slabs' polygonisation (+ exchange),
@@ -329,6 +333,7 @@ private:
         mcb_set_surface_constant(c, iso_);
         mcb_set_scaling(c, sx_, sy_, sz_);
         mcb_set_normals(c, normals_mode());
+        mcb_set_refine_vertices(c, refine_ ? 1 : 0);
         /* marching.cpp:156-170, 481-494.  The reference accepts the mode with its initial distance 0: every cube's iso is
          * then NaN and nothing is drawn; recalculate() short-cuts that case, the GPU only sees positive distances */
         mcb_set_repeat(c, repeat_ && repeat_step_ > 0.f ? 1 : 0, repeat_step_);
@@ -535,6 +540,7 @@ private:
     bool weld_, normals_, seed_mode_, step_mode_, repeat_;
     bool reference_normals_ = false;
     bool analytic_normals_ = false;
+    bool refine_ = false;
     float repeat_step_;
     float seed_[3];
     bool cons_valid_[3], cons_use_[3];

@@ -204,6 +204,36 @@ int mcb_set_seed(mcb_ctx* ctx, int enabled, float x, float y, float z);
  * d = ux*ux + uy*uy + uz*uz, n = u * (1/sqrt(d)) (correctly rounded square root).  The normal points towards increasing f,
  * as mode 1's does.  Like mode 2, mode 3 is not streamed through mcb_set_host_output. */
 int mcb_set_normals(mcb_ctx* ctx, int mode);
+/* Refined vertices (DESIGN.md §13), off by default.  enabled != 0: every soup and welded vertex moves along its own grid edge
+ * to where the equation reaches the surface constant, found by a bracketed root search with the point program (fp32, no
+ * contraction, bit-identical on host and GPU).  Off, nothing changes.  Triangle indices and every count are those of the
+ * unrefined run: the weld decides topology from the unrefined points, then each welded vertex is refined from its own
+ * position.  Normals mode 2 and 3 are computed at the refined positions; mode 1 keeps the emitter's grid normal, blended
+ * along the edge at the unrefined point.  Not streamed through mcb_set_host_output (mcb_host_output_filled() returns 0;
+ * mcb_get_indexed_mesh delivers the refined mesh).  mcb_polygonise returns MCB_E_STATE together with repeating-surface
+ * mode, whose crossing points are extrapolated off their edges.  mcb_inspect_cube is not refined.
+ * A refined position is a function of the input position's bits, the point program, the surface constant, the scale and
+ * the grid's coordinate table c[0..M] only, not of the cube, mode or slab that produced it.  With f(p) = the point program
+ * at (sx*x, sy*y, sz*z), s(v) = v > iso (strict; NaN false) and |.| the absolute value of f - iso:
+ *   1 edge     locate each coordinate in c[0..M] by exact comparisons (binary search).  Exactly two must equal grid
+ *              coordinates and the third lie strictly inside some (c[i], c[i+1]), 0 <= i < M; otherwise p is unchanged
+ *              (a vertex on a grid vertex, anything off the grid).
+ *   2 bracket  a = c[i], b = c[i+1], f at both ends.  s(f(a)) == s(f(b)): p is unchanged (not met on a crossing edge).
+ *              The end with the smaller |.| is the first candidate (the lower one on a tie, a NaN one never wins); when
+ *              it has f == iso exactly the search stops there.
+ *   3 search   x = Marching::interp from a to b, t = (iso - f(a)) / (f(b) - f(a)): the edge's canonical linear point.
+ *              Each step: x not strictly inside (a, b), or NaN -> x = a + (b - a)*0.5f (the next float above a if that
+ *              is not inside); evaluate f(x); stop when f(x) == iso; x replaces the end with its side s(f(x)), its residual
+ *              ga or gb = f(x) - iso; when the same end is replaced twice in a row the other end's residual is halved
+ *              (Illinois).  Then stop when no float lies strictly between a and b, when b - a <= 2^-24 (absolute), or
+ *              after 40 evaluations in all (ends included, MCB_REFINE_EVALS).  Next x: the midpoint when b - a > 0.5 *
+ *              the width two steps earlier (the edge's width before the first step), else the secant point
+ *              a + (b - a)*(ga / (ga - gb)), moved to a + 2^-24 when it is closer than that to a (else to b - 2^-24 when
+ *              closer than that to b), so that once one side has converged the next point lands across the root.
+ *   4 result   the evaluated point with the smallest |.| (ends and every iterate; the earliest on a tie) replaces the
+ *              moving coordinate; the other two keep their bits.  So the refined point is never farther from the level,
+ *              in |.|, than the edge's linear point, and every cube sharing an edge gets the same bits. */
+int mcb_set_refine_vertices(mcb_ctx* ctx, int enabled);
 
 /* The hot path: Marching::recalculate() (marching.cpp:368-384) for this context's slab, entirely on the GPU.
  * On return the triangle soup is resident in device memory in the reference's emission order (cube loop order
@@ -283,8 +313,8 @@ int mcb_get_indexed_mesh_device(mcb_ctx* ctx, const float** vertex_list, const u
  * registered, mcb_polygonise in MCB_MESH_INDEXED mode streams vertex_list / normals / tri_list out range by range
  * while the later ranges are still being produced, and returns when the mesh is on the host — one call, like
  * Marching::recalculate() filling Poly_Data.  normals may be NULL when normals are off.  When a device buffer has to
- * grow first, the mesh does not fit the registered capacities, or normals mode 2 or 3 is on, nothing is
- * streamed: mcb_host_output_filled() returns 0 and mcb_get_indexed_mesh delivers the mesh.  NULL pointers unregister. */
+ * grow first, the mesh does not fit the registered capacities, normals mode 2 or 3 is on, or refined vertices are on,
+ * nothing is streamed: mcb_host_output_filled() returns 0 and mcb_get_indexed_mesh delivers the mesh.  NULL pointers unregister. */
 int mcb_set_host_output(mcb_ctx* ctx, float* vertex_list, uint32_t* tri_list, float* normals, uint64_t cap_vertices,
                         uint64_t cap_triangles);
 int mcb_host_output_filled(const mcb_ctx* ctx);

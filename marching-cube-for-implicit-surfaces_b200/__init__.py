@@ -88,6 +88,7 @@ def _load():
         "mcb_set_scaling": ([vp, f, f, f], i),
         "mcb_set_constraint": ([vp, i, i, f, i], i),
         "mcb_set_normals": ([vp, i], i),
+        "mcb_set_refine_vertices": ([vp, i], i),
         "mcb_set_seed": ([vp, i, f, f, f], i),
         "mcb_set_repeat": ([vp, i, f], i),
         "mcb_inspect_cube": ([vp, f, f, f, C.POINTER(StepData)], i),
@@ -303,6 +304,11 @@ class Context:
 
     def set_normals(self, mode):
         self._ck(lib.mcb_set_normals(self.h, int(mode)))
+
+    def set_refine_vertices(self, enabled):
+        """Refined vertices (include/mcb.h, DESIGN.md §13): every soup and welded vertex moved along its grid edge to where
+        the equation reaches the surface constant; indices and counts unchanged.  Off by default."""
+        self._ck(lib.mcb_set_refine_vertices(self.h, int(bool(enabled))))
 
     def inspect_cube(self, x0, y0, z0):
         """Marching::calculate_step(x0, y0, z0) for one cube, on the GPU."""
@@ -584,6 +590,10 @@ class Marching:
     def set_normals(self, mode):
         self._normals = bool(mode)
         self._ctx.set_normals(mode)
+
+    def set_refined_vertices(self, b):
+        """Extension: include/marching.h Marching::set_refined_vertices (Context.set_refine_vertices)."""
+        self._ctx.set_refine_vertices(b)
 
     def recalculate(self, fetch=True):
         if self._eval is None:

@@ -63,6 +63,7 @@ struct mcb_ctx {
     float iso = 0.f;
     float scale[3] = {1.f, 1.f, 1.f};
     int normals = 1;
+    bool refine = false; /* mcb_set_refine_vertices */
 
     Grid g{};
     bool grid_dirty = true;
@@ -813,6 +814,13 @@ int mcb_set_normals(mcb_ctx* ctx, int mode) {
     return MCB_OK;
 }
 
+int mcb_set_refine_vertices(mcb_ctx* ctx, int enabled) {
+    if (!ctx) return MCB_E_ARG;
+    ctx->refine = enabled != 0;
+    ctx->have_result = false;
+    return MCB_OK;
+}
+
 } /* extern "C" */
 
 namespace {
@@ -845,6 +853,7 @@ struct Run {
     int stage_weld();
     int stage_normal_h();
     int stage_grad_normals(bool soup);
+    int stage_refine(bool soup);
 };
 
 int Run::prepare_buffers() {
@@ -1361,7 +1370,7 @@ int Run::stage_weld() {
     /* streaming: with a registered host destination and everything fitting, weld_emit runs range by range and
      * each finished range of vertices / normals / triangles leaves over PCIe on the copy stream meanwhile */
     constexpr int K = 8;
-    bool stream_out = ctx->h_out_v && ctx->h_out_t && ctx->normals <= 1 && (ctx->normals == 0 || ctx->h_out_n);
+    bool stream_out = ctx->h_out_v && ctx->h_out_t && ctx->normals <= 1 && (ctx->normals == 0 || ctx->h_out_n) && !ctx->refine;
     ctx->streamed = false;
     if (stream_out) {
         MCB_LAUNCH((weld_bounds_kernel), 1, 32, 0, s, B, ctx->d_ctr, ctx->cap_active, K, ctx->d_bounds);
@@ -1436,6 +1445,21 @@ int Run::stage_grad_normals(bool soup) {
     return MCB_OK;
 }
 
+/* Refined vertices (mcb_set_refine_vertices): every soup or welded vertex moved to the equation's root along its grid edge,
+ * after the emitter / weld and before any normals pass that reads the positions */
+int Run::stage_refine(bool soup) {
+    const unsigned grid = (unsigned)ctx->sm_count * 8;
+    const float* c = ctx->d_cs + 1; /* cs[v+1] = c[v] */
+    if (soup)
+        MCB_LAUNCH((refine_vertices_kernel<true>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, g.iso, c, g.M, ctx->d_ctr, ctx->cap_tris,
+                   (float*)ctx->d_pos);
+    else
+        MCB_LAUNCH((refine_vertices_kernel<false>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, g.iso, c, g.M, ctx->d_ctr, ctx->cap_verts,
+                   ctx->d_vlist);
+    launches++;
+    return MCB_OK;
+}
+
 } /* namespace */
 
 extern "C" {
@@ -1455,6 +1479,8 @@ int mcb_polygonise(mcb_ctx* ctx, mcb_counts* out) {
         return fail(ctx, MCB_E_STATE, "seed mode follows one component through the whole grid: it cannot be combined with z-slabs over several GPUs");
     if (ctx->normals == 2 && !(ctx->mesh_mode & MCB_MESH_INDEXED))
         return fail(ctx, MCB_E_STATE, "normal.h normals (mode 2) are defined on the welded mesh: request MCB_MESH_INDEXED");
+    if (ctx->refine && ctx->repeat_on) /* the reference extrapolates those crossing points: they are not on their edges */
+        return fail(ctx, MCB_E_STATE, "refined vertices cannot be combined with repeating-surface mode");
 
     Run run{ctx, g, ctx->eq[0], ctx->stream, false, (ctx->mesh_mode & MCB_MESH_SOUP) != 0, (ctx->mesh_mode & MCB_MESH_INDEXED) != 0,
             nullptr, ClsGeom{}, 0u, (unsigned)ctx->sm_count * 4, 0u};
@@ -1493,10 +1519,12 @@ int mcb_polygonise(mcb_ctx* ctx, mcb_counts* out) {
             if (timing) MCB_CK(cudaEventRecord(ctx->ev[3], s));
         }
         if (run.want_soup && (rc = run.stage_soup()) != MCB_OK) return rc;
+        if (run.want_soup && ctx->refine && (rc = run.stage_refine(true)) != MCB_OK) return rc;
         if (run.want_soup && ctx->normals == 3 && (rc = run.stage_grad_normals(true)) != MCB_OK) return rc;
         if (timing) MCB_CK(cudaEventRecord(ctx->ev[4], s));
         if (run.want_indexed) {
             if ((rc = run.stage_weld()) != MCB_OK) return rc;
+            if (ctx->refine && (rc = run.stage_refine(false)) != MCB_OK) return rc;
             if (ctx->normals == 2 && (rc = run.stage_normal_h()) != MCB_OK) return rc;
             if (ctx->normals == 3 && (rc = run.stage_grad_normals(false)) != MCB_OK) return rc;
         }

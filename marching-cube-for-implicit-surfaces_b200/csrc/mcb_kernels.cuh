@@ -37,6 +37,7 @@
 #include "mcb_bytecode.h"
 #include "mcb_interval.h"
 #include "mcb_launch.h"
+#include "mcb_refine.h"
 #include "mcb_tables.h"
 
 namespace mcbk {
@@ -1328,14 +1329,6 @@ __device__ __forceinline__ void blend_edge_normal(bool fwd, float iso, float f1,
     nz = lz + tt * (hz - lz);
 }
 
-__device__ __forceinline__ float interp_ref(float xs, float xe, float t) {
-    /* Marching::interp, marching.cpp:437-446, with t = (c - v_s) / (v_e - v_s) computed once: the reference calls it
-     * three times per edge with the same field values, so the quotient has the same bits every time */
-    const float v = t * (xe - xs);
-    if (isinf(v) || isnan(v)) return (float)((double)xs + 0.5 * (double)(xe - xs));
-    return xs + v;
-}
-
 template <bool NORMALS, bool IDX32 /* the slab's field has fewer than 2^32 values: 32-bit offsets, one IMAD.WIDE per load address */>
 __global__ void __launch_bounds__(kEmitThreads, kEmitBlocksPerSM)
 emit2_kernel(const Grid g, const float* __restrict__ cs, const float* __restrict__ rinv, const float* __restrict__ F,
@@ -1445,7 +1438,7 @@ emit2_kernel(const Grid g, const float* __restrict__ cs, const float* __restrict
                 const float ca = cc[(oa >> axis) & 1], cb2 = cc[(ob >> axis) & 1];
                 const float f1 = __ldg(F + ia), f2 = __ldg(F + ib);
                 const float tq = (g.iso - f1) / (f2 - f1); /* Marching::interp uses the surface constant itself, also in repeating-surface mode */
-                const float p = interp_ref(ca, cb2, tq);
+                const float p = mcb_interp_ref(ca, cb2, tq);
                 if (NORMALS) { /* central differences times the reciprocals kept in shared memory, blended along the grid edge */
                     const float* ri = crinv + 6 * lc;
                     const float gxa = (__ldg(F + ia + 1) - __ldg(F + ia - 1)) * ri[oa & 1];
@@ -1595,7 +1588,7 @@ __device__ __forceinline__ float weld_edge_point(const WV& W, const CubeEdge& c,
     crossing = (f1 > level) != (f2 > level);
     const int base = (axis == 0 ? c.i : axis == 1 ? c.j : c.k) + 1;
     const float ca = W.cs[base + ((oa >> axis) & 1)], cb = W.cs[base + ((ob >> axis) & 1)];
-    return interp_ref(ca, cb, (g.iso - f1) / (f2 - f1)); /* Marching::interp (marching.cpp:437-446) always uses the surface constant */
+    return mcb_interp_ref(ca, cb, (g.iso - f1) / (f2 - f1)); /* Marching::interp (marching.cpp:437-446) always uses the surface constant */
 }
 __device__ __forceinline__ bool weld_close(float a, float b) { return (double)fabsf(a - b) < 0.000001; } /* marching.h:41 */
 __device__ __forceinline__ unsigned long long weld_key(const Grid& g, const CubeEdge& c) {
@@ -1648,8 +1641,8 @@ __device__ __noinline__ CubeEdge weld_replay(const WV& W, const int G[3], unsign
             const float fl = __ldg(fp), fu = __ldg(fp + (ax == 0 ? (size_t)1 : ax == 1 ? rowp : planep));
             if ((fl > iso) == (fu > iso)) continue;
             const float cl = W.cs[lo_idx], cu = W.cs[lo_idx + 1];
-            const float pf = interp_ref(cl, cu, (g.iso - fl) / (fu - fl)); /* cube edge running lower -> upper */
-            const float pb = interp_ref(cu, cl, (g.iso - fu) / (fl - fu)); /* cube edge running upper -> lower */
+            const float pf = mcb_interp_ref(cl, cu, (g.iso - fl) / (fu - fl)); /* cube edge running lower -> upper */
+            const float pb = mcb_interp_ref(cu, cl, (g.iso - fu) / (fl - fu)); /* cube edge running upper -> lower */
             for (int q = 0; q < 4; q++) {
                 const int hi = 1 - (q >> 1), lo = 1 - (q & 1);
                 CubeEdge o;
@@ -2056,9 +2049,9 @@ weld_emit_kernel(const WV W, const WeldBuffers B, const Counters* __restrict__ c
                     const float f1 = __ldg(pa), f2 = __ldg(pb);
                     const float tq = (g.iso - f1) / (f2 - f1);
                     float* out = vertex_list + 3ull * idx;
-                    out[0] = interp_ref(W.cs[xa], W.cs[xb], tq);
-                    out[1] = interp_ref(W.cs[ya], W.cs[yb], tq);
-                    out[2] = interp_ref(W.cs[za], W.cs[zb], tq);
+                    out[0] = mcb_interp_ref(W.cs[xa], W.cs[xb], tq);
+                    out[1] = mcb_interp_ref(W.cs[ya], W.cs[yb], tq);
+                    out[2] = mcb_interp_ref(W.cs[za], W.cs[zb], tq);
                     if (NORMALS) { /* central differences with IEEE divisions, blended along the grid edge, normalised by 1 / sqrtf */
                         const float* cs = W.cs;
                         const float gxa = (__ldg(pa + 1) - __ldg(pa - 1)) / (cs[xa + 1] - cs[xa - 1]);
@@ -2428,9 +2421,9 @@ __global__ void inspect_cube_kernel(const mcb_program* __restrict__ progs /* [0]
                 const float t = (iso - o.corner_values[a]) / (o.corner_values[b] - o.corner_values[a]);
                 mapper[e] = o.n_edges;
                 o.edge_list[o.n_edges] = e;
-                o.intersect_coord[3 * o.n_edges] = interp_ref(cc[3 * a], cc[3 * b], t);
-                o.intersect_coord[3 * o.n_edges + 1] = interp_ref(cc[3 * a + 1], cc[3 * b + 1], t);
-                o.intersect_coord[3 * o.n_edges + 2] = interp_ref(cc[3 * a + 2], cc[3 * b + 2], t);
+                o.intersect_coord[3 * o.n_edges] = mcb_interp_ref(cc[3 * a], cc[3 * b], t);
+                o.intersect_coord[3 * o.n_edges + 1] = mcb_interp_ref(cc[3 * a + 1], cc[3 * b + 1], t);
+                o.intersect_coord[3 * o.n_edges + 2] = mcb_interp_ref(cc[3 * a + 2], cc[3 * b + 2], t);
                 o.n_edges++;
             }
             const uint64_t row = gtb->tri[o.table_idx];
@@ -2551,6 +2544,32 @@ grad_normals_kernel(const __grid_constant__ mcb_program prog, float sx, float sy
         mcb_grad_normalise(gr, o);
         if (SOUP) reinterpret_cast<float4*>(nrm)[q] = make_float4(o[0], o[1], o[2], 0.f);
         else { nrm[3 * q] = o[0]; nrm[3 * q + 1] = o[1]; nrm[3 * q + 2] = o[2]; }
+    }
+}
+
+/* Refined vertices (mcb_set_refine_vertices): every output vertex strictly inside a grid edge moves, in place, to the root
+ * of the point program along that edge (mcb_refine_vertex, mcb_refine.h), after the emitter (SOUP: float4 (x,y,z,1), 3
+ * per triangle, w kept) or the weld (float3).  cs = the coordinate table c[0..M].  The element count comes from the device
+ * counters, capped by the buffer, so the pass needs no host synchronisation and runs again in a repeated pass. */
+template <bool SOUP>
+__global__ void __launch_bounds__(256)
+refine_vertices_kernel(const __grid_constant__ mcb_program prog, float sx, float sy, float sz, float iso, const float* __restrict__ cs,
+                       int M, const Counters* __restrict__ ctr, unsigned long long cap, float* __restrict__ pos) {
+    unsigned long long n = SOUP ? ctr->triangles : ctr->vertices;
+    if (n > cap) n = cap;
+    if (SOUP) n *= 3;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long q = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += stride) {
+        float p[3];
+        if (SOUP) {
+            const float4 v = reinterpret_cast<const float4*>(pos)[q];
+            p[0] = v.x; p[1] = v.y; p[2] = v.z;
+        } else {
+            p[0] = pos[3 * q]; p[1] = pos[3 * q + 1]; p[2] = pos[3 * q + 2];
+        }
+        if (mcb_refine_vertex(prog.code, prog.n, prog.k, cs, M, iso, sx, sy, sz, p, nullptr) <= 0) continue;
+        if (SOUP) reinterpret_cast<float4*>(pos)[q] = make_float4(p[0], p[1], p[2], 1.f);
+        else { pos[3 * q] = p[0]; pos[3 * q + 1] = p[1]; pos[3 * q + 2] = p[2]; }
     }
 }
 

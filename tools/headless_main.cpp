@@ -9,6 +9,7 @@
 //                [--functions]   (equations and constraints may use sin( cos( sqrt( abs( min( max(: Evaluator::set_function_grammar)
 //                [--analytic-normals]   (normals from the equation's own gradient: Marching::set_analytic_normals)
 //                [--dump-normals out.bin]   (the welded vertex normals, nv*3 f32, or the soup's 3 float4 per triangle)
+//                [--refine-vertices]   (every vertex moved to the equation's root on its grid edge: Marching::set_refined_vertices)
 //
 // Defaults are the reference GUI's (drawer.cpp:39-44): equation "x+y", grid 0.2, scale 1.1, iso 0.
 #include <chrono>
@@ -22,7 +23,7 @@
 static int usage() {
     std::fprintf(stderr, "usage: mcb_headless [--eq S | --eq-file F] [--step h | --res n] [--scale sx sy sz] [--iso c]\n"
                          "                    [--constraint i lhs op rhs] [--no-normals] [--soup] [--ply F] [--dump F] [--repeat n] [--levels d] [--devices n]\n"
-                         "                    [--functions] [--analytic-normals] [--dump-normals F]\n");
+                         "                    [--functions] [--analytic-normals] [--dump-normals F] [--refine-vertices]\n");
     return 2;
 }
 
@@ -58,6 +59,7 @@ int main(int argc, char** argv) {
         } else if (o == "--functions") continue;
         else if (o == "--no-normals") march_maker.set_normals(false);
         else if (o == "--analytic-normals") march_maker.set_analytic_normals(true);
+        else if (o == "--refine-vertices") march_maker.set_refined_vertices(true);
         else if (o == "--soup") march_maker.set_weld(false);
         else if (o == "--ply" && need(1)) ply = argv[++a];
         else if (o == "--dump" && need(1)) dump = argv[++a];
