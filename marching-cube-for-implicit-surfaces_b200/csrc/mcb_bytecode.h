@@ -8,7 +8,8 @@
  * order while each value keeps its role.  All arithmetic is fp32 without FMA contraction; `^` is mcb_powf.
  * The function grammar's unary operators: sin / cos are mcb_sinf / mcb_cosf (mcb_trig.h, glibc's sinf / cosf), sqrt is
  * the correctly rounded square root (sqrtf on the host, __fsqrt_rn on the device), abs clears the sign bit.
- * Its two-argument functions min / max are mcb_minf / mcb_maxf below (IEEE 754-2019 minimumNumber / maximumNumber).
+ * Its two-argument functions min / max are mcb_min / mcb_max below (IEEE 754-2019 minimumNumber / maximumNumber).
+ * Every operation is written once, in the operator table below.
  *
  * Programs travel to the kernels inside the kernel-parameter block, i.e. in the constant bank: every lane of a
  * warp executes the same instruction word, fetched with a uniform constant load.
@@ -16,7 +17,7 @@
 #ifndef MCB_BYTECODE_H
 #define MCB_BYTECODE_H
 
-#if !defined(__CUDACC_RTC__) /* the run-time compiled kernels include this file for mcb_minf / mcb_maxf */
+#if !defined(__CUDACC_RTC__) /* the run-time compiled kernels include this file for mcb_min / mcb_max */
 #include <stdint.h>
 #endif
 
@@ -69,100 +70,20 @@ typedef struct {
 
 #if defined(__CUDACC__)
 #define MCB_BC_FN __host__ __device__ __forceinline__
+#define MCB_BC_MEMBER __host__ __device__ __forceinline__
+#define MCB_BC_NOINLINE static __host__ __device__ __noinline__
 #else
 #define MCB_BC_FN static inline
+#define MCB_BC_MEMBER inline
+#define MCB_BC_NOINLINE static
 #endif
 
-/* min and max of the function grammar: IEEE 754-2019 minimumNumber / maximumNumber.  A NaN operand is ignored (two NaNs
- * give the canonical quiet NaN), -0 < +0, otherwise the smaller / larger operand exactly.  Both are commutative bit for
- * bit, so the lowering may order their operands freely.  Explicit compares and selects, not fminf / fmaxf: C leaves the
- * sign of a zero result of fmin to the implementation.  One source for g++, nvcc and NVRTC (mcb_jit.cpp). */
-MCB_BC_FN float mcb_minf(float a, float b) {
-    const int na = a != a, nb = b != b;
-    if (na || nb) return na && nb ? mcb_u2f(0x7fc00000u) : na ? b : a;
-    if (a == b) return mcb_u2f(mcb_f2u(a) | mcb_f2u(b)); /* equal bits, or +0 and -0: -0 */
-    return a < b ? a : b;
-}
-MCB_BC_FN float mcb_maxf(float a, float b) {
-    const int na = a != a, nb = b != b;
-    if (na || nb) return na && nb ? mcb_u2f(0x7fc00000u) : na ? b : a;
-    if (a == b) return mcb_u2f(mcb_f2u(a) & mcb_f2u(b)); /* equal bits, or +0 and -0: +0 */
-    return a > b ? a : b;
-}
-
-MCB_BC_FN float mcb_binop(uint32_t op, float second, float top) {
-    switch (op) {
-        case MCB_OP_ADD: return second + top;
-        case MCB_OP_SUB: return second - top;
-        case MCB_OP_RSUB: return top - second;
-        case MCB_OP_MUL: return second * top;
-        case MCB_OP_DIV: return second / top;
-        case MCB_OP_RDIV: return top / second;
-        case MCB_OP_POW: return mcb_powf(second, top);
-        case MCB_OP_MIN: return mcb_minf(second, top);
-        case MCB_OP_MAX: return mcb_maxf(second, top);
-        default: return mcb_powf(top, second); /* MCB_OP_RPOW */
-    }
-}
-
-/* The function grammar's functions, fn = 0 sin, 1 cos, 2 sqrt, 3 abs.  Out of line: the scalar interpreters call it
- * rarely and should not carry the inlined fp64 trigonometry in every kernel that interprets a program. */
-#if defined(__CUDACC__)
-static __host__ __device__ __noinline__
-#else
-static
-#endif
-float mcb_fn(uint32_t fn, float v) {
-    switch (fn) {
-        case 0: return mcb_sinf(v);
-        case 1: return mcb_cosf(v);
-        case 2:
-#if defined(__CUDA_ARCH__)
-            return __fsqrt_rn(v);
-#else
-            return sqrtf(v);
-#endif
-        default: return mcb_u2f(mcb_f2u(v) & 0x7fffffffu);
-    }
-}
-
-/* Plain scalar interpreter: one point, memory stack.  Used for the rare, divergent evaluations (ambiguity face
- * centres, mcb_eval_points, constant folding, axis tables); the per-vertex grid kernel has its own register-cached
- * version.  tx/ty/tz = this point's table values per slot (may be NULL when the program has no table loads). */
-MCB_BC_FN float mcb_interp_scalar(const uint32_t* code, int n, const float* k, float x, float y, float z,
-                                  const float* tx, const float* ty, const float* tz) {
-    float st[MCB_MAX_STACK];
-    int sp = 0;
-    for (int pc = 0; pc < n; pc++) {
-        uint32_t w = code[pc], op = MCB_INSN_OP(w), arg = MCB_INSN_ARG(w);
-        switch (op) {
-            case MCB_OP_PUSH_X: st[sp++] = x; break;
-            case MCB_OP_PUSH_Y: st[sp++] = y; break;
-            case MCB_OP_PUSH_Z: st[sp++] = z; break;
-            case MCB_OP_PUSH_K: st[sp++] = k[arg]; break;
-            case MCB_OP_PUSH_TX: st[sp++] = tx[arg]; break;
-            case MCB_OP_PUSH_TY: st[sp++] = ty[arg]; break;
-            case MCB_OP_PUSH_TZ: st[sp++] = tz[arg]; break;
-            case MCB_OP_NEG: st[sp - 1] = -st[sp - 1]; break;
-            case MCB_OP_SIN: case MCB_OP_COS: case MCB_OP_SQRT: case MCB_OP_ABS:
-                st[sp - 1] = mcb_fn(op - MCB_OP_SIN, st[sp - 1]);
-                break;
-            case MCB_OP_END: pc = n; break;
-            default: {
-                float top = st[--sp];
-                st[sp - 1] = mcb_binop(op, st[sp - 1], top);
-            }
-        }
-    }
-    return st[0];
-}
-
-/* ---- analytic normals (mcb_set_normals 3, mcb_eval_gradients) ---------------------------------------------------
- * Forward-mode differentiation of a point program: every stack entry is a dual number, a value and its three partials
- * with respect to the unscaled coordinates.  The value part runs exactly the operations of mcb_interp_scalar, so its bits
- * are those of mcb_eval_points.  The partials follow one fixed fp32 rule per operation of the equation, in the order
- * written, with a the left and b the right operand whatever stack order the lowering chose (the reversed forms swap them
- * back), so the gradient is a function of the operation graph alone:
+/* ---- the operator table ---------------------------------------------------------------------------------------------
+ * Every operation of the grammar, written once for two scalar types, in one source for g++, nvcc and NVRTC (mcb_jit.cpp):
+ *   float     the value that every interpreter computes, on the host and on the device;
+ *   mcb_dual  a value and its three partials with respect to the unscaled coordinates (analytic normals: mcb_set_normals 3,
+ *             mcb_eval_gradients).  Each dual rule computes its value with the float rule above it, so the value part of
+ *             a dual evaluation has the bits of the plain one, then the partials by one fixed fp32 rule:
  *      x, y, z  (sx,0,0) (0,sy,0) (0,0,sz)          constant  0
  *      a+b, a-b ga+-gb                              a*b       ga*b + a*gb
  *      a/b      (ga - q*gb) / b, q = a/b            -a        -ga
@@ -171,9 +92,63 @@ MCB_BC_FN float mcb_interp_scalar(const uint32_t* code, int n, const float* k, f
  *      abs a    sign bit of a set ? -ga : ga
  *      min, max the gradient of the operand whose bits equal the result; (ga+gb)*0.5f when both or neither do
  *               (symmetric, so the free operand order of min / max cannot change a bit)
- * Point programs use no axis tables. */
+ * a is the left and b the right operand as the equation writes them: mcb_binop undoes the reversed stack forms, so a
+ * gradient is a function of the operation graph alone.  All arithmetic is fp32 without FMA contraction (nvcc -fmad=false,
+ * g++ -ffp-contract=off). */
+struct mcb_dual {
+    float v, g[3];
+    mcb_dual() = default;
+    MCB_BC_MEMBER explicit mcb_dual(float c) : v(c), g{0.f, 0.f, 0.f} {} /* a constant */
+    MCB_BC_MEMBER mcb_dual(float c, float gx, float gy, float gz) : v(c), g{gx, gy, gz} {}
+};
 
-/* ln x for the x^y rule: mcb_powf_full's fp64 log2 times ln 2, rounded once.  NaN for x <= 0 or NaN, +inf for +inf. */
+MCB_BC_FN mcb_dual operator+(mcb_dual a, mcb_dual b) {
+    mcb_dual r;
+    r.v = a.v + b.v;
+    for (int c = 0; c < 3; c++) r.g[c] = a.g[c] + b.g[c];
+    return r;
+}
+MCB_BC_FN mcb_dual operator-(mcb_dual a, mcb_dual b) {
+    mcb_dual r;
+    r.v = a.v - b.v;
+    for (int c = 0; c < 3; c++) r.g[c] = a.g[c] - b.g[c];
+    return r;
+}
+MCB_BC_FN mcb_dual operator*(mcb_dual a, mcb_dual b) {
+    mcb_dual r;
+    r.v = a.v * b.v;
+    for (int c = 0; c < 3; c++) r.g[c] = a.g[c] * b.v + a.v * b.g[c];
+    return r;
+}
+MCB_BC_FN mcb_dual operator/(mcb_dual a, mcb_dual b) {
+    mcb_dual r;
+    r.v = a.v / b.v;
+    for (int c = 0; c < 3; c++) r.g[c] = (a.g[c] - r.v * b.g[c]) / b.v;
+    return r;
+}
+MCB_BC_FN mcb_dual operator-(mcb_dual a) {
+    mcb_dual r;
+    r.v = -a.v;
+    for (int c = 0; c < 3; c++) r.g[c] = -a.g[c];
+    return r;
+}
+/* the chain rule of a function of one dual: value v, partials d * ga */
+MCB_BC_FN mcb_dual mcb_chain(float v, float d, mcb_dual a) {
+    mcb_dual r;
+    r.v = v;
+    for (int c = 0; c < 3; c++) r.g[c] = d * a.g[c];
+    return r;
+}
+
+/* a^b is mcb_powf.  x^2 takes the exact fp32 fast path inline; the fp64 algorithm is out of line, one copy per module, so
+ * the grid kernels keep their registers and every kernel that interprets a program does not carry it inlined. */
+MCB_BC_NOINLINE float mcb_pow_call(float a, float b) { return mcb_powf(a, b); }
+MCB_BC_FN float mcb_pow(float a, float b) {
+    float r;
+    if (mcb_f2u(b) == 0x40000000u && mcb_pow2_try(a, &r)) return r;
+    return mcb_pow_call(a, b);
+}
+/* ln x for the a^b rule: mcb_powf_full's fp64 log2 times ln 2, rounded once.  NaN for x <= 0 or NaN, +inf for +inf. */
 MCB_BC_FN float mcb_lnf(float x) {
     uint32_t ix = mcb_f2u(x);
     if (!(x > 0.f)) return mcb_u2f(0x7fc00000u);
@@ -184,93 +159,156 @@ MCB_BC_FN float mcb_lnf(float x) {
     }
     return (float)(mcb_pow_log2(ix) * mcb_u2d(0x3fe62e42fefa39efull) /* ln 2 */);
 }
+MCB_BC_FN mcb_dual mcb_pow(mcb_dual a, mcb_dual b) {
+    const float v = mcb_pow(a.v, b.v);
+    if (b.g[0] == 0.f && b.g[1] == 0.f && b.g[2] == 0.f) return mcb_chain(v, b.v * mcb_pow(a.v, b.v - 1.f), a);
+    mcb_dual r;
+    r.v = v;
+    const float la = mcb_lnf(a.v), ba = b.v / a.v;
+    for (int c = 0; c < 3; c++) r.g[c] = v * (la * b.g[c] + ba * a.g[c]);
+    return r;
+}
 
-MCB_BC_FN float mcb_interp_grad_scalar(const uint32_t* code, int n, const float* k, float x, float y, float z,
-                                       float sx, float sy, float sz, float g[3]) {
-    float st[MCB_MAX_STACK], gs[MCB_MAX_STACK][3];
+/* min and max: IEEE 754-2019 minimumNumber / maximumNumber.  A NaN operand is ignored (two NaNs give the canonical quiet
+ * NaN), -0 < +0, otherwise the smaller / larger operand exactly.  Both are commutative bit for bit, so the lowering may
+ * order their operands freely.  Explicit compares and selects, not fminf / fmaxf: C leaves the sign of a zero result of
+ * fmin to the implementation.  The interval bounds (mcb_interval.h) and the run-time compiled kernels use them too. */
+MCB_BC_FN float mcb_min(float a, float b) {
+    const int na = a != a, nb = b != b;
+    if (na || nb) return na && nb ? mcb_u2f(0x7fc00000u) : na ? b : a;
+    if (a == b) return mcb_u2f(mcb_f2u(a) | mcb_f2u(b)); /* equal bits, or +0 and -0: -0 */
+    return a < b ? a : b;
+}
+MCB_BC_FN float mcb_max(float a, float b) {
+    const int na = a != a, nb = b != b;
+    if (na || nb) return na && nb ? mcb_u2f(0x7fc00000u) : na ? b : a;
+    if (a == b) return mcb_u2f(mcb_f2u(a) & mcb_f2u(b)); /* equal bits, or +0 and -0: +0 */
+    return a > b ? a : b;
+}
+/* the partials of min / max, whose value is v */
+MCB_BC_FN mcb_dual mcb_minmax_grad(float v, mcb_dual a, mcb_dual b) {
+    mcb_dual r;
+    r.v = v;
+    const bool ma = mcb_f2u(a.v) == mcb_f2u(v), mb = mcb_f2u(b.v) == mcb_f2u(v);
+    for (int c = 0; c < 3; c++) r.g[c] = ma && !mb ? a.g[c] : mb && !ma ? b.g[c] : (a.g[c] + b.g[c]) * 0.5f;
+    return r;
+}
+MCB_BC_FN mcb_dual mcb_min(mcb_dual a, mcb_dual b) { return mcb_minmax_grad(mcb_min(a.v, b.v), a, b); }
+MCB_BC_FN mcb_dual mcb_max(mcb_dual a, mcb_dual b) { return mcb_minmax_grad(mcb_max(a.v, b.v), a, b); }
+
+/* sin / cos: mcb_sinf / mcb_cosf (mcb_trig.h, glibc's sinf / cosf), out of line for the reason mcb_pow_call is */
+MCB_BC_NOINLINE float mcb_sin(float a) { return mcb_sinf(a); }
+MCB_BC_NOINLINE float mcb_cos(float a) { return mcb_cosf(a); }
+MCB_BC_FN mcb_dual mcb_sin(mcb_dual a) { return mcb_chain(mcb_sin(a.v), mcb_cos(a.v), a); }
+MCB_BC_FN mcb_dual mcb_cos(mcb_dual a) { return mcb_chain(mcb_cos(a.v), -mcb_sin(a.v), a); }
+
+/* sqrt: correctly rounded on both sides (the device spells it as the intrinsic, so no compile flag can change it) */
+MCB_BC_FN float mcb_sqrt(float a) {
+#if defined(__CUDA_ARCH__)
+    return __fsqrt_rn(a);
+#else
+    return sqrtf(a);
+#endif
+}
+MCB_BC_FN mcb_dual mcb_sqrt(mcb_dual a) {
+    mcb_dual r;
+    r.v = mcb_sqrt(a.v);
+    const float d = r.v + r.v;
+    for (int c = 0; c < 3; c++) r.g[c] = a.g[c] / d;
+    return r;
+}
+
+/* abs clears the sign bit */
+MCB_BC_FN float mcb_abs(float a) { return mcb_u2f(mcb_f2u(a) & 0x7fffffffu); }
+MCB_BC_FN mcb_dual mcb_abs(mcb_dual a) {
+    mcb_dual r = a;
+    r.v = mcb_abs(a.v);
+    if (mcb_f2u(a.v) >> 31)
+        for (int c = 0; c < 3; c++) r.g[c] = -a.g[c];
+    return r;
+}
+
+/* The postfix opcodes on the table: a binary opcode with the operand stack's second and top entries, a unary one with
+ * the top */
+template <typename T>
+MCB_BC_FN T mcb_binop(uint32_t op, T second, T top) {
+    switch (op) {
+        case MCB_OP_ADD: return second + top;
+        case MCB_OP_SUB: return second - top;
+        case MCB_OP_RSUB: return top - second;
+        case MCB_OP_MUL: return second * top;
+        case MCB_OP_DIV: return second / top;
+        case MCB_OP_RDIV: return top / second;
+        case MCB_OP_POW: return mcb_pow(second, top);
+        case MCB_OP_MIN: return mcb_min(second, top);
+        case MCB_OP_MAX: return mcb_max(second, top);
+        default: return mcb_pow(top, second); /* MCB_OP_RPOW */
+    }
+}
+template <typename T>
+MCB_BC_FN T mcb_unop(uint32_t op, T a) {
+    switch (op) {
+        case MCB_OP_NEG: return -a;
+        case MCB_OP_SIN: return mcb_sin(a);
+        case MCB_OP_COS: return mcb_cos(a);
+        case MCB_OP_SQRT: return mcb_sqrt(a);
+        default: return mcb_abs(a); /* MCB_OP_ABS */
+    }
+}
+
+/* Point interpreter: one point, memory stack, on the scalar type T (never deduced: a caller's integer 0 must not turn the
+ * interpreter into integer arithmetic).  tx/ty/tz = this point's table values per slot (may be NULL when the program has
+ * no table loads). */
+template <typename T>
+MCB_BC_FN T mcb_interp_point(const uint32_t* code, int n, const float* k, T x, T y, T z,
+                             const float* tx, const float* ty, const float* tz) {
+    T st[MCB_MAX_STACK];
     int sp = 0;
     for (int pc = 0; pc < n; pc++) {
-        const uint32_t w = code[pc], op = MCB_INSN_OP(w), arg = MCB_INSN_ARG(w);
-        if (op == MCB_OP_END) break;
-        if (op <= MCB_OP_PUSH_K) {
-            st[sp] = op == MCB_OP_PUSH_X ? x : op == MCB_OP_PUSH_Y ? y : op == MCB_OP_PUSH_Z ? z : k[arg];
-            gs[sp][0] = op == MCB_OP_PUSH_X ? sx : 0.f;
-            gs[sp][1] = op == MCB_OP_PUSH_Y ? sy : 0.f;
-            gs[sp][2] = op == MCB_OP_PUSH_Z ? sz : 0.f;
-            sp++;
-            continue;
-        }
-        if (MCB_OP_IS_UNARY(op)) {
-            const float a = st[sp - 1];
-            float* ga = gs[sp - 1];
-            if (op == MCB_OP_NEG) {
-                st[sp - 1] = -a;
-                for (int c = 0; c < 3; c++) ga[c] = -ga[c];
-            } else {
-                const float v = mcb_fn(op - MCB_OP_SIN, a);
-                st[sp - 1] = v;
-                if (op == MCB_OP_SIN || op == MCB_OP_COS) {
-                    const float d = op == MCB_OP_SIN ? mcb_fn(1, a) : -mcb_fn(0, a);
-                    for (int c = 0; c < 3; c++) ga[c] = d * ga[c];
-                } else if (op == MCB_OP_SQRT) {
-                    const float d = v + v;
-                    for (int c = 0; c < 3; c++) ga[c] = ga[c] / d;
-                } else if (mcb_f2u(a) >> 31) {
-                    for (int c = 0; c < 3; c++) ga[c] = -ga[c];
-                }
-            }
-            continue;
-        }
-        const float top = st[--sp], second = st[sp - 1];
-        const bool rev = op == MCB_OP_RSUB || op == MCB_OP_RDIV || op == MCB_OP_RPOW;
-        const float a = rev ? top : second, b = rev ? second : top;
-        float ga[3], gb[3], r[3];
-        for (int c = 0; c < 3; c++) {
-            ga[c] = rev ? gs[sp][c] : gs[sp - 1][c];
-            gb[c] = rev ? gs[sp - 1][c] : gs[sp][c];
-        }
-        const float v = mcb_binop(op, second, top);
+        uint32_t w = code[pc], op = MCB_INSN_OP(w), arg = MCB_INSN_ARG(w);
         switch (op) {
-            case MCB_OP_ADD:
-                for (int c = 0; c < 3; c++) r[c] = ga[c] + gb[c];
+            case MCB_OP_PUSH_X: st[sp++] = x; break;
+            case MCB_OP_PUSH_Y: st[sp++] = y; break;
+            case MCB_OP_PUSH_Z: st[sp++] = z; break;
+            case MCB_OP_PUSH_K: st[sp++] = T(k[arg]); break;
+            case MCB_OP_PUSH_TX: st[sp++] = T(tx[arg]); break;
+            case MCB_OP_PUSH_TY: st[sp++] = T(ty[arg]); break;
+            case MCB_OP_PUSH_TZ: st[sp++] = T(tz[arg]); break;
+            case MCB_OP_NEG: case MCB_OP_SIN: case MCB_OP_COS: case MCB_OP_SQRT: case MCB_OP_ABS:
+                st[sp - 1] = mcb_unop(op, st[sp - 1]);
                 break;
-            case MCB_OP_SUB: case MCB_OP_RSUB:
-                for (int c = 0; c < 3; c++) r[c] = ga[c] - gb[c];
-                break;
-            case MCB_OP_MUL:
-                for (int c = 0; c < 3; c++) r[c] = ga[c] * b + a * gb[c];
-                break;
-            case MCB_OP_DIV: case MCB_OP_RDIV:
-                for (int c = 0; c < 3; c++) r[c] = (ga[c] - v * gb[c]) / b;
-                break;
-            case MCB_OP_MIN: case MCB_OP_MAX: {
-                const uint32_t iv = mcb_f2u(v);
-                const bool ma = mcb_f2u(a) == iv, mb = mcb_f2u(b) == iv;
-                for (int c = 0; c < 3; c++) r[c] = ma && !mb ? ga[c] : mb && !ma ? gb[c] : (ga[c] + gb[c]) * 0.5f;
-                break;
+            case MCB_OP_END: pc = n; break;
+            default: {
+                T top = st[--sp];
+                st[sp - 1] = mcb_binop(op, st[sp - 1], top);
             }
-            default: /* POW, RPOW */
-                if (gb[0] == 0.f && gb[1] == 0.f && gb[2] == 0.f) {
-                    const float d = b * mcb_powf(a, b - 1.f);
-                    for (int c = 0; c < 3; c++) r[c] = d * ga[c];
-                } else {
-                    const float la = mcb_lnf(a), ba = b / a;
-                    for (int c = 0; c < 3; c++) r[c] = v * (la * gb[c] + ba * ga[c]);
-                }
         }
-        st[sp - 1] = v;
-        for (int c = 0; c < 3; c++) gs[sp - 1][c] = r[c];
     }
-    for (int c = 0; c < 3; c++) g[c] = gs[0][c];
     return st[0];
+}
+
+/* Plain values: the rare, divergent evaluations (ambiguity face centres, mcb_eval_points, refined vertices, constant
+ * folding, axis tables); the grid kernels run the fused form below. */
+MCB_BC_FN float mcb_interp_scalar(const uint32_t* code, int n, const float* k, float x, float y, float z,
+                                  const float* tx, const float* ty, const float* tz) {
+    return mcb_interp_point<float>(code, n, k, x, y, z, tx, ty, tz);
+}
+
+/* The value of a point program at (x, y, z) (its bits are those of mcb_interp_scalar) and its gradient g with respect to
+ * the unscaled coordinates, x = sx * unscaled x and so on.  Point programs use no axis tables. */
+MCB_BC_FN float mcb_interp_grad_scalar(const uint32_t* code, int n, const float* k, float x, float y, float z,
+                                       float sx, float sy, float sz, float g[3]) {
+    const mcb_dual r = mcb_interp_point<mcb_dual>(code, n, k, mcb_dual(x, sx, 0.f, 0.f), mcb_dual(y, 0.f, sy, 0.f),
+                                                  mcb_dual(z, 0.f, 0.f, sz), nullptr, nullptr, nullptr);
+    for (int c = 0; c < 3; c++) g[c] = r.g[c];
+    return r.v;
 }
 
 /* The analytic normal of a gradient: m = max |g_i|; (0,0,0) when m is 0, infinite or NaN or a component is NaN; otherwise
  * u = g/m, d = ux*ux + uy*uy + uz*uz (left to right), r = 1/sqrt(d) (correctly rounded, no rsqrt), n = u*r.  Scaling by m
  * first keeps a huge gradient (1/x near 0) a direction instead of an overflow. */
 MCB_BC_FN void mcb_grad_normalise(const float g[3], float out[3]) {
-    const float ax = mcb_u2f(mcb_f2u(g[0]) & 0x7fffffffu), ay = mcb_u2f(mcb_f2u(g[1]) & 0x7fffffffu),
-                az = mcb_u2f(mcb_f2u(g[2]) & 0x7fffffffu);
+    const float ax = mcb_abs(g[0]), ay = mcb_abs(g[1]), az = mcb_abs(g[2]);
     float m = ax > ay ? ax : ay;
     m = m > az ? m : az;
     if (g[0] != g[0] || g[1] != g[1] || g[2] != g[2] || !(m > 0.f) || mcb_f2u(m) == 0x7f800000u) {
@@ -280,11 +318,7 @@ MCB_BC_FN void mcb_grad_normalise(const float g[3], float out[3]) {
     const float ux = g[0] / m, uy = g[1] / m, uz = g[2] / m;
     float d = ux * ux + uy * uy;
     d = d + uz * uz;
-#if defined(__CUDA_ARCH__)
-    const float r = 1.f / __fsqrt_rn(d);
-#else
-    const float r = 1.f / sqrtf(d);
-#endif
+    const float r = 1.f / mcb_sqrt(d);
     out[0] = ux * r; out[1] = uy * r; out[2] = uz * r;
 }
 
@@ -327,23 +361,18 @@ enum {
         }                                                                 \
     } while (0)
 
+static_assert(MCB_F_RPOW - MCB_F_ADD == MCB_OP_RPOW - MCB_OP_ADD && MCB_F_ABS - MCB_F_NEG == MCB_OP_ABS - MCB_OP_NEG,
+              "fused operations ADD..RPOW and NEG..ABS follow their postfix opcodes in order");
+/* One fused word on the operator table: acc = acc (op) v (acc takes the role of the stack's second entry, v of its top),
+ * or v for LOAD / PUSH. */
 MCB_BC_FN float mcb_fop(uint32_t fop, float acc, float v) {
-    switch (fop) {
-        case MCB_F_ADD: return acc + v;
-        case MCB_F_SUB: return acc - v;
-        case MCB_F_RSUB: return v - acc;
-        case MCB_F_MUL: return acc * v;
-        case MCB_F_DIV: return acc / v;
-        case MCB_F_RDIV: return v / acc;
-        case MCB_F_POW: return mcb_powf(acc, v);
-        case MCB_F_RPOW: return mcb_powf(v, acc);
-        case MCB_F_MIN: return mcb_minf(acc, v);
-        case MCB_F_MAX: return mcb_maxf(acc, v);
-        default: return v; /* LOAD, PUSH */
-    }
+    if (fop == MCB_F_LOAD || fop == MCB_F_PUSH) return v;
+    return mcb_binop(fop == MCB_F_MIN ? (uint32_t)MCB_OP_MIN : fop == MCB_F_MAX ? (uint32_t)MCB_OP_MAX : fop - MCB_F_ADD + MCB_OP_ADD,
+                     acc, v);
 }
 
-/* Scalar interpreter of the fused form (host-side checks of mcb::fuse(); the grid kernel has its own). */
+/* Scalar interpreter of the fused form (host-side checks of mcb::fuse(); the grid kernels run the same words through
+ * mcb_fop on their register-tiled accumulators, mcb_kernels.cuh). */
 MCB_BC_FN float mcb_interp_fused_scalar(const uint32_t* code, int n, const float* k, float x, float y, float z,
                                         const float* tx, const float* ty, const float* tz) {
     float st[MCB_MAX_STACK];
@@ -352,8 +381,7 @@ MCB_BC_FN float mcb_interp_fused_scalar(const uint32_t* code, int n, const float
     for (int pc = 0; pc < n; pc++) {
         uint32_t w = code[pc], fop = MCB_FINSN_OP(w), src = MCB_FINSN_SRC(w), arg = MCB_FINSN_ARG(w);
         MCB_FINSN_DECODE(fop, src);
-        if (fop == MCB_F_NEG) { acc = -acc; continue; }
-        if (MCB_F_IS_FN(fop)) { acc = mcb_fn(fop - MCB_F_SIN, acc); continue; }
+        if (fop == MCB_F_NEG || MCB_F_IS_FN(fop)) { acc = mcb_unop(fop - MCB_F_NEG + MCB_OP_NEG, acc); continue; }
         if (fop == MCB_F_PUSH) st[sp++] = acc;
         float v;
         switch (src) {

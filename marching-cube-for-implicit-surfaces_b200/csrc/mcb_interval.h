@@ -27,7 +27,7 @@
  *     taken from analysis; this one rests on the exhaustive run of oracle/trig_exhaustive.c (every finite result of
  *     either function, over all 2^32 inputs, lies in [-1, 1]).  Hoisted sin / cos need no rule at all: their values
  *     are axis-table entries, whose exact minimum and maximum over the box are the leaves;
- *   - min, max (mcb_minf / mcb_maxf): exact and monotone in each argument, [min(a.lo, b.lo), min(a.hi, b.hi)] and the
+ *   - min, max (mcb_min / mcb_max): exact and monotone in each argument, [min(a.lo, b.lo), min(a.hi, b.hi)] and the
  *     same for max.  This rests on the invariant that a known interval never encloses a NaN value: sqrt of a possibly
  *     negative interval, division across 0 and non-finite end points already make the box unknown, so the NaN-ignoring
  *     rule of minimumNumber never applies to a value the interval stands for.  An unknown argument makes the result
@@ -115,8 +115,8 @@ MCB_BC_FN mcb_ival mcb_iv_op(uint32_t fop, mcb_ival acc, mcb_ival v, int* bad) {
         }
         case MCB_F_POW: r = mcb_iv_pow(acc, v, bad); break;
         case MCB_F_RPOW: r = mcb_iv_pow(v, acc, bad); break;
-        case MCB_F_MIN: r.lo = mcb_minf(acc.lo, v.lo); r.hi = mcb_minf(acc.hi, v.hi); break;
-        case MCB_F_MAX: r.lo = mcb_maxf(acc.lo, v.lo); r.hi = mcb_maxf(acc.hi, v.hi); break;
+        case MCB_F_MIN: r.lo = mcb_min(acc.lo, v.lo); r.hi = mcb_min(acc.hi, v.hi); break;
+        case MCB_F_MAX: r.lo = mcb_max(acc.lo, v.lo); r.hi = mcb_max(acc.hi, v.hi); break;
         default: r = v; break; /* LOAD, PUSH */
     }
     if (!mcb_iv_finite(r.lo) || !mcb_iv_finite(r.hi)) *bad = 1;
@@ -134,8 +134,8 @@ MCB_BC_FN mcb_ival mcb_iv_fn(uint32_t fop, mcb_ival a, int* bad) {
             break;
         case MCB_F_SQRT:
             if (!(a.lo >= 0.f)) { *bad = 1; r.lo = r.hi = 0.f; break; }
-            r.lo = mcb_fn(2, a.lo);
-            r.hi = mcb_fn(2, a.hi);
+            r.lo = mcb_sqrt(a.lo);
+            r.hi = mcb_sqrt(a.hi);
             break;
         default: /* sin, cos */
             r.lo = -1.f;

@@ -16,7 +16,7 @@ const char* const kTrigHeader =
 #include "mcb_trig_src.inc" /* mcb_trig.h, likewise */
     ;
 const char* const kBytecodeHeader =
-#include "mcb_bytecode_src.inc" /* mcb_bytecode.h, likewise: mcb_minf / mcb_maxf */
+#include "mcb_bytecode_src.inc" /* mcb_bytecode.h, likewise: mcb_min / mcb_max */
     ;
 
 /* Everything around the generated body.  It restates the tile of eval_field_kernel (mcb_kernels.cuh): a warp owns 128
@@ -49,10 +49,10 @@ __device__ __noinline__ float op_cos(float a) { return mcb_cosf(a); }
 const char* const kHeadSqrtAbs = R"SRC(__device__ __forceinline__ float op_sqrt(float a) { return __fsqrt_rn(a); }
 __device__ __forceinline__ float op_abs(float a) { return __uint_as_float(__float_as_uint(a) & 0x7fffffffu); }
 )SRC";
-/* min / max: the interpreters' own mcb_minf / mcb_maxf (minimumNumber / maximumNumber), also only when used */
+/* min / max: the operator table's mcb_min / mcb_max (minimumNumber / maximumNumber), also only when used */
 const char* const kHeadMinMax = R"SRC(#include "mcb_bytecode.h"
-__device__ __forceinline__ float op_min(float a, float b) { return mcb_minf(a, b); }
-__device__ __forceinline__ float op_max(float a, float b) { return mcb_maxf(a, b); }
+__device__ __forceinline__ float op_min(float a, float b) { return mcb_min(a, b); }
+__device__ __forceinline__ float op_max(float a, float b) { return mcb_max(a, b); }
 )SRC";
 const char* const kHeadPlane = R"SRC(
 extern "C" __global__ void __launch_bounds__(128, MCB_MIN_BLOCKS)

@@ -155,33 +155,6 @@ __global__ void axis_tables_kernel(const uint32_t* __restrict__ slot_code, const
  *     and one vote per vertex and one 16-byte store per tile row.  The comparison against iso is fused here so that
  *     classification never reads the 4 B/vertex field.
  * ------------------------------------------------------------------------------------------------------------- */
-__device__ __noinline__ float powf_call(float a, float b) { return mcb_powf(a, b); } /* one copy, register args */
-
-template <int FOP>
-__device__ __forceinline__ float fused_op(float acc, float v) {
-    switch (FOP) {
-        case MCB_F_ADD: return acc + v;
-        case MCB_F_SUB: return acc - v;
-        case MCB_F_RSUB: return v - acc;
-        case MCB_F_MUL: return acc * v;
-        case MCB_F_DIV: return acc / v;
-        case MCB_F_RDIV: return v / acc;
-        case MCB_F_POW: { /* x^2 first: exact fp32 fast path (mcb_pow.h), the fp64 algorithm only for the rare remainder */
-            float r;
-            if (__float_as_uint(v) == 0x40000000u && mcb_pow2_try(acc, &r)) return r;
-            return powf_call(acc, v);
-        }
-        case MCB_F_RPOW: {
-            float r;
-            if (__float_as_uint(acc) == 0x40000000u && mcb_pow2_try(v, &r)) return r;
-            return powf_call(v, acc);
-        }
-        case MCB_F_MIN: return mcb_minf(acc, v);
-        case MCB_F_MAX: return mcb_maxf(acc, v);
-        default: return v; /* MCB_F_LOAD, MCB_F_PUSH */
-    }
-}
-
 struct EvalLane { /* what an operand fetch needs besides the instruction argument */
     const float* __restrict__ tables;
     int x0, y0, zi; /* the lane's first column (its others: x0 + 32 q), first of the warp's 4 rows, index into the z tables */
@@ -201,25 +174,25 @@ __device__ __forceinline__ void eval_step(float (&acc)[kEvalRows], float*& sp, c
     if (SRC == MCB_SRC_POP) {
         sp -= kEvalLevel;
 #pragma unroll
-        for (int e = 0; e < kEvalRows; e++) acc[e] = fused_op<FOP>(acc[e], sp[e * kEvalThreads]);
+        for (int e = 0; e < kEvalRows; e++) acc[e] = mcb_fop(FOP, acc[e], sp[e * kEvalThreads]);
     } else if (SRC == MCB_SRC_TY) { /* 4 rows of a y-table: 16-byte aligned, same address in every lane */
         const float4 t = __ldg(reinterpret_cast<const float4*>(L.tables + arg + L.y0));
         const float tv[4] = {t.x, t.y, t.z, t.w};
 #pragma unroll
         for (int r = 0; r < 4; r++)
 #pragma unroll
-            for (int q = 0; q < 4; q++) acc[4 * r + q] = fused_op<FOP>(acc[4 * r + q], tv[r]);
+            for (int q = 0; q < 4; q++) acc[4 * r + q] = mcb_fop(FOP, acc[4 * r + q], tv[r]);
     } else if (SRC == MCB_SRC_TX) { /* the lane's 4 columns of an x-table (the tables are padded past the last tile) */
         const float* t = L.tables + arg + L.x0;
         const float tv[4] = {__ldg(t), __ldg(t + QS), __ldg(t + 2 * QS), __ldg(t + 3 * QS)};
 #pragma unroll
         for (int r = 0; r < 4; r++)
 #pragma unroll
-            for (int q = 0; q < 4; q++) acc[4 * r + q] = fused_op<FOP>(acc[4 * r + q], tv[q]);
+            for (int q = 0; q < 4; q++) acc[4 * r + q] = mcb_fop(FOP, acc[4 * r + q], tv[q]);
     } else { /* one value for all 16 vertices of the lane */
         const float u = SRC == MCB_SRC_K ? prog.k[arg] : __ldg(L.tables + arg + L.zi);
 #pragma unroll
-        for (int e = 0; e < kEvalRows; e++) acc[e] = fused_op<FOP>(acc[e], u);
+        for (int e = 0; e < kEvalRows; e++) acc[e] = mcb_fop(FOP, acc[e], u);
     }
 }
 
@@ -251,7 +224,7 @@ __device__ __forceinline__ void eval_pair(float (&acc)[kEvalRows], uint32_t arg_
 #pragma unroll
     for (int r = 0; r < 4; r++)
 #pragma unroll
-        for (int q = 0; q < 4; q++) acc[4 * r + q] = fused_op<FOP>(a.at(r, q), b.at(r, q));
+        for (int q = 0; q < 4; q++) acc[4 * r + q] = mcb_fop(FOP, a.at(r, q), b.at(r, q));
 }
 #define MCB_HANDLER_SPILL 55 /* push the accumulator on the memory stack; the new value comes from the next (pair) word */
 #define MCB_HANDLER_FN(FOP) (56 + (FOP) - MCB_F_SIN) /* sin, cos, sqrt, abs of the accumulator: 56..59 (function grammar) */
@@ -277,27 +250,24 @@ constexpr int kEvalTileX = 128; /* columns per warp tile */
 constexpr int kEvalTileY = 4;   /* rows per warp tile */
 static_assert(kEvalRows == 16, "a lane carries a 4 x 4 patch");
 
-/* The function grammar's functions on the 16 accumulators (handlers 56..59).  sin / cos: the fp64 restatement of glibc's
- * sinf / cosf (mcb_trig.h) out of line, one copy; sqrt: correctly rounded. */
-__device__ __noinline__ float sinf_call(float a) { return mcb_sinf(a); }
-__device__ __noinline__ float cosf_call(float a) { return mcb_cosf(a); }
+/* The function grammar's functions on the 16 accumulators (handlers 56..59) */
 __device__ __forceinline__ void eval_fn(float (&acc)[kEvalRows], uint32_t handler) {
     switch (handler) {
         case MCB_HANDLER_FN(MCB_F_SIN):
 #pragma unroll
-            for (int e = 0; e < kEvalRows; e++) acc[e] = sinf_call(acc[e]);
+            for (int e = 0; e < kEvalRows; e++) acc[e] = mcb_sin(acc[e]);
             break;
         case MCB_HANDLER_FN(MCB_F_COS):
 #pragma unroll
-            for (int e = 0; e < kEvalRows; e++) acc[e] = cosf_call(acc[e]);
+            for (int e = 0; e < kEvalRows; e++) acc[e] = mcb_cos(acc[e]);
             break;
         case MCB_HANDLER_FN(MCB_F_SQRT):
 #pragma unroll
-            for (int e = 0; e < kEvalRows; e++) acc[e] = __fsqrt_rn(acc[e]);
+            for (int e = 0; e < kEvalRows; e++) acc[e] = mcb_sqrt(acc[e]);
             break;
         default: /* abs */
 #pragma unroll
-            for (int e = 0; e < kEvalRows; e++) acc[e] = __uint_as_float(__float_as_uint(acc[e]) & 0x7fffffffu);
+            for (int e = 0; e < kEvalRows; e++) acc[e] = mcb_abs(acc[e]);
             break;
     }
 }

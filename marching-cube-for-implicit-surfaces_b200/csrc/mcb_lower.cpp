@@ -363,7 +363,7 @@ struct Lowerer {
             case '*': op = MCB_OP_MUL; break;
             case '-': op = right_first ? MCB_OP_RSUB : MCB_OP_SUB; break;
             case '/': op = right_first ? MCB_OP_RDIV : MCB_OP_DIV; break;
-            case 'm': op = MCB_OP_MIN; break; /* commutative bit for bit (mcb_minf): either order, no reversed form */
+            case 'm': op = MCB_OP_MIN; break; /* commutative bit for bit (mcb_min): either order, no reversed form */
             case 'M': op = MCB_OP_MAX; break;
             default: op = right_first ? MCB_OP_RPOW : MCB_OP_POW; break;
         }

@@ -76,8 +76,8 @@ MCB_BC_FN int mcb_refine_vertex(const uint32_t* code, int n, const float* k, con
     const bool sa = fa > iso; /* the classifier's predicate: strict, NaN counts as false */
     if (sa == (fb > iso)) return MCB_REFINE_SAME_SIGN;
     int evals = 2;
-    float best = a, bd = mcb_u2f(mcb_f2u(fa - iso) & 0x7fffffffu);
-    const float db = mcb_u2f(mcb_f2u(fb - iso) & 0x7fffffffu);
+    float best = a, bd = mcb_abs(fa - iso);
+    const float db = mcb_abs(fb - iso);
     if (mcb_refine_better(db, bd)) { best = b; bd = db; }
     if (bd != 0.f) {
         float ga = fa - iso, gb = fb - iso;            /* Illinois-weighted residuals of the two ends */
@@ -92,7 +92,7 @@ MCB_BC_FN int mcb_refine_vertex(const uint32_t* code, int n, const float* k, con
             q[ax] = x;
             const float fx = mcb_interp_scalar(code, n, k, sx * q[0], sy * q[1], sz * q[2], 0, 0, 0);
             evals++;
-            const float dx = mcb_u2f(mcb_f2u(fx - iso) & 0x7fffffffu);
+            const float dx = mcb_abs(fx - iso);
             if (mcb_refine_better(dx, bd)) { best = x; bd = dx; }
             if (fx == iso) break;
             if ((fx > iso) == sa) {

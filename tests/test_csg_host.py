@@ -124,7 +124,7 @@ def _product_eval(host, eq, a, b):
 
 
 def test_min_max_on_special_pairs_equal_the_definition_and_the_oracle(host):
-    """mcb_minf / mcb_maxf (the host build of csrc/mcb_bytecode.h, through the point interpreter: `min(x,y)` is
+    """mcb_min / mcb_max (the host build of csrc/mcb_bytecode.h, through the point interpreter: `min(x,y)` is
     PUSH_X PUSH_Y MIN) against the numpy statement of the definition, the oracle's plain-C restatement called directly and
     the oracle's walk; sign of zero included, NaN as a class."""
     a, b = special_pairs()
