@@ -78,7 +78,7 @@ struct mcb_ctx {
     Counters* d_ctr = nullptr;
     Counters* h_ctr = nullptr; /* pinned */
     unsigned long long* d_ent = nullptr;    /* classify -> compact scratch: one entry per active item of every tile */
-    uint32_t* d_tile_u32 = nullptr;         /* [5][cap_tiles]: entries, active cubes, triangles, and the two exclusive prefixes */
+    uint32_t* d_tile_u32 = nullptr;         /* [3][cap_tiles]: entries, active cubes, triangles of every tile; [2][tile groups]: the sums per group */
     unsigned long long* d_amb = nullptr;    /* [cap_amb][2] ambiguous cubes awaiting the face-centre test */
     uint32_t cap_amb = 0;
     size_t cap_tile_entries = 0;
@@ -284,6 +284,13 @@ int install_equation(mcb_ctx* ctx, int slot, const char* equation) {
     return MCB_OK;
 }
 
+size_t tile_groups(size_t tiles) { return (tiles + kTileGroup - 1) / kTileGroup; }
+
+/* the per-group tile sums start at zero in every classify pass (classify_kernel and ambiguity_kernel add to them) */
+cudaError_t clear_tile_groups(const mcb_ctx* ctx, cudaStream_t s) {
+    return cudaMemsetAsync(ctx->d_tile_u32 + 3 * ctx->cap_tiles, 0, 2 * tile_groups(ctx->cap_tiles) * 4, s);
+}
+
 /* Tiling of the classify pass: runs of whole cube rows, at most kClsItemCap items, at least ~4 tiles per SM
  * (DESIGN.md, classify). */
 ClsGeom classify_geometry(const mcb_ctx* ctx, const Grid& g, unsigned* tiles) {
@@ -335,7 +342,7 @@ int setup_grid(mcb_ctx* ctx) {
         if (ctx->d_tile_u32) cudaFree(ctx->d_tile_u32);
         ctx->d_tile_u32 = nullptr;
         ctx->cap_tiles = 0;
-        MCB_CK(cudaMalloc((void**)&ctx->d_tile_u32, 5 * tiles * 4));
+        MCB_CK(cudaMalloc((void**)&ctx->d_tile_u32, (3 * tiles + 2 * tile_groups(tiles)) * 4));
         ctx->cap_tiles = tiles;
     }
     const size_t entries = tiles * (size_t)cg0.tile_rows * cg0.WC; /* worst case: every item active */
@@ -842,12 +849,13 @@ struct Run {
     int encode_program(mcb_program& launch, bool& has_pow, bool& has_fn, bool& has_minmax, bool blocks);
     int ensure_block_buffers(FieldBlocks* fb, BlockDims* bd);
     int launch_block_eval(const FieldBlocks& fb, const uint32_t* list, const unsigned* count);
+    int fork_block_clears();
     int stage_eval_blocks();
     int stage_fill();
     int launch_eval_jit();
     int stage_tables();
     int stage_eval();
-    int stage_classify();
+    int stage_classify(bool rerun);
     int stage_seed();
     int stage_soup();
     int stage_weld();
@@ -1072,7 +1080,7 @@ int launch_constraints(Run& r) {
     int first = 1;
     for (int i = 0; i < 3; i++) {
         if (!(ctx->cons[i].in_use && ctx->eq[i + 1].valid)) continue;
-        MCB_LAUNCH((eval_constraint_kernel), (unsigned)((words + 7) / 8), 256, 0, r.s, ctx->eq[i + 1].point, r.g, ctx->d_cs, ctx->cons[i].op,
+        MCB_LAUNCH_PDL((eval_constraint_kernel), (unsigned)((words + 7) / 8), 256, 0, r.s, ctx->eq[i + 1].point, r.g, ctx->d_cs, ctx->cons[i].op,
                    ctx->cons[i].rhs, first, ctx->d_V, words);
         first = 0;
         r.launches++;
@@ -1100,11 +1108,11 @@ int Run::stage_eval() {
         mcb_program launch;
         bool has_pow, has_fn, has_minmax;
         if ((rc = encode_program(launch, has_pow, has_fn, has_minmax, false)) != MCB_OK) return rc;
-        if (has_minmax && (has_pow || has_fn)) MCB_LAUNCH((eval_field_kernel<true, true, true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
-        else if (has_minmax) MCB_LAUNCH((eval_field_kernel<false, true, false, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
-        else if (has_fn) MCB_LAUNCH((eval_field_kernel<true, true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
-        else if (has_pow) MCB_LAUNCH((eval_field_kernel<true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
-        else MCB_LAUNCH((eval_field_kernel<false, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        if (has_minmax && (has_pow || has_fn)) MCB_LAUNCH_PDL((eval_field_kernel<true, true, true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        else if (has_minmax) MCB_LAUNCH_PDL((eval_field_kernel<false, true, false, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        else if (has_fn) MCB_LAUNCH_PDL((eval_field_kernel<true, true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        else if (has_pow) MCB_LAUNCH_PDL((eval_field_kernel<true, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
+        else MCB_LAUNCH_PDL((eval_field_kernel<false, true>), blocks, kEvalThreads, smem, s, launch, g, ctx->d_tables, ctx->d_F, ctx->d_S, rgpp);
         launches++;
     }
     return launch_constraints(*this);
@@ -1182,9 +1190,10 @@ int Run::launch_block_eval(const FieldBlocks& fb, const uint32_t* list, const un
     return MCB_OK;
 }
 
-/* K1, block-field mode (MCB_FIELD_SPARSE / MCB_FIELD_AUTO): interval classes per 32 x 4 x 4 vertex block, field values
- * and signs only in the undecided blocks, the candidate map for classify (mcb_kernels.cuh, "decide, evaluate, skip") */
-int Run::stage_eval_blocks() {
+/* Block-field mode, before the axis tables: the buffers of the stage, and the three clears on the side stream, which run
+ * under the tables, the bounds and the super-block classes (none of them reads the cleared arrays); block_class, the
+ * first kernel that writes into them, waits for fork_ev[1].  Nothing here sits between two kernels on the main stream. */
+int Run::fork_block_clears() {
     FieldBlocks fb;
     BlockDims bd;
     int rc = ensure_block_buffers(&fb, &bd);
@@ -1193,20 +1202,7 @@ int Run::stage_eval_blocks() {
         MCB_CK(cudaMemsetAsync(ctx->d_F, 0xff, (size_t)g.NZ * g.NV * g.P * sizeof(float), s));
         MCB_CK(cudaMemsetAsync(ctx->d_S, 0x5a, (size_t)g.NZ * g.NV * g.WP * sizeof(uint32_t), s));
     }
-    ctx->field_is_sparse = true;
-    ctx->jit_used = false;
-    if (jit_wanted(ctx, eq)) {
-        const mcb_ctx::JitKernel* jk = nullptr;
-        rc = jit_module(ctx, eq, &jk);
-        if (rc == MCB_OK) { ctx->jit_used = true; ctx->jit_cur = jk; }
-        else if (rc == kJitDeferred) ctx->jit_note = "compiling in the background";
-        else if (ctx->jit == MCB_JIT_ON) return rc;
-        else ctx->jit_note = ctx->err;
-    }
     const size_t nblocks = (size_t)bd.nbx * bd.nby * bd.nbz;
-    const unsigned nsuper = (unsigned)bd.nbx * (unsigned)bd.nsy * (unsigned)bd.nsz;
-    /* the three clears run on the side stream while the bounds and the super-block classes are computed; block_class, the
-     * first kernel that writes into the cleared arrays, waits for them */
     cudaStream_t side = ctx->copy_stream;
     MCB_CK(cudaEventRecord(ctx->fork_ev[0], s));
     MCB_CK(cudaStreamWaitEvent(side, ctx->fork_ev[0], 0));
@@ -1214,18 +1210,40 @@ int Run::stage_eval_blocks() {
     MCB_CK(cudaMemsetAsync(ctx->d_fflags, 0, nblocks, side));
     MCB_CK(cudaMemsetAsync(ctx->d_bcls, 0xFF, nblocks, side)); /* kClsInherit: the super-block's verdict holds unless the fine pass says otherwise */
     MCB_CK(cudaEventRecord(ctx->fork_ev[1], side));
-    MCB_LAUNCH((axis_bounds_kernel), dim3((unsigned)((3 * bd.spa * bd.nb + 127) / 128), 2u), 128, 0, s, ctx->d_tables, g, bd, eq.c.n_axis_slots[0],
+    return MCB_OK;
+}
+
+/* K1, block-field mode (MCB_FIELD_SPARSE / MCB_FIELD_AUTO): interval classes per 32 x 4 x 4 vertex block, field values
+ * and signs only in the undecided blocks, the candidate map for classify (mcb_kernels.cuh, "decide, evaluate, skip") */
+int Run::stage_eval_blocks() {
+    FieldBlocks fb;
+    BlockDims bd;
+    int rc = ensure_block_buffers(&fb, &bd);
+    if (rc != MCB_OK) return rc;
+    ctx->field_is_sparse = true;
+    ctx->jit_used = false;
+    if (jit_wanted(ctx, eq)) {
+        const mcb_ctx::JitKernel* jk = nullptr;
+        rc = jit_module(ctx, eq, &jk);
+        if (rc == MCB_OK) { ctx->jit_used = true; ctx->jit_cur = jk; }
+        else if (rc == kJitDeferred) ctx->jit_note = "compiling in the background";
+        else if (ctx->jit == MCB_JIT_ON) { cudaStreamWaitEvent(s, ctx->fork_ev[1], 0); return rc; } /* the clears are joined on every path */
+        else ctx->jit_note = ctx->err;
+    }
+    const unsigned nsuper = (unsigned)bd.nbx * (unsigned)bd.nsy * (unsigned)bd.nsz;
+    cudaStream_t side = ctx->copy_stream;
+    MCB_LAUNCH_PDL((axis_bounds_kernel), dim3((unsigned)((3 * bd.spa * bd.nb + 127) / 128), 2u), 128, 0, s, ctx->d_tables, g, bd, eq.c.n_axis_slots[0],
                eq.c.n_axis_slots[1], eq.c.n_axis_slots[2], ctx->d_bounds_iv);
-    MCB_LAUNCH((super_class_kernel), (nsuper + 127) / 128, 128, 0, s, eq.grid, g, bd, ctx->d_bounds_iv, ctx->decide_blocks ? 1 : 0, ctx->d_scls,
+    MCB_LAUNCH_PDL((super_class_kernel), (nsuper + 127) / 128, 128, 0, s, eq.grid, g, bd, ctx->d_bounds_iv, ctx->decide_blocks ? 1 : 0, ctx->d_scls,
                ctx->d_slist, ctx->d_ctr);
-    MCB_CK(cudaStreamWaitEvent(s, ctx->fork_ev[1], 0));
-    MCB_LAUNCH((block_class_kernel), (unsigned)ctx->sm_count * 8, 256, 0, s, eq.grid, g, bd, ctx->d_bounds_iv, ctx->d_slist, ctx->decide_blocks ? 1 : 0,
+    MCB_CK(cudaStreamWaitEvent(s, ctx->fork_ev[1], 0)); /* the clears (fork_block_clears) */
+    MCB_LAUNCH_PDL((block_class_kernel), (unsigned)ctx->sm_count * 8, 256, 0, s, eq.grid, g, bd, ctx->d_bounds_iv, ctx->d_slist, ctx->decide_blocks ? 1 : 0,
                ctx->d_bcls, ctx->d_fflags, ctx->d_elist, ctx->d_cand, ctx->d_ctr);
     /* Two latency-bound kernels that touch disjoint blocks — the sign words of the decided neighbours, the field of the
      * undecided blocks — run side by side: the first on the side stream, joined before anything reads the sign planes */
     MCB_CK(cudaEventRecord(ctx->fork_ev[0], s));
     MCB_CK(cudaStreamWaitEvent(side, ctx->fork_ev[0], 0));
-    MCB_LAUNCH((decided_signs_kernel), (unsigned)ctx->sm_count * 8, 256, 0, side, g, bd, ctx->d_elist, ctx->d_ctr, ctx->d_bcls, ctx->d_scls, ctx->d_S);
+    MCB_LAUNCH_PDL((decided_signs_kernel), (unsigned)ctx->sm_count * 8, 256, 0, side, g, bd, ctx->d_elist, ctx->d_ctr, ctx->d_bcls, ctx->d_scls, ctx->d_S);
     MCB_CK(cudaEventRecord(ctx->fork_ev[1], side));
     launches += 4;
     rc = launch_block_eval(fb, ctx->d_elist, &ctx->d_ctr->eval_blocks);
@@ -1234,21 +1252,25 @@ int Run::stage_eval_blocks() {
     return launch_constraints(*this);
 }
 
-/* K2: classification (per tile, independent) -> face-centre tests of the ambiguous cubes -> scan of the tile totals ->
- * compaction */
-int Run::stage_classify() {
+/* K2: classification (per tile, independent) -> face-centre tests of the ambiguous cubes -> compaction (each tile's
+ * base from the tile totals before it).  `rerun`: a repeated pass after buffer growth, whose counters need resetting —
+ * the first pass finds them zeroed at the start of the call, and the evaluation stage writes none of them. */
+int Run::stage_classify(bool rerun) {
     int rc;
-    MCB_CK(cudaMemsetAsync(ctx->d_ctr, 0, kCountersClassifyBytes, s)); /* the evaluation stage's counters stay */
+    if (rerun) {
+        MCB_CK(cudaMemsetAsync(ctx->d_ctr, 0, kCountersClassifyBytes, s)); /* the evaluation stage's counters stay */
+        MCB_CK(clear_tile_groups(ctx, s));
+    }
     uint32_t* tu = ctx->d_tile_u32;
-    const size_t ct = ctx->cap_tiles;
+    const size_t ct = ctx->cap_tiles, ng = tile_groups(ct);
     const bool skip = ctx->field_is_sparse; /* the candidate map of the block-field mode */
-    const ClsScratch sc{ctx->d_ent, tu, tu + ct, tu + 2 * ct, tu + 3 * ct, tu + 4 * ct, ctx->d_amb, ctx->cap_amb, cg.tile_rows * cg.WC,
+    const ClsScratch sc{ctx->d_ent, tu, tu + ct, tu + 2 * ct, tu + 3 * ct, tu + 3 * ct + ng, ctx->d_amb, ctx->cap_amb, cg.tile_rows * cg.WC,
                         skip ? ctx->d_cand : nullptr, (uint32_t)((g.M + 3) / 4), (uint32_t)((cg.WC + 63) / 64)};
     const uint32_t* cw = nullptr;
     if (g.repeat) { /* per-cube iso levels: the corner signs come from the field, item by item */
         const unsigned long long items = (unsigned long long)cg.total_rows * cg.WC;
         if ((rc = ensure(ctx, &ctx->d_cw, &ctx->cap_cw, (size_t)items * 8)) != MCB_OK) return rc;
-        MCB_LAUNCH((repeat_words_kernel), (unsigned)ctx->sm_count * 8, 256, 0, s, g, ctx->d_F, cg.WC, ctx->d_cw, items);
+        MCB_LAUNCH_PDL((repeat_words_kernel), (unsigned)ctx->sm_count * 8, 256, 0, s, g, ctx->d_F, cg.WC, ctx->d_cw, items);
         launches++;
         cw = ctx->d_cw;
     }
@@ -1259,16 +1281,15 @@ int Run::stage_classify() {
     const FieldBlocks apron = skip ? FieldBlocks{ctx->bd.nbx, ctx->bd.nby, ctx->bd.nbz, ctx->d_fflags, ctx->d_flist} : FieldBlocks{0, 0, 0, nullptr, nullptr};
 #define MCB_CLASSIFY(HAS_V, REPEAT)                                                                                                   \
     do {                                                                                                                              \
-        MCB_LAUNCH((classify_kernel<HAS_V, REPEAT>), tiles, kClsThreads, kClsSmemBytes, s, g, ctx->d_cls, ctx->d_S, dV, cg, sc, ctx->d_ctr, cw); \
-        MCB_LAUNCH((ambiguity_kernel<REPEAT>), amb_ctas, 128, 0, s, eq.point, g, ctx->d_cs, ctx->d_cls, sc, ctx->d_ctr, ctx->d_F);          \
-        MCB_LAUNCH((tile_scan_kernel), 1, 1024, 0, s, sc, tiles, ctx->d_ctr);                                                             \
-        MCB_LAUNCH((compact_kernel<REPEAT>), tiles, kClsThreads, 0, s, g, ctx->d_cls, ctx->d_S, dV, cg, sc, ctx->d_rec, ctx->d_trioff,     \
-                   ctx->cap_active, items, cw, apron);                                                                                 \
+        MCB_LAUNCH_PDL((classify_kernel<HAS_V, REPEAT>), tiles, kClsThreads, kClsSmemBytes, s, g, ctx->d_cls, ctx->d_S, dV, cg, sc, ctx->d_ctr, cw); \
+        MCB_LAUNCH_PDL((ambiguity_kernel<REPEAT>), amb_ctas, 128, 0, s, eq.point, g, ctx->d_cs, ctx->d_cls, sc, ctx->d_ctr, ctx->d_F);          \
+        MCB_LAUNCH_PDL((compact_kernel<REPEAT>), tiles, kClsThreads, 0, s, g, ctx->d_cls, ctx->d_S, dV, cg, sc, ctx->d_ctr, ctx->d_rec,        \
+                       ctx->d_trioff, ctx->cap_active, items, cw, apron);                                                              \
     } while (0)
     if (cw) { if (dV) MCB_CLASSIFY(true, true); else MCB_CLASSIFY(false, true); }
     else { if (dV) MCB_CLASSIFY(true, false); else MCB_CLASSIFY(false, false); }
 #undef MCB_CLASSIFY
-    launches += 4;
+    launches += 3;
     return MCB_OK;
 }
 
@@ -1282,7 +1303,7 @@ int Run::stage_fill() {
     int rc = ensure_block_buffers(&fb, &bd);
     if (rc != MCB_OK) return rc;
     const size_t nb = (size_t)fb.nbx * fb.nby * fb.nbz;
-    MCB_LAUNCH((field_list_kernel), (unsigned)((nb / 16 + 256) / 256), 256, 0, s, fb, (unsigned)nb, ctx->d_ctr); /* the blocks compact_kernel marked */
+    MCB_LAUNCH_PDL((field_list_kernel), (unsigned)((nb / 16 + 256) / 256), 256, 0, s, fb, (unsigned)nb, ctx->d_ctr); /* the blocks compact_kernel marked */
     launches += 1;
     return launch_block_eval(fb, ctx->d_flist, &ctx->d_ctr->field_blocks);
 }
@@ -1346,7 +1367,7 @@ int Run::stage_soup() {
     const bool idx32 = (unsigned long long)g.NZ * g.NV * g.P < (1ull << 32) - 2ull * g.NV * g.P; /* offsets +- one plane stay below 2^32 */
     const unsigned grid = (unsigned)ctx->sm_count * (unsigned)kEmitBlocksPerSM; /* one resident wave: emit2 hands out chunks itself */
 #define MCB_SOUP(NRM, I32)                                                                                                            \
-    MCB_LAUNCH((emit2_kernel<NRM, I32>), grid, kEmitThreads, 0, s, g, ctx->d_cs, rinv, ctx->d_F, ctx->d_cls, ctx->d_rec, ctx->d_trioff, \
+    MCB_LAUNCH_PDL((emit2_kernel<NRM, I32>), grid, kEmitThreads, 0, s, g, ctx->d_cs, rinv, ctx->d_F, ctx->d_cls, ctx->d_rec, ctx->d_trioff, \
                ctx->d_ctr, ctx->cap_active, ctx->cap_tris, ctx->d_pos, NRM ? ctx->d_nrm : nullptr)
     if (ctx->normals == 1) { if (idx32) MCB_SOUP(true, true); else MCB_SOUP(true, false); }
     else { if (idx32) MCB_SOUP(false, true); else MCB_SOUP(false, false); }
@@ -1362,11 +1383,11 @@ int Run::stage_weld() {
     const WeldView W{g, ctx->d_cs, ctx->d_F, any_constraint ? ctx->d_V : nullptr, ctx->seed_on ? ctx->d_item : nullptr, cg.WC};
     const WeldViewT<true> WR{W.g, W.cs, W.F, W.V, W.present, W.WC}; /* repeating-surface mode: same view, level checks compiled in */
     const WeldBuffers B{ctx->d_rec, ctx->d_trioff, ctx->d_item, ctx->d_vinfo, ctx->d_chunk_new, cg.WC};
-    if (g.repeat) MCB_LAUNCH((weld_count_kernel), eblocks * 2, kWeldThreads, 0, s, WR, B, ctx->d_ctr, ctx->cap_active);
-    else if (W.V != nullptr || W.present != nullptr) MCB_LAUNCH((weld_count_kernel), eblocks * 2, kWeldThreads, 0, s, W, B, ctx->d_ctr, ctx->cap_active);
-    else MCB_LAUNCH((weld_count_fast_kernel), eblocks * 4, kWeldCubes, 0, s, W, B, ctx->d_cls, ctx->d_ctr, ctx->cap_active);
-    MCB_LAUNCH((weld_scan_kernel), 1, 1024, 0, s, ctx->d_chunk_new, ctx->d_ctr, ctx->cap_active);
-    MCB_LAUNCH((weld_base_kernel), eblocks * 2, kWeldCubes, 0, s, B, ctx->d_ctr, ctx->cap_active);
+    if (g.repeat) MCB_LAUNCH_PDL((weld_count_kernel<WeldViewT<true>>), eblocks * 2, kWeldThreads, 0, s, WR, B, ctx->d_ctr, ctx->cap_active);
+    else if (W.V != nullptr || W.present != nullptr) MCB_LAUNCH_PDL((weld_count_kernel<WeldView>), eblocks * 2, kWeldThreads, 0, s, W, B, ctx->d_ctr, ctx->cap_active);
+    else MCB_LAUNCH_PDL((weld_count_fast_kernel), eblocks * 4, kWeldCubes, 0, s, W, B, ctx->d_cls, ctx->d_ctr, ctx->cap_active);
+    MCB_LAUNCH_PDL((weld_scan_kernel), 1, 1024, 0, s, ctx->d_chunk_new, ctx->d_ctr, ctx->cap_active);
+    MCB_LAUNCH_PDL((weld_base_kernel), eblocks * 2, kWeldCubes, 0, s, B, ctx->d_ctr, ctx->cap_active);
     /* streaming: with a registered host destination and everything fitting, weld_emit runs range by range and
      * each finished range of vertices / normals / triangles leaves over PCIe on the copy stream meanwhile */
     constexpr int K = 8;
@@ -1387,7 +1408,7 @@ int Run::stage_weld() {
         const unsigned long long cb = stream_out ? ctx->h_bounds[3 * j] : 0ull, ce = stream_out ? ctx->h_bounds[3 * j + 3] : ~0ull;
         if (stream_out && cb == ce) continue;
 #define MCB_WELD_EMIT(NRM, VIEW)                                                                                              \
-    MCB_LAUNCH((weld_emit_kernel<NRM>), eblocks * 2, kWeldThreads, 0, s, VIEW, B, ctx->d_ctr, ctx->cap_active, ctx->cap_verts, ctx->cap_itris, \
+    MCB_LAUNCH_PDL((weld_emit_kernel<NRM, std::decay<decltype(VIEW)>::type>), eblocks * 2, kWeldThreads, 0, s, VIEW, B, ctx->d_ctr, ctx->cap_active, ctx->cap_verts, ctx->cap_itris, \
                                                                ctx->d_vlist, NRM ? ctx->d_vnrm : nullptr, ctx->d_tlist, cb, ce)
         if (ctx->normals == 1) { if (g.repeat) MCB_WELD_EMIT(true, WR); else MCB_WELD_EMIT(true, W); }
         else { if (g.repeat) MCB_WELD_EMIT(false, WR); else MCB_WELD_EMIT(false, W); }
@@ -1436,10 +1457,10 @@ int Run::stage_normal_h() {
 int Run::stage_grad_normals(bool soup) {
     const unsigned grid = (unsigned)ctx->sm_count * 8;
     if (soup)
-        MCB_LAUNCH((grad_normals_kernel<true>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, ctx->d_ctr, ctx->cap_tris,
+        MCB_LAUNCH_PDL((grad_normals_kernel<true>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, ctx->d_ctr, ctx->cap_tris,
                    (const float*)ctx->d_pos, (float*)ctx->d_nrm);
     else
-        MCB_LAUNCH((grad_normals_kernel<false>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, ctx->d_ctr, ctx->cap_verts,
+        MCB_LAUNCH_PDL((grad_normals_kernel<false>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, ctx->d_ctr, ctx->cap_verts,
                    ctx->d_vlist, ctx->d_vnrm);
     launches++;
     return MCB_OK;
@@ -1451,10 +1472,10 @@ int Run::stage_refine(bool soup) {
     const unsigned grid = (unsigned)ctx->sm_count * 8;
     const float* c = ctx->d_cs + 1; /* cs[v+1] = c[v] */
     if (soup)
-        MCB_LAUNCH((refine_vertices_kernel<true>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, g.iso, c, g.M, ctx->d_ctr, ctx->cap_tris,
+        MCB_LAUNCH_PDL((refine_vertices_kernel<true>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, g.iso, c, g.M, ctx->d_ctr, ctx->cap_tris,
                    (float*)ctx->d_pos);
     else
-        MCB_LAUNCH((refine_vertices_kernel<false>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, g.iso, c, g.M, ctx->d_ctr, ctx->cap_verts,
+        MCB_LAUNCH_PDL((refine_vertices_kernel<false>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, g.iso, c, g.M, ctx->d_ctr, ctx->cap_verts,
                    ctx->d_vlist);
     launches++;
     return MCB_OK;
@@ -1497,6 +1518,8 @@ int mcb_polygonise(mcb_ctx* ctx, mcb_counts* out) {
     const bool blocks = ctx->field_mode != MCB_FIELD_DENSE && !g.repeat;
     const bool timing = ctx->stage_timing;
     MCB_CK(cudaMemsetAsync(ctx->d_ctr, 0, sizeof(Counters), s));
+    MCB_CK(clear_tile_groups(ctx, s)); /* here, before the chain: the first classify pass starts without a clear between kernels */
+    if (blocks && (rc = run.fork_block_clears()) != MCB_OK) return rc;
     if (timing) MCB_CK(cudaEventRecord(ctx->ev[0], s));
     if ((rc = run.stage_tables()) != MCB_OK) return rc;
     if (timing) MCB_CK(cudaEventRecord(ctx->ev[1], s));
@@ -1507,8 +1530,8 @@ int mcb_polygonise(mcb_ctx* ctx, mcb_counts* out) {
     bool need_classify = true;
     for (;;) { /* repeated only when an output buffer had to grow (mcb_counts::reruns) */
         if (need_classify) {
-            if ((rc = run.stage_classify()) != MCB_OK) return rc;
-            /* several GPUs: this slab's triangle count is final now (tile_scan_kernel) — its all-gather is enqueued here, on
+            if ((rc = run.stage_classify(reruns > 0)) != MCB_OK) return rc;
+            /* several GPUs: this slab's triangle count is final now (compact_kernel's last block) — its all-gather is enqueued here, on
              * the side stream, so that NCCL's launch cost hides behind the emission instead of following the call.  Once
              * per call: a repeated pass (buffer growth) must not add a collective the other ranks do not have */
             if (ctx->comm_auto && ctx->nccl_comm && reruns == 0 && (rc = comm_enqueue(ctx)) != MCB_OK) return rc;

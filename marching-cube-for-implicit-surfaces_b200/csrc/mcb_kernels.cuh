@@ -25,6 +25,13 @@
  *   K4  weld_count/scan/base/emit        the reference's welded, indexed mesh
  *   K5  nh_*                             normal.h normals on the welded mesh
  *   K7  inspect_cube                     calculate_step for one cube (step-by-step mode)
+ *
+ * The wait rule.  The kernels of a call follow each other on one stream, most of them launched with MCB_LAUNCH_PDL
+ * (mcb_launch.h), so that a kernel's blocks are placed while its predecessor drains.  Such a kernel opens with
+ * MCB_GRID_WAIT(): before it, nothing but arithmetic on the parameters and shared-memory set-up — no global load or
+ * store, counters and atomics included.  The wait returns once the predecessor has completed and its writes are visible;
+ * that predecessor waited for its own, so everything earlier in the call is covered too.  MCB_GRID_DEPENDENTS() right
+ * after it lets the next grid be placed during this one's tail.  A kernel without the wait is launched with MCB_LAUNCH.
  */
 #pragma once
 
@@ -100,7 +107,7 @@ struct Counters {
     unsigned int error; /* 2 = 2^31 or more triangles in the slab */
     unsigned int field_blocks, amb_n; /* blocks the apron refill wrote; ambiguous cubes appended to the face-test list */
     unsigned long long nh_vertices, nh_triangles; /* what the normal.h stage works on: the mesh, or nothing when it is truncated */
-    /* ---- everything above is reset before every classify pass; what follows belongs to the evaluation stage ---- */
+    /* ---- everything above is zero before every classify pass (the call's clear, or the re-run's); what follows belongs to the evaluation stage ---- */
     unsigned int eval_blocks, eval_supers; /* block-field mode: 32 x 4 x 4 vertex blocks / 32 x 16 x 16 super-blocks the interval test could not decide */
     unsigned int emit_next, emit_done;     /* emit2: next chunk to hand out / blocks that have finished (the last one resets both) */
 };
@@ -361,6 +368,8 @@ template <bool HAS_POW, bool STORE_F, bool HAS_FN = false, bool HAS_MINMAX = fal
 __global__ void __launch_bounds__(kEvalThreads, HAS_POW || HAS_FN ? 8 : 10)
 eval_field_kernel(const __grid_constant__ mcb_program prog, const Grid g, const float* __restrict__ tables,
                   float* __restrict__ F, uint32_t* __restrict__ S, int row_groups) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     MCB_DYNAMIC_SMEM(float, stack_smem); /* [level][16][kEvalThreads] */
     const int lane = threadIdx.x & 31;
     const int cx = (int)blockIdx.x;                                            /* 128-column tile of the row */
@@ -460,6 +469,8 @@ eval_blocks_kernel(const __grid_constant__ mcb_program prog, const Grid g, const
  * and zero-filled to a multiple of 16), a warp reserves its entries with one atomic. */
 __global__ void __launch_bounds__(256)
 field_list_kernel(const FieldBlocks fb, unsigned nblocks, Counters* __restrict__ ctr) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     const unsigned g16 = blockIdx.x * blockDim.x + threadIdx.x; /* group of 16 flags */
     const int lane = threadIdx.x & 31;
     uint4 f = make_uint4(0u, 0u, 0u, 0u);
@@ -516,6 +527,8 @@ constexpr int kSuper = 4; /* blocks per super-block in y and z */
 __global__ void __launch_bounds__(128)
 axis_bounds_kernel(const float* __restrict__ tables, const Grid g, const BlockDims bd, int nsx, int nsy, int nsz,
                    mcb_ival* __restrict__ B /* [2][3][spa][nb]: level 0 blocks, level 1 super-blocks */) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     const int level = blockIdx.y;
     if (idx >= 3 * bd.spa * bd.nb) return;
@@ -554,6 +567,8 @@ __global__ void __launch_bounds__(128)
 super_class_kernel(const __grid_constant__ mcb_program prog /* fused grid program, slot numbers as arguments */, const Grid g,
                    const BlockDims bd, const mcb_ival* __restrict__ B, int decide /* 0: everything is "undecided" (tests) */,
                    uint8_t* __restrict__ scls, uint32_t* __restrict__ slist, Counters* __restrict__ ctr) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     const unsigned n = (unsigned)bd.nbx * (unsigned)bd.nsy * (unsigned)bd.nsz;
     const unsigned idx = blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
@@ -580,6 +595,8 @@ block_class_kernel(const __grid_constant__ mcb_program prog, const Grid g, const
                    uint8_t* __restrict__ flags /* preset to 0 */, uint32_t* __restrict__ list,
                    unsigned long long* __restrict__ cand /* preset to 0: one bit per cube block, cmw words per (layer group, row group) */,
                    Counters* __restrict__ ctr) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     const unsigned nsuper = ctr->eval_supers;
     const int lane = threadIdx.x & 31;
     const unsigned stride = gridDim.x * blockDim.x;
@@ -638,6 +655,8 @@ __device__ __forceinline__ void write_decided_signs(const Grid& g, uint32_t* __r
 __global__ void __launch_bounds__(256)
 decided_signs_kernel(const Grid g, const BlockDims bd, const uint32_t* __restrict__ list, const Counters* __restrict__ ctr,
                      uint8_t* __restrict__ cls, const uint8_t* __restrict__ scls, uint32_t* __restrict__ S) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     const unsigned n = ctr->eval_blocks;
     const int lane = threadIdx.x & 31;
     const unsigned nwarps = gridDim.x * (blockDim.x >> 5);
@@ -693,6 +712,8 @@ decided_signs_all_kernel(const Grid g, const BlockDims bd, uint8_t* __restrict__
 __global__ void __launch_bounds__(256)
 eval_constraint_kernel(const __grid_constant__ mcb_program prog, const Grid g, const float* __restrict__ cs,
                        int op, float rhs, int first, uint32_t* __restrict__ V, long long total_words) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     const int lane = threadIdx.x & 31;
     const long long widx = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
     if (widx >= total_words) return;
@@ -734,10 +755,11 @@ eval_constraint_kernel(const __grid_constant__ mcb_program prog, const Grid g, c
  *          the field — and, when it redirects, the bit in the item's entry and the triangle-count difference of row
  *          255-code, applied to the entry and to the tile total with atomics.  Dense lanes: a tile with one
  *          ambiguous cube no longer holds up a whole block, and the test is evaluated once, not twice.
- *     tile_scan_kernel (one block): exclusive scan of the per-tile totals; grand totals to the counters.
- *     compact_kernel (one block per tile; tiles without an active item leave at once):
- *       C2 per chunk of 32 list entries a packed shuffle scan, then one lane per active item writes its cubes'
- *          records in loop order at tile base + chunk base + lane offset.
+ *     compact_kernel (one block per tile; tiles without an active item leave at once, except the last):
+ *       C2 the tile's base: the sum of the earlier tiles' totals (final once ambiguity_kernel is done; a few thousand
+ *          words from L2); the last tile's block also writes the grand totals to the counters.  Per chunk of 32 list
+ *          entries a packed shuffle scan, then one lane per active item writes its cubes' records in loop order at
+ *          tile base + chunk base + lane offset.
  * ------------------------------------------------------------------------------------------------------------- */
 constexpr int kClsWarps = kClsThreads / 32;
 constexpr int kClsItemCap = 8192; /* items per tile: bitmap 1 KB + active-item list 16 KB of shared memory */
@@ -833,6 +855,8 @@ __device__ __forceinline__ void repeat_item_words(const uint32_t* __restrict__ C
 }
 __global__ void __launch_bounds__(256)
 repeat_words_kernel(const Grid g, const float* __restrict__ F, uint32_t WC, uint32_t* __restrict__ Cw, unsigned long long items) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     const int lane = threadIdx.x & 31;
     const size_t rowp = (size_t)g.P, planep = (size_t)g.NV * g.P;
     for (unsigned long long item = (unsigned long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); item < items;
@@ -877,13 +901,14 @@ __device__ __forceinline__ void view_item(ItemView& it, uint32_t item_local, uin
     if (V != nullptr && it.m) it.m &= valid_mask(V, idx, (uint32_t)g.WP, plane);
 }
 
-struct ClsScratch {          /* global scratch handed from classify_kernel to ambiguity / tile_scan / compact */
+constexpr uint32_t kTileGroupLog = 8, kTileGroup = 1u << kTileGroupLog; /* a group's sums stay below 2^32 */
+struct ClsScratch {          /* global scratch handed from classify_kernel to ambiguity / compact */
     unsigned long long* ent; /* [tiles][tile_items]  one entry per active item of the tile, loop order (layout above) */
     uint32_t* nz;            /* [tiles]  number of entries */
     uint32_t* tile_a;        /* [tiles]  active cubes of the tile */
     uint32_t* tile_t;        /* [tiles]  triangles of the tile (ambiguity_kernel corrects it) */
-    uint32_t* base_a;        /* [tiles]  exclusive prefixes (tile_scan_kernel) */
-    uint32_t* base_t;
+    uint32_t* grp_a;         /* [ceil(tiles / kTileGroup)]  the same sums per group of tiles, zeroed before the pass, */
+    uint32_t* grp_t;         /*   so that compact_kernel's base reads a group total per earlier group, not every tile */
     unsigned long long* amb; /* [cap_amb][2]  entry index | bit << 40 | face << 45 | code << 48 ;  i | j << 12 | k << 24 */
     uint32_t cap_amb;
     uint32_t tile_items;     /* tile_rows * WC */
@@ -901,6 +926,8 @@ __global__ void __launch_bounds__(kClsThreads, 4)
 classify_kernel(const Grid g, const ClsTables* __restrict__ gtb, const uint32_t* __restrict__ S, const uint32_t* __restrict__ V,
                 const ClsGeom q, const ClsScratch sc, Counters* __restrict__ ctr,
                 const uint32_t* __restrict__ Cw /* repeating-surface mode: corner words, else nullptr */) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     MCB_DYNAMIC_SMEM(uint32_t, cls_smem);
     uint32_t* bitmap = cls_smem;                                          /* [kClsChunkCap] one bit per item */
     uint16_t* list = reinterpret_cast<uint16_t*>(cls_smem + kClsChunkCap); /* [kClsItemCap] active items, loop order */
@@ -1080,6 +1107,8 @@ classify_kernel(const Grid g, const ClsTables* __restrict__ gtb, const uint32_t*
         sc.nz[tile] = nz;
         sc.tile_a[tile] = ta;                  /* < 2^19 cubes */
         sc.tile_t[tile] = tt;                  /* ambiguity_kernel corrects it afterwards */
+        atomicAdd(sc.grp_a + (tile >> kTileGroupLog), ta);
+        atomicAdd(sc.grp_t + (tile >> kTileGroupLog), tt);
     }
 }
 
@@ -1088,6 +1117,8 @@ template <bool REPEAT>
 __global__ void __launch_bounds__(128)
 ambiguity_kernel(const __grid_constant__ mcb_program point_prog, const Grid g, const float* __restrict__ cs,
                  const ClsTables* __restrict__ gtb, const ClsScratch sc, Counters* __restrict__ ctr, const float* __restrict__ F) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     const uint32_t n = min(ctr->amb_n, sc.cap_amb);
     uint32_t redirected = 0;
     for (uint32_t a = blockIdx.x * blockDim.x + threadIdx.x; a < n; a += gridDim.x * blockDim.x) {
@@ -1101,73 +1132,60 @@ ambiguity_kernel(const __grid_constant__ mcb_program point_prog, const Grid g, c
         /* one atomic sets the cube's redirect bit and moves the item's triangle count: the count field cannot underflow,
          * every partial sum of corrections is at least minus the triangles counted for those cubes */
         atomicAdd(sc.ent + entry, (1ull << (32 + b)) + (unsigned long long)((long long)delta * 64));
-        if (delta) atomicAdd(sc.tile_t + entry / sc.tile_items, (uint32_t)delta);
+        if (delta) {
+            const uint32_t t = (uint32_t)(entry / sc.tile_items);
+            atomicAdd(sc.tile_t + t, (uint32_t)delta);
+            atomicAdd(sc.grp_t + (t >> kTileGroupLog), (uint32_t)delta);
+        }
     }
     if (redirected) atomicAdd(&ctr->redirected, (unsigned long long)redirected);
 }
 
-/* Exclusive scan of the per-tile totals: a few thousand tiles, one block, kTileScanPer consecutive tiles per thread.
- * Grand totals -> counters. */
-constexpr int kTileScanPer = 8;
-__global__ void __launch_bounds__(1024)
-tile_scan_kernel(const ClsScratch sc, uint32_t tiles, Counters* __restrict__ ctr) {
-    __shared__ unsigned long long warp_a[32], warp_t[32];
-    __shared__ unsigned long long carry_a, carry_t;
-    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-    if (t == 0) { carry_a = 0; carry_t = 0; }
-    __syncthreads();
-    for (uint32_t b0 = 0; b0 < tiles; b0 += 1024u * kTileScanPer) {
-        const uint32_t i0 = b0 + (uint32_t)t * kTileScanPer;
-        uint32_t va[kTileScanPer], vt[kTileScanPer];
-        unsigned long long sa = 0, st = 0;
-#pragma unroll
-        for (int q = 0; q < kTileScanPer; q++) {
-            va[q] = i0 + q < tiles ? sc.tile_a[i0 + q] : 0u;
-            vt[q] = i0 + q < tiles ? sc.tile_t[i0 + q] : 0u;
-            sa += va[q]; st += vt[q];
-        }
-        unsigned long long ia = sa, it = st;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const unsigned long long ua = __shfl_up_sync(0xffffffffu, ia, d), ut = __shfl_up_sync(0xffffffffu, it, d);
-            if (lane >= d) { ia += ua; it += ut; }
-        }
-        if (lane == 31) { warp_a[warp] = ia; warp_t[warp] = it; }
-        __syncthreads();
-        unsigned long long ba = carry_a, bt = carry_t;
-        for (int w2 = 0; w2 < warp; w2++) { ba += warp_a[w2]; bt += warp_t[w2]; }
-        unsigned long long ra = ba + ia - sa, rt = bt + it - st;
-#pragma unroll
-        for (int q = 0; q < kTileScanPer; q++) {
-            if (i0 + q < tiles) { sc.base_a[i0 + q] = (uint32_t)ra; sc.base_t[i0 + q] = (uint32_t)rt; }
-            ra += va[q]; rt += vt[q];
-        }
-        __syncthreads();
-        if (t == 1023) { carry_a = ba + ia; carry_t = bt + it; }
-        __syncthreads();
-    }
-    if (t == 0) {
-        ctr->active = carry_a;
-        ctr->triangles = carry_t;
-        ctr->ambiguous = ctr->amb_n;
-        if (carry_t >= (1ull << 31)) ctr->error = 2u; /* >= 2^31 triangles in one slab: beyond any output buffer */
-    }
-}
-
 template <bool REPEAT>
-__global__ void __launch_bounds__(kClsThreads)
+__global__ void __launch_bounds__(kClsThreads, 5) /* 48 registers, as before the tile bases moved in: no spill */
 compact_kernel(const Grid g, const ClsTables* __restrict__ gtb, const uint32_t* __restrict__ S, const uint32_t* __restrict__ V,
-               const ClsGeom q, const ClsScratch sc, unsigned long long* __restrict__ rec, uint32_t* __restrict__ trioff,
-               unsigned long long cap_active, unsigned long long* __restrict__ item_info /* nullptr unless the weld needs it */,
+               const ClsGeom q, const ClsScratch sc, Counters* __restrict__ ctr, unsigned long long* __restrict__ rec,
+               uint32_t* __restrict__ trioff, unsigned long long cap_active, unsigned long long* __restrict__ item_info /* nullptr unless the weld needs it */,
                const uint32_t* __restrict__ Cw /* repeating-surface mode, else nullptr */,
                const FieldBlocks fb /* block-field mode: flags != nullptr, the apron blocks are marked here */) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     __shared__ uint32_t chunk_a[kClsChunkCap], chunk_t[kClsChunkCap]; /* per 32 list entries */
     __shared__ uint32_t warp_x[kClsWarps], warp_y[kClsWarps];
+    __shared__ unsigned long long warp_ba[kClsWarps], warp_bt[kClsWarps], base_s[2];
 
     const uint32_t tile = blockIdx.x;
     const uint32_t nz = sc.nz[tile];
-    if (nz == 0) return; /* uniform per block */
+    const bool last = tile == gridDim.x - 1u; /* the grid is one block per tile */
+    if (nz == 0 && !last) return; /* uniform per block */
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+
+    /* the tile's exclusive bases (read back from base_s in C2): every tile and group total is final once ambiguity_kernel
+     * is done; the earlier groups' totals, then the earlier tiles of this tile's group */
+    {
+        unsigned long long sa = 0, st = 0;
+        const uint32_t g0 = tile >> kTileGroupLog;
+        for (uint32_t i = threadIdx.x; i < g0; i += kClsThreads) { sa += sc.grp_a[i]; st += sc.grp_t[i]; }
+        for (uint32_t i = (g0 << kTileGroupLog) + threadIdx.x; i < tile; i += kClsThreads) { sa += sc.tile_a[i]; st += sc.tile_t[i]; }
+#pragma unroll
+        for (int d = 16; d; d >>= 1) { sa += __shfl_xor_sync(0xffffffffu, sa, d); st += __shfl_xor_sync(0xffffffffu, st, d); }
+        if (lane == 0) { warp_ba[warp] = sa; warp_bt[warp] = st; }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            unsigned long long ba = 0, bt = 0;
+#pragma unroll
+            for (int w2 = 0; w2 < kClsWarps; w2++) { ba += warp_ba[w2]; bt += warp_bt[w2]; }
+            base_s[0] = ba; base_s[1] = bt;
+            if (last) {
+                const unsigned long long total_t = bt + sc.tile_t[tile];
+                ctr->active = ba + sc.tile_a[tile];
+                ctr->triangles = total_t;
+                ctr->ambiguous = ctr->amb_n;
+                if (total_t >= (1ull << 31)) ctr->error = 2u; /* >= 2^31 triangles in one slab: beyond any output buffer */
+            }
+        }
+    }
+    if (nz == 0) return; /* the last tile's block, done with the totals */
     const unsigned long long* __restrict__ gent = sc.ent + (size_t)tile * sc.tile_items;
     const uint32_t row0 = tile * q.tile_rows;
 
@@ -1215,7 +1233,7 @@ compact_kernel(const Grid g, const ClsTables* __restrict__ gtb, const uint32_t* 
     /* ---- C2: write the compacted records in loop order -------------------------------------------------------- */
     const uint32_t WP = (uint32_t)g.WP, plane = (uint32_t)g.NV * WP, M = (uint32_t)g.M;
     const uint32_t kz0 = row0 / M, j0 = row0 - kz0 * M;
-    const unsigned long long tile_a = sc.base_a[tile], tile_t = sc.base_t[tile];
+    const unsigned long long tile_a = base_s[0], tile_t = base_s[1];
     for (uint32_t kb = (uint32_t)warp * 32u; kb < nz; kb += kClsThreads) {
         const uint32_t k = kb + (uint32_t)lane;
         const unsigned long long e = k < nz ? gent[k] : 0ull;
@@ -1305,6 +1323,8 @@ emit2_kernel(const Grid g, const float* __restrict__ cs, const float* __restrict
              const ClsTables* __restrict__ gtb, const unsigned long long* __restrict__ rec, const uint32_t* __restrict__ trioff,
              Counters* ctr, unsigned long long cap_active, unsigned long long cap_tris,
              float4* __restrict__ pos, float4* __restrict__ nrm) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     static_assert(kEmitSlots >= 12 && kEmitCubes <= 256 && kEmitCubes <= kEmitThreads, "a cube's edges fit one run; a thread per cube in phase 1");
     __shared__ float4 eslot[NORMALS ? kEmitSlots : 1];    /* crossing edge: coordinate along its axis, normal */
     __shared__ float epos_only[NORMALS ? 1 : kEmitSlots];
@@ -1780,6 +1800,8 @@ __device__ __forceinline__ uint32_t weld_load_chunk(WeldChunk& sh, const unsigne
 template <class WV>
 __global__ void __launch_bounds__(kWeldThreads)
 weld_count_kernel(const WV W, const WeldBuffers B, const Counters* __restrict__ ctr, unsigned long long cap_active) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     __shared__ WeldChunk sh;
     unsigned long long A = ctr->active;
     if (A > cap_active) A = cap_active;
@@ -1828,6 +1850,8 @@ weld_count_kernel(const WV W, const WeldBuffers B, const Counters* __restrict__ 
 __global__ void __launch_bounds__(kWeldCubes, 12)
 weld_count_fast_kernel(const WeldView W, const WeldBuffers B, const ClsTables* __restrict__ gtb, const Counters* __restrict__ ctr,
                        unsigned long long cap_active) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     __shared__ uint32_t warp_s[kWeldCubes / 32];
     const Grid& g = W.g;
     unsigned long long A = ctr->active;
@@ -1896,6 +1920,8 @@ weld_count_fast_kernel(const WeldView W, const WeldBuffers B, const ClsTables* _
 constexpr int kWeldScanPer = 8;
 __global__ void __launch_bounds__(1024)
 weld_scan_kernel(uint32_t* __restrict__ chunk_new, Counters* __restrict__ ctr, unsigned long long cap_active) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     __shared__ unsigned long long warp_tot[32];
     __shared__ unsigned long long carry_s;
     unsigned long long A = ctr->active;
@@ -1930,6 +1956,8 @@ weld_scan_kernel(uint32_t* __restrict__ chunk_new, Counters* __restrict__ ctr, u
 /* per-cube first vertex index: chunk base + exclusive scan of the new-vertex counts inside the chunk */
 __global__ void __launch_bounds__(kWeldCubes)
 weld_base_kernel(const WeldBuffers B, const Counters* __restrict__ ctr, unsigned long long cap_active) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     __shared__ uint32_t warp_s[kWeldCubes / 32];
     unsigned long long A = ctr->active;
     if (A > cap_active) A = cap_active;
@@ -1972,6 +2000,8 @@ weld_emit_kernel(const WV W, const WeldBuffers B, const Counters* __restrict__ c
                  unsigned long long cap_verts, unsigned long long cap_tris, float* __restrict__ vertex_list,
                  float* __restrict__ vertex_nrm, uint32_t* __restrict__ tri_list, unsigned long long chunk_begin,
                  unsigned long long chunk_end /* chunks [begin,end) of kWeldCubes cubes: the host streams the mesh out range by range */) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     __shared__ WeldChunk sh;
     __shared__ uint32_t eidx[kWeldCubes * 12]; /* welded vertex index of [cube][edge] */
     __shared__ uint8_t tri2cube[kWeldCubes * 5]; /* chunk-local triangle -> local cube (a cube has at most 5) */
@@ -2498,6 +2528,8 @@ template <bool SOUP>
 __global__ void __launch_bounds__(256)
 grad_normals_kernel(const __grid_constant__ mcb_program prog, float sx, float sy, float sz, const Counters* __restrict__ ctr,
                     unsigned long long cap, const float* __restrict__ pos, float* __restrict__ nrm) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     unsigned long long n = SOUP ? ctr->triangles : ctr->vertices;
     if (n > cap) n = cap;
     if (SOUP) n *= 3;
@@ -2525,6 +2557,8 @@ template <bool SOUP>
 __global__ void __launch_bounds__(256)
 refine_vertices_kernel(const __grid_constant__ mcb_program prog, float sx, float sy, float sz, float iso, const float* __restrict__ cs,
                        int M, const Counters* __restrict__ ctr, unsigned long long cap, float* __restrict__ pos) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
     unsigned long long n = SOUP ? ctr->triangles : ctr->vertices;
     if (n > cap) n = cap;
     if (SOUP) n *= 3;
