@@ -98,7 +98,9 @@ public:
 
     bool recalculate() {
         if (!ensure_ctx()) return false;
+        error_.clear();
         if (step_mode_ && !seed_mode_) { unpin_all(); return step_once(); } /* marching.cpp:386-428 */
+        if (dc_ && devices_ > 1) { error_ = "dual contouring runs on one device: a quad needs the cubes on both sides of a slab boundary"; return false; }
         if (devices_ > 1 && weld_ && !seed_mode_ && !(repeat_ && !(repeat_step_ > 0.f))) return recalculate_on_devices();
         /* reset_all_data() of the reference (marching.cpp:293-305), except that vertex_list / tri_list keep their storage
          * AND their size until the new mesh is in: the GPU streams the new Poly_Data straight into them (below) */
@@ -108,14 +110,14 @@ public:
         /* welded: the GPU builds Poly_Data's own layout (vertex_list + tri_list, numbered and welded like
          * add_step_to_poly_data, marching.cpp:599-654); unwelded: the float4 triangle soup */
         mcb_set_seed(ctx_, seed_mode_ ? 1 : 0, seed_[0], seed_[1], seed_[2]); /* marching.cpp:310-331, as a set (loop order) */
-        mcb_set_mesh_mode(ctx_, weld_ ? MCB_MESH_INDEXED : MCB_MESH_SOUP);
+        mcb_set_mesh_mode(ctx_, dc_ ? MCB_MESH_DC : weld_ ? MCB_MESH_INDEXED : MCB_MESH_SOUP);
         if (repeat_ && !(repeat_step_ > 0.f)) { /* distance 0: NaN iso levels, no cube is active */
             poly_data.vertex_list.clear(); poly_data.tri_list.clear();
             soup_.clear(); normals_soup_.clear(); vertex_normals_.clear();
             poly_data.step_data.step_i = -1;
             return true;
         }
-        if (weld_) {
+        if (weld_ || dc_) {
             /* Poly_Data's vectors, page-locked where they are, are the destination of the device's copy engine: while the
              * later parts of the mesh are still being welded the earlier ones are already crossing PCIe, and the call
              * returns with Poly_Data filled (drawer.cpp:795-801 reads it next).  That needs the vectors to be large
@@ -123,7 +125,7 @@ public:
              * repeated or shrinking configuration; a growing one takes the plain copy below once, then streams again. */
             const size_t cv = poly_data.vertex_list.size() / 3, ct = poly_data.tri_list.size() / 3;
             const bool with_n = normals_mode() == 1;
-            bool stream = cv > 0 && ct > 0 && normals_mode() <= 1 && !refine_ && (!with_n || vertex_normals_.size() / 3 >= cv);
+            bool stream = cv > 0 && ct > 0 && normals_mode() <= 1 && !refine_ && !dc_ && (!with_n || vertex_normals_.size() / 3 >= cv);
             if (stream) stream = pin(pin_v_, poly_data.vertex_list) && pin(pin_t_, poly_data.tri_list) && (!with_n || pin(pin_n_, vertex_normals_));
             mcb_set_host_output(ctx_, stream ? poly_data.vertex_list.data() : nullptr, stream ? poly_data.tri_list.data() : nullptr,
                                 stream && with_n ? vertex_normals_.data() : nullptr, stream ? cv : 0, stream ? ct : 0);
@@ -283,6 +285,13 @@ public:
      * DESIGN.md §13), on every context of set_devices; indices and counts unchanged.  false (default): the reference's
      * linear interpolation */
     void set_refined_vertices(bool b) { refine_ = b; }
+    /* true: Poly_Data holds the dual-contoured mesh (MCB_MESH_DC, DESIGN.md §14): one vertex per active cube, on the
+     * surface's sharp edges and corners, whatever set_weld says.  Normals are the analytic ones (mode 3), or normal.h's with
+     * set_reference_normals(true) and set_analytic_normals(false).  One device only: with set_devices(n > 1) recalculate()
+     * returns false and last_error() says why.  false (default): marching cubes */
+    void set_dual_contouring(bool b) { dc_ = b; }
+    /* why the last recalculate() returned false */
+    const char* last_error() const { return !error_.empty() ? error_.c_str() : ctx_ ? mcb_last_error(ctx_) : ""; }
     bool set_slab(int k_begin, int k_end) { slab_[0] = k_begin; slab_[1] = k_end; have_slab_ = true; return true; }
     const mcb_counts& last_counts() const { return counts_; }
     /* set_devices(n > 1): wall time of the phases of the last recalculate(), ms: the slabs' polygonisation (+ exchange),
@@ -325,7 +334,10 @@ private:
         if (have_slab_ && mcb_set_slab(ctx_, slab_[0], slab_[1]) != MCB_OK) return false;
         return true;
     }
-    int normals_mode() const { return normals_ ? (analytic_normals_ ? 3 : weld_ && reference_normals_ ? 2 : 1) : 0; }
+    int normals_mode() const {
+        if (dc_) return normals_ ? (reference_normals_ && !analytic_normals_ ? 2 : 3) : 0; /* mode 1 lives on grid edges */
+        return normals_ ? (analytic_normals_ ? 3 : weld_ && reference_normals_ ? 2 : 1) : 0;
+    }
     bool push_parameters() { return push_parameters(ctx_); }
     bool push_parameters(mcb_ctx* c) {
         mcb_set_grammar(c, evaluator_->grammar()); /* Evaluator::set_function_grammar */
@@ -541,6 +553,8 @@ private:
     bool reference_normals_ = false;
     bool analytic_normals_ = false;
     bool refine_ = false;
+    bool dc_ = false;
+    std::string error_;
     float repeat_step_;
     float seed_[3];
     bool cons_valid_[3], cons_use_[3];

@@ -81,6 +81,30 @@ typedef struct {
 /* What mcb_polygonise leaves in device memory (mcb_set_mesh_mode; default MCB_MESH_SOUP). */
 #define MCB_MESH_SOUP 1     /* triangle soup: 3 float4 positions (+ 3 float4 normals) per triangle, emission order */
 #define MCB_MESH_INDEXED 2  /* Poly_Data layout: welded vertex_list (xyz floats) + tri_list (3 indices per triangle) */
+/* Dual contouring (DESIGN.md §14), used alone (with MCB_MESH_SOUP or MCB_MESH_INDEXED: MCB_E_ARG): one vertex per active cube
+ * placed on the surface's sharp edges and corners, one quad (two triangles) per crossing grid edge, in the indexed-mesh
+ * buffers (mcb_get_indexed_mesh / _device, mcb_set_index_base as usual).  mcb_counts: vertices == active, triangles = the DC
+ * triangles, active / ambiguous / redirected keep their classification meaning, mesh_mode = 4.  Normals mode 0, 2 (normal.h on
+ * this mesh) and 3 (the gradient at each vertex); mode 1 is MCB_E_STATE.  mcb_polygonise returns MCB_E_STATE with seed mode,
+ * repeating-surface mode, a slab that is not the full grid or a communicator of several ranks.  Never streamed through
+ * mcb_set_host_output.  Constraints: a skipped cube has no vertex and a quad that needs it is dropped.  Crossing points are
+ * always refined; mcb_set_refine_vertices has no effect on this mesh.  The rule, fp32 without contraction, bit-identical on
+ * host and GPU (csrc/mcb_qef.h):
+ *   1 edge    each crossing grid edge (s(f) differs at its ends, s(v) = v > iso): p = mcb_set_refine_vertices' rule applied
+ *             to Marching::interp from the lower to the upper end; n = the mode 3 normal at p.  Computed once, by the first
+ *             active cube in loop order that contains the edge.  n = (0,0,0) adds no plane.
+ *   2 vertex  per active cube, its crossing edges in edge order 0..11: mass point c = (sum p_k) / m; A = sum n n^T,
+ *             r = sum n_k (n_k . (p_k - c)); cyclic Jacobi on A, pairs (0,1) (0,2) (1,2), 6 sweeps, a rotation skipped
+ *             when its off-diagonal entry is 0; eigenvalues below 0.01 * the largest dropped (x = c when the largest is 0);
+ *             x = c + sum_kept ((v_i . r) / l_i) v_i, each coordinate clamped to the cube [c[i], c[i+1]].
+ *   3 quads   each crossing grid edge whose four cubes are active (none on the grid's outer faces): emitted by the cube whose
+ *             corner (i+1, j+1, k+1) it touches, its x, y, z edges in that order, owners in loop order; vertices = the four
+ *             cubes in the order (0,0), (1,0), (1,1), (0,1) over the edge's other axes (y,z / z,x / x,y), reversed when the
+ *             lower end has s = 1, so that triangles face increasing f as the reference's tri_table triangles do; split along
+ *             the shorter diagonal (squared lengths, w0-w2 on a tie) into (w0 w1 w2)(w0 w2 w3) or (w0 w1 w3)(w1 w2 w3).
+ *   4 numbers vertex q = active cube q of mcb_get_active's order; a cube whose only crossing edges lie on the grid's outer
+ *             faces keeps a vertex no triangle uses. */
+#define MCB_MESH_DC 4
 
 /* ---- library / host-only helpers (no GPU needed) ---------------------------------------------------------- */
 
@@ -296,7 +320,7 @@ int mcb_jit_check_grammar(const char* equation, int grammar, char* log, size_t c
  * class, which never reads the field back, uses MCB_FIELD_AUTO. */
 int mcb_set_field_mode(mcb_ctx* ctx, int mode);
 
-/* MCB_MESH_SOUP, MCB_MESH_INDEXED or both (3).  The indexed mesh is what Marching::recalculate() leaves in
+/* MCB_MESH_SOUP, MCB_MESH_INDEXED or both (3), or MCB_MESH_DC alone.  The indexed mesh is what Marching::recalculate() leaves in
  * Poly_Data (marching.h:26-30): vertices welded and numbered as add_step_to_poly_data / add_point do it
  * (marching.cpp:599-654, tolerance comparator marching.h:38-54), triangles in emission order. */
 int mcb_set_mesh_mode(mcb_ctx* ctx, int mode);

@@ -23,6 +23,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libmcb200.so")
 
 MESH_SOUP, MESH_INDEXED = 1, 2
+MESH_DC = 4  # dual contouring, used alone: one vertex per active cube on sharp edges and corners (include/mcb.h, DESIGN.md §14)
 FIELD_DENSE, FIELD_SPARSE, FIELD_AUTO = 0, 1, 2
 JIT_OFF, JIT_ON, JIT_AUTO = 0, 1, 2
 GRAMMAR_REFERENCE, GRAMMAR_FUNCTIONS = 0, 1  # the reference's equation language / the same plus sin( cos( sqrt( abs( min( max(
@@ -355,7 +356,8 @@ class Context:
         self._ck(lib.mcb_set_stage_timing(self.h, int(bool(enabled))))
 
     def set_mesh_mode(self, mode):
-        """MESH_SOUP (float4 triangle soup), MESH_INDEXED (welded Poly_Data layout) or both (3)."""
+        """MESH_SOUP (float4 triangle soup), MESH_INDEXED (welded Poly_Data layout), both (3), or MESH_DC alone (the
+        dual-contoured mesh in the indexed layout, read with get_indexed_mesh)."""
         self._ck(lib.mcb_set_mesh_mode(self.h, int(mode)))
 
     def get_indexed_mesh(self, normals=False):
@@ -594,6 +596,10 @@ class Marching:
     def set_refined_vertices(self, b):
         """Extension: include/marching.h Marching::set_refined_vertices (Context.set_refine_vertices)."""
         self._ctx.set_refine_vertices(b)
+
+    def set_dual_contouring(self, b):
+        """Extension: include/marching.h Marching::set_dual_contouring — Poly_Data holds the dual-contoured mesh (MESH_DC)."""
+        self._ctx.set_mesh_mode(MESH_DC if b else MESH_INDEXED)
 
     def recalculate(self, fetch=True):
         if self._eval is None:

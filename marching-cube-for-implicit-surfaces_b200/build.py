@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmcb200.so")
 SOURCES = ["mcb_api.cu", "mcb_lower.cpp", "mcb_jit.cpp"]
 HEADERS = [os.path.join("..", "..", "tools", "headless_main.cpp"), os.path.join("..", "..", "include", "marching.h"),
-           os.path.join("..", "..", "include", "evaluator.h"), "mcb_kernels.cuh", "mcb_jit.h", "mcb_bytecode.h", "mcb_refine.h", "mcb_pow.h", "mcb_trig.h", "mcb_interval.h", "mcb_tables.h", "mcb_tri_words.inc", "mcb_lower.h",
+           os.path.join("..", "..", "include", "evaluator.h"), "mcb_kernels.cuh", "mcb_jit.h", "mcb_bytecode.h", "mcb_refine.h", "mcb_qef.h", "mcb_pow.h", "mcb_trig.h", "mcb_interval.h", "mcb_tables.h", "mcb_tri_words.inc", "mcb_lower.h",
            os.path.join("..", "..", "include", "mcb.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-fmad=false",

@@ -162,6 +162,9 @@ struct mcb_ctx {
     unsigned long long* d_vinfo = nullptr; /* per active cube: first new vertex | new-edge mask | on-vertex mask */
     uint32_t* d_chunk_new = nullptr;
     unsigned long long cap_weld = 0;       /* cubes the two arrays above are sized for */
+    float4* d_dc_slots = nullptr;          /* dual contouring: [12 * cap_dc] Hermite data per (active cube, local edge) */
+    uint32_t* d_dc_u32 = nullptr;          /* [cap_dc] triangles per cube | [cap_dc] their exclusive scan | scan block sums */
+    unsigned long long cap_dc = 0;
     cudaEvent_t ev[9] = {};
     /* sparse-field mode (mcb_set_field_mode): the field is only written in 32 x 4 x 4 vertex blocks around the surface */
     int field_mode = MCB_FIELD_DENSE;
@@ -398,6 +401,17 @@ int ensure_weld_scratch(mcb_ctx* ctx, const Grid& g) {
     MCB_CK(cudaMalloc((void**)&ctx->d_vinfo, ctx->cap_active * 8));
     MCB_CK(cudaMalloc((void**)&ctx->d_chunk_new, (ctx->cap_active / kWeldCubes + 2) * 4));
     ctx->cap_weld = ctx->cap_active;
+    return MCB_OK;
+}
+
+int ensure_dc_scratch(mcb_ctx* ctx) {
+    if (ctx->cap_dc >= ctx->cap_active && ctx->d_dc_slots) return MCB_OK;
+    cudaFree(ctx->d_dc_slots); cudaFree(ctx->d_dc_u32);
+    ctx->d_dc_slots = nullptr; ctx->d_dc_u32 = nullptr; ctx->cap_dc = 0;
+    const unsigned long long n = ctx->cap_active;
+    MCB_CK(cudaMalloc((void**)&ctx->d_dc_slots, 12 * n * sizeof(float4)));
+    MCB_CK(cudaMalloc((void**)&ctx->d_dc_u32, (2 * n + n / kScanBlock + 2) * 4));
+    ctx->cap_dc = n;
     return MCB_OK;
 }
 
@@ -639,7 +653,7 @@ void mcb_destroy(mcb_ctx* ctx) {
     cudaFree(ctx->d_rec); cudaFree(ctx->d_trioff); cudaFree(ctx->d_pos); cudaFree(ctx->d_nrm);
     cudaFree(ctx->d_vlist); cudaFree(ctx->d_vnrm); cudaFree(ctx->d_tlist); cudaFree(ctx->d_item); cudaFree(ctx->d_vinfo);
     cudaFree(ctx->d_chunk_new); cudaFree(ctx->d_fn); cudaFree(ctx->d_nh_count); cudaFree(ctx->d_nh_start); cudaFree(ctx->d_nh_cursor);
-    cudaFree(ctx->d_nh_sums); cudaFree(ctx->d_nh_adj);
+    cudaFree(ctx->d_nh_sums); cudaFree(ctx->d_nh_adj); cudaFree(ctx->d_dc_slots); cudaFree(ctx->d_dc_u32);
     cudaFree(ctx->d_mark); cudaFree(ctx->d_changed); cudaFree(ctx->d_seed_u32); cudaFree(ctx->d_rec2); cudaFree(ctx->d_trioff2);
     for (auto& e : ctx->ev) if (e) cudaEventDestroy(e);
     for (auto& e : ctx->seg_ev) if (e) cudaEventDestroy(e);
@@ -862,6 +876,7 @@ struct Run {
     int stage_normal_h();
     int stage_grad_normals(bool soup);
     int stage_refine(bool soup);
+    int stage_dc();
 };
 
 int Run::prepare_buffers() {
@@ -1481,6 +1496,28 @@ int Run::stage_refine(bool soup) {
     return MCB_OK;
 }
 
+/* K8: the dual-contoured mesh (MCB_MESH_DC) into the indexed-mesh buffers, in place of the soup and the weld */
+int Run::stage_dc() {
+    int rc;
+    if ((rc = ensure_dc_scratch(ctx)) != MCB_OK) return rc;
+    ctx->streamed = false; /* never streamed to registered host buffers */
+    const WeldView W{g, ctx->d_cs, ctx->d_F, any_constraint ? ctx->d_V : nullptr, nullptr, cg.WC};
+    const WeldBuffers B{ctx->d_rec, ctx->d_trioff, ctx->d_item, nullptr, nullptr, cg.WC};
+    const unsigned grid = (unsigned)ctx->sm_count * 8;
+    const unsigned long long n = ctx->cap_dc;
+    uint32_t *tcount = ctx->d_dc_u32, *toff = tcount + n, *sums = toff + n;
+    const unsigned long long* nd = &ctx->d_ctr->dc_n;
+    MCB_LAUNCH_PDL((dc_edges_kernel), grid, 256, 0, s, eq.point, W, ctx->d_rec, ctx->d_ctr, ctx->cap_active, ctx->d_dc_slots);
+    MCB_LAUNCH_PDL((dc_vertex_kernel), grid, 256, 0, s, W, B, ctx->d_ctr, ctx->cap_verts, (const float4*)ctx->d_dc_slots, ctx->d_vlist, tcount);
+    MCB_LAUNCH((scan_block_sums_kernel), eblocks, kScanBlock, 0, s, tcount, nd, sums);
+    MCB_LAUNCH((scan_sums_kernel), 1, kScanBlock, 0, s, sums, nd);
+    MCB_LAUNCH((scan_apply_kernel), eblocks, kScanBlock, 0, s, tcount, sums, nd, toff);
+    MCB_LAUNCH_PDL((dc_emit_kernel), grid, 256, 0, s, W, B, ctx->d_ctr, ctx->cap_verts, ctx->cap_itris, (const float*)ctx->d_vlist, tcount, toff,
+                   ctx->d_tlist);
+    launches += 6;
+    return MCB_OK;
+}
+
 } /* namespace */
 
 extern "C" {
@@ -1498,12 +1535,21 @@ int mcb_polygonise(mcb_ctx* ctx, mcb_counts* out) {
     if (ctx->repeat_on && ctx->seed_on) return fail(ctx, MCB_E_STATE, "repeating-surface mode and seed mode cannot be combined");
     if (ctx->seed_on && ctx->nccl_comm && ctx->comm_nranks > 1)
         return fail(ctx, MCB_E_STATE, "seed mode follows one component through the whole grid: it cannot be combined with z-slabs over several GPUs");
-    if (ctx->normals == 2 && !(ctx->mesh_mode & MCB_MESH_INDEXED))
+    if (ctx->normals == 2 && !(ctx->mesh_mode & (MCB_MESH_INDEXED | MCB_MESH_DC)))
         return fail(ctx, MCB_E_STATE, "normal.h normals (mode 2) are defined on the welded mesh: request MCB_MESH_INDEXED");
     if (ctx->refine && ctx->repeat_on) /* the reference extrapolates those crossing points: they are not on their edges */
         return fail(ctx, MCB_E_STATE, "refined vertices cannot be combined with repeating-surface mode");
+    const bool dc = ctx->mesh_mode == MCB_MESH_DC;
+    if (dc) {
+        if (ctx->normals == 1)
+            return fail(ctx, MCB_E_STATE, "dual contouring: normals mode 1 is defined on grid edges; use mode 0, 2 or 3");
+        if (ctx->seed_on) return fail(ctx, MCB_E_STATE, "dual contouring cannot be combined with seed mode");
+        if (ctx->repeat_on) return fail(ctx, MCB_E_STATE, "dual contouring cannot be combined with repeating-surface mode");
+        if (g.kb != 0 || g.ke != g.M || (ctx->nccl_comm && ctx->comm_nranks > 1))
+            return fail(ctx, MCB_E_STATE, "dual contouring needs the full grid on one context: a quad needs the cubes on both sides of a slab boundary");
+    }
 
-    Run run{ctx, g, ctx->eq[0], ctx->stream, false, (ctx->mesh_mode & MCB_MESH_SOUP) != 0, (ctx->mesh_mode & MCB_MESH_INDEXED) != 0,
+    Run run{ctx, g, ctx->eq[0], ctx->stream, false, (ctx->mesh_mode & MCB_MESH_SOUP) != 0, (ctx->mesh_mode & (MCB_MESH_INDEXED | MCB_MESH_DC)) != 0,
             nullptr, ClsGeom{}, 0u, (unsigned)ctx->sm_count * 4, 0u};
     for (int i = 0; i < 3; i++) run.any_constraint |= ctx->cons[i].in_use && ctx->eq[i + 1].valid;
     if ((rc = run.prepare_buffers()) != MCB_OK) return rc;
@@ -1545,9 +1591,13 @@ int mcb_polygonise(mcb_ctx* ctx, mcb_counts* out) {
         if (run.want_soup && ctx->refine && (rc = run.stage_refine(true)) != MCB_OK) return rc;
         if (run.want_soup && ctx->normals == 3 && (rc = run.stage_grad_normals(true)) != MCB_OK) return rc;
         if (timing) MCB_CK(cudaEventRecord(ctx->ev[4], s));
-        if (run.want_indexed) {
+        if (dc) {
+            if ((rc = run.stage_dc()) != MCB_OK) return rc;
+        } else if (run.want_indexed) {
             if ((rc = run.stage_weld()) != MCB_OK) return rc;
             if (ctx->refine && (rc = run.stage_refine(false)) != MCB_OK) return rc;
+        }
+        if (run.want_indexed) {
             if (ctx->normals == 2 && (rc = run.stage_normal_h()) != MCB_OK) return rc;
             if (ctx->normals == 3 && (rc = run.stage_grad_normals(false)) != MCB_OK) return rc;
         }
@@ -1690,7 +1740,7 @@ int mcb_jit_check_grammar(const char* equation, int grammar, char* log, size_t c
 }
 
 int mcb_set_mesh_mode(mcb_ctx* ctx, int mode) {
-    if (!ctx || mode < 1 || mode > 3) return MCB_E_ARG;
+    if (!ctx || !((mode >= 1 && mode <= 3) || mode == MCB_MESH_DC)) return MCB_E_ARG; /* MCB_MESH_DC is used alone */
     ctx->mesh_mode = mode;
     ctx->have_result = false;
     return MCB_OK;
@@ -1711,7 +1761,7 @@ int mcb_get_indexed_mesh(mcb_ctx* ctx, float* vertex_list, uint32_t* tri_list, f
     int rc = enter(ctx);
     if (rc != MCB_OK) return rc;
     if (!ctx->have_result) return fail(ctx, MCB_E_STATE, "mcb_polygonise has not run since the last change");
-    if (!(ctx->last.mesh_mode & MCB_MESH_INDEXED)) return fail(ctx, MCB_E_STATE, "the indexed mesh was not requested (mcb_set_mesh_mode)");
+    if (!(ctx->last.mesh_mode & (MCB_MESH_INDEXED | MCB_MESH_DC))) return fail(ctx, MCB_E_STATE, "the indexed mesh was not requested (mcb_set_mesh_mode)");
     const uint64_t Vn = ctx->last.vertices, T = ctx->last.triangles;
     if ((vertex_list || normals) && Vn > cap_vertices) return fail(ctx, MCB_E_CAPACITY, "vertex buffer too small");
     if (tri_list && T > cap_triangles) return fail(ctx, MCB_E_CAPACITY, "triangle buffer too small");
@@ -1739,7 +1789,7 @@ int mcb_set_index_base(mcb_ctx* ctx, uint32_t base) {
 int mcb_get_indexed_mesh_device(mcb_ctx* ctx, const float** vertex_list, const uint32_t** tri_list, const float** normals) {
     if (!ctx) return MCB_E_ARG;
     if (!ctx->have_result) return fail(ctx, MCB_E_STATE, "mcb_polygonise has not run since the last change");
-    if (!(ctx->last.mesh_mode & MCB_MESH_INDEXED)) return fail(ctx, MCB_E_STATE, "the indexed mesh was not requested (mcb_set_mesh_mode)");
+    if (!(ctx->last.mesh_mode & (MCB_MESH_INDEXED | MCB_MESH_DC))) return fail(ctx, MCB_E_STATE, "the indexed mesh was not requested (mcb_set_mesh_mode)");
     if (vertex_list) *vertex_list = ctx->d_vlist;
     if (tri_list) *tri_list = ctx->d_tlist;
     if (normals) *normals = ctx->normals ? ctx->d_vnrm : nullptr;

@@ -24,6 +24,7 @@
  *   K3  emit<NORMALS>                    triangle soup, one thread per crossing edge, coalesced float4 stores
  *   K4  weld_count/scan/base/emit        the reference's welded, indexed mesh
  *   K5  nh_*                             normal.h normals on the welded mesh
+ *   K8  dc_edges, dc_vertex, dc_emit     dual contouring (MCB_MESH_DC) in place of K3 / K4
  *   K7  inspect_cube                     calculate_step for one cube (step-by-step mode)
  *
  * The wait rule.  The kernels of a call follow each other on one stream, most of them launched with MCB_LAUNCH_PDL
@@ -44,6 +45,7 @@
 #include "mcb_bytecode.h"
 #include "mcb_interval.h"
 #include "mcb_launch.h"
+#include "mcb_qef.h"
 #include "mcb_refine.h"
 #include "mcb_tables.h"
 
@@ -110,6 +112,7 @@ struct Counters {
     /* ---- everything above is zero before every classify pass (the call's clear, or the re-run's); what follows belongs to the evaluation stage ---- */
     unsigned int eval_blocks, eval_supers; /* block-field mode: 32 x 4 x 4 vertex blocks / 32 x 16 x 16 super-blocks the interval test could not decide */
     unsigned int emit_next, emit_done;     /* emit2: next chunk to hand out / blocks that have finished (the last one resets both) */
+    unsigned long long dc_n;               /* dual contouring: active cubes the stage works on (active, capped by the records) */
 };
 constexpr size_t kCountersClassifyBytes = offsetof(Counters, eval_blocks);
 
@@ -2574,6 +2577,158 @@ refine_vertices_kernel(const __grid_constant__ mcb_program prog, float sx, float
         if (mcb_refine_vertex(prog.code, prog.n, prog.k, cs, M, iso, sx, sy, sz, p, nullptr) <= 0) continue;
         if (SOUP) reinterpret_cast<float4*>(pos)[q] = make_float4(p[0], p[1], p[2], 1.f);
         else { pos[3 * q] = p[0]; pos[3 * q + 1] = p[1]; pos[3 * q + 2] = p[2]; }
+    }
+}
+
+/* ---------------------------------------------------------------------------------------------------------------
+ * K8  dual contouring (MCB_MESH_DC, mcb_qef.h, DESIGN.md §14), after compact in place of the soup and the weld.  One
+ *     vertex per active cube, numbered like the record list; a cube is found through the weld's per-word look-up
+ *     (compact_kernel's item words: first record | active mask).  A cube that contains a crossing edge is active exactly
+ *     when it lies in the grid and passes the constraints (weld_cube_ok), so no sign has to be read outside the cube
+ *     that asks.
+ *       dc_edges   per active cube: Hermite data (refined coordinate, unit normal; one float4) of every crossing edge it is
+ *                  the first cube in loop order to contain, into slot 12 * record + local edge
+ *       dc_vertex  per active cube: its crossing edges' Hermite data from their computing cubes, the QEF vertex, and two
+ *                  triangles for each of its three quad edges (through its corner (i+1, j+1, k+1)) whose cubes are active
+ *       scan       exclusive scan of those counts (scan_block_sums / scan_sums / scan_apply)
+ *       dc_emit    the triangles, split along the quad's shorter diagonal
+ *     Sizes come from the device counters (dc_n = active capped by the records), so nothing waits for the host; a pass
+ *     whose buffers were too small writes what fits and is repeated.
+ * ------------------------------------------------------------------------------------------------------------- */
+__device__ __forceinline__ void dc_corners(const Grid& g, const float* __restrict__ F, int i, int j, int k, float f[8]) {
+    const size_t rowp = (size_t)g.P, planep = (size_t)g.NV * g.P;
+    const float* f0 = F + (size_t)(k - g.kb + 1) * planep + (size_t)(j + 1) * rowp + (i + 1);
+#pragma unroll
+    for (int v = 0; v < 8; v++) {
+        const int o = mcb_corner_ofs(v);
+        f[v] = __ldg(f0 + (size_t)(o >> 2) * planep + (size_t)((o >> 1) & 1) * rowp + (o & 1));
+    }
+}
+/* field value at the lower end of edge e (the end with the smaller coordinate) */
+__device__ __forceinline__ float dc_lower_value(const float f[8], int e) {
+    const int a = mcb_edge_a(e), b = mcb_edge_b(e);
+    return mcb_corner_ofs(a) < mcb_corner_ofs(b) ? f[a] : f[b];
+}
+/* the first cube in loop order that contains the grid edge and is active */
+__device__ __forceinline__ CubeEdge dc_computing_cube(const WeldView& W, int i, int j, int k, int e, const GridEdge& E) {
+    CubeEdge o{i, j, k, e};
+    weld_owner_fast(W, E, o);
+    return o;
+}
+
+__global__ void __launch_bounds__(256)
+dc_edges_kernel(const __grid_constant__ mcb_program prog, const WeldView W, const unsigned long long* __restrict__ rec,
+                Counters* __restrict__ ctr, unsigned long long cap_active, float4* __restrict__ slots) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
+    const Grid& g = W.g;
+    const unsigned long long A = ctr->active, n = A < cap_active ? A : cap_active;
+    if (blockIdx.x == 0 && threadIdx.x == 0) { ctr->vertices = A; ctr->triangles = 0ull; ctr->dc_n = n; }
+    const float* c = W.cs + 1; /* c[v] = cs[v+1] */
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long q = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += stride) {
+        const unsigned long long r = rec[q];
+        const int i = (int)(r & 0xFFF), j = (int)((r >> 12) & 0xFFF), k = (int)((r >> 24) & 0xFFF);
+        float f[8];
+        dc_corners(g, W.F, i, j, k, f);
+        for (int e = 0; e < 12; e++) {
+            if ((f[mcb_edge_a(e)] > g.iso) == (f[mcb_edge_b(e)] > g.iso)) continue;
+            const GridEdge E = grid_edge_of(i, j, k, e);
+            const CubeEdge o = dc_computing_cube(W, i, j, k, e, E);
+            if (o.i != i || o.j != j || o.k != k) continue;
+            const float lo[3] = {c[E.vx], c[E.vy], c[E.vz]};
+            const int ia = E.axis == 0 ? E.vx : E.axis == 1 ? E.vy : E.vz;
+            const bool a_low = mcb_corner_ofs(mcb_edge_a(e)) < mcb_corner_ofs(mcb_edge_b(e));
+            const float flo = a_low ? f[mcb_edge_a(e)] : f[mcb_edge_b(e)], fhi = a_low ? f[mcb_edge_b(e)] : f[mcb_edge_a(e)];
+            float h[4];
+            mcb_dc_edge(prog.code, prog.n, prog.k, c, g.M, g.iso, g.sx, g.sy, g.sz, lo, E.axis, ia, flo, fhi, h);
+            slots[12 * q + e] = make_float4(h[0], h[1], h[2], h[3]);
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256)
+dc_vertex_kernel(const WeldView W, const WeldBuffers B, const Counters* __restrict__ ctr, unsigned long long cap_verts,
+                 const float4* __restrict__ slots, float* __restrict__ vlist, uint32_t* __restrict__ tcount) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
+    const Grid& g = W.g;
+    const unsigned long long n = ctr->dc_n;
+    const float* c = W.cs + 1;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long q = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += stride) {
+        const unsigned long long r = B.rec[q];
+        const int i = (int)(r & 0xFFF), j = (int)((r >> 12) & 0xFFF), k = (int)((r >> 24) & 0xFFF);
+        float f[8];
+        dc_corners(g, W.F, i, j, k, f);
+        float pts[12][3], nrm[12][3];
+        int m = 0;
+        for (int e = 0; e < 12; e++) {
+            if ((f[mcb_edge_a(e)] > g.iso) == (f[mcb_edge_b(e)] > g.iso)) continue;
+            const GridEdge E = grid_edge_of(i, j, k, e);
+            const CubeEdge o = dc_computing_cube(W, i, j, k, e, E);
+            const uint32_t idx = weld_find_cube(B, g, o.i, o.j, o.k);
+            const float4 h = idx < n ? slots[12ull * idx + o.e] : make_float4(0.f, 0.f, 0.f, 0.f); /* else: truncated records, repeated */
+            pts[m][0] = c[E.vx]; pts[m][1] = c[E.vy]; pts[m][2] = c[E.vz];
+            pts[m][E.axis] = h.x;
+            nrm[m][0] = h.y; nrm[m][1] = h.z; nrm[m][2] = h.w;
+            m++;
+        }
+        const float lo[3] = {c[i], c[j], c[k]}, hi[3] = {c[i + 1], c[j + 1], c[k + 1]};
+        float x[3];
+        mcb_qef_vertex(pts, nrm, m, lo, hi, x, nullptr);
+        if (q < cap_verts) { vlist[3 * q] = x[0]; vlist[3 * q + 1] = x[1]; vlist[3 * q + 2] = x[2]; }
+        uint32_t t = 0;
+        for (int axis = 0; axis < 3; axis++) {
+            const int e = mcb_dc_quad_edge(axis);
+            if ((f[mcb_edge_a(e)] > g.iso) == (f[mcb_edge_b(e)] > g.iso)) continue;
+            int cb[4][3];
+            mcb_dc_quad_cubes(i, j, k, axis, false, cb);
+            bool ok = true;
+            for (int s = 1; s < 4; s++) ok = ok && weld_cube_ok(W, cb[s][0], cb[s][1], cb[s][2]);
+            if (ok) t += 2;
+        }
+        tcount[q] = t;
+    }
+}
+
+__global__ void __launch_bounds__(256)
+dc_emit_kernel(const WeldView W, const WeldBuffers B, Counters* __restrict__ ctr, unsigned long long cap_verts, unsigned long long cap_tris,
+               const float* __restrict__ vlist, const uint32_t* __restrict__ tcount, const uint32_t* __restrict__ toff,
+               uint32_t* __restrict__ tlist) {
+    MCB_GRID_WAIT();
+    MCB_GRID_DEPENDENTS();
+    const Grid& g = W.g;
+    const unsigned long long n = ctr->dc_n;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (unsigned long long q = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += stride) {
+        if (q == n - 1) ctr->triangles = (unsigned long long)toff[q] + tcount[q];
+        if (tcount[q] == 0) continue;
+        const unsigned long long r = B.rec[q];
+        const int i = (int)(r & 0xFFF), j = (int)((r >> 12) & 0xFFF), k = (int)((r >> 24) & 0xFFF);
+        float f[8];
+        dc_corners(g, W.F, i, j, k, f);
+        unsigned long long t = toff[q];
+        for (int axis = 0; axis < 3; axis++) {
+            const int e = mcb_dc_quad_edge(axis);
+            if ((f[mcb_edge_a(e)] > g.iso) == (f[mcb_edge_b(e)] > g.iso)) continue;
+            int cb[4][3];
+            mcb_dc_quad_cubes(i, j, k, axis, dc_lower_value(f, e) > g.iso, cb);
+            bool ok = true;
+            for (int s = 0; s < 4; s++) ok = ok && weld_cube_ok(W, cb[s][0], cb[s][1], cb[s][2]);
+            if (!ok) continue;
+            uint32_t w[4];
+            float p[4][3];
+            for (int s = 0; s < 4; s++) {
+                w[s] = weld_find_cube(B, g, cb[s][0], cb[s][1], cb[s][2]);
+                const unsigned long long v = w[s] < cap_verts ? w[s] : 0ull; /* else: the pass is repeated with room */
+                p[s][0] = vlist[3 * v]; p[s][1] = vlist[3 * v + 1]; p[s][2] = vlist[3 * v + 2];
+            }
+            const bool d02 = mcb_dc_split02(p[0], p[1], p[2], p[3]);
+            const uint32_t tri[6] = {w[0], w[1], d02 ? w[2] : w[3], d02 ? w[0] : w[1], w[2], w[3]};
+            for (int h = 0; h < 2; h++, t++)
+                if (t < cap_tris) { tlist[3 * t] = tri[3 * h]; tlist[3 * t + 1] = tri[3 * h + 1]; tlist[3 * t + 2] = tri[3 * h + 2]; }
+        }
     }
 }
 

@@ -10,6 +10,7 @@
 //                [--analytic-normals]   (normals from the equation's own gradient: Marching::set_analytic_normals)
 //                [--dump-normals out.bin]   (the welded vertex normals, nv*3 f32, or the soup's 3 float4 per triangle)
 //                [--refine-vertices]   (every vertex moved to the equation's root on its grid edge: Marching::set_refined_vertices)
+//                [--dual-contouring]   (the dual-contoured mesh, sharp edges and corners kept: Marching::set_dual_contouring)
 //
 // Defaults are the reference GUI's (drawer.cpp:39-44): equation "x+y", grid 0.2, scale 1.1, iso 0.
 #include <chrono>
@@ -23,7 +24,8 @@
 static int usage() {
     std::fprintf(stderr, "usage: mcb_headless [--eq S | --eq-file F] [--step h | --res n] [--scale sx sy sz] [--iso c]\n"
                          "                    [--constraint i lhs op rhs] [--no-normals] [--soup] [--ply F] [--dump F] [--repeat n] [--levels d] [--devices n]\n"
-                         "                    [--functions] [--analytic-normals] [--dump-normals F] [--refine-vertices]\n");
+                         "                    [--functions] [--analytic-normals] [--dump-normals F] [--refine-vertices]\n"
+                         "                    [--dual-contouring]\n");
     return 2;
 }
 
@@ -60,6 +62,7 @@ int main(int argc, char** argv) {
         else if (o == "--no-normals") march_maker.set_normals(false);
         else if (o == "--analytic-normals") march_maker.set_analytic_normals(true);
         else if (o == "--refine-vertices") march_maker.set_refined_vertices(true);
+        else if (o == "--dual-contouring") march_maker.set_dual_contouring(true);
         else if (o == "--soup") march_maker.set_weld(false);
         else if (o == "--ply" && need(1)) ply = argv[++a];
         else if (o == "--dump" && need(1)) dump = argv[++a];
@@ -83,7 +86,10 @@ int main(int argc, char** argv) {
     int steady_n = 0;
     for (int r = 0; r < repeat; r++) {
         const auto t0 = std::chrono::steady_clock::now();
-        if (!march_maker.recalculate()) { std::fprintf(stderr, "recalculate failed (is there a CUDA device? there is no CPU fallback)\n"); return 1; }
+        if (!march_maker.recalculate()) {
+            std::fprintf(stderr, "recalculate failed: %s (is there a CUDA device? there is no CPU fallback)\n", march_maker.last_error());
+            return 1;
+        }
         const double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
         if (ms < best_ms) best_ms = ms;
         if (r == 0) {                                   /* context creation, buffer growth; NVRTC works in the background */
