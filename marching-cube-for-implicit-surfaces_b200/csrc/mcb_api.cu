@@ -28,14 +28,49 @@ using namespace mcbk;
 
 namespace {
 
+/* Device memory (pinned host memory when Pinned) for at least size() elements of T, owned: the destructor frees it.
+ * grow(n) keeps the allocation when it holds n elements already, and otherwise replaces it without copying the
+ * contents; when the new allocation fails the buffer is left empty. */
+template <class T, bool Pinned = false>
+class Buf {
+public:
+    Buf() = default;
+    Buf(Buf&& o) noexcept { swap(o); }
+    Buf& operator=(Buf o) noexcept { swap(o); return *this; } /* the old allocation leaves with `o` */
+    ~Buf() { release(); }
+    cudaError_t grow(size_t n) {
+        if (p_ && n_ >= n) return cudaSuccess;
+        release();
+        const cudaError_t e = Pinned ? cudaMallocHost((void**)&p_, n * sizeof(T)) : cudaMalloc((void**)&p_, n * sizeof(T));
+        if (e != cudaSuccess) { p_ = nullptr; return e; }
+        n_ = n;
+        return cudaSuccess;
+    }
+    void swap(Buf& o) noexcept { std::swap(p_, o.p_); std::swap(n_, o.n_); }
+    size_t size() const { return n_; }
+    T* get() const { return p_; }
+    operator T*() const { return p_; }
+    T* operator->() const { return p_; }
+
+private:
+    void release() {
+        if (p_) Pinned ? cudaFreeHost(p_) : cudaFree(p_);
+        p_ = nullptr;
+        n_ = 0;
+    }
+    T* p_ = nullptr;
+    size_t n_ = 0;
+};
+template <class T> using PinnedBuf = Buf<T, true>;
+
 struct EqSlot {
     bool valid = false;
     mcb::Compiled c;
     mcb_program point; /* full expression at an arbitrary point */
     mcb_program grid;  /* full expression on the grid, hoisted subtrees as table operands, fused accumulator form */
-    uint32_t* d_slot_code = nullptr;
-    SlotDesc* d_slots = nullptr;
-    float* d_kpool = nullptr;
+    Buf<uint32_t> d_slot_code;
+    Buf<SlotDesc> d_slots;
+    Buf<float> d_kpool;
     int n_const = 0, n_axis = 0, max_per_axis = 1;
 };
 
@@ -67,36 +102,35 @@ struct mcb_ctx {
 
     Grid g{};
     bool grid_dirty = true;
-    float* d_cs = nullptr;
+    /* The counts cap_* below say how many items the kernels may write to the buffers beside them.  Each is at most the
+     * size of every buffer it describes: it is zeroed before they grow and set once they all have, so that a failed
+     * growth is retried by the next call. */
+    Buf<float> d_cs;
     size_t rinv_ofs = 0; /* d_cs + rinv_ofs: 1 / (c[v+1] - c[v-1]) per stored coordinate */
-    float* d_F = nullptr;
-    uint32_t* d_S = nullptr;
-    uint32_t* d_V = nullptr;
-    float* d_tables = nullptr;
-    size_t cap_F = 0, cap_S = 0, cap_V = 0, cap_tables = 0, cap_cs = 0;
-    ClsTables* d_cls = nullptr;
-    Counters* d_ctr = nullptr;
-    Counters* h_ctr = nullptr; /* pinned */
-    unsigned long long* d_ent = nullptr;    /* classify -> compact scratch: one entry per active item of every tile */
-    uint32_t* d_tile_u32 = nullptr;         /* [3][cap_tiles]: entries, active cubes, triangles of every tile; [2][tile groups]: the sums per group */
-    unsigned long long* d_amb = nullptr;    /* [cap_amb][2] ambiguous cubes awaiting the face-centre test */
+    Buf<float> d_F;
+    Buf<uint32_t> d_S;
+    Buf<uint32_t> d_V;
+    Buf<float> d_tables;
+    Buf<ClsTables> d_cls;
+    Buf<Counters> d_ctr;
+    PinnedBuf<Counters> h_ctr;
+    Buf<unsigned long long> d_ent;          /* classify -> compact scratch: one entry per active item of every tile */
+    Buf<uint32_t> d_tile_u32;               /* [3][cap_tiles]: entries, active cubes, triangles of every tile; [2][tile groups]: the sums per group */
+    Buf<unsigned long long> d_amb;          /* [cap_amb][2] ambiguous cubes awaiting the face-centre test */
     uint32_t cap_amb = 0;
-    size_t cap_tile_entries = 0;
     size_t cap_tiles = 0;
-    unsigned long long* d_rec = nullptr;
-    uint32_t* d_trioff = nullptr;
+    Buf<unsigned long long> d_rec;          /* [cap_active] */
+    Buf<uint32_t> d_trioff;                 /* [cap_active] */
     unsigned long long cap_active = 0;
-    float4* d_pos = nullptr;
-    float4* d_nrm = nullptr;
+    Buf<float4> d_pos;                      /* [3 * cap_tris] */
+    Buf<float4> d_nrm;                      /* [3 * cap_tris] with normals on, else empty */
     unsigned long long cap_tris = 0;
-    bool nrm_allocated = false;
     int mesh_mode = MCB_MESH_SOUP;
     /* welded, indexed mesh (Poly_Data layout) */
-    float* d_vlist = nullptr;      /* [3 * cap_verts] */
-    float* d_vnrm = nullptr;       /* [3 * cap_verts] */
-    uint32_t* d_tlist = nullptr;   /* [3 * cap_itris] */
+    Buf<float> d_vlist;            /* [3 * cap_verts] */
+    Buf<float> d_vnrm;             /* [3 * cap_verts] with normals on, else empty */
+    Buf<uint32_t> d_tlist;         /* [3 * cap_itris] */
     unsigned long long cap_verts = 0, cap_itris = 0;
-    bool vnrm_allocated = false;
     /* host output registered with mcb_set_host_output: the indexed mesh is streamed out while it is produced */
     float* h_out_v = nullptr;
     uint32_t* h_out_t = nullptr;
@@ -105,8 +139,8 @@ struct mcb_ctx {
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t seg_ev[9] = {};
     cudaEvent_t fork_ev[2] = {};    /* evaluation stage: decided_signs runs on copy_stream next to the block evaluation */
-    unsigned long long* d_bounds = nullptr;
-    unsigned long long* h_bounds = nullptr; /* pinned */
+    Buf<unsigned long long> d_bounds;
+    PinnedBuf<unsigned long long> h_bounds;
     bool streamed = false;                  /* the last polygonise delivered the mesh to the registered buffers */
     /* seed mode (mcb_set_seed) */
     bool seed_on = false;
@@ -126,45 +160,39 @@ struct mcb_ctx {
     float ms_compile = 0.f;        /* host time of the NVRTC compile it had to do (0 when cached) */
     bool repeat_on = false;        /* repeating-surface mode (mcb_set_repeat) */
     float repeat_step = 0.f;
-    uint32_t* d_cw = nullptr;      /* [items][8] corner words of every 32-cube item, repeating-surface mode only */
-    size_t cap_cw = 0;
+    Buf<uint32_t> d_cw;            /* [items][8] corner words of every 32-cube item, repeating-surface mode only */
     float seed[3] = {0.f, 0.f, 0.f};
     /* z-slabs over several GPUs (mcb_comm_*): the NCCL communicator and the device-side placement of this slab */
     void* nccl_comm = nullptr;
     int comm_rank = 0, comm_nranks = 1;
     cudaStream_t comm_stream = nullptr;
     cudaEvent_t comm_ready = nullptr, comm_done = nullptr;
-    unsigned long long* d_comm = nullptr;   /* [2 + nranks]: two staging slots for this slab's count, then the gathered counts */
-    unsigned long long* h_comm = nullptr;   /* pinned copy of the gathered counts */
+    Buf<unsigned long long> d_comm;         /* [2 + nranks]: two staging slots for this slab's count, then the gathered counts */
+    PinnedBuf<unsigned long long> h_comm;   /* the gathered counts */
     int comm_flip = 0;
     bool comm_pending = false;
     std::vector<double> layer_cost;         /* [M] cost of every cube layer as the last (re)balance saw it */
     std::vector<int> comm_cuts;             /* [nranks + 1] the slabs of the last (re)balance */
     bool comm_auto = false;                 /* mcb_comm_set_auto: mcb_polygonise enqueues the exchange itself, as soon as the count is final */
-    uint32_t* d_layer_hist = nullptr;       /* [cap_layer_hist] triangles per global cube layer */
-    size_t cap_layer_hist = 0;
-    uint8_t* d_mark = nullptr;
-    uint32_t* d_changed = nullptr;
-    uint32_t* d_seed_u32 = nullptr; /* keep | ktri | pa | pt, cap_seed entries each, then the block sums */
-    unsigned long long* d_rec2 = nullptr;
-    uint32_t* d_trioff2 = nullptr;
-    unsigned long long cap_seed = 0;
+    Buf<uint32_t> d_layer_hist;             /* [M] triangles per global cube layer */
+    /* seed mode, for cap_active cubes */
+    Buf<uint8_t> d_mark;
+    Buf<uint32_t> d_changed;
+    Buf<uint32_t> d_seed_u32;      /* keep | ktri | pa | pt, cap_active entries each, then the scan's block sums */
+    Buf<unsigned long long> d_rec2; /* the kept records, swapped with d_rec */
+    Buf<uint32_t> d_trioff2;
     /* normal.h normals (mcb_set_normals 2): face normals, vertex -> corner CSR */
-    float* d_fn = nullptr;
-    uint32_t* d_nh_count = nullptr;
-    uint32_t* d_nh_start = nullptr;
-    uint32_t* d_nh_cursor = nullptr;
-    uint32_t* d_nh_sums = nullptr;
-    uint32_t* d_nh_adj = nullptr;
-    unsigned long long cap_nh_verts = 0, cap_nh_tris = 0;
-    unsigned long long* d_item = nullptr;  /* per 32-cube word: first record | active mask << 32 (compact -> weld) */
-    size_t cap_items = 0;
-    unsigned long long* d_vinfo = nullptr; /* per active cube: first new vertex | new-edge mask | on-vertex mask */
-    uint32_t* d_chunk_new = nullptr;
-    unsigned long long cap_weld = 0;       /* cubes the two arrays above are sized for */
-    float4* d_dc_slots = nullptr;          /* dual contouring: [12 * cap_dc] Hermite data per (active cube, local edge) */
-    uint32_t* d_dc_u32 = nullptr;          /* [cap_dc] triangles per cube | [cap_dc] their exclusive scan | scan block sums */
-    unsigned long long cap_dc = 0;
+    Buf<float> d_fn;
+    Buf<uint32_t> d_nh_count;
+    Buf<uint32_t> d_nh_start;
+    Buf<uint32_t> d_nh_cursor;
+    Buf<uint32_t> d_nh_sums;
+    Buf<uint32_t> d_nh_adj;
+    Buf<unsigned long long> d_item;  /* per 32-cube word: first record | active mask << 32 (compact -> weld) */
+    Buf<unsigned long long> d_vinfo; /* per active cube: first new vertex | new-edge mask | on-vertex mask */
+    Buf<uint32_t> d_chunk_new;
+    Buf<float4> d_dc_slots;          /* dual contouring: [12 * cap_active] Hermite data per (active cube, local edge) */
+    Buf<uint32_t> d_dc_u32;          /* [cap_active] triangles per cube | [cap_active] their exclusive scan | scan block sums */
     cudaEvent_t ev[9] = {};
     /* sparse-field mode (mcb_set_field_mode): the field is only written in 32 x 4 x 4 vertex blocks around the surface */
     int field_mode = MCB_FIELD_DENSE;
@@ -174,17 +202,15 @@ struct mcb_ctx {
     bool stage_timing = true;      /* mcb_set_stage_timing: CUDA events around the stages (mcb_counts::ms_*) */
     uint32_t index_base = 0;        /* mcb_set_index_base: added to every index mcb_get_indexed_mesh delivers */
     uint32_t index_base_applied = 0; /* what d_tlist currently carries (0 after every polygonisation) */
-    uint8_t* d_fflags = nullptr;   /* [cap_fblocks] 2 = evaluated (undecided block), 1 = apron block to refill, 0 = untouched */
-    uint8_t* d_bcls = nullptr;     /* [cap_fblocks] interval class of every 32 x 4 x 4 vertex block */
-    uint32_t* d_flist = nullptr;   /* [cap_fblocks] apron blocks */
-    uint32_t* d_elist = nullptr;   /* [cap_fblocks] undecided blocks */
-    unsigned long long* d_cand = nullptr; /* [cap_cand] one bit per cube block that may hold an active cube */
-    uint32_t* d_slist = nullptr;   /* [cap_scls] undecided super-blocks */
-    uint8_t* d_scls = nullptr;     /* [cap_scls] interval class of every 32 x 16 x 16 super-block */
-    size_t cap_scls = 0;
+    Buf<uint8_t> d_fflags;         /* [blocks] 2 = evaluated (undecided block), 1 = apron block to refill, 0 = untouched */
+    Buf<uint8_t> d_bcls;           /* [blocks] interval class of every 32 x 4 x 4 vertex block */
+    Buf<uint32_t> d_flist;         /* [blocks] apron blocks */
+    Buf<uint32_t> d_elist;         /* [blocks] undecided blocks */
+    Buf<unsigned long long> d_cand; /* one bit per cube block that may hold an active cube */
+    Buf<uint32_t> d_slist;         /* [super-blocks] undecided super-blocks */
+    Buf<uint8_t> d_scls;           /* [super-blocks] interval class of every 32 x 16 x 16 super-block */
     BlockDims bd{};                /* block geometry of the last block-field run (mcb_get_cases completes the sign words with it) */
-    mcb_ival* d_bounds_iv = nullptr; /* [3][slots][nb] table bounds per block of each axis */
-    size_t cap_fblocks = 0, cap_cand = 0, cap_bounds_iv = 0;
+    Buf<mcb_ival> d_bounds_iv;     /* [3][slots][nb] table bounds per block of each axis */
     mcb_counts last{};
     bool have_result = false;
 };
@@ -207,15 +233,6 @@ int fail(mcb_ctx* ctx, int code, const std::string& msg) {
     return code;
 }
 
-template <class T>
-int ensure(mcb_ctx* ctx, T** p, size_t* cap, size_t need) {
-    if (*cap >= need && *p) return MCB_OK;
-    if (*p) { cudaFree(*p); *p = nullptr; *cap = 0; }
-    MCB_CK(cudaMalloc((void**)p, need * sizeof(T)));
-    *cap = need;
-    return MCB_OK;
-}
-
 /* The reference's grid loop, marching.cpp:372-377: fp32 accumulation, bound rounded from a double expression. */
 std::vector<float> reference_axis(float step) {
     std::vector<float> c;
@@ -236,13 +253,6 @@ void fill_program(mcb_program& p, const std::vector<uint32_t>& code, const std::
     std::copy(k.begin(), k.end(), p.k);
 }
 
-void free_slot(EqSlot& s) {
-    if (s.d_slot_code) cudaFree(s.d_slot_code);
-    if (s.d_slots) cudaFree(s.d_slots);
-    if (s.d_kpool) cudaFree(s.d_kpool);
-    s.d_slot_code = nullptr; s.d_slots = nullptr; s.d_kpool = nullptr;
-}
-
 int install_equation(mcb_ctx* ctx, int slot, const char* equation) {
     mcb::Compiled c;
     std::string err;
@@ -250,10 +260,6 @@ int install_equation(mcb_ctx* ctx, int slot, const char* equation) {
     if (rc != MCB_OK) return fail(ctx, rc, err);
 
     EqSlot ns;
-    struct Guard { /* frees the new slot's device memory on every early return */
-        EqSlot* s;
-        ~Guard() { if (s) free_slot(*s); }
-    } guard{&ns};
     ns.c = c;
     ns.valid = true;
     std::vector<SlotDesc> descs;
@@ -264,12 +270,12 @@ int install_equation(mcb_ctx* ctx, int slot, const char* equation) {
     }
     ns.max_per_axis = std::max(1, std::max(c.n_axis_slots[0], std::max(c.n_axis_slots[1], c.n_axis_slots[2])));
     if (!descs.empty()) {
-        MCB_CK(cudaMalloc((void**)&ns.d_slot_code, std::max<size_t>(1, c.slot_code.size()) * sizeof(uint32_t)));
-        MCB_CK(cudaMalloc((void**)&ns.d_slots, descs.size() * sizeof(SlotDesc)));
+        MCB_CK(ns.d_slot_code.grow(std::max<size_t>(1, c.slot_code.size())));
+        MCB_CK(ns.d_slots.grow(descs.size()));
         MCB_CK(cudaMemcpyAsync(ns.d_slot_code, c.slot_code.data(), c.slot_code.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
         MCB_CK(cudaMemcpyAsync(ns.d_slots, descs.data(), descs.size() * sizeof(SlotDesc), cudaMemcpyHostToDevice, ctx->stream));
     }
-    MCB_CK(cudaMalloc((void**)&ns.d_kpool, MCB_MAX_K * sizeof(float)));
+    MCB_CK(ns.d_kpool.grow(MCB_MAX_K));
     MCB_CK(cudaMemcpyAsync(ns.d_kpool, c.kpool.data(), c.kpool.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     if (ns.n_const > 0) {
         /* constant subtrees are folded ON THE DEVICE by the same interpreter that evaluates the field */
@@ -280,9 +286,7 @@ int install_equation(mcb_ctx* ctx, int slot, const char* equation) {
     MCB_CK(cudaStreamSynchronize(ctx->stream));
     fill_program(ns.point, ns.c.point_code, ns.c.kpool);
     fill_program(ns.grid, ns.c.grid_fused, ns.c.kpool);
-    free_slot(ctx->eq[slot]);
-    ctx->eq[slot] = ns;
-    guard.s = nullptr; /* the slot owns the allocations now */
+    ctx->eq[slot] = std::move(ns);
     ctx->have_result = false;
     return MCB_OK;
 }
@@ -330,104 +334,54 @@ int setup_grid(mcb_ctx* ctx) {
     for (size_t q = g.NV; q < ncs; q++) cs[q] = cs[g.NV - 1];
     for (int v = 1; v + 1 < g.NV; v++) cs[ncs + v] = 1.0f / (cs[v + 1] - cs[v - 1]);
     ctx->rinv_ofs = ncs;
-    int rc;
-    if ((rc = ensure(ctx, &ctx->d_cs, &ctx->cap_cs, cs.size())) != MCB_OK) return rc;
+    MCB_CK(ctx->d_cs.grow(cs.size()));
     MCB_CK(cudaMemcpyAsync(ctx->d_cs, cs.data(), cs.size() * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     MCB_CK(cudaStreamSynchronize(ctx->stream)); /* cs is a stack vector */
     const size_t nF = (size_t)g.NZ * g.NV * g.P + 64;
     const size_t nS = (size_t)g.NZ * g.NV * g.WP + 64;
-    if ((rc = ensure(ctx, &ctx->d_F, &ctx->cap_F, nF)) != MCB_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_S, &ctx->cap_S, nS)) != MCB_OK) return rc;
+    MCB_CK(ctx->d_F.grow(nF));
+    MCB_CK(ctx->d_S.grow(nS));
     unsigned tiles_now = 0;
     const ClsGeom cg0 = classify_geometry(ctx, g, &tiles_now);
     const size_t tiles = (size_t)tiles_now + 1;
     if (tiles > ctx->cap_tiles) {
-        if (ctx->d_tile_u32) cudaFree(ctx->d_tile_u32);
-        ctx->d_tile_u32 = nullptr;
         ctx->cap_tiles = 0;
-        MCB_CK(cudaMalloc((void**)&ctx->d_tile_u32, (3 * tiles + 2 * tile_groups(tiles)) * 4));
+        MCB_CK(ctx->d_tile_u32.grow(3 * tiles + 2 * tile_groups(tiles)));
         ctx->cap_tiles = tiles;
     }
-    const size_t entries = tiles * (size_t)cg0.tile_rows * cg0.WC; /* worst case: every item active */
-    if (entries > ctx->cap_tile_entries) {
-        if (ctx->d_ent) cudaFree(ctx->d_ent);
-        ctx->d_ent = nullptr;
-        ctx->cap_tile_entries = 0;
-        MCB_CK(cudaMalloc((void**)&ctx->d_ent, entries * 8));
-        ctx->cap_tile_entries = entries;
-    }
+    MCB_CK(ctx->d_ent.grow(tiles * (size_t)cg0.tile_rows * cg0.WC)); /* worst case: every item active */
     if (!ctx->d_amb) {
+        MCB_CK(ctx->d_amb.grow(2 * (size_t)(1u << 18)));
         ctx->cap_amb = 1u << 18;
-        MCB_CK(cudaMalloc((void**)&ctx->d_amb, (size_t)ctx->cap_amb * 16));
     }
     ctx->grid_dirty = false;
     return MCB_OK;
 }
 
-int ensure_records(mcb_ctx* ctx, unsigned long long need) {
-    if (ctx->cap_active >= need) return MCB_OK;
-    if (ctx->d_rec) cudaFree(ctx->d_rec);
-    if (ctx->d_trioff) cudaFree(ctx->d_trioff);
-    ctx->d_rec = nullptr; ctx->d_trioff = nullptr; ctx->cap_active = 0;
-    MCB_CK(cudaMalloc((void**)&ctx->d_rec, need * 8));
-    MCB_CK(cudaMalloc((void**)&ctx->d_trioff, need * 4));
-    ctx->cap_active = need;
+/* the records of cap_active cubes */
+int grow_records(mcb_ctx* ctx, unsigned long long n) {
+    if (ctx->cap_active >= n) return MCB_OK;
+    ctx->cap_active = 0;
+    MCB_CK(ctx->d_rec.grow(n));
+    MCB_CK(ctx->d_trioff.grow(n));
+    ctx->cap_active = n;
     return MCB_OK;
 }
 
-int ensure_soup(mcb_ctx* ctx, unsigned long long need, bool normals) {
-    if (ctx->cap_tris >= need && (!normals || ctx->nrm_allocated)) return MCB_OK;
-    need = std::max(need, ctx->cap_tris);
-    if (ctx->d_pos) cudaFree(ctx->d_pos);
-    if (ctx->d_nrm) cudaFree(ctx->d_nrm);
-    ctx->d_pos = nullptr; ctx->d_nrm = nullptr; ctx->cap_tris = 0; ctx->nrm_allocated = false;
-    MCB_CK(cudaMalloc((void**)&ctx->d_pos, need * 3 * sizeof(float4)));
-    if (normals) {
-        MCB_CK(cudaMalloc((void**)&ctx->d_nrm, need * 3 * sizeof(float4)));
-        ctx->nrm_allocated = true;
-    }
-    ctx->cap_tris = need;
+/* the soup of cap_tris triangles: positions, and normals unless they are off */
+int grow_soup(mcb_ctx* ctx, unsigned long long n, bool normals) {
+    if (ctx->cap_tris >= n && (!normals || ctx->d_nrm)) return MCB_OK;
+    n = std::max(n, ctx->cap_tris);
+    ctx->cap_tris = 0;
+    MCB_CK(ctx->d_pos.grow(3 * n));
+    if (normals) MCB_CK(ctx->d_nrm.grow(3 * n));
+    else ctx->d_nrm = {};
+    ctx->cap_tris = n;
     return MCB_OK;
 }
 
-int ensure_weld_scratch(mcb_ctx* ctx, const Grid& g) {
-    const size_t items = (size_t)(g.ke - g.kb) * g.M * ((g.M + 31) / 32);
-    int rc;
-    if ((rc = ensure(ctx, &ctx->d_item, &ctx->cap_items, items)) != MCB_OK) return rc;
-    if (ctx->cap_weld >= ctx->cap_active && ctx->d_vinfo) return MCB_OK;
-    if (ctx->d_vinfo) cudaFree(ctx->d_vinfo);
-    if (ctx->d_chunk_new) cudaFree(ctx->d_chunk_new);
-    ctx->d_vinfo = nullptr; ctx->d_chunk_new = nullptr; ctx->cap_weld = 0;
-    MCB_CK(cudaMalloc((void**)&ctx->d_vinfo, ctx->cap_active * 8));
-    MCB_CK(cudaMalloc((void**)&ctx->d_chunk_new, (ctx->cap_active / kWeldCubes + 2) * 4));
-    ctx->cap_weld = ctx->cap_active;
-    return MCB_OK;
-}
-
-int ensure_dc_scratch(mcb_ctx* ctx) {
-    if (ctx->cap_dc >= ctx->cap_active && ctx->d_dc_slots) return MCB_OK;
-    cudaFree(ctx->d_dc_slots); cudaFree(ctx->d_dc_u32);
-    ctx->d_dc_slots = nullptr; ctx->d_dc_u32 = nullptr; ctx->cap_dc = 0;
-    const unsigned long long n = ctx->cap_active;
-    MCB_CK(cudaMalloc((void**)&ctx->d_dc_slots, 12 * n * sizeof(float4)));
-    MCB_CK(cudaMalloc((void**)&ctx->d_dc_u32, (2 * n + n / kScanBlock + 2) * 4));
-    ctx->cap_dc = n;
-    return MCB_OK;
-}
-
-int ensure_seed_scratch(mcb_ctx* ctx) {
-    if (ctx->cap_seed >= ctx->cap_active && ctx->d_mark) return MCB_OK;
-    cudaFree(ctx->d_mark); cudaFree(ctx->d_seed_u32); cudaFree(ctx->d_rec2); cudaFree(ctx->d_trioff2);
-    ctx->d_mark = nullptr; ctx->d_seed_u32 = nullptr; ctx->d_rec2 = nullptr; ctx->d_trioff2 = nullptr; ctx->cap_seed = 0;
-    const unsigned long long n = ctx->cap_active;
-    MCB_CK(cudaMalloc((void**)&ctx->d_mark, n));
-    MCB_CK(cudaMalloc((void**)&ctx->d_seed_u32, (4 * n + n / kScanBlock + 2) * 4));
-    MCB_CK(cudaMalloc((void**)&ctx->d_rec2, n * 8));
-    MCB_CK(cudaMalloc((void**)&ctx->d_trioff2, n * 4));
-    if (!ctx->d_changed) MCB_CK(cudaMalloc((void**)&ctx->d_changed, 4));
-    ctx->cap_seed = n;
-    return MCB_OK;
-}
+/* an exclusive scan of n entries needs n / kScanBlock + 2 block sums (Run::scan) */
+size_t scan_sums(size_t n) { return n / kScanBlock + 2; }
 
 /* Marching::get_starting_seed_grid (marching.cpp:104-113), as cube indices: floor(((seed/scale) - (-1)) / step), fp32 */
 void seed_cube(const mcb_ctx* ctx, int out[3]) {
@@ -437,43 +391,19 @@ void seed_cube(const mcb_ctx* ctx, int out[3]) {
     }
 }
 
-int ensure_normal_h_scratch(mcb_ctx* ctx) {
-    if (ctx->cap_nh_verts < ctx->cap_verts || !ctx->d_nh_count) {
-        cudaFree(ctx->d_nh_count); cudaFree(ctx->d_nh_start); cudaFree(ctx->d_nh_cursor); cudaFree(ctx->d_nh_sums);
-        ctx->d_nh_count = ctx->d_nh_start = ctx->d_nh_cursor = ctx->d_nh_sums = nullptr; ctx->cap_nh_verts = 0;
-        MCB_CK(cudaMalloc((void**)&ctx->d_nh_count, ctx->cap_verts * 4));
-        MCB_CK(cudaMalloc((void**)&ctx->d_nh_start, ctx->cap_verts * 4));
-        MCB_CK(cudaMalloc((void**)&ctx->d_nh_cursor, ctx->cap_verts * 4));
-        MCB_CK(cudaMalloc((void**)&ctx->d_nh_sums, (ctx->cap_verts / kScanBlock + 2) * 4));
-        ctx->cap_nh_verts = ctx->cap_verts;
-    }
-    if (ctx->cap_nh_tris < ctx->cap_itris || !ctx->d_fn) {
-        cudaFree(ctx->d_fn); cudaFree(ctx->d_nh_adj);
-        ctx->d_fn = nullptr; ctx->d_nh_adj = nullptr; ctx->cap_nh_tris = 0;
-        MCB_CK(cudaMalloc((void**)&ctx->d_fn, ctx->cap_itris * 3 * sizeof(float)));
-        MCB_CK(cudaMalloc((void**)&ctx->d_nh_adj, ctx->cap_itris * 3 * sizeof(uint32_t)));
-        ctx->cap_nh_tris = ctx->cap_itris;
-    }
-    return MCB_OK;
-}
-
-int ensure_indexed(mcb_ctx* ctx, unsigned long long verts, unsigned long long tris, bool normals) {
-    if (ctx->cap_verts < verts || !ctx->d_vlist || (normals && !ctx->vnrm_allocated)) {
+/* the indexed mesh: cap_verts vertices, their normals unless they are off, cap_itris triangles */
+int grow_indexed(mcb_ctx* ctx, unsigned long long verts, unsigned long long tris, bool normals) {
+    if (ctx->cap_verts < verts || (normals && !ctx->d_vnrm)) {
         verts = std::max(verts, ctx->cap_verts);
-        if (ctx->d_vlist) cudaFree(ctx->d_vlist);
-        if (ctx->d_vnrm) cudaFree(ctx->d_vnrm);
-        ctx->d_vlist = nullptr; ctx->d_vnrm = nullptr; ctx->cap_verts = 0; ctx->vnrm_allocated = false;
-        MCB_CK(cudaMalloc((void**)&ctx->d_vlist, verts * 3 * sizeof(float)));
-        if (normals) {
-            MCB_CK(cudaMalloc((void**)&ctx->d_vnrm, verts * 3 * sizeof(float)));
-            ctx->vnrm_allocated = true;
-        }
+        ctx->cap_verts = 0;
+        MCB_CK(ctx->d_vlist.grow(3 * verts));
+        if (normals) MCB_CK(ctx->d_vnrm.grow(3 * verts));
+        else ctx->d_vnrm = {};
         ctx->cap_verts = verts;
     }
-    if (ctx->cap_itris < tris || !ctx->d_tlist) {
-        if (ctx->d_tlist) cudaFree(ctx->d_tlist);
-        ctx->d_tlist = nullptr; ctx->cap_itris = 0;
-        MCB_CK(cudaMalloc((void**)&ctx->d_tlist, tris * 3 * sizeof(uint32_t)));
+    if (ctx->cap_itris < tris) {
+        ctx->cap_itris = 0;
+        MCB_CK(ctx->d_tlist.grow(3 * tris));
         ctx->cap_itris = tris;
     }
     return MCB_OK;
@@ -599,10 +529,10 @@ int mcb_create(int device, mcb_ctx** out) {
         if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return bail(MCB_E_CUDA);
     for (auto& e : ctx->fork_ev)
         if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) return bail(MCB_E_CUDA);
-    if (cudaMalloc((void**)&ctx->d_bounds, 3 * 9 * 8) != cudaSuccess) return bail(MCB_E_NOMEM);
-    if (cudaMallocHost((void**)&ctx->h_bounds, 3 * 9 * 8) != cudaSuccess) return bail(MCB_E_NOMEM);
-    if (cudaMalloc((void**)&ctx->d_ctr, sizeof(Counters)) != cudaSuccess) return bail(MCB_E_NOMEM);
-    if (cudaMallocHost((void**)&ctx->h_ctr, sizeof(Counters)) != cudaSuccess) return bail(MCB_E_NOMEM);
+    if (ctx->d_bounds.grow(3 * 9) != cudaSuccess) return bail(MCB_E_NOMEM);
+    if (ctx->h_bounds.grow(3 * 9) != cudaSuccess) return bail(MCB_E_NOMEM);
+    if (ctx->d_ctr.grow(1) != cudaSuccess) return bail(MCB_E_NOMEM);
+    if (ctx->h_ctr.grow(1) != cudaSuccess) return bail(MCB_E_NOMEM);
     ClsTables tb;
     int8_t face[256];
     mcb_build_ambiguity_faces(face);
@@ -613,7 +543,7 @@ int mcb_create(int device, mcb_ctx** out) {
         tb.emask[q] = 0;
         for (int e = 0; e < 12; e++) tb.emask[q] |= (uint16_t)((((q >> mcb_edge_a(e)) ^ (q >> mcb_edge_b(e))) & 1) << e);
     }
-    if (cudaMalloc((void**)&ctx->d_cls, sizeof(ClsTables)) != cudaSuccess) return bail(MCB_E_NOMEM);
+    if (ctx->d_cls.grow(1) != cudaSuccess) return bail(MCB_E_NOMEM);
     if (cudaMemcpy(ctx->d_cls, &tb, sizeof tb, cudaMemcpyHostToDevice) != cudaSuccess) return bail(MCB_E_CUDA);
     {
         const int stack_bytes = MCB_MAX_STACK * kEvalRows * kEvalThreads * (int)sizeof(float);
@@ -643,28 +573,14 @@ void mcb_destroy(mcb_ctx* ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    for (auto& s : ctx->eq) free_slot(s);
     for (auto& kv : ctx->jit_cache) if (kv.second.lib) cudaLibraryUnload(kv.second.lib);
-    cudaFree(ctx->d_fflags); cudaFree(ctx->d_flist); cudaFree(ctx->d_cw); cudaFree(ctx->d_bcls); cudaFree(ctx->d_elist); cudaFree(ctx->d_cand); cudaFree(ctx->d_scls); cudaFree(ctx->d_slist);
-    cudaFree(ctx->d_bounds_iv); cudaFree(ctx->d_ent); cudaFree(ctx->d_tile_u32); cudaFree(ctx->d_amb);
-    cudaFree(ctx->d_cs); cudaFree(ctx->d_F); cudaFree(ctx->d_S); cudaFree(ctx->d_V); cudaFree(ctx->d_tables);
-    cudaFree(ctx->d_cls); cudaFree(ctx->d_ctr);
-    if (ctx->h_ctr) cudaFreeHost(ctx->h_ctr);
-    cudaFree(ctx->d_rec); cudaFree(ctx->d_trioff); cudaFree(ctx->d_pos); cudaFree(ctx->d_nrm);
-    cudaFree(ctx->d_vlist); cudaFree(ctx->d_vnrm); cudaFree(ctx->d_tlist); cudaFree(ctx->d_item); cudaFree(ctx->d_vinfo);
-    cudaFree(ctx->d_chunk_new); cudaFree(ctx->d_fn); cudaFree(ctx->d_nh_count); cudaFree(ctx->d_nh_start); cudaFree(ctx->d_nh_cursor);
-    cudaFree(ctx->d_nh_sums); cudaFree(ctx->d_nh_adj); cudaFree(ctx->d_dc_slots); cudaFree(ctx->d_dc_u32);
-    cudaFree(ctx->d_mark); cudaFree(ctx->d_changed); cudaFree(ctx->d_seed_u32); cudaFree(ctx->d_rec2); cudaFree(ctx->d_trioff2);
     for (auto& e : ctx->ev) if (e) cudaEventDestroy(e);
     for (auto& e : ctx->seg_ev) if (e) cudaEventDestroy(e);
     for (auto& e : ctx->fork_ev) if (e) cudaEventDestroy(e);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     mcb_comm_finalize(ctx);
-    cudaFree(ctx->d_layer_hist);
-    cudaFree(ctx->d_bounds);
-    if (ctx->h_bounds) cudaFreeHost(ctx->h_bounds);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
-    delete ctx;
+    delete ctx; /* frees the buffers, with the context's device current */
 }
 
 const char* mcb_last_error(const mcb_ctx* ctx) { return ctx ? ctx->err.c_str() : "null context"; }
@@ -697,18 +613,15 @@ int mcb_eval_points(mcb_ctx* ctx, int slot, const float* xyz, float* out, size_t
     if (slot < 0 || slot > 3 || !ctx->eq[slot].valid) return fail(ctx, MCB_E_STATE, "no equation in that slot");
     if (n == 0) return MCB_OK;
     if (!xyz || !out) return fail(ctx, MCB_E_ARG, "null buffer");
-    float *d_in = nullptr, *d_out = nullptr;
-    MCB_CK(cudaMalloc((void**)&d_in, n * 3 * sizeof(float)));
-    cudaError_t e = cudaMalloc((void**)&d_out, n * sizeof(float));
-    if (e != cudaSuccess) { cudaFree(d_in); return fail(ctx, MCB_E_NOMEM, "cudaMalloc"); }
+    Buf<float> d_in, d_out;
+    MCB_CK(d_in.grow(n * 3));
+    MCB_CK(d_out.grow(n));
     float sx = apply_scale ? ctx->scale[0] : 1.f, sy = apply_scale ? ctx->scale[1] : 1.f, sz = apply_scale ? ctx->scale[2] : 1.f;
-    cudaMemcpyAsync(d_in, xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    MCB_CK(cudaMemcpyAsync(d_in, xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     MCB_LAUNCH((eval_points_kernel), (unsigned)((n + 127) / 128), 128, 0, ctx->stream, ctx->eq[slot].point, d_in, d_out, (long long)n, sx, sy, sz);
-    cudaMemcpyAsync(out, d_out, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
-    e = cudaStreamSynchronize(ctx->stream);
-    cudaError_t e2 = cudaGetLastError();
-    cudaFree(d_in); cudaFree(d_out);
-    if (e != cudaSuccess || e2 != cudaSuccess) return fail(ctx, MCB_E_CUDA, std::string("eval_points: ") + cudaGetErrorString(e != cudaSuccess ? e : e2));
+    MCB_CK(cudaMemcpyAsync(out, d_out, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    MCB_CK(cudaStreamSynchronize(ctx->stream));
+    MCB_CK(cudaGetLastError());
     return MCB_OK;
 }
 
@@ -718,18 +631,15 @@ int mcb_eval_gradients(mcb_ctx* ctx, int slot, const float* xyz, float* grad, si
     if (slot < 0 || slot > 3 || !ctx->eq[slot].valid) return fail(ctx, MCB_E_STATE, "no equation in that slot");
     if (n == 0) return MCB_OK;
     if (!xyz || !grad) return fail(ctx, MCB_E_ARG, "null buffer");
-    float *d_in = nullptr, *d_out = nullptr;
-    MCB_CK(cudaMalloc((void**)&d_in, n * 3 * sizeof(float)));
-    cudaError_t e = cudaMalloc((void**)&d_out, n * 3 * sizeof(float));
-    if (e != cudaSuccess) { cudaFree(d_in); return fail(ctx, MCB_E_NOMEM, "cudaMalloc"); }
+    Buf<float> d_in, d_out;
+    MCB_CK(d_in.grow(n * 3));
+    MCB_CK(d_out.grow(n * 3));
     float sx = apply_scale ? ctx->scale[0] : 1.f, sy = apply_scale ? ctx->scale[1] : 1.f, sz = apply_scale ? ctx->scale[2] : 1.f;
-    cudaMemcpyAsync(d_in, xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    MCB_CK(cudaMemcpyAsync(d_in, xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
     MCB_LAUNCH((eval_gradients_kernel), (unsigned)((n + 127) / 128), 128, 0, ctx->stream, ctx->eq[slot].point, d_in, d_out, (long long)n, sx, sy, sz);
-    cudaMemcpyAsync(grad, d_out, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream);
-    e = cudaStreamSynchronize(ctx->stream);
-    cudaError_t e2 = cudaGetLastError();
-    cudaFree(d_in); cudaFree(d_out);
-    if (e != cudaSuccess || e2 != cudaSuccess) return fail(ctx, MCB_E_CUDA, std::string("eval_gradients: ") + cudaGetErrorString(e != cudaSuccess ? e : e2));
+    MCB_CK(cudaMemcpyAsync(grad, d_out, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    MCB_CK(cudaStreamSynchronize(ctx->stream));
+    MCB_CK(cudaGetLastError());
     return MCB_OK;
 }
 
@@ -787,10 +697,10 @@ int mcb_inspect_cube(mcb_ctx* ctx, float x0, float y0, float z0, mcb_step_data* 
     if (rc != MCB_OK) return rc;
     if (!out) return fail(ctx, MCB_E_ARG, "null output");
     if (!ctx->eq[0].valid) return fail(ctx, MCB_E_STATE, "no surface equation");
-    mcb_program* d_progs = nullptr;
-    StepOut* d_out = nullptr;
-    MCB_CK(cudaMalloc((void**)&d_progs, 4 * sizeof(mcb_program)));
-    if (cudaMalloc((void**)&d_out, sizeof(StepOut)) != cudaSuccess) { cudaFree(d_progs); return fail(ctx, MCB_E_NOMEM, "cudaMalloc"); }
+    Buf<mcb_program> d_progs;
+    Buf<StepOut> d_out;
+    MCB_CK(d_progs.grow(4));
+    MCB_CK(d_out.grow(1));
     InspectCons cons{};
     int slots[3] = {0, 0, 0};
     for (int i = 0; i < 3; i++) {
@@ -798,14 +708,12 @@ int mcb_inspect_cube(mcb_ctx* ctx, float x0, float y0, float z0, mcb_step_data* 
         cons.op[cons.n] = ctx->cons[i].op; cons.rhs[cons.n] = ctx->cons[i].rhs; slots[cons.n] = i + 1; cons.n++;
     }
     for (int sl = 0; sl < 4; sl++)
-        if (ctx->eq[sl].valid) cudaMemcpyAsync(d_progs + sl, &ctx->eq[sl].point, sizeof(mcb_program), cudaMemcpyHostToDevice, ctx->stream);
+        if (ctx->eq[sl].valid) MCB_CK(cudaMemcpyAsync(d_progs + sl, &ctx->eq[sl].point, sizeof(mcb_program), cudaMemcpyHostToDevice, ctx->stream));
     MCB_LAUNCH((inspect_cube_kernel), 1, 1, 0, ctx->stream, d_progs, cons, slots[0], slots[1], slots[2], x0, y0, z0, ctx->step, ctx->scale[0],
                                                   ctx->scale[1], ctx->scale[2], ctx->iso, ctx->repeat_on ? 1 : 0, ctx->repeat_step, ctx->d_cls, d_out);
-    cudaMemcpyAsync(out, d_out, sizeof(StepOut), cudaMemcpyDeviceToHost, ctx->stream);
-    cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    cudaError_t e2 = cudaGetLastError();
-    cudaFree(d_progs); cudaFree(d_out);
-    if (e != cudaSuccess || e2 != cudaSuccess) return fail(ctx, MCB_E_CUDA, std::string("inspect_cube: ") + cudaGetErrorString(e != cudaSuccess ? e : e2));
+    MCB_CK(cudaMemcpyAsync(out, d_out, sizeof(StepOut), cudaMemcpyDeviceToHost, ctx->stream));
+    MCB_CK(cudaStreamSynchronize(ctx->stream));
+    MCB_CK(cudaGetLastError());
     return MCB_OK;
 }
 
@@ -861,8 +769,9 @@ struct Run {
 
     int prepare_buffers();
     int encode_program(mcb_program& launch, bool& has_pow, bool& has_fn, bool& has_minmax, bool blocks);
-    int ensure_block_buffers(FieldBlocks* fb, BlockDims* bd);
+    int grow_block_buffers(FieldBlocks* fb, BlockDims* bd);
     int launch_block_eval(const FieldBlocks& fb, const uint32_t* list, const unsigned* count);
+    void scan(const uint32_t* in, const unsigned long long* n, uint32_t* sums, uint32_t* out);
     int fork_block_clears();
     int stage_eval_blocks();
     int stage_fill();
@@ -881,22 +790,18 @@ struct Run {
 
 int Run::prepare_buffers() {
     int rc;
-    const size_t ntab = (size_t)3 * eq.max_per_axis * g.P + 256; /* the last 128-column tile reads past the pitch */
-    if ((rc = ensure(ctx, &ctx->d_tables, &ctx->cap_tables, ntab)) != MCB_OK) return rc;
-    if (any_constraint) {
-        const size_t nS = (size_t)g.NZ * g.NV * g.WP + 64;
-        if ((rc = ensure(ctx, &ctx->d_V, &ctx->cap_V, nS)) != MCB_OK) return rc;
-    }
+    MCB_CK(ctx->d_tables.grow((size_t)3 * eq.max_per_axis * g.P + 256)); /* the last 128-column tile reads past the pitch */
+    if (any_constraint) MCB_CK(ctx->d_V.grow((size_t)g.NZ * g.NV * g.WP + 64));
     if (ctx->cap_active == 0) {
         unsigned long long guess = std::max<unsigned long long>(1ull << 16, 8ull * g.M * g.M);
         guess = std::min<unsigned long long>(guess, (unsigned long long)(g.ke - g.kb) * g.M * g.M);
-        if ((rc = ensure_records(ctx, std::max<unsigned long long>(guess, 1024))) != MCB_OK) return rc;
+        if ((rc = grow_records(ctx, std::max<unsigned long long>(guess, 1024))) != MCB_OK) return rc;
     }
-    if (want_soup && (ctx->cap_tris == 0 || (ctx->normals && !ctx->nrm_allocated))) {
-        if ((rc = ensure_soup(ctx, std::max<unsigned long long>(2 * ctx->cap_active, 1024), ctx->normals != 0)) != MCB_OK) return rc;
+    if (want_soup && (ctx->cap_tris == 0 || (ctx->normals && !ctx->d_nrm))) {
+        if ((rc = grow_soup(ctx, std::max<unsigned long long>(2 * ctx->cap_active, 1024), ctx->normals != 0)) != MCB_OK) return rc;
     }
     if (want_indexed) {
-        if ((rc = ensure_indexed(ctx, std::max<unsigned long long>(ctx->cap_verts, std::max<unsigned long long>(ctx->cap_active + ctx->cap_active / 4, 1024)),
+        if ((rc = grow_indexed(ctx, std::max<unsigned long long>(ctx->cap_verts, std::max<unsigned long long>(ctx->cap_active + ctx->cap_active / 4, 1024)),
                                  std::max<unsigned long long>(ctx->cap_itris, std::max<unsigned long long>(2 * ctx->cap_active, 1024)), ctx->normals != 0)) != MCB_OK) return rc;
     }
     return MCB_OK;
@@ -1134,7 +1039,7 @@ int Run::stage_eval() {
 }
 
 /* the 32 x 4 x 4 vertex blocks of the slab and everything indexed by them */
-int Run::ensure_block_buffers(FieldBlocks* fb, BlockDims* bd) {
+int Run::grow_block_buffers(FieldBlocks* fb, BlockDims* bd) {
     bd->nbx = g.P / kFieldBlockX;
     bd->nby = (g.NV + kFieldBlockY - 1) / kFieldBlockY;
     bd->nbz = (g.NZ + kFieldBlockZ - 1) / kFieldBlockZ;
@@ -1147,27 +1052,21 @@ int Run::ensure_block_buffers(FieldBlocks* fb, BlockDims* bd) {
     bd->ckb = (g.ke - g.kb + 3) / 4;
     const size_t nb = (size_t)bd->nbx * bd->nby * bd->nbz;
     if (nb >= (1ull << 32)) return fail(ctx, MCB_E_CAPACITY, "too many field blocks: split the grid into more z-slabs");
-    if (ctx->cap_fblocks < nb) {
-        cudaFree(ctx->d_fflags); cudaFree(ctx->d_flist); cudaFree(ctx->d_bcls); cudaFree(ctx->d_elist);
-        ctx->d_fflags = nullptr; ctx->d_flist = nullptr; ctx->d_bcls = nullptr; ctx->d_elist = nullptr; ctx->cap_fblocks = 0;
-        if (cudaMalloc((void**)&ctx->d_fflags, nb + 16) != cudaSuccess || cudaMalloc((void**)&ctx->d_flist, (nb + 16) * sizeof(uint32_t)) != cudaSuccess ||
-            cudaMalloc((void**)&ctx->d_bcls, nb + 16) != cudaSuccess || cudaMalloc((void**)&ctx->d_elist, (nb + 16) * sizeof(uint32_t)) != cudaSuccess)
-            return fail(ctx, MCB_E_NOMEM, "cudaMalloc of the field-block lists failed");
+    /* the four grow together, and zeroed: the smallest decides, so that a growth that failed part-way is completed by the
+     * next call whatever grid it brings */
+    if (std::min({ctx->d_fflags.size(), ctx->d_flist.size(), ctx->d_bcls.size(), ctx->d_elist.size()}) < nb + 16) {
+        MCB_CK(ctx->d_fflags.grow(nb + 16));
+        MCB_CK(ctx->d_flist.grow(nb + 16));
+        MCB_CK(ctx->d_bcls.grow(nb + 16));
+        MCB_CK(ctx->d_elist.grow(nb + 16));
         MCB_CK(cudaMemsetAsync(ctx->d_fflags, 0, nb + 16, s)); /* the padding field_list_kernel reads stays zero */
         MCB_CK(cudaMemsetAsync(ctx->d_bcls, 0, nb + 16, s));
-        ctx->cap_fblocks = nb;
     }
-    int rc;
-    if ((rc = ensure(ctx, &ctx->d_bounds_iv, &ctx->cap_bounds_iv, (size_t)2 * 3 * bd->spa * bd->nb)) != MCB_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_cand, &ctx->cap_cand, (size_t)((bd->WC + 63) / 64) * bd->cjb * bd->ckb)) != MCB_OK) return rc;
+    MCB_CK(ctx->d_bounds_iv.grow((size_t)2 * 3 * bd->spa * bd->nb));
+    MCB_CK(ctx->d_cand.grow((size_t)((bd->WC + 63) / 64) * bd->cjb * bd->ckb));
     const size_t nsup = (size_t)bd->nbx * bd->nsy * bd->nsz;
-    if (ctx->cap_scls < nsup) {
-        cudaFree(ctx->d_scls); cudaFree(ctx->d_slist);
-        ctx->d_scls = nullptr; ctx->d_slist = nullptr; ctx->cap_scls = 0;
-        MCB_CK(cudaMalloc((void**)&ctx->d_scls, nsup));
-        MCB_CK(cudaMalloc((void**)&ctx->d_slist, nsup * sizeof(uint32_t)));
-        ctx->cap_scls = nsup;
-    }
+    MCB_CK(ctx->d_scls.grow(nsup));
+    MCB_CK(ctx->d_slist.grow(nsup));
     *fb = FieldBlocks{bd->nbx, bd->nby, bd->nbz, ctx->d_fflags, ctx->d_flist};
     ctx->bd = *bd;
     return MCB_OK;
@@ -1211,7 +1110,7 @@ int Run::launch_block_eval(const FieldBlocks& fb, const uint32_t* list, const un
 int Run::fork_block_clears() {
     FieldBlocks fb;
     BlockDims bd;
-    int rc = ensure_block_buffers(&fb, &bd);
+    int rc = grow_block_buffers(&fb, &bd);
     if (rc != MCB_OK) return rc;
     if (ctx->poison_field) { /* tests: a read of a field value or a sign word nobody wrote must show */
         MCB_CK(cudaMemsetAsync(ctx->d_F, 0xff, (size_t)g.NZ * g.NV * g.P * sizeof(float), s));
@@ -1233,7 +1132,7 @@ int Run::fork_block_clears() {
 int Run::stage_eval_blocks() {
     FieldBlocks fb;
     BlockDims bd;
-    int rc = ensure_block_buffers(&fb, &bd);
+    int rc = grow_block_buffers(&fb, &bd);
     if (rc != MCB_OK) return rc;
     ctx->field_is_sparse = true;
     ctx->jit_used = false;
@@ -1271,7 +1170,6 @@ int Run::stage_eval_blocks() {
  * base from the tile totals before it).  `rerun`: a repeated pass after buffer growth, whose counters need resetting —
  * the first pass finds them zeroed at the start of the call, and the evaluation stage writes none of them. */
 int Run::stage_classify(bool rerun) {
-    int rc;
     if (rerun) {
         MCB_CK(cudaMemsetAsync(ctx->d_ctr, 0, kCountersClassifyBytes, s)); /* the evaluation stage's counters stay */
         MCB_CK(clear_tile_groups(ctx, s));
@@ -1280,18 +1178,22 @@ int Run::stage_classify(bool rerun) {
     const size_t ct = ctx->cap_tiles, ng = tile_groups(ct);
     const bool skip = ctx->field_is_sparse; /* the candidate map of the block-field mode */
     const ClsScratch sc{ctx->d_ent, tu, tu + ct, tu + 2 * ct, tu + 3 * ct, tu + 3 * ct + ng, ctx->d_amb, ctx->cap_amb, cg.tile_rows * cg.WC,
-                        skip ? ctx->d_cand : nullptr, (uint32_t)((g.M + 3) / 4), (uint32_t)((cg.WC + 63) / 64)};
+                        skip ? ctx->d_cand.get() : nullptr, (uint32_t)((g.M + 3) / 4), (uint32_t)((cg.WC + 63) / 64)};
     const uint32_t* cw = nullptr;
     if (g.repeat) { /* per-cube iso levels: the corner signs come from the field, item by item */
         const unsigned long long items = (unsigned long long)cg.total_rows * cg.WC;
-        if ((rc = ensure(ctx, &ctx->d_cw, &ctx->cap_cw, (size_t)items * 8)) != MCB_OK) return rc;
+        MCB_CK(ctx->d_cw.grow((size_t)items * 8));
         MCB_LAUNCH_PDL((repeat_words_kernel), (unsigned)ctx->sm_count * 8, 256, 0, s, g, ctx->d_F, cg.WC, ctx->d_cw, items);
         launches++;
         cw = ctx->d_cw;
     }
     const bool need_items = want_indexed || ctx->seed_on; /* per-word record index for the weld / the seed walk */
-    if (need_items && (rc = ensure_weld_scratch(ctx, g)) != MCB_OK) return rc;
-    unsigned long long* items = need_items ? ctx->d_item : nullptr;
+    if (need_items) { /* and the weld's scratch, sized for the records this pass writes */
+        MCB_CK(ctx->d_item.grow((size_t)cg.total_rows * cg.WC));
+        MCB_CK(ctx->d_vinfo.grow(ctx->cap_active));
+        MCB_CK(ctx->d_chunk_new.grow(ctx->cap_active / kWeldCubes + 2));
+    }
+    unsigned long long* items = need_items ? ctx->d_item.get() : nullptr;
     const unsigned amb_ctas = (unsigned)ctx->sm_count * 2;
     const FieldBlocks apron = skip ? FieldBlocks{ctx->bd.nbx, ctx->bd.nby, ctx->bd.nbz, ctx->d_fflags, ctx->d_flist} : FieldBlocks{0, 0, 0, nullptr, nullptr};
 #define MCB_CLASSIFY(HAS_V, REPEAT)                                                                                                   \
@@ -1315,7 +1217,7 @@ int Run::stage_classify(bool rerun) {
 int Run::stage_fill() {
     FieldBlocks fb;
     BlockDims bd;
-    int rc = ensure_block_buffers(&fb, &bd);
+    int rc = grow_block_buffers(&fb, &bd);
     if (rc != MCB_OK) return rc;
     const size_t nb = (size_t)fb.nbx * fb.nby * fb.nbz;
     MCB_LAUNCH_PDL((field_list_kernel), (unsigned)((nb / 16 + 256) / 256), 256, 0, s, fb, (unsigned)nb, ctx->d_ctr); /* the blocks compact_kernel marked */
@@ -1325,12 +1227,15 @@ int Run::stage_fill() {
 
 /* K6: keep the component of the seed cube (marching.cpp:42-137, 310-331) */
 int Run::stage_seed() {
-    int rc;
     MCB_CK(cudaMemcpyAsync(ctx->h_ctr, ctx->d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
     MCB_CK(cudaStreamSynchronize(s));
     if (ctx->h_ctr->active <= ctx->cap_active) { /* otherwise the records are truncated: the re-run comes first */
-        if ((rc = ensure_seed_scratch(ctx)) != MCB_OK) return rc;
-        const unsigned long long n = ctx->cap_seed;
+        const unsigned long long n = ctx->cap_active;
+        MCB_CK(ctx->d_mark.grow(n));
+        MCB_CK(ctx->d_seed_u32.grow(4 * n + scan_sums(n)));
+        MCB_CK(ctx->d_rec2.grow(n)); /* swapped with d_rec below: both hold cap_active records either way */
+        MCB_CK(ctx->d_trioff2.grow(n));
+        MCB_CK(ctx->d_changed.grow(1));
         uint32_t *keep = ctx->d_seed_u32, *ktri = keep + n, *pa = ktri + n, *pt = pa + n, *sums = pt + n;
         const SeedBuffers SB{ctx->d_rec, ctx->d_item, cg.WC, ctx->d_mark, ctx->d_changed};
         const WeldView W{g, ctx->d_cs, ctx->d_F, dV, nullptr, cg.WC};
@@ -1356,17 +1261,13 @@ int Run::stage_seed() {
         }
         const unsigned long long* na = &ctx->d_ctr->active;
         MCB_LAUNCH((seed_flags_kernel), sblocks, 256, 0, s, SB, ctx->d_cls, ctx->d_ctr, ctx->cap_active, keep, ktri);
-        MCB_LAUNCH((scan_block_sums_kernel), sblocks / 2, kScanBlock, 0, s, keep, na, sums);
-        MCB_LAUNCH((scan_sums_kernel), 1, kScanBlock, 0, s, sums, na);
-        MCB_LAUNCH((scan_apply_kernel), sblocks / 2, kScanBlock, 0, s, keep, sums, na, pa);
-        MCB_LAUNCH((scan_block_sums_kernel), sblocks / 2, kScanBlock, 0, s, ktri, na, sums);
-        MCB_LAUNCH((scan_sums_kernel), 1, kScanBlock, 0, s, sums, na);
-        MCB_LAUNCH((scan_apply_kernel), sblocks / 2, kScanBlock, 0, s, ktri, sums, na, pt);
+        scan(keep, na, sums, pa);
+        scan(ktri, na, sums, pt);
         MCB_LAUNCH((seed_scatter_kernel), sblocks, 256, 0, s, SB, keep, ktri, pa, pt, ctx->d_ctr, ctx->cap_active, ctx->d_rec2, ctx->d_trioff2);
         MCB_LAUNCH((seed_commit_kernel), 1, 1, 0, s, ctx->d_ctr);
-        std::swap(ctx->d_rec, ctx->d_rec2);
-        std::swap(ctx->d_trioff, ctx->d_trioff2);
-        launches += 9;
+        ctx->d_rec.swap(ctx->d_rec2);
+        ctx->d_trioff.swap(ctx->d_trioff2);
+        launches += 3;
         if (want_indexed) { /* the weld must only see the kept cubes: rebuild the per-word look-up from scratch */
             MCB_CK(cudaMemsetAsync(ctx->d_item, 0, (size_t)(g.ke - g.kb) * g.M * cg.WC * 8, s));
             MCB_LAUNCH((seed_items_kernel), sblocks, 256, 0, s, ctx->d_rec, g, cg.WC, ctx->d_ctr, ctx->d_item);
@@ -1376,6 +1277,14 @@ int Run::stage_seed() {
     return MCB_OK;
 }
 
+/* exclusive scan of in[0 .. *n) into out; sums: scan_sums(capacity) entries of scratch */
+void Run::scan(const uint32_t* in, const unsigned long long* n, uint32_t* sums, uint32_t* out) {
+    MCB_LAUNCH((scan_block_sums_kernel), eblocks, kScanBlock, 0, s, in, n, sums);
+    MCB_LAUNCH((scan_sums_kernel), 1, kScanBlock, 0, s, sums, n);
+    MCB_LAUNCH((scan_apply_kernel), eblocks, kScanBlock, 0, s, in, sums, n, out);
+    launches += 3;
+}
+
 /* K3: interpolation + coalesced float4 emission of the triangle soup */
 int Run::stage_soup() {
     const float* rinv = ctx->d_cs + ctx->rinv_ofs;
@@ -1383,7 +1292,7 @@ int Run::stage_soup() {
     const unsigned grid = (unsigned)ctx->sm_count * (unsigned)kEmitBlocksPerSM; /* one resident wave: emit2 hands out chunks itself */
 #define MCB_SOUP(NRM, I32)                                                                                                            \
     MCB_LAUNCH_PDL((emit2_kernel<NRM, I32>), grid, kEmitThreads, 0, s, g, ctx->d_cs, rinv, ctx->d_F, ctx->d_cls, ctx->d_rec, ctx->d_trioff, \
-               ctx->d_ctr, ctx->cap_active, ctx->cap_tris, ctx->d_pos, NRM ? ctx->d_nrm : nullptr)
+               ctx->d_ctr, ctx->cap_active, ctx->cap_tris, ctx->d_pos, NRM ? ctx->d_nrm.get() : nullptr)
     if (ctx->normals == 1) { if (idx32) MCB_SOUP(true, true); else MCB_SOUP(true, false); }
     else { if (idx32) MCB_SOUP(false, true); else MCB_SOUP(false, false); }
 #undef MCB_SOUP
@@ -1393,9 +1302,7 @@ int Run::stage_soup() {
 
 /* K4: the reference's welded, indexed mesh (Poly_Data::vertex_list / tri_list) */
 int Run::stage_weld() {
-    int rc;
-    if ((rc = ensure_weld_scratch(ctx, g)) != MCB_OK) return rc;
-    const WeldView W{g, ctx->d_cs, ctx->d_F, any_constraint ? ctx->d_V : nullptr, ctx->seed_on ? ctx->d_item : nullptr, cg.WC};
+    const WeldView W{g, ctx->d_cs, ctx->d_F, any_constraint ? ctx->d_V.get() : nullptr, ctx->seed_on ? ctx->d_item.get() : nullptr, cg.WC};
     const WeldViewT<true> WR{W.g, W.cs, W.F, W.V, W.present, W.WC}; /* repeating-surface mode: same view, level checks compiled in */
     const WeldBuffers B{ctx->d_rec, ctx->d_trioff, ctx->d_item, ctx->d_vinfo, ctx->d_chunk_new, cg.WC};
     if (g.repeat) MCB_LAUNCH_PDL((weld_count_kernel<WeldViewT<true>>), eblocks * 2, kWeldThreads, 0, s, WR, B, ctx->d_ctr, ctx->cap_active);
@@ -1424,7 +1331,7 @@ int Run::stage_weld() {
         if (stream_out && cb == ce) continue;
 #define MCB_WELD_EMIT(NRM, VIEW)                                                                                              \
     MCB_LAUNCH_PDL((weld_emit_kernel<NRM, std::decay<decltype(VIEW)>::type>), eblocks * 2, kWeldThreads, 0, s, VIEW, B, ctx->d_ctr, ctx->cap_active, ctx->cap_verts, ctx->cap_itris, \
-                                                               ctx->d_vlist, NRM ? ctx->d_vnrm : nullptr, ctx->d_tlist, cb, ce)
+                                                               ctx->d_vlist, NRM ? ctx->d_vnrm.get() : nullptr, ctx->d_tlist, cb, ce)
         if (ctx->normals == 1) { if (g.repeat) MCB_WELD_EMIT(true, WR); else MCB_WELD_EMIT(true, W); }
         else { if (g.repeat) MCB_WELD_EMIT(false, WR); else MCB_WELD_EMIT(false, W); }
 #undef MCB_WELD_EMIT
@@ -1452,19 +1359,21 @@ int Run::stage_weld() {
 
 /* K5: CalculateNormal (normal.h:3-42) on the welded mesh, bit-exact */
 int Run::stage_normal_h() {
-    int rc;
-    if ((rc = ensure_normal_h_scratch(ctx)) != MCB_OK) return rc;
+    MCB_CK(ctx->d_nh_count.grow(ctx->cap_verts));
+    MCB_CK(ctx->d_nh_start.grow(ctx->cap_verts));
+    MCB_CK(ctx->d_nh_cursor.grow(ctx->cap_verts));
+    MCB_CK(ctx->d_nh_sums.grow(scan_sums(ctx->cap_verts)));
+    MCB_CK(ctx->d_fn.grow(3 * ctx->cap_itris));
+    MCB_CK(ctx->d_nh_adj.grow(3 * ctx->cap_itris));
     const unsigned long long* nv = &ctx->d_ctr->nh_vertices;
     MCB_LAUNCH((nh_gate_kernel), 1, 1, 0, s, ctx->d_ctr, ctx->cap_active, ctx->cap_verts, ctx->cap_itris);
     MCB_CK(cudaMemsetAsync(ctx->d_nh_count, 0, ctx->cap_verts * 4, s));
     MCB_CK(cudaMemsetAsync(ctx->d_nh_cursor, 0, ctx->cap_verts * 4, s));
     MCB_LAUNCH((nh_face_normals_kernel), eblocks * 2, 256, 0, s, ctx->d_vlist, ctx->d_tlist, ctx->d_ctr, ctx->cap_itris, ctx->d_fn, ctx->d_nh_count);
-    MCB_LAUNCH((scan_block_sums_kernel), eblocks, kScanBlock, 0, s, ctx->d_nh_count, nv, ctx->d_nh_sums);
-    MCB_LAUNCH((scan_sums_kernel), 1, kScanBlock, 0, s, ctx->d_nh_sums, nv);
-    MCB_LAUNCH((scan_apply_kernel), eblocks, kScanBlock, 0, s, ctx->d_nh_count, ctx->d_nh_sums, nv, ctx->d_nh_start);
+    scan(ctx->d_nh_count, nv, ctx->d_nh_sums, ctx->d_nh_start);
     MCB_LAUNCH((nh_fill_kernel), eblocks * 2, 256, 0, s, ctx->d_tlist, ctx->d_ctr, ctx->cap_itris, ctx->d_nh_start, ctx->d_nh_cursor, ctx->d_nh_adj);
     MCB_LAUNCH((nh_accumulate_kernel), eblocks * 4, 128, 0, s, ctx->d_fn, ctx->d_nh_start, ctx->d_nh_count, ctx->d_nh_adj, ctx->d_ctr, ctx->cap_verts, ctx->d_vnrm);
-    launches += 7;
+    launches += 4;
     return MCB_OK;
 }
 
@@ -1473,7 +1382,7 @@ int Run::stage_grad_normals(bool soup) {
     const unsigned grid = (unsigned)ctx->sm_count * 8;
     if (soup)
         MCB_LAUNCH_PDL((grad_normals_kernel<true>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, ctx->d_ctr, ctx->cap_tris,
-                   (const float*)ctx->d_pos, (float*)ctx->d_nrm);
+                   (const float*)ctx->d_pos.get(), (float*)ctx->d_nrm.get());
     else
         MCB_LAUNCH_PDL((grad_normals_kernel<false>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, ctx->d_ctr, ctx->cap_verts,
                    ctx->d_vlist, ctx->d_vnrm);
@@ -1488,7 +1397,7 @@ int Run::stage_refine(bool soup) {
     const float* c = ctx->d_cs + 1; /* cs[v+1] = c[v] */
     if (soup)
         MCB_LAUNCH_PDL((refine_vertices_kernel<true>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, g.iso, c, g.M, ctx->d_ctr, ctx->cap_tris,
-                   (float*)ctx->d_pos);
+                   (float*)ctx->d_pos.get());
     else
         MCB_LAUNCH_PDL((refine_vertices_kernel<false>), grid, 256, 0, s, eq.point, g.sx, g.sy, g.sz, g.iso, c, g.M, ctx->d_ctr, ctx->cap_verts,
                    ctx->d_vlist);
@@ -1498,23 +1407,21 @@ int Run::stage_refine(bool soup) {
 
 /* K8: the dual-contoured mesh (MCB_MESH_DC) into the indexed-mesh buffers, in place of the soup and the weld */
 int Run::stage_dc() {
-    int rc;
-    if ((rc = ensure_dc_scratch(ctx)) != MCB_OK) return rc;
+    const unsigned long long n = ctx->cap_active;
+    MCB_CK(ctx->d_dc_slots.grow(12 * n));
+    MCB_CK(ctx->d_dc_u32.grow(2 * n + scan_sums(n)));
     ctx->streamed = false; /* never streamed to registered host buffers */
-    const WeldView W{g, ctx->d_cs, ctx->d_F, any_constraint ? ctx->d_V : nullptr, nullptr, cg.WC};
+    const WeldView W{g, ctx->d_cs, ctx->d_F, any_constraint ? ctx->d_V.get() : nullptr, nullptr, cg.WC};
     const WeldBuffers B{ctx->d_rec, ctx->d_trioff, ctx->d_item, nullptr, nullptr, cg.WC};
     const unsigned grid = (unsigned)ctx->sm_count * 8;
-    const unsigned long long n = ctx->cap_dc;
     uint32_t *tcount = ctx->d_dc_u32, *toff = tcount + n, *sums = toff + n;
     const unsigned long long* nd = &ctx->d_ctr->dc_n;
     MCB_LAUNCH_PDL((dc_edges_kernel), grid, 256, 0, s, eq.point, W, ctx->d_rec, ctx->d_ctr, ctx->cap_active, ctx->d_dc_slots);
     MCB_LAUNCH_PDL((dc_vertex_kernel), grid, 256, 0, s, W, B, ctx->d_ctr, ctx->cap_verts, (const float4*)ctx->d_dc_slots, ctx->d_vlist, tcount);
-    MCB_LAUNCH((scan_block_sums_kernel), eblocks, kScanBlock, 0, s, tcount, nd, sums);
-    MCB_LAUNCH((scan_sums_kernel), 1, kScanBlock, 0, s, sums, nd);
-    MCB_LAUNCH((scan_apply_kernel), eblocks, kScanBlock, 0, s, tcount, sums, nd, toff);
+    scan(tcount, nd, sums, toff);
     MCB_LAUNCH_PDL((dc_emit_kernel), grid, 256, 0, s, W, B, ctx->d_ctr, ctx->cap_verts, ctx->cap_itris, (const float*)ctx->d_vlist, tcount, toff,
                    ctx->d_tlist);
-    launches += 6;
+    launches += 3;
     return MCB_OK;
 }
 
@@ -1553,7 +1460,7 @@ int mcb_polygonise(mcb_ctx* ctx, mcb_counts* out) {
             nullptr, ClsGeom{}, 0u, (unsigned)ctx->sm_count * 4, 0u};
     for (int i = 0; i < 3; i++) run.any_constraint |= ctx->cons[i].in_use && ctx->eq[i + 1].valid;
     if ((rc = run.prepare_buffers()) != MCB_OK) return rc;
-    run.dV = run.any_constraint ? ctx->d_V : nullptr;
+    run.dV = run.any_constraint ? ctx->d_V.get() : nullptr;
     run.cg = classify_geometry(ctx, g, &run.tiles);
     cudaStream_t s = ctx->stream;
     uint32_t reruns = 0;
@@ -1612,27 +1519,26 @@ int mcb_polygonise(mcb_ctx* ctx, mcb_counts* out) {
         bool again = false;
         need_classify = false;
         if (needA > ctx->cap_active) {
-            if ((rc = ensure_records(ctx, needA + needA / 8 + 1024)) != MCB_OK) return rc;
+            if ((rc = grow_records(ctx, needA + needA / 8 + 1024)) != MCB_OK) return rc;
             need_classify = true;
             again = true;
         }
         if (ctx->h_ctr->amb_n > ctx->cap_amb) { /* more ambiguous cubes than the face-test list holds: counts are provisional */
             const uint32_t want = ctx->h_ctr->amb_n + ctx->h_ctr->amb_n / 8 + 1024;
-            cudaFree(ctx->d_amb);
-            ctx->d_amb = nullptr; ctx->cap_amb = 0;
-            MCB_CK(cudaMalloc((void**)&ctx->d_amb, (size_t)want * 16));
+            ctx->cap_amb = 0;
+            MCB_CK(ctx->d_amb.grow(2 * (size_t)want));
             ctx->cap_amb = want;
             need_classify = true;
             again = true;
         }
         if (run.want_soup && needT > ctx->cap_tris) {
-            if ((rc = ensure_soup(ctx, needT + needT / 8 + 1024, ctx->normals != 0)) != MCB_OK) return rc;
+            if ((rc = grow_soup(ctx, needT + needT / 8 + 1024, ctx->normals != 0)) != MCB_OK) return rc;
             again = true;
         }
         if (run.want_indexed && (needT > ctx->cap_itris || needV > ctx->cap_verts || need_classify)) {
             /* with truncated records the vertex count is a lower bound: size generously, the re-run settles it */
             const unsigned long long v = std::max(needV + needV / 8 + 1024, need_classify ? needA + needA / 4 : 0ull);
-            if ((rc = ensure_indexed(ctx, v, needT + needT / 8 + 1024, ctx->normals != 0)) != MCB_OK) return rc;
+            if ((rc = grow_indexed(ctx, v, needT + needT / 8 + 1024, ctx->normals != 0)) != MCB_OK) return rc;
             again = true;
         }
         if (!again) break;
@@ -1792,21 +1698,21 @@ int mcb_get_indexed_mesh_device(mcb_ctx* ctx, const float** vertex_list, const u
     if (!(ctx->last.mesh_mode & (MCB_MESH_INDEXED | MCB_MESH_DC))) return fail(ctx, MCB_E_STATE, "the indexed mesh was not requested (mcb_set_mesh_mode)");
     if (vertex_list) *vertex_list = ctx->d_vlist;
     if (tri_list) *tri_list = ctx->d_tlist;
-    if (normals) *normals = ctx->normals ? ctx->d_vnrm : nullptr;
+    if (normals) *normals = ctx->normals ? ctx->d_vnrm.get() : nullptr;
     return MCB_OK;
 }
 
 int mcb_counts_device(mcb_ctx* ctx, const uint64_t** counts) {
     if (!ctx || !counts) return MCB_E_ARG;
-    *counts = reinterpret_cast<const uint64_t*>(ctx->d_ctr);
+    *counts = reinterpret_cast<const uint64_t*>(ctx->d_ctr.get());
     return MCB_OK;
 }
 
 int mcb_get_mesh_device(mcb_ctx* ctx, const float** pos4, const float** nrm4) {
     if (!ctx) return MCB_E_ARG;
     if (!ctx->have_result) return fail(ctx, MCB_E_STATE, "mcb_polygonise has not run since the last change");
-    if (pos4) *pos4 = (const float*)ctx->d_pos;
-    if (nrm4) *nrm4 = ctx->normals == 1 || ctx->normals == 3 ? (const float*)ctx->d_nrm : nullptr;
+    if (pos4) *pos4 = (const float*)ctx->d_pos.get();
+    if (nrm4) *nrm4 = ctx->normals == 1 || ctx->normals == 3 ? (const float*)ctx->d_nrm.get() : nullptr;
     return MCB_OK;
 }
 
@@ -1822,19 +1728,17 @@ int mcb_get_cases(mcb_ctx* ctx, uint8_t* cube_code, uint8_t* table_idx) {
         const unsigned nblocks = (unsigned)ctx->bd.nbx * (unsigned)ctx->bd.nby * (unsigned)ctx->bd.nbz;
         MCB_LAUNCH((decided_signs_all_kernel), (nblocks + 255) / 256, 256, 0, ctx->stream, g, ctx->bd, ctx->d_bcls, ctx->d_scls, ctx->d_S);
     }
-    uint8_t *d_code = nullptr, *d_tidx = nullptr;
-    MCB_CK(cudaMalloc((void**)&d_code, (size_t)n));
-    if (cudaMalloc((void**)&d_tidx, (size_t)n) != cudaSuccess) { cudaFree(d_code); return fail(ctx, MCB_E_NOMEM, "cudaMalloc"); }
-    MCB_LAUNCH((dense_codes_kernel), (unsigned)((n + 255) / 256), 256, 0, ctx->stream, g, ctx->d_S, any_constraint ? ctx->d_V : nullptr, d_code, d_tidx, n,
-                                                                             g.repeat ? ctx->d_cw : nullptr, (uint32_t)((g.M + 31) / 32));
+    Buf<uint8_t> d_code, d_tidx;
+    MCB_CK(d_code.grow((size_t)n));
+    MCB_CK(d_tidx.grow((size_t)n));
+    MCB_LAUNCH((dense_codes_kernel), (unsigned)((n + 255) / 256), 256, 0, ctx->stream, g, ctx->d_S, any_constraint ? ctx->d_V.get() : nullptr, d_code, d_tidx, n,
+                                                                             g.repeat ? ctx->d_cw.get() : nullptr, (uint32_t)((g.M + 31) / 32));
     if (ctx->last.active)
         MCB_LAUNCH((scatter_tidx_kernel), (unsigned)((ctx->last.active + 255) / 256), 256, 0, ctx->stream, g, ctx->d_rec, ctx->last.active, d_tidx);
-    if (cube_code) cudaMemcpyAsync(cube_code, d_code, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream);
-    if (table_idx) cudaMemcpyAsync(table_idx, d_tidx, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream);
-    cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    cudaError_t e2 = cudaGetLastError();
-    cudaFree(d_code); cudaFree(d_tidx);
-    if (e != cudaSuccess || e2 != cudaSuccess) return fail(ctx, MCB_E_CUDA, std::string("get_cases: ") + cudaGetErrorString(e != cudaSuccess ? e : e2));
+    if (cube_code) MCB_CK(cudaMemcpyAsync(cube_code, d_code, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (table_idx) MCB_CK(cudaMemcpyAsync(table_idx, d_tidx, (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    MCB_CK(cudaStreamSynchronize(ctx->stream));
+    MCB_CK(cudaGetLastError());
     return MCB_OK;
 }
 
@@ -1989,7 +1893,7 @@ int mcb_layer_triangles(mcb_ctx* ctx, uint32_t* per_layer) {
     if (!ctx->have_result) return fail(ctx, MCB_E_STATE, "mcb_polygonise has not run since the last change");
     if (!per_layer) return fail(ctx, MCB_E_ARG, "null buffer");
     const size_t M = (size_t)ctx->g.M;
-    if ((rc = ensure(ctx, &ctx->d_layer_hist, &ctx->cap_layer_hist, M)) != MCB_OK) return rc;
+    MCB_CK(ctx->d_layer_hist.grow(M));
     MCB_CK(cudaMemsetAsync(ctx->d_layer_hist, 0, M * 4, ctx->stream));
     MCB_LAUNCH((layer_hist_kernel), (unsigned)ctx->sm_count * 4, 256, 0, ctx->stream, ctx->d_rec, ctx->d_trioff, ctx->d_ctr, ctx->cap_active, ctx->d_layer_hist);
     MCB_CK(cudaMemcpyAsync(per_layer, ctx->d_layer_hist + ctx->g.kb, (size_t)(ctx->g.ke - ctx->g.kb) * 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2019,8 +1923,8 @@ int mcb_comm_finalize(mcb_ctx* ctx) {
     if (ctx->comm_stream) { cudaStreamDestroy(ctx->comm_stream); ctx->comm_stream = nullptr; }
     if (ctx->comm_ready) { cudaEventDestroy(ctx->comm_ready); ctx->comm_ready = nullptr; }
     if (ctx->comm_done) { cudaEventDestroy(ctx->comm_done); ctx->comm_done = nullptr; }
-    cudaFree(ctx->d_comm); ctx->d_comm = nullptr;
-    if (ctx->h_comm) { cudaFreeHost(ctx->h_comm); ctx->h_comm = nullptr; }
+    ctx->d_comm = {};
+    ctx->h_comm = {};
     ctx->comm_nranks = 1; ctx->comm_rank = 0; ctx->comm_pending = false;
     return MCB_OK;
 }
@@ -2039,8 +1943,8 @@ int mcb_comm_init(mcb_ctx* ctx, const void* id128, int rank, int nranks) {
     MCB_CK(cudaStreamCreateWithFlags(&ctx->comm_stream, cudaStreamNonBlocking));
     MCB_CK(cudaEventCreateWithFlags(&ctx->comm_ready, cudaEventDisableTiming));
     MCB_CK(cudaEventCreateWithFlags(&ctx->comm_done, cudaEventDisableTiming));
-    MCB_CK(cudaMalloc((void**)&ctx->d_comm, (size_t)(2 + nranks) * 8));
-    MCB_CK(cudaMallocHost((void**)&ctx->h_comm, (size_t)nranks * 8));
+    MCB_CK(ctx->d_comm.grow((size_t)(2 + nranks)));
+    MCB_CK(ctx->h_comm.grow((size_t)nranks));
     int k0, k1;
     if ((rc = mcb_slab_range(ctx->M, rank, nranks, &k0, &k1)) != MCB_OK) return fail(ctx, rc, "fewer cube layers than ranks");
     return mcb_set_slab(ctx, k0, k1);
@@ -2082,7 +1986,7 @@ int mcb_comm_balance(mcb_ctx* ctx, double fixed_cost_per_layer, int* k_begin, in
     if (!ctx->nccl_comm) return fail(ctx, MCB_E_STATE, "mcb_comm_init has not been called");
     if (!ctx->have_result) return fail(ctx, MCB_E_STATE, "mcb_polygonise has not run since the last change: nothing to balance by");
     const size_t M = (size_t)ctx->g.M;
-    if ((rc = ensure(ctx, &ctx->d_layer_hist, &ctx->cap_layer_hist, M)) != MCB_OK) return rc;
+    MCB_CK(ctx->d_layer_hist.grow(M));
     MCB_CK(cudaMemsetAsync(ctx->d_layer_hist, 0, M * 4, ctx->stream));
     MCB_LAUNCH((layer_hist_kernel), (unsigned)ctx->sm_count * 4, 256, 0, ctx->stream, ctx->d_rec, ctx->d_trioff, ctx->d_ctr, ctx->cap_active, ctx->d_layer_hist);
     /* one collective at a time per communicator: an all-gather still in flight on the side stream goes first */

@@ -312,13 +312,45 @@ inline bool fence_free(void* p) {
     fence_map().erase(it);
     return true;
 }
+/* Allocation accounting for the tests (tests/test_emu_buffers.py): the live allocations, the number of cudaMalloc /
+ * cudaMallocHost calls, and a switch that makes the n-th following call fail with cudaErrorMemoryAllocation. */
+struct Allocs {
+    std::mutex m;
+    std::map<void*, size_t> live;
+    long long calls = 0, fail_in = 0;
+};
+inline Allocs& allocs() { static Allocs a; return a; }
 } /* namespace emu */
+extern "C" __attribute__((used, visibility("default"))) inline void mcb_emu_alloc_stats(long long* live, long long* calls) {
+    std::lock_guard<std::mutex> lk(emu::allocs().m);
+    *live = (long long)emu::allocs().live.size();
+    *calls = emu::allocs().calls;
+}
+/* n > 0: the n-th cudaMalloc / cudaMallocHost from now on fails (once); 0: none does */
+extern "C" __attribute__((used, visibility("default"))) inline void mcb_emu_fail_alloc(long long n) {
+    std::lock_guard<std::mutex> lk(emu::allocs().m);
+    emu::allocs().fail_in = n;
+}
 template <class T> static inline cudaError_t cudaMalloc(T** p, size_t n) {
+    emu::Allocs& a = emu::allocs();
+    std::lock_guard<std::mutex> lk(a.m);
+    a.calls++;
+    if (a.fail_in > 0 && --a.fail_in == 0) { *p = nullptr; return cudaErrorMemoryAllocation; }
     *p = emu::fence_on() ? (T*)emu::fence_alloc(n) : (T*)aligned_alloc(256, (n + 255) / 256 * 256 + 256);
-    return *p ? cudaSuccess : cudaErrorMemoryAllocation;
+    if (!*p) return cudaErrorMemoryAllocation;
+    a.live[(void*)*p] = n;
+    return cudaSuccess;
 }
 template <class T> static inline cudaError_t cudaMallocHost(T** p, size_t n) { return cudaMalloc(p, n); }
-static inline cudaError_t cudaFree(void* p) { if (p && !emu::fence_free(p)) free(p); return cudaSuccess; }
+static inline cudaError_t cudaFree(void* p) {
+    if (!p) return cudaSuccess;
+    {
+        std::lock_guard<std::mutex> lk(emu::allocs().m);
+        emu::allocs().live.erase(p);
+    }
+    if (!emu::fence_free(p)) free(p);
+    return cudaSuccess;
+}
 static inline cudaError_t cudaFreeHost(void* p) { return cudaFree(p); }
 static inline cudaError_t cudaHostRegister(void*, size_t, unsigned) { return cudaSuccess; }
 static inline cudaError_t cudaHostUnregister(void*) { return cudaSuccess; }
